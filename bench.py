@@ -2,6 +2,7 @@
 """bench.py — throughput of the KOMB hot path (hits -> graph -> k-core -> CORE-A).
 
     python bench.py [--gpus N] [--steps K] [--warmup W] [--impl ours|reference] [--no-configs] [--no-cpu-baseline]
+                    [--dump-outputs DIR]
     (KOMB_BENCH_ONLY_CONFIG=cfg3|cfg4_eighth|cfg4|cfg5 at N > 1: run the step and only that secondary config)
 
 One "step" = one pass of the whole hot path over one synthetic batch (BASELINE.json configs[1]: 1 M unitigs,
@@ -363,6 +364,31 @@ def cfg4_hits_device(n, r_lo, r_cnt, p, seed, chunk=1 << 25):
     return torch.cat([mates[0][0], mates[1][0]]), torch.cat([mates[0][1], mates[1][1]])
 
 
+DUMP_SAMPLE = 1 << 20      # entries of one output written whole; a longer output is written as a seeded sample
+
+
+def dump_outputs(out_dir: str, r: dict) -> None:
+    """--dump-outputs: what the last timed step hands its caller (kombgpu_graph_results: canonical edge list, degree,
+    coreness, CORE-A score) as float64 .npy files, so that two builds can be compared output for output.  An output
+    longer than DUMP_SAMPLE entries is written at DUMP_SAMPLE positions drawn with a fixed seed from its length;
+    vertex_index.npy / edge_index.npy hold the positions written.  counts.npy = [n_vertices, n_edges]."""
+    d = Path(out_dir)
+    d.mkdir(parents=True, exist_ok=True)
+
+    def positions(count: int) -> np.ndarray:
+        if count <= DUMP_SAMPLE:
+            return np.arange(count, dtype=np.int64)
+        return np.sort(np.random.default_rng(0).choice(count, DUMP_SAMPLE, replace=False))
+
+    n, E = r["degree"].shape[0], r["u"].shape[0]
+    vi, ei = positions(n), positions(E)
+    arrays = {"counts": np.array([n, E]), "vertex_index": vi, "edge_index": ei,
+              "degree": r["degree"][vi], "coreness": r["coreness"][vi], "score": r["score"][vi],
+              "edges_u": r["u"][ei], "edges_v": r["v"][ei]}
+    for name, a in arrays.items():
+        np.save(d / f"{name}.npy", a.astype(np.float64))   # ids and counts stay below 2^53: exact in float64
+
+
 def certificate_single(core, col, deg, n, chunk=1 << 27):
     import torch
     ge = torch.zeros(n, dtype=torch.int32, device="cuda"); gt = torch.zeros(n, dtype=torch.int32, device="cuda")
@@ -494,15 +520,24 @@ def run_ours(args):
     sampler.start()
     ev = [(torch.cuda.Event(enable_timing=True), torch.cuda.Event(enable_timing=True)) for _ in range(args.steps)]
     stats = []
+    last_graph = None
     torch.cuda.synchronize()
     for i in range(args.steps):
         flush.fill_(i & 0xff)                 # L2 flush between timed iterations (outside the events)
         torch.cuda.synchronize()
         ev[i][0].record(stream)
-        stats.append(step_device())
+        if args.dump_outputs and i == args.steps - 1:
+            # the last step's graph outlives its timed window so that its results can be written below
+            st_last, last_graph = step_device(keep=True)
+            stats.append(st_last)
+        else:
+            stats.append(step_device())
         ev[i][1].record(stream)
     torch.cuda.synchronize()
     clocks = sampler.stop()
+    if last_graph is not None:
+        dump_outputs(args.dump_outputs, last_graph.results(komb_b200.KEY_REF32))
+        last_graph.close()
     step_ms = [a.elapsed_time(b) for a, b in ev]
     ms_per_step = float(np.mean(step_ms))
     st = stats[-1]
@@ -515,7 +550,8 @@ def run_ours(args):
 
     if args.profile:
         print(json.dumps({"profile_run": True, "ms_per_step": ms_per_step, "launches_per_step": st["kernel_launches"],
-                          "ms_build": ms_build, "ms_peel": ms_peel, "ms_corea": ms_corea}), flush=True)
+                          "ms_build": ms_build, "ms_peel": ms_peel, "ms_corea": ms_corea,
+                          "dumped_outputs": args.dump_outputs}), flush=True)
         ctx.close()
         return
 
@@ -590,6 +626,9 @@ def run_ours(args):
         "gpu_launches": int(sum(s["kernel_launches"] for s in stats)),
         "parity": parity,
         "clocks": clocks,
+        # set when the last timed step kept its graph past its end event (--dump-outputs): not like for like with a run
+        # without the flag
+        "dumped_outputs": args.dump_outputs,
     }
     del rk_d, ut_d
     if not args.no_configs:
@@ -937,7 +976,13 @@ def main():
     ap.add_argument("--no-configs", action="store_true", help="skip the secondary BASELINE configs (cfg3 / cfg4 / cfg5)")
     ap.add_argument("--profile", action="store_true",
                     help="minimal run for ncu: 1 warm-up + the timed steps only, no e2e / CPU legs")
+    ap.add_argument("--dump-outputs", metavar="DIR",
+                    help="write what the last timed step computed to DIR/<name>.npy (float64; single-GPU path)")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
+    if args.dump_outputs and (args.gpus != 1 or args.impl != "ours" or int(os.environ.get("WORLD_SIZE", "1")) != 1):
+        ap.error("--dump-outputs writes the single-GPU path's outputs: use it with --gpus 1 --impl ours, in one process")
     if args.impl == "reference":
         run_reference_arm(args)
     else:

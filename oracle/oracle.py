@@ -234,6 +234,56 @@ def densest_block_greedy(n: int, edges: np.ndarray, weight, workdir) -> dict:
     return {"density": density, "rows": np.sort(ids[:nr]), "cols": np.sort(ids[nr:nr + nc])}
 
 
+def densest_block_serial(n: int, edges: np.ndarray, weight=None) -> dict:
+    """The serial greedy peel of CombineCoreA::runMerge (src/CombineCoreA.h:56-186) restated over a binary heap, with
+    `removed` cleared (the reference reads it uninitialised, :105-109) and ties between equal priorities broken by the
+    smaller id (the reference's HashIndexedMinHeap has its own tie order).  A row and a column copy of every unitig,
+    priority weight + degree; the copy of least priority goes (the row on a strict <), its neighbours' other copies
+    lose one; the densest remainder seen wins (strict >, :134).  Density is in the reference's units,
+    (2 sum w + 2 E(S)) / (rows + columns left)."""
+    import heapq
+    u, v = unpack_edges(edges)
+    u, v = u.astype(np.int64), v.astype(np.int64)
+    w = np.zeros(n, np.float64) if weight is None else np.asarray(weight, np.float64)
+    adj = [[] for _ in range(n)]
+    for a, b in zip(u.tolist(), v.tolist()):
+        adj[a].append(b)
+        adj[b].append(a)
+    prio = [[float(w[i]) + len(adj[i]) for i in range(n)] for _ in range(2)]      # [0]: rows, [1]: columns
+    heaps = [[(p, i) for i, p in enumerate(prio[0])], [(p, i) for i, p in enumerate(prio[1])]]
+    for h in heaps:
+        heapq.heapify(h)
+    removed = [bytearray(n), bytearray(n)]
+    suspicious = 2.0 * float(w.sum()) + 2.0 * float(u.shape[0])
+
+    def peek(mode):
+        h = heaps[mode]
+        while h and (removed[mode][h[0][1]] or h[0][0] != prio[mode][h[0][1]]):
+            heapq.heappop(h)                            # stale entry: removed, or its priority was refreshed since
+        return h[0] if h else None
+
+    order, modes = [0] * (2 * n), [0] * (2 * n)
+    best, best_left, left = 0.0, 0, 2 * n
+    while left >= 1:
+        r, c = peek(0), peek(1)
+        mode = 0 if r is not None and (c is None or r[0] < c[0]) else 1
+        p, node = heapq.heappop(heaps[mode])
+        suspicious -= p
+        left -= 1
+        order[left], modes[left] = node, mode
+        if left >= 1 and suspicious / left > best:
+            best, best_left = suspicious / left, left
+        removed[mode][node] = 1
+        other = 1 - mode
+        for dst in adj[node]:
+            if not removed[other][dst]:
+                prio[other][dst] -= 1.0
+                heapq.heappush(heaps[other], (prio[other][dst], dst))
+    rows = [order[i] for i in range(best_left) if modes[i] == 0]
+    cols = [order[i] for i in range(best_left) if modes[i] == 1]
+    return {"density": best, "rows": np.sort(np.array(rows, np.int64)), "cols": np.sort(np.array(cols, np.int64))}
+
+
 def max_core_truss(n: int, edges: np.ndarray, core: np.ndarray) -> dict:
     """Kgraph::runTruss (src/graph.cpp:486-563) restated, for SMALL graphs (pure Python): the induced subgraph of the
     vertices of maximal coreness (:470-476, :502), igraph_trussness of its edges (:508; the largest k such that the edge

@@ -168,39 +168,52 @@ def _dyadic_weights(rng, n):
 
 
 def test_densest_block_checkers(oracle_mod, tmp_path):
-    """The bulk densest-block checker (oracle.densest_block_bulk) against the reference's serial greedy run over the
-    reference's own HashIndexedMinHeap (oracle/_ref/densest_ref): both approximate the same optimum, so they bound
-    each other (bulk <= OPT_sym <= OPT_b <= 2 greedy; greedy <= OPT_b <= 2 OPT_sym <= 4 (1 + eps) bulk), and on a
-    planted clique both find it."""
-    if not oracle_mod.REF_DENSEST.exists():
-        pytest.skip("oracle/_ref/densest_ref not built (needs /root/reference)")
+    """The bulk densest-block checker (oracle.densest_block_bulk) against the serial greedy of runMerge: both
+    approximate the same optimum, so they bound each other (bulk <= OPT_sym <= OPT_b <= 2 greedy; greedy <= OPT_b <=
+    2 OPT_sym <= 4 (1 + eps) bulk), and on a planted clique both find it.  The greedy is the restatement
+    (oracle.densest_block_serial) and, where oracle/_ref has been built from the reference tree, also the reference's
+    own loop over its HashIndexedMinHeap (oracle/_ref/densest_ref)."""
     from komb_b200 import synth
+
+    def greedies(n, edges, w):
+        out = [oracle_mod.densest_block_serial(n, edges, w)]
+        if oracle_mod.REF_DENSEST.exists():
+            out.append(oracle_mod.densest_block_greedy(n, edges, w, tmp_path))
+        return out
+
     rng = np.random.default_rng(11)
     for seed, n, m, weighted in [(1, 200, 1500, False), (2, 800, 9000, True), (3, 50, 80, True), (4, 1500, 4000, False)]:
         u, v = synth.rmat_edges(11, m, n_vertices=n, seed=seed)
         edges = oracle_mod.simplify(u, v)
         w = _dyadic_weights(rng, n) if weighted else None
-        for eps in (0.0, 0.5):
-            bulk = oracle_mod.densest_block_bulk(n, edges, w, eps)
-            greedy = oracle_mod.densest_block_greedy(n, edges, w, tmp_path)
-            assert bulk["density"] <= 2.0 * greedy["density"] * (1 + 1e-12)
-            assert greedy["density"] <= 4.0 * (1.0 + eps) * bulk["density"] * (1 + 1e-12)
-            # the reported density is the density of the reported block
-            mem = bulk["member"]
-            eu, ev = oracle_mod.unpack_edges(edges)
-            inside = int((mem[eu] & mem[ev]).sum())
-            ws = float(w[mem].sum()) if weighted else 0.0
-            assert bulk["n_vertices"] == int(mem.sum()) and bulk["n_edges"] == inside
-            assert bulk["density"] == (ws + inside) / mem.sum()
+        eu, ev = oracle_mod.unpack_edges(edges)
+        for greedy in greedies(n, edges, w):
+            # the greedy's density is that of its rows and columns: weights of both plus the adjacency entries between
+            rows, cols = np.zeros(n, bool), np.zeros(n, bool)
+            rows[greedy["rows"]] = True
+            cols[greedy["cols"]] = True
+            wg = float(w[rows].sum() + w[cols].sum()) if weighted else 0.0
+            entries = int((rows[eu] & cols[ev]).sum() + (rows[ev] & cols[eu]).sum())
+            assert greedy["density"] == pytest.approx((wg + entries) / (rows.sum() + cols.sum()), rel=1e-12)
+            for eps in (0.0, 0.5):
+                bulk = oracle_mod.densest_block_bulk(n, edges, w, eps)
+                assert bulk["density"] <= 2.0 * greedy["density"] * (1 + 1e-12)
+                assert greedy["density"] <= 4.0 * (1.0 + eps) * bulk["density"] * (1 + 1e-12)
+                # the reported density is the density of the reported block
+                mem = bulk["member"]
+                inside = int((mem[eu] & mem[ev]).sum())
+                ws = float(w[mem].sum()) if weighted else 0.0
+                assert bulk["n_vertices"] == int(mem.sum()) and bulk["n_edges"] == inside
+                assert bulk["density"] == (ws + inside) / mem.sum()
     # K_30 planted in a sparse graph: the clique is the densest block for both (density (30 - 1) / 2)
     iu, iv = np.triu_indices(30, k=1)
     u = np.concatenate([iu + 7, rng.integers(0, 3000, 3000)]).astype(np.uint32)
     v = np.concatenate([iv + 7, rng.integers(0, 3000, 3000)]).astype(np.uint32)
     edges = oracle_mod.simplify(u, v)
     bulk = oracle_mod.densest_block_bulk(3000, edges, None, 0.1)
-    greedy = oracle_mod.densest_block_greedy(3000, edges, None, tmp_path)
     assert set(np.flatnonzero(bulk["member"])) >= set(range(7, 37)) and bulk["density"] >= 14.5
-    assert set(greedy["rows"]) >= set(range(7, 37)) and greedy["density"] >= 14.5
+    for greedy in greedies(3000, edges, None):
+        assert set(greedy["rows"]) >= set(range(7, 37)) and greedy["density"] >= 14.5
     # degenerate inputs
     assert oracle_mod.densest_block_bulk(0, np.zeros(0, np.uint64))["n_vertices"] == 0
     one = oracle_mod.densest_block_bulk(5, np.zeros(0, np.uint64), np.array([0.0, 2.0, 0.5, 0.0, 0.0]), 0.5)
