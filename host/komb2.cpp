@@ -11,7 +11,12 @@
 //              (default "ref32" reproduces the reference's int32 wrap, quirk Q5);
 //              KOMB_TOKENIZE=host tokenises and interns the SAM text on the host (default with one GPU: on the device,
 //              kombgpu_sam_parse); KOMB_OUTPUT=host formats the three files on the host (default with device
-//              tokenisation: on the device, kombgpu_graph_format); KOMB_TIMING=1 prints wall-clock marks.
+//              tokenisation: on the device, kombgpu_graph_format); KOMB_TIMING=1 prints wall-clock marks;
+//              KOMB_UNITIG_FASTA=anomalous, =truss or =anomalous,truss also writes the -u FASTA's records of the
+//              anomalous unitigs (CORE-A above the IQR fence q3 + 1.5 (q3 - q1)) to <outdir>/anomalous_unitigs.fasta and
+//              of the unitigs on the max-truss edges of the maximal core to <outdir>/truss_unitigs.fasta, indexed, joined
+//              and copied on the device (truss needs one GPU: not with KOMB_GPU_DEVICES).  Unset, the FASTA is only
+//              opened, as the reference does.
 #include <omp.h>
 
 #include <chrono>
@@ -47,7 +52,31 @@ int main(int argc, const char **argv) {
         }
     }
 
+    // checked before any device work
+    bool fasta_anomalous = false, fasta_truss = false;
+    if (const char *uf = getenv("KOMB_UNITIG_FASTA")) {
+        const std::string list(uf);
+        for (size_t b = 0; b <= list.size();) {
+            size_t e = list.find(',', b);
+            if (e == std::string::npos) e = list.size();
+            const std::string w = list.substr(b, e - b);
+            if (w == "anomalous") fasta_anomalous = true;
+            else if (w == "truss") fasta_truss = true;
+            else if (!(w.empty() && list.empty())) {
+                fprintf(stderr, "komb2: KOMB_UNITIG_FASTA=%s: unknown word '%s' (expected anomalous, truss or anomalous,truss)\n", uf, w.c_str());
+                return EXIT_FAILURE;
+            }
+            b = e + 1;
+        }
+        if (fasta_truss && devices.size() > 1) {
+            fprintf(stderr, "komb2: KOMB_UNITIG_FASTA=%s: truss_unitigs.fasta needs one GPU (the graph partitioned over KOMB_GPU_DEVICES has "
+                            "no truss)\n", uf);
+            return EXIT_FAILURE;
+        }
+    }
+
     komb::Kgraph kg((uint32_t)opt.threads, (uint64_t)opt.readlen, device, key_mode, devices);
+    kg.setUnitigFasta(fasta_anomalous, fasta_truss);
     komb::HitTable hits;
     komb::MappedFile sam1, sam2;  // the hit table points into these until the ids exist
     auto begin_komb = std::chrono::steady_clock::now();
@@ -76,7 +105,7 @@ int main(int argc, const char **argv) {
             std::chrono::duration_cast<std::chrono::microseconds>(post_core - post_generate).count() / 1000000.0);
     fprintf(stdout, "\nTime elapsed for combineFile: %.3f s\n", 0.0);
 
-    kg.anomalyDetection(opt.output, true);
+    kg.anomalyDetection(opt.output, true, opt.input_unitigs, hits);
     fprintf(stdout, "\nTime elapsed for anomalyDetection: %.3f s\n", komb::seconds_since(post_core));
     fprintf(stdout, "Identified anomalous unitigs\n");
     fprintf(stdout, "Created anomalouss unitigs file\n");

@@ -278,6 +278,56 @@ int kombgpu_graph_max_core_edges(const kombgpu_graph *g, uint32_t *u, uint32_t *
 /* The unitigs on edges of maximal trussness (original ids, ascending); n_truss_vertices entries. */
 int kombgpu_graph_truss_vertices(const kombgpu_graph *g, uint32_t *vids);
 
+/* ---- the unitig FASTA: sequences of the unitigs the analysis singles out --------------------------------------
+ *
+ * FASTA records.  The input is the bytes of one FASTA file.  A record starts at a '>' at offset 0 or right after a
+ * '\n' and ends where the next record starts, or at the end of the file.  Its name is the bytes after '>' up to the
+ * first of ' ' '\t' '\r' '\n' '\v' '\f' -- the rule by which bwa-mem2 (kseq) derives the SAM RNAME, so names in the
+ * FASTA match RNAMEs in the SAM.  Sequence lines are never parsed: wrapped records, CRLF line endings and header
+ * descriptions pass through unchanged.  KOMBGPU_EINVAL, with a message, for non-whitespace bytes before the first
+ * record, an empty name, or two records with the same name (the join would be ambiguous).  An empty file has zero
+ * records.
+ *
+ * Join.  Every vertex gets the record whose name equals its unitig name, compared byte for byte (a hash alone never
+ * decides a match).  Vertices without a record are counted (*n_missing); that is not an error at join time.
+ *
+ * Anomalous unitigs (IQR fence on CORE-A).  s = the n scores sorted ascending; each quartile as
+ * numpy.percentile(..., method="linear") computes it, in float64: h = n p - p for p = 0.25 and 0.75, i = floor(h),
+ * j = min(i + 1, n - 1), t = h - i, d = s[j] - s[i], q = s[i] + d t when t < 0.5, else q = s[j] - d (1 - t).  Then
+ * fence = q3 + whisker (q3 - q1), and vertex v is anomalous iff score[v] > fence (strictly); whisker is usually 1.5.
+ * NaN scores are KOMBGPU_EINVAL; negative scores are allowed; n = 0 selects nothing and reports zeros.  There is no
+ * parity claim against the reference's getMedian / splitAnomalousUnitigs: their sources are not in this tree and the
+ * reference disables them; the rule above is the spec.
+ *
+ * Extraction.  The bytes of the selected vertices' records, copied verbatim, in the order of the FASTA file; a '\n' is
+ * appended only when the file's last record is unterminated and selected.  A selected vertex without a record is
+ * KOMBGPU_EINVAL, and the message names one such vertex id and its unitig name.  The output stays on the device until
+ * kombgpu_fasta_extract_fetch copies it (into page-locked memory from kombgpu_pinned_alloc for full PCIe rate). */
+typedef struct kombgpu_fasta kombgpu_fasta;
+/* Upload `size` bytes of FASTA text and index its records on the device. */
+int kombgpu_fasta_load(kombgpu_ctx *ctx, const char *text, uint64_t size, kombgpu_fasta **out);
+void kombgpu_fasta_destroy(kombgpu_fasta *fa);
+/* records and bytes of the file; either pointer may be NULL */
+int kombgpu_fasta_counts(const kombgpu_fasta *fa, uint32_t *n_records, uint64_t *n_bytes);
+/* vertex -> record.  The vertex names are those of the kombgpu_hits the graph was built from (spans of its device copy
+ * of the SAM text; same context), or a packed host table: name v is bytes [offsets[v], offsets[v + 1]) of `bytes`
+ * (n + 1 offsets).  A join replaces the previous one. */
+int kombgpu_fasta_join_hits(kombgpu_fasta *fa, const kombgpu_hits *names, uint32_t *n_missing);
+int kombgpu_fasta_join_names(kombgpu_fasta *fa, const char *bytes, const uint64_t *offsets, uint32_t n, uint32_t *n_missing);
+/* mask: n host bytes, nonzero = selected, n = the vertices of the last join; *bytes = size of the output text */
+int kombgpu_fasta_extract(kombgpu_fasta *fa, const uint8_t *mask, uint32_t n, uint64_t *bytes);
+int kombgpu_fasta_extract_fetch(kombgpu_fasta *fa, char *dst);
+/* CUDA-event times of the upload, the index (record starts, names, table), the last join and the last extraction, and
+ * the kernels launched for this FASTA; any pointer may be NULL */
+int kombgpu_fasta_timing(const kombgpu_fasta *fa, float *ms_upload, float *ms_index, float *ms_join, float *ms_extract,
+                         uint64_t *kernel_launches);
+/* IQR fence on CORE-A over n host scores, or over the graph's own (needs kombgpu_graph_corea first, else
+ * KOMBGPU_ESTATE).  member (optional): n bytes, 1 for the anomalous unitigs.  Any output pointer may be NULL. */
+int kombgpu_anomalous(kombgpu_ctx *ctx, const double *score, uint32_t n, double whisker, double *q1, double *q3,
+                      double *fence, uint32_t *n_selected, uint8_t *member);
+int kombgpu_graph_anomalous(kombgpu_graph *g, double whisker, double *q1, double *q3, double *fence,
+                            uint32_t *n_selected, uint8_t *member);
+
 /* The whole path in one call, host buffers in and out: what komb2 does between readSAM and its three writers
  * (getEdgeInfo ... anomalyDetection, src/komb2.cpp:104-132).  Same results as kombgpu_build_graph followed by
  * kombgpu_graph_results; the difference is scheduling: the edge list is final half-way through the build (the CSR

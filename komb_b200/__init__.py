@@ -6,6 +6,6 @@ path: alignment hits -> unitig adjacency graph -> k-core -> CORE-A score.
 """
 from . import synth  # noqa: F401
 from ._lib import KEY_EXACT64, KEY_REF32, KombGpuError  # noqa: F401
-from .api import Context, Graph  # noqa: F401
+from .api import Context, Fasta, Graph  # noqa: F401
 
 __all__ = ["Context", "Graph", "KombGpuError", "KEY_REF32", "KEY_EXACT64", "synth"]

@@ -110,6 +110,19 @@ SIGNATURES = {
     "kombgpu_graph_format_fetch": (c_int, [c_void_p, c_int, c_void_p, c_int]),
     "kombgpu_graph_format_wait": (c_int, [c_void_p]),
     "kombgpu_format_corea": (c_int, [c_void_p, c_void_p, c_uint32, c_void_p, c_uint64, POINTER(c_uint64)]),
+    # the unitig FASTA: index, join, anomalous selection, extraction
+    "kombgpu_fasta_load": (c_int, [c_void_p, c_char_p, c_uint64, POINTER(c_void_p)]),
+    "kombgpu_fasta_destroy": (None, [c_void_p]),
+    "kombgpu_fasta_counts": (c_int, [c_void_p, POINTER(c_uint32), POINTER(c_uint64)]),
+    "kombgpu_fasta_join_hits": (c_int, [c_void_p, c_void_p, POINTER(c_uint32)]),
+    "kombgpu_fasta_join_names": (c_int, [c_void_p, c_char_p, c_void_p, c_uint32, POINTER(c_uint32)]),
+    "kombgpu_fasta_extract": (c_int, [c_void_p, c_void_p, c_uint32, POINTER(c_uint64)]),
+    "kombgpu_fasta_extract_fetch": (c_int, [c_void_p, c_void_p]),
+    "kombgpu_fasta_timing": (c_int, [c_void_p, POINTER(c_float), POINTER(c_float), POINTER(c_float), POINTER(c_float), POINTER(c_uint64)]),
+    "kombgpu_anomalous": (c_int, [c_void_p, c_void_p, c_uint32, c_double, POINTER(c_double), POINTER(c_double), POINTER(c_double),
+                                  POINTER(c_uint32), c_void_p]),
+    "kombgpu_graph_anomalous": (c_int, [c_void_p, c_double, POINTER(c_double), POINTER(c_double), POINTER(c_double), POINTER(c_uint32),
+                                        c_void_p]),
     # multi-GPU partition interface
     "kombgpu_local_edges_dev": (c_int, [c_void_p, c_void_p, c_void_p, c_uint64, c_uint32, POINTER(c_void_p)]),
     "kombgpu_edgeset_from_pairs_dev": (c_int, [c_void_p, c_void_p, c_void_p, c_uint64, c_uint32, POINTER(c_void_p)]),

@@ -176,6 +176,24 @@ class Context:
         self._check(self._lib.kombgpu_sam_parse(self._h, arr, sizes, n, byref(h)))
         return Hits(self, h, texts)
 
+    def fasta(self, text: bytes) -> "Fasta":
+        """Upload the bytes of a FASTA file and index its records on the device (kombgpu_fasta_load)."""
+        text = bytes(text)
+        h = c_void_p()
+        self._check(self._lib.kombgpu_fasta_load(self._h, text, len(text), byref(h)))
+        return Fasta(self, h)
+
+    def anomalous(self, score, whisker: float = 1.5) -> dict:
+        """IQR fence on CORE-A over host scores (kombgpu_anomalous): q1, q3, fence, n_selected and the member mask."""
+        sc = _host(score, np.float64)
+        if sc.ndim != 1:
+            raise ValueError("expected a 1-D array of scores")
+        member = np.zeros(sc.shape[0], np.uint8)
+        q1, q3, fence, ns = c_double(), c_double(), c_double(), c_uint32()
+        self._check(self._lib.kombgpu_anomalous(self._h, _ptr(sc), sc.shape[0], float(whisker), byref(q1), byref(q3), byref(fence), byref(ns),
+                                                _ptr(member)))
+        return {"q1": q1.value, "q3": q3.value, "fence": fence.value, "n_selected": ns.value, "member": member.astype(bool)}
+
     def graph_from_edges(self, u, v, n_vertices: int) -> "Graph":
         return self._pair_call(self._lib.kombgpu_graph_from_edges, self._lib.kombgpu_graph_from_edges_dev,
                                u, v, int(n_vertices))
@@ -256,6 +274,65 @@ class Hits:
         g = c_void_p()
         self._ctx._check(self._lib.kombgpu_build_graph_hits(self._h, byref(g)))
         return Graph(self._ctx, g, self)
+
+
+class Fasta:
+    """A FASTA file indexed on the device (kombgpu_fasta): join its records to a graph's vertices by name, then copy
+    out the records of selected vertices."""
+
+    def __init__(self, ctx: Context, handle: c_void_p):
+        self._ctx, self._lib, self._h = ctx, ctx._lib, handle
+
+    def close(self):
+        if getattr(self, "_h", None):
+            self._lib.kombgpu_fasta_destroy(self._h)
+            self._h = None
+
+    def __del__(self):
+        try:
+            self.close()
+        except Exception:
+            pass
+
+    def __enter__(self):
+        return self
+
+    def __exit__(self, *exc):
+        self.close()
+
+    def counts(self) -> dict:
+        nr, nb = c_uint32(), c_uint64()
+        self._ctx._check(self._lib.kombgpu_fasta_counts(self._h, byref(nr), byref(nb)))
+        return {"n_records": nr.value, "n_bytes": nb.value}
+
+    def join(self, hits: "Hits | None" = None, names=None) -> int:
+        """vertex -> record by name: the vertex names of `hits` (the device copy of the SAM text), or a host list of
+        names (bytes), vertex v = names[v].  Returns the number of vertices without a record."""
+        if (hits is None) == (names is None):
+            raise ValueError("pass exactly one of hits= and names=")
+        miss = c_uint32()
+        if hits is not None:
+            self._ctx._check(self._lib.kombgpu_fasta_join_hits(self._h, hits._h, byref(miss)))
+        else:
+            names = [bytes(x) for x in names]
+            off = np.zeros(len(names) + 1, np.uint64)
+            np.cumsum([len(x) for x in names], out=off[1:])
+            self._ctx._check(self._lib.kombgpu_fasta_join_names(self._h, b"".join(names), _ptr(off), len(names), byref(miss)))
+        return miss.value
+
+    def extract(self, mask) -> bytes:
+        """The records of the vertices with a true mask entry, verbatim, in file order (kombgpu_fasta_extract)."""
+        m = np.ascontiguousarray(np.asarray(mask).astype(bool).astype(np.uint8))
+        n = c_uint64()
+        self._ctx._check(self._lib.kombgpu_fasta_extract(self._h, _ptr(m), m.shape[0], byref(n)))
+        buf = ctypes.create_string_buffer(max(n.value, 1))
+        self._ctx._check(self._lib.kombgpu_fasta_extract_fetch(self._h, buf))
+        return buf.raw[:n.value]
+
+    def timing(self) -> dict:
+        up, ix, jn, ex, l = ctypes.c_float(), ctypes.c_float(), ctypes.c_float(), ctypes.c_float(), c_uint64()
+        self._ctx._check(self._lib.kombgpu_fasta_timing(self._h, byref(up), byref(ix), byref(jn), byref(ex), byref(l)))
+        return {"ms_upload": up.value, "ms_index": ix.value, "ms_join": jn.value, "ms_extract": ex.value, "kernel_launches": l.value}
 
 
 class Graph:
@@ -429,6 +506,14 @@ class Graph:
         self._ctx._check(self._lib.kombgpu_graph_truss_vertices(self._h, _ptr(tv)))
         return {"n_core_vertices": nc.value, "n_core_edges": mc.value, "max_trussness": tm.value, "u": u, "v": v, "trussness": tr,
                 "truss_vertices": tv}
+
+    def anomalous(self, whisker: float = 1.5) -> dict:
+        """IQR fence on the graph's own CORE-A scores (kombgpu_graph_anomalous; needs corea() first)."""
+        n, _ = self.counts()
+        member = np.zeros(n, np.uint8)
+        q1, q3, fence, ns = c_double(), c_double(), c_double(), c_uint32()
+        self._ctx._check(self._lib.kombgpu_graph_anomalous(self._h, float(whisker), byref(q1), byref(q3), byref(fence), byref(ns), _ptr(member)))
+        return {"q1": q1.value, "q3": q3.value, "fence": fence.value, "n_selected": ns.value, "member": member.astype(bool)}
 
     def stats(self) -> dict:
         st = Stats()

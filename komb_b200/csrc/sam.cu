@@ -27,6 +27,7 @@
 
 #include "graph.cuh"
 #include "primitives.cuh"
+#include "strings.cuh"
 
 struct kombgpu_hits {
     kombgpu_ctx *ctx = nullptr;
@@ -90,25 +91,6 @@ struct LineStartOut {
             if (((words[j >> 2] >> (8 * (j & 3))) & 0xffu) == 0x0au) start[++k] = base + c * 16 + j + 1;
     }
 };
-
-__device__ __forceinline__ uint64_t hash_span(const unsigned char *__restrict__ p, uint32_t len, uint64_t seed) {
-    uint64_t h = seed ^ ((uint64_t)len * 0xff51afd7ed558ccdull);
-    uint32_t i = 0;
-    for (; i + 8 <= len; i += 8) {
-        uint64_t w = 0;
-#pragma unroll
-        for (int b = 0; b < 8; ++b) w |= (uint64_t)p[i + b] << (8 * b);
-        h = (h ^ w) * 0xc2b2ae3d27d4eb4full;
-        h ^= h >> 29;
-    }
-    uint64_t w = 0;
-    for (int b = 0; i < len; ++i, ++b) w |= (uint64_t)p[i] << (8 * b);
-    h = (h ^ w) * 0x165667b19e3779f9ull;
-    h ^= h >> 32;
-    h *= 0xd6e8feb86659fd93ull;
-    h ^= h >> 32;
-    return h;
-}
 
 // next token of [p, end) under strtok(.., "\t") rules: leading tabs are skipped
 __device__ __forceinline__ bool next_token(const unsigned char *__restrict__ t, uint64_t &p, uint64_t end, uint64_t &s, uint32_t &len) {
