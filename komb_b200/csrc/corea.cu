@@ -1,16 +1,18 @@
 // corea.cu — stage 3: CORE-A anomaly score.
 //
 // Restates CoreA::getAnomalyScore / fractionalRank (src/CoreA.h:109-187):
-//   key_i   = coreness_i * n + degree_i            (int32 wrap = "ref32", quirk Q5)
+//   key_i   = coreness_i * n + degree_i            (int32 wrap = "ref32", quirk Q5; int64 = "exact64")
 //   a_i     = descending average-tie rank of degree_i
 //   b_i     = descending average-tie rank of key_i
 //   score_i = | ln a_i - ln b_i |
 // The reference ranks in O(n * distinct values); here
 //   degree ranks: histogram over [0, max degree] -> prefix scan -> rank LUT
 //   key ranks   : radix sort of (key << 32 | vertex) -> run boundaries -> rank
+// exact64 keys are ranked as the pair (coreness + degree / n, degree % n), which
+// orders exactly like coreness * n + degree, also for degrees >= n.
 // Ranks are exact half-integers in FP64 (class [s, e) of the ascending order has
 // descending average rank n - (s + e - 1) / 2); only ln() can differ from glibc,
-// by <= 1 ulp, far inside the 1e-6 relative tolerance the path is held to.
+// by <= 1 ulp: the scores are held to 6e-14 absolute of the exact ranks' logs.
 #include <cstdlib>
 #include <cstring>
 
@@ -27,6 +29,19 @@ constexpr int kSmemBins = 4096;
 inline uint32_t grid_for(uint64_t n, int per_block, uint32_t cap) {
     uint32_t g = ceil_div_u64(n ? n : 1, per_block);
     return g < cap ? g : cap;
+}
+
+// exact64 key coreness * n + degree as the pair (high, low) = (coreness + degree / n, degree % n): the degree's
+// multiples of n carried into the coreness, so the pair orders exactly like the int64 key even for degrees >= n
+__device__ __forceinline__ uint2 exact_pair(int32_t core, int32_t deg, uint32_t n) {
+    uint32_t c = (uint32_t)core, d = (uint32_t)deg;
+    if (d >= n) { c += d / n; d %= n; }
+    return make_uint2(c, d);
+}
+// bit widths of the two fields of exact_pair over coreness <= max_core, degree <= max_deg (n >= 1)
+inline void exact_pair_bits(uint32_t max_core, uint32_t max_deg, uint32_t n, int *core_bits, int *deg_bits) {
+    *core_bits = bits_for((uint64_t)max_core + max_deg / n);
+    *deg_bits = bits_for(max_deg < n ? max_deg : n - 1);
 }
 
 // mm[0] = max degree, mm[1] = max coreness, mm[2] = 1 if any value is negative (input validation)
@@ -93,10 +108,10 @@ __global__ void __launch_bounds__(kThreads) pack_rank_keys_kernel(const int32_t 
             // (int32)(coreness * n + degree) with two's complement wrap; flip the sign bit for unsigned order
             hi = ((uint32_t)core[i] * n + (uint32_t)deg[i]) ^ 0x80000000u;
         } else if (mode == 1) {
-            // exact: order of coreness * n + degree == lexicographic (coreness, degree) since degree < n
-            hi = ((uint32_t)core[i] << deg_bits) | (uint32_t)deg[i];
+            const uint2 p = exact_pair(core[i], deg[i], n);
+            hi = (p.x << deg_bits) | p.y;
         } else if (mode == 2) {
-            hi = (uint32_t)deg[i];   // wide fallback, first sort: by degree
+            hi = exact_pair(core[i], deg[i], n).y;   // wide fallback, first sort: by the low field
         } else {
             hi = 0;
         }
@@ -104,27 +119,30 @@ __global__ void __launch_bounds__(kThreads) pack_rank_keys_kernel(const int32_t 
     }
 }
 
-// wide fallback, second sort: re-key the degree-sorted sequence by coreness
-__global__ void __launch_bounds__(kThreads) rekey_by_core_kernel(const int32_t *__restrict__ core, uint32_t n,
-                                                                 uint64_t *__restrict__ keys) {
-    for (uint64_t i = (uint64_t)blockIdx.x * blockDim.x + threadIdx.x; i < n; i += (uint64_t)gridDim.x * blockDim.x) {
+// wide fallback, second sort: re-key the sequence sorted by the low field by the high field
+// (`count` keys; `n` is the vertex count of the whole graph)
+__global__ void __launch_bounds__(kThreads) rekey_by_core_kernel(const int32_t *__restrict__ core, const int32_t *__restrict__ deg,
+                                                                 uint32_t count, uint32_t n, uint64_t *__restrict__ keys) {
+    for (uint64_t i = (uint64_t)blockIdx.x * blockDim.x + threadIdx.x; i < count; i += (uint64_t)gridDim.x * blockDim.x) {
         uint32_t v = (uint32_t)keys[i];
-        keys[i] = ((uint64_t)(uint32_t)core[v] << 32) | v;
+        keys[i] = ((uint64_t)exact_pair(core[v], deg[v], n).x << 32) | v;
     }
 }
 
-// class heads of the sorted sequence.  wide = compare (coreness, degree) through
+// class heads of the sorted sequence.  wide = compare the exact64 pairs through
 // the vertex id instead of the packed high word.
 struct ClassFlagIn {
     const uint64_t *keys;
     const int32_t *core;
     const int32_t *deg;
+    uint32_t n;
     int wide;
     __device__ uint32_t operator()(uint64_t i) const {
         if (i == 0) return 1u;
         if (!wide) return (keys[i] >> 32) != (keys[i - 1] >> 32) ? 1u : 0u;
         uint32_t a = (uint32_t)keys[i], b = (uint32_t)keys[i - 1];
-        return (core[a] != core[b] || deg[a] != deg[b]) ? 1u : 0u;
+        const uint2 pa = exact_pair(core[a], deg[a], n), pb = exact_pair(core[b], deg[b], n);
+        return (pa.x != pb.x || pa.y != pb.y) ? 1u : 0u;
     }
 };
 struct ClassFlagOut {
@@ -168,8 +186,8 @@ __global__ void __launch_bounds__(kThreads) score_kernel(const uint64_t *__restr
 
 // ---- small key spaces: no sort at all.  When (max coreness + 1) x (max degree + 1) is small (the usual unitig graph:
 // a few dozen coreness levels, a few hundred degrees) the (coreness, degree) pairs are counted in a 2-D histogram;
-// without int32 wrap the key coreness * n + degree orders like the pair, so the key ranks are a prefix scan over the
-// bins (the same LUT trick as the degree ranks, whose histogram is the bins' column sums).
+// while no degree reaches n and (ref32) nothing wraps, the key coreness * n + degree orders like the pair, so the key
+// ranks are a prefix scan over the bins (the same LUT trick as the degree ranks, whose histogram is the bins' column sums).
 constexpr uint32_t kPairBinsSmem = 12288;        // 48 KB of shared-memory counters
 constexpr uint64_t kPairBinsMax = 1ull << 22;    // above this the sort-based path is used
 
@@ -242,12 +260,12 @@ int corea_scores(kombgpu_ctx *ctx, const int32_t *core, const int32_t *deg, uint
     if (h_mm[2]) return ctx_fail(ctx, KOMBGPU_EINVAL, "negative coreness or degree");
     const uint32_t max_deg = (uint32_t)h_mm[0], max_core = (uint32_t)h_mm[1];
 
-    // small key space and no int32 wrap of coreness * n + degree: ranks from the 2-D histogram, no sort
+    // small key space: ranks from the 2-D histogram, no sort.  The keys order like the raw pair (coreness, degree) only
+    // while no degree >= n carries into the coreness and, for ref32, coreness * n + degree does not wrap.
     const uint64_t n_pair_bins = (uint64_t)(max_core + 1) * (uint64_t)(max_deg + 1);
-    // ref32 keys order like the pair only while coreness * n + degree neither wraps nor lets a degree >= n carry into the coreness
-    const bool wraps = key_mode == KOMBGPU_KEY_REF32 && ((uint64_t)max_core * n + max_deg > 0x7fffffffull || max_deg >= n);
+    const bool pair_order = max_deg < n && (key_mode == KOMBGPU_KEY_EXACT64 || (uint64_t)max_core * n + max_deg <= 0x7fffffffull);
     const bool no_lut = getenv("KOMBGPU_COREA_SORT") != nullptr;   // A/B runs and tests: force the sort-based path
-    if (n_pair_bins <= kPairBinsMax && !wraps && !no_lut) {
+    if (n_pair_bins <= kPairBinsMax && pair_order && !no_lut) {
         const uint32_t n_deg = max_deg + 1, n_core = max_core + 1, nb = (uint32_t)n_pair_bins;
         DevBuf<uint32_t> pair, dh;
         DevBuf<double> key_lut, deg_lut;
@@ -297,19 +315,20 @@ int corea_scores(kombgpu_ctx *ctx, const int32_t *core, const int32_t *deg, uint
         int np = plan_radix_passes(32, 64, 0, 0, passes);
         KG_TRY(radix_sort_u64(ctx, ka.p, kb.p, n, passes, np, &sorted));
     } else {
-        const int db = bits_for(max_deg), cb = bits_for(max_core);
+        int cb, db;
+        exact_pair_bits(max_core, max_deg, n, &cb, &db);
         if (db + cb <= 32) {
             KG_LAUNCH(ctx, pack_rank_keys_kernel, grid_for(n, kThreads, cap), kThreads, 0, core, deg, n, n, 1, db, ka.p);
             int np = plan_radix_passes(32, 32 + db + cb, 0, 0, passes);
             KG_TRY(radix_sort_u64(ctx, ka.p, kb.p, n, passes, np, &sorted));
         } else {
-            // (coreness, degree) does not fit 32 bits: LSD over the two fields with a re-key in between
+            // the pair does not fit 32 bits: LSD over its two fields with a re-key in between
             wide = 1;
             KG_LAUNCH(ctx, pack_rank_keys_kernel, grid_for(n, kThreads, cap), kThreads, 0, core, deg, n, n, 2, 0, ka.p);
             int np = plan_radix_passes(32, 32 + db, 0, 0, passes);
             KG_TRY(radix_sort_u64(ctx, ka.p, kb.p, n, passes, np, &sorted));
             uint64_t *other = sorted == ka.p ? kb.p : ka.p;
-            KG_LAUNCH(ctx, rekey_by_core_kernel, grid_for(n, kThreads, cap), kThreads, 0, core, n, sorted);
+            KG_LAUNCH(ctx, rekey_by_core_kernel, grid_for(n, kThreads, cap), kThreads, 0, core, deg, n, n, sorted);
             np = plan_radix_passes(32, 32 + cb, 0, 0, passes);
             uint64_t *sorted2 = sorted;
             KG_TRY(radix_sort_u64(ctx, sorted, other, n, passes, np, &sorted2));
@@ -323,7 +342,7 @@ int corea_scores(kombgpu_ctx *ctx, const int32_t *core, const int32_t *deg, uint
     KG_ALLOC(ctx, cls, n);
     if (!n_classes || !max_bits) return ctx_fail(ctx, KOMBGPU_ENOMEM, "workspace");
     KG_CUDA(ctx, cudaMemsetAsync(max_bits.p, 0, sizeof(unsigned long long), ctx->stream));
-    KG_TRY((device_scan<uint32_t>(ctx, n, ClassFlagIn{sorted, core, deg, wide}, ClassFlagOut{head_pos.p, cls.p}, n_classes.p)));
+    KG_TRY((device_scan<uint32_t>(ctx, n, ClassFlagIn{sorted, core, deg, n, wide}, ClassFlagOut{head_pos.p, cls.p}, n_classes.p)));
     KG_LAUNCH(ctx, score_kernel, grid_for(n, kThreads, cap), kThreads, 0, sorted, cls.p, head_pos.p, n_classes.p, deg, lut.p, n,
               score, max_bits.p);
     unsigned long long h_bits = 0;
@@ -362,8 +381,12 @@ __global__ void __launch_bounds__(kThreads) class_keys_kernel(const uint64_t *__
     for (uint64_t c = (uint64_t)blockIdx.x * blockDim.x + threadIdx.x; c < n_classes; c += (uint64_t)gridDim.x * blockDim.x) {
         const uint32_t h = head_pos[c];
         const uint32_t v = (uint32_t)sorted[h];
-        dkey[c] = key_mode == KOMBGPU_KEY_REF32 ? (uint64_t)(((uint32_t)core[v] * n_global + (uint32_t)deg[v]) ^ 0x80000000u)
-                                                : (((uint64_t)(uint32_t)core[v] << 32) | (uint32_t)deg[v]);
+        if (key_mode == KOMBGPU_KEY_REF32) {
+            dkey[c] = (uint64_t)(((uint32_t)core[v] * n_global + (uint32_t)deg[v]) ^ 0x80000000u);
+        } else {
+            const uint2 p = exact_pair(core[v], deg[v], n_global);
+            dkey[c] = ((uint64_t)p.x << 32) | p.y;
+        }
         dhead[c] = h;
     }
 }
@@ -460,7 +483,8 @@ int dist_corea(kombgpu_dist_graph *g, int key_mode) {
             int np = plan_radix_passes(32, 64, 0, 0, passes);
             KG_TRY(radix_sort_u64(ctx, ka.p, kb.p, n_local, passes, np, &sorted));
         } else {
-            const int db = bits_for(max_deg), cb = bits_for(max_core);
+            int cb, db;
+            exact_pair_bits(max_core, max_deg, n, &cb, &db);
             if (db + cb <= 32) {
                 KG_LAUNCH(ctx, pack_rank_keys_kernel, grid_for(n_local, kThreads, cap), kThreads, 0, g->core, g->deg, n_local, n, 1, db, ka.p);
                 int np = plan_radix_passes(32, 32 + db + cb, 0, 0, passes);
@@ -471,7 +495,7 @@ int dist_corea(kombgpu_dist_graph *g, int key_mode) {
                 int np = plan_radix_passes(32, 32 + db, 0, 0, passes);
                 KG_TRY(radix_sort_u64(ctx, ka.p, kb.p, n_local, passes, np, &sorted));
                 uint64_t *other = sorted == ka.p ? kb.p : ka.p;
-                KG_LAUNCH(ctx, rekey_by_core_kernel, grid_for(n_local, kThreads, cap), kThreads, 0, g->core, n_local, sorted);
+                KG_LAUNCH(ctx, rekey_by_core_kernel, grid_for(n_local, kThreads, cap), kThreads, 0, g->core, g->deg, n_local, n, sorted);
                 np = plan_radix_passes(32, 32 + cb, 0, 0, passes);
                 uint64_t *sorted2 = sorted;
                 KG_TRY(radix_sort_u64(ctx, sorted, other, n_local, passes, np, &sorted2));
@@ -483,7 +507,7 @@ int dist_corea(kombgpu_dist_graph *g, int key_mode) {
     KG_ALLOC(ctx, head_pos, n_local);
     KG_ALLOC(ctx, cls, n_local);
     if (!d_classes) return ctx_fail(ctx, KOMBGPU_ENOMEM, "workspace");
-    KG_TRY((device_scan<uint32_t>(ctx, n_local, ClassFlagIn{sorted, g->core, g->deg, wide}, ClassFlagOut{head_pos.p, cls.p}, d_classes.p)));
+    KG_TRY((device_scan<uint32_t>(ctx, n_local, ClassFlagIn{sorted, g->core, g->deg, n, wide}, ClassFlagOut{head_pos.p, cls.p}, d_classes.p)));
     uint32_t n_classes = 0;
     KG_TRY(read_back(ctx, d_classes.p, &n_classes, 1));
 

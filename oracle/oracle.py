@@ -151,6 +151,47 @@ def corea_ranks(core: np.ndarray, deg: np.ndarray, key_mode: int = KEY_REF32):
     return rd, rk
 
 
+# Every ranking path builds its ranks as exact half-integers in FP64, so a score can differ from |ln rd - ln rk| of the
+# exact ranks only by the rounding of two log() calls and one subtraction: a few ulp of ln(2^32) < 23, about 1e-14.
+# A key rank off by one half at rank r moves a score by about 0.5 / r, which is 2.3e-10 even at r = 2^31.
+COREA_ATOL = 6e-14
+
+
+def check_corea_ranks(got: np.ndarray, rd: np.ndarray, rk: np.ndarray, atol: float = COREA_ATOL) -> None:
+    """Assert that the scores `got` are |ln rd - ln rk| of the exact descending average ranks (degree ranks rd, key
+    ranks rk) within `atol` absolute, and that vertices with the same rank pair have bit-identical scores."""
+    got = np.asarray(got)
+    assert got.dtype == np.float64 and got.shape == rd.shape == rk.shape, (got.dtype, got.shape, rd.shape, rk.shape)
+    exp = np.abs(np.log(rd) - np.log(rk))
+    err = np.abs(got - exp)
+    bad = np.flatnonzero(~(err <= atol))          # NaN fails too
+    if bad.size:
+        i = int(bad[np.argmax(np.nan_to_num(err[bad], nan=np.inf))])
+        raise AssertionError(f"{bad.size} CORE-A scores off by more than {atol:g}; worst at vertex {i}: got {got[i]!r}, "
+                             f"expected {exp[i]!r} (degree rank {rd[i]}, key rank {rk[i]})")
+    if got.size > 1:
+        o = np.lexsort((rk, rd))
+        same = (rd[o[1:]] == rd[o[:-1]]) & (rk[o[1:]] == rk[o[:-1]])
+        bits = got.view(np.uint64)[o]
+        split = np.flatnonzero(same & (bits[1:] != bits[:-1]))
+        if split.size:
+            a, b = int(o[split[0]]), int(o[split[0] + 1])
+            raise AssertionError(f"vertices {a} and {b} share the rank pair ({rd[a]}, {rk[a]}) but score {got[a]!r} "
+                                 f"and {got[b]!r}")
+
+
+def check_corea(got: np.ndarray, core: np.ndarray, deg: np.ndarray, key_mode: int, ranking: bool = True) -> None:
+    """The exact CORE-A check: `got` against the oracle's exact ranks (check_corea_ranks) and, with `ranking`, the
+    anomaly ranking (descending score, ties by vertex id) identical to the oracle's.  Leave `ranking` off for
+    random (coreness, degree) arrays: their many near-tied scores of different rank pairs order by the last bit of
+    log()."""
+    rd, rk = corea_ranks(core, deg, key_mode)
+    check_corea_ranks(got, rd, rk)
+    if ranking:
+        exp = corea(core, deg, key_mode)
+        assert np.array_equal(np.argsort(-got, kind="stable"), np.argsort(-exp, kind="stable")), "anomaly ranking differs"
+
+
 def densest_core(core: np.ndarray, edges: np.ndarray) -> dict:
     """Checker for kombgpu_graph_densest_core: the k-core maximising edges / vertices (equal density: the larger
     block; k = smallest coreness inside the block).
