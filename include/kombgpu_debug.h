@@ -22,6 +22,11 @@ int kombgpu_debug_sort_u64(kombgpu_ctx *ctx, uint64_t n, int lo_bits, int hi_bit
  * coreness (kombgpu_coreness peels once per graph), so one build serves many timed peels. */
 int kombgpu_debug_peel_again(kombgpu_graph *g);
 
+/* tests/test_pair_chunks_gpu.py, tools/pair_chunk_probe.py: the number of chunks a graph built from hits or pairs
+ * reduced its clique pairs in.  1 is the one-shot path; the chunked path runs when the pairs reach 2^32 or, with
+ * KOMBGPU_PAIR_CHUNK=<pairs> set, when they exceed that many (the chunk size).  0 for a graph adopted from a CSR. */
+int kombgpu_debug_build_chunks(const kombgpu_graph *g, uint32_t *n_chunks);
+
 #ifdef __cplusplus
 }
 #endif

@@ -79,6 +79,7 @@ SIGNATURES = {
     "kombgpu_analyse_hits_csr": (c_int, [c_void_p, c_void_p, c_void_p, c_uint64, c_uint32, c_int, c_uint64, c_void_p, c_void_p, c_void_p,
                                          c_void_p, c_void_p, POINTER(c_void_p)]),
     "kombgpu_debug_peel_again": (c_int, [c_void_p]),
+    "kombgpu_debug_build_chunks": (c_int, [c_void_p, POINTER(c_uint32)]),
     "kombgpu_degree": (c_int, [c_void_p, c_void_p]),
     "kombgpu_coreness": (c_int, [c_void_p, c_void_p]),
     "kombgpu_corea": (c_int, [c_void_p, c_void_p, c_void_p, c_uint32, c_int, c_void_p]),

@@ -515,6 +515,13 @@ class Graph:
         self._ctx._check(self._lib.kombgpu_graph_anomalous(self._h, float(whisker), byref(q1), byref(q3), byref(fence), byref(ns), _ptr(member)))
         return {"q1": q1.value, "q3": q3.value, "fence": fence.value, "n_selected": ns.value, "member": member.astype(bool)}
 
+    def build_chunks(self) -> int:
+        """Chunks the build reduced its clique pairs in: 1 for the one-shot path (measurement aid,
+        include/kombgpu_debug.h)."""
+        n = c_uint32()
+        self._ctx._check(self._lib.kombgpu_debug_build_chunks(self._h, byref(n)))
+        return n.value
+
     def stats(self) -> dict:
         st = Stats()
         self._ctx._check(self._lib.kombgpu_graph_stats(self._h, byref(st)))

@@ -190,12 +190,13 @@ struct SegPairsOut {
 constexpr int kEmitItems = 8;
 constexpr int kEmitTile = kThreads * kEmitItems;  // outputs per CTA
 
-// tile_seg[t] = last segment s with seg_base[s] <= t * kEmitTile
+// Pairs [base, end) of the global pair index are emitted to pairs[0, end - base): the whole list in one shot (base 0)
+// or one chunk of it.  tile_seg[t] = last segment s with seg_base[s] <= base + t * kEmitTile
 __global__ void __launch_bounds__(kThreads) emit_partition_kernel(const uint64_t *__restrict__ seg_base, uint32_t n_seg,
-                                                                  uint32_t n_tiles, uint32_t *__restrict__ tile_seg) {
+                                                                  uint32_t n_tiles, uint64_t base, uint32_t *__restrict__ tile_seg) {
     uint32_t t = blockIdx.x * blockDim.x + threadIdx.x;
     if (t >= n_tiles) return;
-    uint64_t p = (uint64_t)t * kEmitTile;
+    uint64_t p = base + (uint64_t)t * kEmitTile;
     uint32_t lo = 0, hi = n_seg;  // invariant: seg_base[lo] <= p, (hi == n_seg or seg_base[hi] > p)
     while (hi - lo > 1) {
         uint32_t mid = lo + (hi - lo) / 2;
@@ -208,15 +209,17 @@ __global__ void __launch_bounds__(kThreads) emit_pairs_kernel(const uint64_t *__
                                                               const uint32_t *__restrict__ seg_head,
                                                               const uint64_t *__restrict__ seg_base, uint32_t n_seg,
                                                               const uint32_t *__restrict__ tile_seg, uint32_t n_tiles,
-                                                              uint64_t n_pairs, uint64_t *__restrict__ pairs) {
+                                                              uint64_t base, uint64_t end, uint64_t *__restrict__ pairs) {
     __shared__ uint64_t s_base[kEmitTile + 2];
     __shared__ uint32_t s_head[kEmitTile + 2];
     const uint32_t tile = blockIdx.x;
-    const uint64_t p0 = (uint64_t)tile * kEmitTile;
-    const uint64_t p1 = min(n_pairs, p0 + kEmitTile);
+    const uint64_t p0 = base + (uint64_t)tile * kEmitTile;
+    const uint64_t p1 = min(end, p0 + kEmitTile);
     const uint32_t s_first = tile_seg[tile];
     const uint32_t s_last = tile + 1 < n_tiles ? tile_seg[tile + 1] : n_seg - 1;
-    const uint32_t cnt = s_last - s_first + 1;  // <= kEmitTile + 1: every segment is non-empty
+    // every segment is non-empty, so the tile's pairs lie in its first kEmitTile segments (the last tile of a chunk
+    // may see every later segment up to n_seg - 1)
+    const uint32_t cnt = min(s_last - s_first + 1, (uint32_t)kEmitTile + 1);
     for (uint32_t i = threadIdx.x; i < cnt; i += kThreads) {
         s_base[i] = seg_base[s_first + i];
         s_head[i] = seg_head[s_first + i];
@@ -239,7 +242,7 @@ __global__ void __launch_bounds__(kThreads) emit_pairs_kernel(const uint64_t *__
         uint64_t a = t - b * (b - 1) / 2;
         const uint64_t h = s_head[lo];
         const uint32_t ua = (uint32_t)hits[h + a], ub = (uint32_t)hits[h + b];  // distinct; ascending only after a sort
-        pairs[p] = ((uint64_t)min(ua, ub) << 32) | max(ua, ub);
+        pairs[p - base] = ((uint64_t)min(ua, ub) << 32) | max(ua, ub);
     }
 }
 
@@ -280,6 +283,98 @@ struct CompactEdgesMult {
         }
         mult[pos] = (uint32_t)r;
     }
+};
+
+// ---- chunked path: merge of two sorted unique (key, count) lists ---------------------------------------------
+// A is the running edge list, B one chunk's.  Merge path over the merged sequence with both copies of a shared key
+// (A's first); a B key equal to the A key before it is a duplicate: it is dropped and its count added to A's.  An
+// output lands at its merged position minus the duplicates before it, so one counting pass (duplicates per tile)
+// and a scan over the tiles give every write position, and the output size is known before it is allocated.
+
+// part[t] = A elements among the first t * kMergeTile merged elements (A before B on equal keys)
+__global__ void __launch_bounds__(kThreads) unique_merge_partition_kernel(const uint64_t *__restrict__ a, uint64_t n_a,
+                                                                          const uint64_t *__restrict__ b, uint64_t n_b,
+                                                                          uint32_t n_tiles, uint64_t *__restrict__ part) {
+    const uint32_t t = blockIdx.x * blockDim.x + threadIdx.x;
+    if (t > n_tiles) return;
+    const uint64_t diag = min((uint64_t)t * kMergeTile, n_a + n_b);
+    uint64_t lo = diag > n_b ? diag - n_b : 0, hi = min(diag, n_a);
+    while (lo < hi) {
+        const uint64_t mid = lo + (hi - lo) / 2;
+        if (a[mid] <= b[diag - 1 - mid]) lo = mid + 1; else hi = mid;
+    }
+    part[t] = lo;
+}
+
+// kWrite = false: tile_dups[t] = B duplicates in tile t.  kWrite = true: tile_dups[t] = duplicates in the tiles before
+// t; writes the merged unique keys and their summed counts (saturating at 2^32 - 1).
+template <bool kWrite>
+__global__ void __launch_bounds__(kThreads) unique_merge_kernel(const uint64_t *__restrict__ a, const uint32_t *__restrict__ a_cnt,
+                                                                uint64_t n_a, const uint64_t *__restrict__ b,
+                                                                const uint32_t *__restrict__ b_cnt, uint64_t n_b,
+                                                                const uint64_t *__restrict__ part, uint32_t *__restrict__ tile_dups,
+                                                                uint64_t *__restrict__ out, uint32_t *__restrict__ out_cnt) {
+    // s_key = [A[a0 - 1] | the tile's A keys | its B keys | B[b0 + cb]]; ~0 (a loop, never a key) where absent
+    __shared__ uint64_t s_key[kMergeTile + 2];
+    __shared__ uint32_t s_scan[kThreads / 32 + 1];
+    const uint32_t tile = blockIdx.x;
+    const uint64_t o0 = (uint64_t)tile * kMergeTile;
+    const uint32_t count = (uint32_t)min((uint64_t)kMergeTile, n_a + n_b - o0);
+    const uint64_t a0 = part[tile], b0 = o0 - a0;
+    const uint32_t ca = (uint32_t)(part[tile + 1] - a0), cb = count - ca;
+    for (uint32_t i = threadIdx.x; i < count + 2; i += kThreads) {
+        uint64_t k = ~0ull;
+        if (i == 0) { if (a0 > 0) k = a[a0 - 1]; }
+        else if (i <= ca) k = a[a0 + i - 1];
+        else if (i <= count) k = b[b0 + (i - 1 - ca)];
+        else if (b0 + cb < n_b) k = b[b0 + cb];
+        s_key[i] = k;
+    }
+    __syncthreads();
+    const uint64_t *s_a = s_key + 1, *s_b = s_key + 1 + ca;   // s_a[-1] = A[a0 - 1], s_b[cb] = B[b0 + cb]
+    const uint32_t diag = min(threadIdx.x * kMergeItems, count);
+    const uint32_t ia0 = merge_path(diag, ca, cb, [&](uint32_t i) { return s_a[i]; }, [&](uint32_t j) { return s_b[j]; });
+    const uint32_t ib0 = diag - ia0;
+    uint32_t ia = ia0, ib = ib0, dups = 0;
+#pragma unroll
+    for (int j = 0; j < kMergeItems; ++j) {
+        if (diag + j >= count) break;
+        if (ia < ca && (ib >= cb || s_a[ia] <= s_b[ib])) ++ia;
+        else { dups += s_a[(int)ia - 1] == s_b[ib]; ++ib; }
+    }
+    uint32_t tile_total;
+    const uint32_t before = block_excl_scan_add<uint32_t, kThreads>(dups, s_scan, &tile_total);
+    if (!kWrite) {
+        if (threadIdx.x == 0) tile_dups[tile] = tile_total;
+        return;
+    }
+    uint64_t pos = o0 + diag - tile_dups[tile] - before;
+    ia = ia0; ib = ib0;
+#pragma unroll
+    for (int j = 0; j < kMergeItems; ++j) {
+        if (diag + j >= count) break;
+        if (ia < ca && (ib >= cb || s_a[ia] <= s_b[ib])) {
+            const uint64_t k = s_a[ia];
+            uint64_t c = a_cnt[a0 + ia];
+            if (s_b[ib] == k) c += b_cnt[b0 + ib];   // its B copy follows (possibly in the next tile)
+            out[pos] = k;
+            out_cnt[pos] = (uint32_t)min(c, (uint64_t)0xffffffffu);
+            ++pos; ++ia;
+        } else {
+            const uint64_t k = s_b[ib];
+            if (s_a[(int)ia - 1] != k) { out[pos] = k; out_cnt[pos] = b_cnt[b0 + ib]; ++pos; }
+            ++ib;
+        }
+    }
+}
+
+struct ReadU32 {
+    const uint32_t *x;
+    __device__ uint32_t operator()(uint64_t i) const { return x[i]; }
+};
+struct WriteU32Prefix {
+    uint32_t *x;
+    __device__ void operator()(uint64_t i, uint32_t prefix, uint32_t) const { x[i] = prefix; }
 };
 
 // ---- CSR ---------------------------------------------------------------------------
@@ -440,10 +535,100 @@ struct AnyHeadFlag {  // unique of sorted directed entries (no loop test: routed
     __device__ uint32_t operator()(uint64_t i) const { return (i == 0 || keys[i] != keys[i - 1]) ? 1u : 0u; }
 };
 
-// hits -> all clique pairs, sorted (duplicates still in).  pa / pb are the ping-pong buffers.
+// ---- chunked path -----------------------------------------------------------------------------------------------
+// A clique of k unitigs emits C(k, 2) pairs, so P outgrows the edge count E by far on repeats.  When P reaches 2^32 (or
+// exceeds KOMBGPU_PAIR_CHUNK), the pairs are emitted, sorted and reduced to (key, count) a chunk at a time, and each
+// chunk is merged into the running edge list: device memory holds one chunk of pairs plus O(E + H).
+
+constexpr uint64_t kPairChunk = (1ull << 30) - (1ull << 20);   // below 2^30: every chunk sorts with the single-read passes
+
+// the chunk size when P takes the chunked path, else 0
+uint64_t pair_chunk(uint64_t n_pairs) {
+    uint64_t cap = 0;
+    if (const char *e = getenv("KOMBGPU_PAIR_CHUNK")) cap = strtoull(e, nullptr, 10);   // tests and A/B runs
+    if (cap && n_pairs > cap) return min(cap, (uint64_t)0xffffffffu);   // a chunk's counts are 32-bit
+    return n_pairs >= (1ull << 32) ? kPairChunk : 0;
+}
+
+// where the edge list (and its multiplicities) go when the chunked path runs
+struct EdgeSink {
+    DevBuf<uint64_t> *edges;
+    uint64_t *n_edges;
+    DevBuf<uint32_t> *mult;   // optional
+    uint32_t *n_chunks;       // optional
+    bool done = false;        // set when the chunked path produced the edge list
+};
+
+// emit(p0, p1, dst) writes the canonical keys of pairs [p0, p1) to dst[0, p1 - p0)
+template <typename Emit>
+int chunked_edges(kombgpu_ctx *ctx, uint64_t n_pairs, uint64_t chunk, int bn, Emit emit, EdgeSink *sink) {
+    DevBuf<uint64_t> ka, kb, run, next;
+    DevBuf<uint32_t> ccnt, run_cnt, next_cnt, d_cnt(ctx, 1);
+    KG_ALLOC(ctx, ka, chunk);
+    KG_ALLOC(ctx, kb, chunk);
+    KG_ALLOC(ctx, ccnt, chunk);
+    if (!d_cnt) return ctx_fail(ctx, KOMBGPU_ENOMEM, "workspace");
+    RadixPass passes[8];
+    const int np = plan_radix_passes(0, bn, 32, 32 + bn, passes);
+    uint64_t n_run = 0;
+    uint32_t n_chunks = 0;
+    for (uint64_t p0 = 0; p0 < n_pairs; p0 += chunk, ++n_chunks) {
+        const uint64_t n_c = min(chunk, n_pairs - p0);
+        // emit, sort, reduce to sorted unique (key, count) in the other ping-pong buffer
+        KG_TRY(emit(p0, p0 + n_c, ka.p));
+        uint64_t *sorted = ka.p;
+        KG_TRY(radix_sort_u64(ctx, ka.p, kb.p, n_c, passes, np, &sorted));
+        uint64_t *cuniq = sorted == ka.p ? kb.p : ka.p;
+        KG_TRY((device_scan<uint32_t>(ctx, n_c, EdgeFlagIn{sorted}, CompactEdgesMult{sorted, n_c, cuniq, ccnt.p}, d_cnt.p)));
+        uint32_t n_u = 0;
+        KG_TRY(read_back(ctx, d_cnt.p, &n_u, 1));
+        if (n_u == 0) continue;
+        // merge into the running list: count the duplicates per tile, then the output size, then write
+        const uint64_t n_m = n_run + n_u;
+        const uint32_t n_tiles = ceil_div_u64(n_m, kMergeTile);
+        DevBuf<uint64_t> part;
+        DevBuf<uint32_t> tile_dups;
+        KG_ALLOC(ctx, part, (size_t)n_tiles + 1);
+        KG_ALLOC(ctx, tile_dups, n_tiles);
+        KG_LAUNCH(ctx, unique_merge_partition_kernel, grid_for((uint64_t)n_tiles + 1, kThreads), kThreads, 0, run.p, n_run, cuniq,
+                  (uint64_t)n_u, n_tiles, part.p);
+        KG_LAUNCH(ctx, unique_merge_kernel<false>, n_tiles, kThreads, 0, run.p, run_cnt.p, n_run, cuniq, ccnt.p, (uint64_t)n_u,
+                  part.p, tile_dups.p, nullptr, nullptr);
+        KG_TRY((device_scan<uint32_t>(ctx, n_tiles, ReadU32{tile_dups.p}, WriteU32Prefix{tile_dups.p}, d_cnt.p)));
+        uint32_t n_dups = 0;
+        KG_TRY(read_back(ctx, d_cnt.p, &n_dups, 1));
+        const uint64_t n_out = n_m - n_dups;
+        if (n_out >= (1ull << 32))
+            return ctx_fail(ctx, KOMBGPU_EINVAL, "%llu simple edges exceed the 2^32 per-device edge limit",
+                            (unsigned long long)n_out);
+        KG_ALLOC(ctx, next, n_out);
+        KG_ALLOC(ctx, next_cnt, n_out);
+        KG_LAUNCH(ctx, unique_merge_kernel<true>, n_tiles, kThreads, 0, run.p, run_cnt.p, n_run, cuniq, ccnt.p, (uint64_t)n_u,
+                  part.p, tile_dups.p, next.p, next_cnt.p);
+        // the running list only grows: give the old one back to the device rather than to the context's cache
+        ws_release(ctx, run.take());
+        ws_release(ctx, run_cnt.take());
+        run = std::move(next);
+        run_cnt = std::move(next_cnt);
+        n_run = n_out;
+    }
+    if (!run) KG_ALLOC(ctx, run, 0);
+    *sink->edges = std::move(run);
+    *sink->n_edges = n_run;
+    if (sink->mult) {
+        if (!run_cnt) KG_ALLOC(ctx, run_cnt, 0);
+        *sink->mult = std::move(run_cnt);
+    }
+    if (sink->n_chunks) *sink->n_chunks = n_chunks;
+    sink->done = true;
+    return KOMBGPU_OK;
+}
+
+// hits -> all clique pairs, sorted (duplicates still in).  pa / pb are the ping-pong buffers.  With a sink, a P that
+// takes the chunked path goes straight to the sink's edge list (sink->done; pa / pb stay empty).
 int hits_to_sorted_pairs(kombgpu_ctx *ctx, const uint32_t *read_key, const uint32_t *unitig, uint64_t n_hits,
                          uint32_t n_vertices, DevBuf<uint64_t> &pa, DevBuf<uint64_t> &pb, uint64_t **psorted_out,
-                         uint64_t *n_pairs_out, kombgpu_stats *st, bool sort_pairs = true) {
+                         uint64_t *n_pairs_out, kombgpu_stats *st, bool sort_pairs = true, EdgeSink *sink = nullptr) {
     if (n_hits >= (1ull << 32)) return ctx_fail(ctx, KOMBGPU_EINVAL, "n_hits >= 2^32 is not supported on one device");
     const int bn = bits_for(n_vertices > 0 ? n_vertices - 1 : 0);
     st->n_hits = n_hits;
@@ -526,6 +711,19 @@ int hits_to_sorted_pairs(kombgpu_ctx *ctx, const uint32_t *read_key, const uint3
     KG_TRY(read_back(ctx, d_tot.p, &n_pairs, 1));
     st->n_pairs = n_pairs;
     *n_pairs_out = n_pairs;
+    if (const uint64_t chunk = sink ? pair_chunk(n_pairs) : 0) {
+        // 3'. chunks of pairs, each emitted from its global pair index (a chunk may start inside a read's clique)
+        DevBuf<uint32_t> tile_seg;
+        KG_ALLOC(ctx, tile_seg, ceil_div_u64(chunk, kEmitTile));
+        auto emit = [&](uint64_t p0, uint64_t p1, uint64_t *dst) -> int {
+            const uint32_t n_tiles = ceil_div_u64(p1 - p0, kEmitTile);
+            KG_LAUNCH(ctx, emit_partition_kernel, grid_for(n_tiles, kThreads), kThreads, 0, seg_base.p, n_seg, n_tiles, p0, tile_seg.p);
+            KG_LAUNCH(ctx, emit_pairs_kernel, n_tiles, kThreads, 0, hits, seg_head.p, seg_base.p, n_seg, tile_seg.p, n_tiles, p0, p1,
+                      dst);
+            return KOMBGPU_OK;
+        };
+        return chunked_edges(ctx, n_pairs, chunk, bn, emit, sink);
+    }
     if (n_pairs >= (1ull << 32))
         return ctx_fail(ctx, KOMBGPU_EINVAL, "%llu clique pairs exceed the 2^32 per-device limit", (unsigned long long)n_pairs);
 
@@ -537,9 +735,9 @@ int hits_to_sorted_pairs(kombgpu_ctx *ctx, const uint32_t *read_key, const uint3
         const uint32_t n_tiles = ceil_div_u64(n_pairs, kEmitTile);
         DevBuf<uint32_t> tile_seg;
         KG_ALLOC(ctx, tile_seg, n_tiles);
-        KG_LAUNCH(ctx, emit_partition_kernel, grid_for(n_tiles, kThreads), kThreads, 0, seg_base.p, n_seg, n_tiles, tile_seg.p);
+        KG_LAUNCH(ctx, emit_partition_kernel, grid_for(n_tiles, kThreads), kThreads, 0, seg_base.p, n_seg, n_tiles, 0ull, tile_seg.p);
         KG_LAUNCH(ctx, emit_pairs_kernel, n_tiles, kThreads, 0, hits, seg_head.p, seg_base.p, n_seg, tile_seg.p, n_tiles,
-                  n_pairs, pa.p);
+                  0ull, n_pairs, pa.p);
         if (sort_pairs) {
             int npp = plan_radix_passes(0, bn, 32, 32 + bn, passes);
             KG_TRY(radix_sort_u64(ctx, pa.p, pb.p, n_pairs, passes, npp, &psorted));
@@ -621,15 +819,35 @@ int lower_bounds_hi(kombgpu_ctx *ctx, const uint64_t *keys, uint64_t count, cons
 }
 
 int hits_to_edges(kombgpu_ctx *ctx, const uint32_t *read_key, const uint32_t *unitig, uint64_t n_hits, uint32_t n_vertices,
-                  DevBuf<uint64_t> &edges, uint64_t *n_edges, kombgpu_stats *st, DevBuf<uint32_t> *mult) {
+                  DevBuf<uint64_t> &edges, uint64_t *n_edges, kombgpu_stats *st, DevBuf<uint32_t> *mult, uint32_t *n_chunks) {
     DevBuf<uint64_t> pa, pb;
     uint64_t *psorted = nullptr, n_pairs = 0;
-    KG_TRY(hits_to_sorted_pairs(ctx, read_key, unitig, n_hits, n_vertices, pa, pb, &psorted, &n_pairs, st));
+    EdgeSink sink{&edges, n_edges, mult, n_chunks};
+    KG_TRY(hits_to_sorted_pairs(ctx, read_key, unitig, n_hits, n_vertices, pa, pb, &psorted, &n_pairs, st, true, &sink));
+    if (sink.done) return KOMBGPU_OK;
+    if (n_chunks) *n_chunks = 1;
     return unique_edges(ctx, psorted, n_pairs, edges, n_edges, mult);
 }
 
 int pairs_to_edges(kombgpu_ctx *ctx, const uint32_t *u, const uint32_t *v, uint64_t n_pairs, uint32_t n_vertices,
-                   DevBuf<uint64_t> &edges, uint64_t *n_edges, DevBuf<uint32_t> *mult) {
+                   DevBuf<uint64_t> &edges, uint64_t *n_edges, DevBuf<uint32_t> *mult, uint32_t *n_chunks) {
+    if (const uint64_t chunk = pair_chunk(n_pairs)) {
+        // chunks of the input, packed and range-checked as the one-shot path does
+        DevBuf<uint32_t> info(ctx, 2);
+        if (!info) return ctx_fail(ctx, KOMBGPU_ENOMEM, "workspace");
+        KG_CUDA(ctx, cudaMemsetAsync(info.p, 0, 2 * sizeof(uint32_t), ctx->stream));
+        auto emit = [&](uint64_t p0, uint64_t p1, uint64_t *dst) -> int {
+            KG_LAUNCH(ctx, pack_pairs_kernel, min(grid_for(p1 - p0, kThreads), 148u * 16u), kThreads, 0, u + p0, v + p0, p1 - p0,
+                      n_vertices, dst, info.p);
+            uint32_t h_info[2] = {0, 0};
+            KG_TRY(read_back(ctx, info.p, h_info, 2));
+            if (h_info[1]) return ctx_fail(ctx, KOMBGPU_EINVAL, "edge endpoint >= n_vertices (%u)", n_vertices);
+            return KOMBGPU_OK;
+        };
+        EdgeSink sink{&edges, n_edges, mult, n_chunks};
+        return chunked_edges(ctx, n_pairs, chunk, bits_for(n_vertices > 0 ? n_vertices - 1 : 0), emit, &sink);
+    }
+    if (n_chunks) *n_chunks = 1;
     DevBuf<uint64_t> ka, kb;
     uint64_t *sorted = nullptr;
     KG_TRY(pairs_to_sorted_keys(ctx, u, v, n_pairs, n_vertices, ka, kb, &sorted));
@@ -804,7 +1022,7 @@ int build_from_pairs(kombgpu_ctx *ctx, const uint32_t *u, const uint32_t *v, uin
     uint64_t E = 0;
     g->st.n_pairs = n_pairs;
     DevBuf<uint32_t> mult;
-    KG_TRY(pairs_to_edges(ctx, u, v, n_pairs, n_vertices, edges, &E, &mult));
+    KG_TRY(pairs_to_edges(ctx, u, v, n_pairs, n_vertices, edges, &E, &mult, &g->build_chunks));
     g->mult = mult.take();
     return csr_from_edges(ctx, edges, E, n_vertices, g);
 }
@@ -814,7 +1032,7 @@ int build_from_hits(kombgpu_ctx *ctx, const uint32_t *read_key, const uint32_t *
     DevBuf<uint64_t> edges;
     uint64_t E = 0;
     DevBuf<uint32_t> mult;
-    KG_TRY(hits_to_edges(ctx, read_key, unitig, n_hits, n_vertices, edges, &E, &g->st, &mult));
+    KG_TRY(hits_to_edges(ctx, read_key, unitig, n_hits, n_vertices, edges, &E, &g->st, &mult, &g->build_chunks));
     g->mult = mult.take();
     return csr_from_edges(ctx, edges, E, n_vertices, g);
 }

@@ -77,6 +77,17 @@ void ws_free(kombgpu_ctx *ctx, void *p) {
         if (b.ptr == p) { b.in_use = false; return; }
 }
 
+void ws_release(kombgpu_ctx *ctx, void *p) {
+    if (!p) return;
+    for (size_t i = 0; i < ctx->arena.size(); ++i)
+        if (ctx->arena[i].ptr == p) {
+            cudaStreamSynchronize(ctx->stream);
+            cudaFree(p);
+            ctx->arena.erase(ctx->arena.begin() + i);
+            return;
+        }
+}
+
 void ws_trim(kombgpu_ctx *ctx) {
     cudaStreamSynchronize(ctx->stream);
     for (size_t i = 0; i < ctx->arena.size();) {
@@ -438,6 +449,13 @@ int kombgpu_debug_peel_again(kombgpu_graph *g) {
     return kombgpu_coreness(g, nullptr);
 }
 
+// measurement aid (include/kombgpu_debug.h): how many chunks the build reduced its pairs in
+int kombgpu_debug_build_chunks(const kombgpu_graph *g, uint32_t *n_chunks) {
+    if (!g || !n_chunks) return KOMBGPU_EINVAL;
+    *n_chunks = g->build_chunks;
+    return KOMBGPU_OK;
+}
+
 int kombgpu_corea(kombgpu_ctx *ctx, const int32_t *coreness, const int32_t *degree, uint32_t n, int key_mode, double *score) {
     if (!ctx) return KOMBGPU_EINVAL;
     if (n && (!coreness || !degree || !score)) return ctx_fail(ctx, KOMBGPU_EINVAL, "null argument");
@@ -565,7 +583,7 @@ static int analyse_hits_impl(kombgpu_ctx *ctx, const uint32_t *read_key, const u
         DevBuf<uint64_t> edges;
         DevBuf<uint32_t> mult;
         uint64_t E = 0;
-        if (rc == KOMBGPU_OK) rc = hits_to_edges(ctx, da.p, db.p, n_hits, n_vertices, edges, &E, &g->st, &mult);
+        if (rc == KOMBGPU_OK) rc = hits_to_edges(ctx, da.p, db.p, n_hits, n_vertices, edges, &E, &g->st, &mult, &g->build_chunks);
         g->mult = mult.take();
         if (rc == KOMBGPU_OK && v && E > edge_capacity)
             rc = ctx_fail(ctx, KOMBGPU_EINVAL, "%llu edges do not fit the caller's edge buffers (%llu)", (unsigned long long)E,

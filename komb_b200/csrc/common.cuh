@@ -53,6 +53,8 @@ int ctx_fail(kombgpu_ctx *ctx, int code, const char *fmt, ...);
 // block handed back with ws_free may be reused by the next launch immediately.
 void *ws_alloc(kombgpu_ctx *ctx, size_t bytes);
 void ws_free(kombgpu_ctx *ctx, void *p);
+// hand a block back to the device at once (a buffer that keeps growing, so the cache could never reuse it)
+void ws_release(kombgpu_ctx *ctx, void *p);
 void ws_trim(kombgpu_ctx *ctx);
 
 // RAII holder for workspace blocks.

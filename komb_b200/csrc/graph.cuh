@@ -13,6 +13,7 @@ struct kombgpu_graph {
     uint32_t *col = nullptr;     // [2E]  neighbours, every row ascending
     uint32_t *fwd_start = nullptr; // [n+1] forward index of the edge list: edges [fwd_start[u], fwd_start[u+1]) have source u
     uint32_t *mult = nullptr;    // [E]   pairs (reads, or input duplicates) that support each edge
+    uint32_t build_chunks = 0;   // chunks the pairs were reduced in (1: one shot; 0: adopted from a CSR)
     int32_t *deg = nullptr;      // [n]
     int32_t *core = nullptr;     // [n]   after peel
     double *score = nullptr;     // [n]   after CORE-A
@@ -43,10 +44,13 @@ int build_from_pairs(kombgpu_ctx *ctx, const uint32_t *u, const uint32_t *v, uin
 
 // building blocks of stage 1 shared with the partitioned (multi-GPU) path (build.cu)
 // `mult` (optional): receives, per unique edge, how many emitted pairs collapsed into it
+// Any number of pairs: from 2^32 on (or above KOMBGPU_PAIR_CHUNK) they are reduced in chunks; `n_chunks` (optional)
+// receives how many (1 for the one-shot path).
 int hits_to_edges(kombgpu_ctx *ctx, const uint32_t *read_key, const uint32_t *unitig, uint64_t n_hits, uint32_t n_vertices,
-                  DevBuf<uint64_t> &edges, uint64_t *n_edges, kombgpu_stats *st, DevBuf<uint32_t> *mult = nullptr);
+                  DevBuf<uint64_t> &edges, uint64_t *n_edges, kombgpu_stats *st, DevBuf<uint32_t> *mult = nullptr,
+                  uint32_t *n_chunks = nullptr);
 int pairs_to_edges(kombgpu_ctx *ctx, const uint32_t *u, const uint32_t *v, uint64_t n_pairs, uint32_t n_vertices,
-                   DevBuf<uint64_t> &edges, uint64_t *n_edges, DevBuf<uint32_t> *mult = nullptr);
+                   DevBuf<uint64_t> &edges, uint64_t *n_edges, DevBuf<uint32_t> *mult = nullptr, uint32_t *n_chunks = nullptr);
 int hits_to_pairs(kombgpu_ctx *ctx, const uint32_t *read_key, const uint32_t *unitig, uint64_t n_hits, uint32_t n_vertices,
                   DevBuf<uint64_t> &pairs, uint64_t *n_pairs, kombgpu_stats *st);
 int pairs_to_keys(kombgpu_ctx *ctx, const uint32_t *u, const uint32_t *v, uint64_t n_pairs, uint32_t n_vertices, DevBuf<uint64_t> &keys);

@@ -82,6 +82,35 @@ def metagenome_hits(n_unitigs: int, n_read_pairs: int, seed: int = 11, alpha: fl
     return mates[0], mates[1]
 
 
+def repeat_family_hits(n_unitigs: int = 200_000, family_size: int = 2000, overlap: int = 300, n_families: int = 3,
+                       reads_per_family: int = 750, n_background: int = 100_000, seed: int = 21) -> tuple[HitSet, HitSet]:
+    """Repeats under `bwa mem -a`: every read of a repeat family hits all of the family's unitigs, so one read emits
+    C(family_size, 2) clique pairs (the defaults give 4 497 750 000 from the families: more than 2^32).
+
+    Family f holds `family_size` unitigs, `overlap` of them shared with family f + 1; ids are scrambled over
+    [0, n_unitigs).  Each family read lists its unitigs in its own shuffled order, split over the two mates with 200
+    unitigs (a tenth of the family) in both.  The families' reads come first, then `n_background` cfg2-style read pairs
+    (metagenome_hits).  Both mate files are in read order."""
+    rng = np.random.Generator(np.random.PCG64(seed))
+    step = family_size - overlap
+    fams = [scramble_ids(np.arange(f * step, f * step + family_size, dtype=np.uint32), n_unitigs) for f in range(n_families)]
+    both = family_size // 10
+    split = (family_size + both) // 2
+    rk = [[], []]
+    ut = [[], []]
+    r = 0
+    for fam in fams:
+        for _ in range(reads_per_family):
+            order = rng.permutation(fam)
+            for m, part in enumerate((order[:split], order[split - both:])):
+                rk[m].append(np.full(part.shape[0], r, np.uint32))
+                ut[m].append(part)
+            r += 1
+    b1, b2 = metagenome_hits(n_unitigs, n_background, seed=seed + 1, read_offset=r)
+    return (HitSet(np.concatenate(rk[0] + [b1.read_key]), np.concatenate(ut[0] + [b1.unitig])),
+            HitSet(np.concatenate(rk[1] + [b2.read_key]), np.concatenate(ut[1] + [b2.unitig])))
+
+
 def render_sam(hits: HitSet, n_unitigs: int, mate: int, unmapped_every: int = 0,
                with_header: bool = True, qname_suffix: bool = True) -> bytes:
     """Render a hit set as SAM text the reference tokeniser accepts
