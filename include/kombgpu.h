@@ -436,7 +436,9 @@ int kombgpu_corea_dev(kombgpu_ctx *ctx, const int32_t *coreness_dev, const int32
  *
  *   build   every rank turns ITS reads' hits into clique pairs, stores each pair straight into the receive buffer
  *           of the rank that owns min(u, v); the owner sorts + deduplicates, sends the reversed copy of every edge
- *           to the owner of max(u, v), and both halves become the owner's CSR rows
+ *           to the owner of max(u, v), and both halves become the owner's CSR rows.  From 2^32 pairs over all
+ *           ranks on, the pairs go in rounds (fewer than 2^30 routed to an owner per round) that every owner
+ *           merges into its slice of the edge list
  *   peel    one persistent kernel per GPU; a rank logs the unitigs it peels and copies the new part of its log into
  *           every peer (4 bytes per peeled unitig cross a link, whatever its degree); every rank decrements ITS
  *           neighbours of each logged unitig; ranks meet once per cascade generation through flags in peer memory
@@ -491,7 +493,13 @@ typedef struct kombgpu_dist_stats {
 
 /* Stage 1..3 over all ranks, collective.  Inputs are device pointers on the rank's device: the hits of THIS
  * rank's reads (both mates, global unitig ids; a read's hits must all be on one rank), or this rank's share of an
- * edge list.  Results stay on the device until fetched. */
+ * edge list.  Results stay on the device until fetched.
+ * Limits per rank: n_hits < 2^32, distinct (read, unitig) hits < 2^31, edges whose u it owns (n_fwd_local) < 2^32
+ * and adjacency entries of its rows (n_directed_local) < 2^32 (KOMBGPU_EINVAL otherwise).  The clique pairs, those a
+ * rank emits (or passes in) and those routed to it, are not limited: from 2^32 pairs over all ranks on they are
+ * emitted, routed, sorted and merged in rounds, so a rank holds one round of them.  The results do not depend on
+ * the rounds.  When one rank fails, every rank returns an error (the failing rank its own) and the contexts and
+ * the communicator stay usable. */
 int kombgpu_dist_build_hits_dev(kombgpu_comm *comm, const uint32_t *read_key_dev, const uint32_t *unitig_dev,
                                 uint64_t n_hits, uint32_t n_vertices_global, kombgpu_dist_graph **out);
 int kombgpu_dist_build_pairs_dev(kombgpu_comm *comm, const uint32_t *u_dev, const uint32_t *v_dev, uint64_t n_pairs,

@@ -27,6 +27,11 @@ int kombgpu_debug_peel_again(kombgpu_graph *g);
  * KOMBGPU_PAIR_CHUNK=<pairs> set, when they exceed that many (the chunk size).  0 for a graph adopted from a CSR. */
 int kombgpu_debug_build_chunks(const kombgpu_graph *g, uint32_t *n_chunks);
 
+/* tests/test_dist_pair_chunks_gpu.py, tools/dist_pair_chunk_probe.py: the number of rounds a multi-GPU build emitted,
+ * routed and reduced its clique pairs in.  1 is the one-shot path; the rounds run when the pairs of all ranks reach
+ * 2^32 or, with KOMBGPU_PAIR_CHUNK=<pairs> set, when some rank's pairs exceed that many (the pairs per rank and round). */
+int kombgpu_debug_dist_build_rounds(const kombgpu_dist_graph *g, uint32_t *n_rounds);
+
 #ifdef __cplusplus
 }
 #endif

@@ -80,6 +80,7 @@ SIGNATURES = {
                                          c_void_p, c_void_p, POINTER(c_void_p)]),
     "kombgpu_debug_peel_again": (c_int, [c_void_p]),
     "kombgpu_debug_build_chunks": (c_int, [c_void_p, POINTER(c_uint32)]),
+    "kombgpu_debug_dist_build_rounds": (c_int, [c_void_p, POINTER(c_uint32)]),
     "kombgpu_degree": (c_int, [c_void_p, c_void_p]),
     "kombgpu_coreness": (c_int, [c_void_p, c_void_p]),
     "kombgpu_corea": (c_int, [c_void_p, c_void_p, c_void_p, c_uint32, c_int, c_void_p]),

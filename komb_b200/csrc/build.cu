@@ -540,12 +540,9 @@ struct AnyHeadFlag {  // unique of sorted directed entries (no loop test: routed
 // exceeds KOMBGPU_PAIR_CHUNK), the pairs are emitted, sorted and reduced to (key, count) a chunk at a time, and each
 // chunk is merged into the running edge list: device memory holds one chunk of pairs plus O(E + H).
 
-constexpr uint64_t kPairChunk = (1ull << 30) - (1ull << 20);   // below 2^30: every chunk sorts with the single-read passes
-
 // the chunk size when P takes the chunked path, else 0
 uint64_t pair_chunk(uint64_t n_pairs) {
-    uint64_t cap = 0;
-    if (const char *e = getenv("KOMBGPU_PAIR_CHUNK")) cap = strtoull(e, nullptr, 10);   // tests and A/B runs
+    const uint64_t cap = pair_chunk_env();
     if (cap && n_pairs > cap) return min(cap, (uint64_t)0xffffffffu);   // a chunk's counts are 32-bit
     return n_pairs >= (1ull << 32) ? kPairChunk : 0;
 }
@@ -556,194 +553,36 @@ struct EdgeSink {
     uint64_t *n_edges;
     DevBuf<uint32_t> *mult;   // optional
     uint32_t *n_chunks;       // optional
-    bool done = false;        // set when the chunked path produced the edge list
 };
 
 // emit(p0, p1, dst) writes the canonical keys of pairs [p0, p1) to dst[0, p1 - p0)
 template <typename Emit>
 int chunked_edges(kombgpu_ctx *ctx, uint64_t n_pairs, uint64_t chunk, int bn, Emit emit, EdgeSink *sink) {
-    DevBuf<uint64_t> ka, kb, run, next;
-    DevBuf<uint32_t> ccnt, run_cnt, next_cnt, d_cnt(ctx, 1);
+    DevBuf<uint64_t> ka, kb;
+    DevBuf<uint32_t> ccnt;
     KG_ALLOC(ctx, ka, chunk);
     KG_ALLOC(ctx, kb, chunk);
     KG_ALLOC(ctx, ccnt, chunk);
-    if (!d_cnt) return ctx_fail(ctx, KOMBGPU_ENOMEM, "workspace");
     RadixPass passes[8];
     const int np = plan_radix_passes(0, bn, 32, 32 + bn, passes);
-    uint64_t n_run = 0;
+    EdgeRun run;
     uint32_t n_chunks = 0;
     for (uint64_t p0 = 0; p0 < n_pairs; p0 += chunk, ++n_chunks) {
         const uint64_t n_c = min(chunk, n_pairs - p0);
-        // emit, sort, reduce to sorted unique (key, count) in the other ping-pong buffer
+        // emit, sort, reduce to sorted unique (key, count) in the other ping-pong buffer, merge into the running list
         KG_TRY(emit(p0, p0 + n_c, ka.p));
         uint64_t *sorted = ka.p;
         KG_TRY(radix_sort_u64(ctx, ka.p, kb.p, n_c, passes, np, &sorted));
-        uint64_t *cuniq = sorted == ka.p ? kb.p : ka.p;
-        KG_TRY((device_scan<uint32_t>(ctx, n_c, EdgeFlagIn{sorted}, CompactEdgesMult{sorted, n_c, cuniq, ccnt.p}, d_cnt.p)));
-        uint32_t n_u = 0;
-        KG_TRY(read_back(ctx, d_cnt.p, &n_u, 1));
-        if (n_u == 0) continue;
-        // merge into the running list: count the duplicates per tile, then the output size, then write
-        const uint64_t n_m = n_run + n_u;
-        const uint32_t n_tiles = ceil_div_u64(n_m, kMergeTile);
-        DevBuf<uint64_t> part;
-        DevBuf<uint32_t> tile_dups;
-        KG_ALLOC(ctx, part, (size_t)n_tiles + 1);
-        KG_ALLOC(ctx, tile_dups, n_tiles);
-        KG_LAUNCH(ctx, unique_merge_partition_kernel, grid_for((uint64_t)n_tiles + 1, kThreads), kThreads, 0, run.p, n_run, cuniq,
-                  (uint64_t)n_u, n_tiles, part.p);
-        KG_LAUNCH(ctx, unique_merge_kernel<false>, n_tiles, kThreads, 0, run.p, run_cnt.p, n_run, cuniq, ccnt.p, (uint64_t)n_u,
-                  part.p, tile_dups.p, nullptr, nullptr);
-        KG_TRY((device_scan<uint32_t>(ctx, n_tiles, ReadU32{tile_dups.p}, WriteU32Prefix{tile_dups.p}, d_cnt.p)));
-        uint32_t n_dups = 0;
-        KG_TRY(read_back(ctx, d_cnt.p, &n_dups, 1));
-        const uint64_t n_out = n_m - n_dups;
-        if (n_out >= (1ull << 32))
-            return ctx_fail(ctx, KOMBGPU_EINVAL, "%llu simple edges exceed the 2^32 per-device edge limit",
-                            (unsigned long long)n_out);
-        KG_ALLOC(ctx, next, n_out);
-        KG_ALLOC(ctx, next_cnt, n_out);
-        KG_LAUNCH(ctx, unique_merge_kernel<true>, n_tiles, kThreads, 0, run.p, run_cnt.p, n_run, cuniq, ccnt.p, (uint64_t)n_u,
-                  part.p, tile_dups.p, next.p, next_cnt.p);
-        // the running list only grows: give the old one back to the device rather than to the context's cache
-        ws_release(ctx, run.take());
-        ws_release(ctx, run_cnt.take());
-        run = std::move(next);
-        run_cnt = std::move(next_cnt);
-        n_run = n_out;
+        KG_TRY(merge_sorted_chunk(ctx, sorted, n_c, sorted == ka.p ? kb.p : ka.p, ccnt.p, &run));
     }
-    if (!run) KG_ALLOC(ctx, run, 0);
-    *sink->edges = std::move(run);
-    *sink->n_edges = n_run;
+    if (!run.keys) KG_ALLOC(ctx, run.keys, 0);
+    *sink->edges = std::move(run.keys);
+    *sink->n_edges = run.n;
     if (sink->mult) {
-        if (!run_cnt) KG_ALLOC(ctx, run_cnt, 0);
-        *sink->mult = std::move(run_cnt);
+        if (!run.cnt) KG_ALLOC(ctx, run.cnt, 0);
+        *sink->mult = std::move(run.cnt);
     }
     if (sink->n_chunks) *sink->n_chunks = n_chunks;
-    sink->done = true;
-    return KOMBGPU_OK;
-}
-
-// hits -> all clique pairs, sorted (duplicates still in).  pa / pb are the ping-pong buffers.  With a sink, a P that
-// takes the chunked path goes straight to the sink's edge list (sink->done; pa / pb stay empty).
-int hits_to_sorted_pairs(kombgpu_ctx *ctx, const uint32_t *read_key, const uint32_t *unitig, uint64_t n_hits,
-                         uint32_t n_vertices, DevBuf<uint64_t> &pa, DevBuf<uint64_t> &pb, uint64_t **psorted_out,
-                         uint64_t *n_pairs_out, kombgpu_stats *st, bool sort_pairs = true, EdgeSink *sink = nullptr) {
-    if (n_hits >= (1ull << 32)) return ctx_fail(ctx, KOMBGPU_EINVAL, "n_hits >= 2^32 is not supported on one device");
-    const int bn = bits_for(n_vertices > 0 ? n_vertices - 1 : 0);
-    st->n_hits = n_hits;
-
-    // 1. (read, unitig) keys, sorted + unique  == per-read unitig SETS, mates merged
-    DevBuf<uint64_t> ha, hb;
-    DevBuf<uint32_t> info(ctx, 5);
-    KG_ALLOC(ctx, ha, n_hits);
-    KG_ALLOC(ctx, hb, n_hits);
-    if (!info) return ctx_fail(ctx, KOMBGPU_ENOMEM, "workspace");
-    const uint32_t info0[5] = {0, 0, 0, 0xffffffffu, 0};   // max key, error, descents, first descent, read too long
-    KG_CUDA(ctx, cudaMemcpyAsync(info.p, info0, sizeof(info0), cudaMemcpyHostToDevice, ctx->stream));
-    if (n_hits)
-        KG_LAUNCH(ctx, pack_hits_kernel, min(grid_for(n_hits, kThreads), 148u * 16u), kThreads, 0, read_key, unitig, n_hits,
-                  n_vertices, ha.p, info.p);
-    uint32_t h_info[5] = {0, 0, 0, 0, 0};
-    KG_TRY(read_back(ctx, info.p, h_info, 5));
-    if (h_info[1]) return ctx_fail(ctx, KOMBGPU_EINVAL, "unitig id >= n_vertices (%u)", n_vertices);
-    DevBuf<uint32_t> d_cnt(ctx, 1);
-    if (!d_cnt) return ctx_fail(ctx, KOMBGPU_ENOMEM, "workspace");
-    uint64_t *sorted = ha.p, *other = hb.p;
-    uint32_t n_uniq = 0;
-    RadixPass passes[8];
-    bool grouped = false;   // unique hits grouped by read without a sort?
-    DevBuf<uint64_t> hc;    // third buffer of the merge path (see below)
-    if (n_hits && h_info[2] <= 1 && !getenv("KOMBGPU_NO_MERGE")) {
-        // The reads arrive in file order (at most two runs of non-decreasing keys: the two mate files): a stable
-        // merge by read key replaces the radix sort (6 passes for cfg2), and since the per-read unitig SET is all
-        // the path needs, duplicates inside a read are found by looking back through the read.
-        uint64_t *by_read = ha.p;
-        if (h_info[2] == 1) {
-            const uint32_t n_a = h_info[3], n_b = (uint32_t)(n_hits - n_a);
-            const uint32_t n_tiles = ceil_div_u64(n_hits, kMergeTile);
-            DevBuf<uint32_t> part;
-            KG_ALLOC(ctx, part, (size_t)n_tiles + 1);
-            KG_LAUNCH(ctx, merge_partition_kernel, grid_for((uint64_t)n_tiles + 1, kThreads), kThreads, 0, ha.p, n_a, ha.p + n_a, n_b,
-                      n_tiles, part.p);
-            KG_LAUNCH(ctx, merge_runs_kernel, n_tiles, kThreads, 0, ha.p, n_a, ha.p + n_a, n_b, part.p, hb.p);
-            by_read = hb.p;
-        }
-        // compaction needs a third buffer only when the merge used both: the packed input is dead after the merge,
-        // but a read that is too long sends us back to it, so keep it and compact into scratch
-        uint64_t *dst = by_read == ha.p ? hb.p : nullptr;
-        if (!dst) { KG_ALLOC(ctx, hc, n_hits); dst = hc.p; }
-        KG_TRY((device_scan<uint32_t>(ctx, n_hits, FirstInReadFlag{by_read, info.p + 4}, CompactKeysU64{by_read, dst}, d_cnt.p)));
-        uint32_t too_long = 0;
-        KG_TRY(read_back(ctx, info.p + 4, &too_long, 1));
-        if (!too_long) {
-            KG_TRY(read_back(ctx, d_cnt.p, &n_uniq, 1));
-            grouped = true;
-            other = dst;
-        }
-    }
-    if (!grouped) {
-        int np = plan_radix_passes(0, bn, 32, 32 + bits_for(h_info[0]), passes);
-        KG_TRY(radix_sort_u64(ctx, ha.p, hb.p, n_hits, passes, np, &sorted));
-        other = sorted == ha.p ? hb.p : ha.p;
-        KG_TRY((device_scan<uint32_t>(ctx, n_hits, HeadFlagU64{sorted}, CompactKeysU64{sorted, other}, d_cnt.p)));
-        KG_TRY(read_back(ctx, d_cnt.p, &n_uniq, 1));
-    }
-    const uint64_t *hits = other;  // unique hits grouped by read (sorted when the general path ran), n_uniq of them
-    st->n_unique_hits = n_uniq;
-    // the segment scan below carries two 32-bit counters in one word whose top two bits are the scan's status flags
-    if (n_uniq >= (1u << 31)) return ctx_fail(ctx, KOMBGPU_EINVAL, "%u distinct (read, unitig) hits exceed the 2^31 per-device limit", n_uniq);
-
-    // 2. reads with >= 2 unitigs -> segments; pairs per segment -> offsets
-    DevBuf<uint32_t> seg_head, seg_tail;
-    DevBuf<uint64_t> d_tot(ctx, 1);
-    KG_ALLOC(ctx, seg_head, (size_t)n_uniq / 2 + 1);
-    KG_ALLOC(ctx, seg_tail, (size_t)n_uniq / 2 + 1);
-    if (!d_tot) return ctx_fail(ctx, KOMBGPU_ENOMEM, "workspace");
-    KG_TRY((device_scan<uint64_t>(ctx, n_uniq, SegFlagIn{hits, n_uniq}, SegFlagOut{seg_head.p, seg_tail.p}, d_tot.p)));
-    uint64_t seg_tot = 0;
-    KG_TRY(read_back(ctx, d_tot.p, &seg_tot, 1));
-    const uint32_t n_seg = (uint32_t)(seg_tot >> 32);
-    DevBuf<uint64_t> seg_base;
-    KG_ALLOC(ctx, seg_base, (size_t)n_seg + 1);
-    KG_TRY((device_scan<uint64_t>(ctx, n_seg, SegPairsIn{seg_head.p, seg_tail.p}, SegPairsOut{seg_base.p}, d_tot.p)));
-    uint64_t n_pairs = 0;
-    KG_TRY(read_back(ctx, d_tot.p, &n_pairs, 1));
-    st->n_pairs = n_pairs;
-    *n_pairs_out = n_pairs;
-    if (const uint64_t chunk = sink ? pair_chunk(n_pairs) : 0) {
-        // 3'. chunks of pairs, each emitted from its global pair index (a chunk may start inside a read's clique)
-        DevBuf<uint32_t> tile_seg;
-        KG_ALLOC(ctx, tile_seg, ceil_div_u64(chunk, kEmitTile));
-        auto emit = [&](uint64_t p0, uint64_t p1, uint64_t *dst) -> int {
-            const uint32_t n_tiles = ceil_div_u64(p1 - p0, kEmitTile);
-            KG_LAUNCH(ctx, emit_partition_kernel, grid_for(n_tiles, kThreads), kThreads, 0, seg_base.p, n_seg, n_tiles, p0, tile_seg.p);
-            KG_LAUNCH(ctx, emit_pairs_kernel, n_tiles, kThreads, 0, hits, seg_head.p, seg_base.p, n_seg, tile_seg.p, n_tiles, p0, p1,
-                      dst);
-            return KOMBGPU_OK;
-        };
-        return chunked_edges(ctx, n_pairs, chunk, bn, emit, sink);
-    }
-    if (n_pairs >= (1ull << 32))
-        return ctx_fail(ctx, KOMBGPU_EINVAL, "%llu clique pairs exceed the 2^32 per-device limit", (unsigned long long)n_pairs);
-
-    // 3. emit all pairs, sort
-    KG_ALLOC(ctx, pa, n_pairs);
-    if (sort_pairs) KG_ALLOC(ctx, pb, n_pairs);
-    uint64_t *psorted = pa.p;
-    if (n_pairs) {
-        const uint32_t n_tiles = ceil_div_u64(n_pairs, kEmitTile);
-        DevBuf<uint32_t> tile_seg;
-        KG_ALLOC(ctx, tile_seg, n_tiles);
-        KG_LAUNCH(ctx, emit_partition_kernel, grid_for(n_tiles, kThreads), kThreads, 0, seg_base.p, n_seg, n_tiles, 0ull, tile_seg.p);
-        KG_LAUNCH(ctx, emit_pairs_kernel, n_tiles, kThreads, 0, hits, seg_head.p, seg_base.p, n_seg, tile_seg.p, n_tiles,
-                  0ull, n_pairs, pa.p);
-        if (sort_pairs) {
-            int npp = plan_radix_passes(0, bn, 32, 32 + bn, passes);
-            KG_TRY(radix_sort_u64(ctx, pa.p, pb.p, n_pairs, passes, npp, &psorted));
-        }
-    }
-    *psorted_out = psorted;
     return KOMBGPU_OK;
 }
 
@@ -818,32 +657,196 @@ int lower_bounds_hi(kombgpu_ctx *ctx, const uint64_t *keys, uint64_t count, cons
     return read_back(ctx, d_i.p, idx_host, nb);
 }
 
+uint64_t pair_chunk_env() {
+    const char *e = getenv("KOMBGPU_PAIR_CHUNK");   // tests and A/B runs
+    return e ? strtoull(e, nullptr, 10) : 0;
+}
+
+int merge_sorted_chunk(kombgpu_ctx *ctx, const uint64_t *sorted, uint64_t n_c, uint64_t *cuniq, uint32_t *ccnt, EdgeRun *run) {
+    DevBuf<uint32_t> d_cnt(ctx, 1);
+    if (!d_cnt) return ctx_fail(ctx, KOMBGPU_ENOMEM, "workspace");
+    KG_TRY((device_scan<uint32_t>(ctx, n_c, EdgeFlagIn{sorted}, CompactEdgesMult{sorted, n_c, cuniq, ccnt}, d_cnt.p)));
+    uint32_t n_u = 0;
+    KG_TRY(read_back(ctx, d_cnt.p, &n_u, 1));
+    if (n_u == 0) return KOMBGPU_OK;
+    // merge into the running list: count the duplicates per tile, then the output size, then write
+    const uint64_t n_run = run->n, n_m = n_run + n_u;
+    const uint32_t n_tiles = ceil_div_u64(n_m, kMergeTile);
+    DevBuf<uint64_t> part, next;
+    DevBuf<uint32_t> tile_dups, next_cnt;
+    KG_ALLOC(ctx, part, (size_t)n_tiles + 1);
+    KG_ALLOC(ctx, tile_dups, n_tiles);
+    KG_LAUNCH(ctx, unique_merge_partition_kernel, grid_for((uint64_t)n_tiles + 1, kThreads), kThreads, 0, run->keys.p, n_run, cuniq,
+              (uint64_t)n_u, n_tiles, part.p);
+    KG_LAUNCH(ctx, unique_merge_kernel<false>, n_tiles, kThreads, 0, run->keys.p, run->cnt.p, n_run, cuniq, ccnt, (uint64_t)n_u,
+              part.p, tile_dups.p, nullptr, nullptr);
+    KG_TRY((device_scan<uint32_t>(ctx, n_tiles, ReadU32{tile_dups.p}, WriteU32Prefix{tile_dups.p}, d_cnt.p)));
+    uint32_t n_dups = 0;
+    KG_TRY(read_back(ctx, d_cnt.p, &n_dups, 1));
+    const uint64_t n_out = n_m - n_dups;
+    if (n_out >= (1ull << 32))
+        return ctx_fail(ctx, KOMBGPU_EINVAL, "%llu simple edges exceed the 2^32 per-device edge limit", (unsigned long long)n_out);
+    KG_ALLOC(ctx, next, n_out);
+    KG_ALLOC(ctx, next_cnt, n_out);
+    KG_LAUNCH(ctx, unique_merge_kernel<true>, n_tiles, kThreads, 0, run->keys.p, run->cnt.p, n_run, cuniq, ccnt, (uint64_t)n_u,
+              part.p, tile_dups.p, next.p, next_cnt.p);
+    // the running list only grows: give the old one back to the device rather than to the context's cache
+    ws_release(ctx, run->keys.take());
+    ws_release(ctx, run->cnt.take());
+    run->keys = std::move(next);
+    run->cnt = std::move(next_cnt);
+    run->n = n_out;
+    return KOMBGPU_OK;
+}
+
+int HitPairs::emit(uint64_t p0, uint64_t p1, uint64_t *dst) {
+    if (p1 <= p0) return KOMBGPU_OK;
+    const uint32_t n_tiles = ceil_div_u64(p1 - p0, kEmitTile);
+    if (tile_seg.count < n_tiles) KG_ALLOC(ctx, tile_seg, n_tiles);
+    KG_LAUNCH(ctx, emit_partition_kernel, grid_for(n_tiles, kThreads), kThreads, 0, seg_base.p, n_seg, n_tiles, p0, tile_seg.p);
+    KG_LAUNCH(ctx, emit_pairs_kernel, n_tiles, kThreads, 0, hits, seg_head.p, seg_base.p, n_seg, tile_seg.p, n_tiles, p0, p1, dst);
+    return KOMBGPU_OK;
+}
+
+void HitPairs::release() {
+    ha.release(); hb.release(); hc.release(); seg_base.release();
+    seg_head.release(); seg_tail.release(); tile_seg.release();
+    hits = nullptr;
+}
+
+int count_hit_pairs(kombgpu_ctx *ctx, const uint32_t *read_key, const uint32_t *unitig, uint64_t n_hits, uint32_t n_vertices,
+                    HitPairs *hp, kombgpu_stats *st) {
+    if (n_hits >= (1ull << 32)) return ctx_fail(ctx, KOMBGPU_EINVAL, "n_hits >= 2^32 is not supported on one device");
+    const int bn = bits_for(n_vertices > 0 ? n_vertices - 1 : 0);
+    hp->ctx = ctx;
+    st->n_hits = n_hits;
+    DevBuf<uint64_t> &ha = hp->ha, &hb = hp->hb;
+
+    // 1. (read, unitig) keys, sorted + unique  == per-read unitig SETS, mates merged
+    DevBuf<uint32_t> info(ctx, 5);
+    KG_ALLOC(ctx, ha, n_hits);
+    KG_ALLOC(ctx, hb, n_hits);
+    if (!info) return ctx_fail(ctx, KOMBGPU_ENOMEM, "workspace");
+    const uint32_t info0[5] = {0, 0, 0, 0xffffffffu, 0};   // max key, error, descents, first descent, read too long
+    KG_CUDA(ctx, cudaMemcpyAsync(info.p, info0, sizeof(info0), cudaMemcpyHostToDevice, ctx->stream));
+    if (n_hits)
+        KG_LAUNCH(ctx, pack_hits_kernel, min(grid_for(n_hits, kThreads), 148u * 16u), kThreads, 0, read_key, unitig, n_hits,
+                  n_vertices, ha.p, info.p);
+    uint32_t h_info[5] = {0, 0, 0, 0, 0};
+    KG_TRY(read_back(ctx, info.p, h_info, 5));
+    if (h_info[1]) return ctx_fail(ctx, KOMBGPU_EINVAL, "unitig id >= n_vertices (%u)", n_vertices);
+    DevBuf<uint32_t> d_cnt(ctx, 1);
+    if (!d_cnt) return ctx_fail(ctx, KOMBGPU_ENOMEM, "workspace");
+    uint64_t *sorted = ha.p, *other = hb.p;
+    uint32_t n_uniq = 0;
+    RadixPass passes[8];
+    bool grouped = false;   // unique hits grouped by read without a sort?
+    if (n_hits && h_info[2] <= 1 && !getenv("KOMBGPU_NO_MERGE")) {
+        // The reads arrive in file order (at most two runs of non-decreasing keys: the two mate files): a stable
+        // merge by read key replaces the radix sort (6 passes for cfg2), and since the per-read unitig SET is all
+        // the path needs, duplicates inside a read are found by looking back through the read.
+        uint64_t *by_read = ha.p;
+        if (h_info[2] == 1) {
+            const uint32_t n_a = h_info[3], n_b = (uint32_t)(n_hits - n_a);
+            const uint32_t n_tiles = ceil_div_u64(n_hits, kMergeTile);
+            DevBuf<uint32_t> part;
+            KG_ALLOC(ctx, part, (size_t)n_tiles + 1);
+            KG_LAUNCH(ctx, merge_partition_kernel, grid_for((uint64_t)n_tiles + 1, kThreads), kThreads, 0, ha.p, n_a, ha.p + n_a, n_b,
+                      n_tiles, part.p);
+            KG_LAUNCH(ctx, merge_runs_kernel, n_tiles, kThreads, 0, ha.p, n_a, ha.p + n_a, n_b, part.p, hb.p);
+            by_read = hb.p;
+        }
+        // compaction needs a third buffer only when the merge used both: the packed input is dead after the merge,
+        // but a read that is too long sends us back to it, so keep it and compact into scratch
+        uint64_t *dst = by_read == ha.p ? hb.p : nullptr;
+        if (!dst) { KG_ALLOC(ctx, hp->hc, n_hits); dst = hp->hc.p; }
+        KG_TRY((device_scan<uint32_t>(ctx, n_hits, FirstInReadFlag{by_read, info.p + 4}, CompactKeysU64{by_read, dst}, d_cnt.p)));
+        uint32_t too_long = 0;
+        KG_TRY(read_back(ctx, info.p + 4, &too_long, 1));
+        if (!too_long) {
+            KG_TRY(read_back(ctx, d_cnt.p, &n_uniq, 1));
+            grouped = true;
+            other = dst;
+        }
+    }
+    if (!grouped) {
+        int np = plan_radix_passes(0, bn, 32, 32 + bits_for(h_info[0]), passes);
+        KG_TRY(radix_sort_u64(ctx, ha.p, hb.p, n_hits, passes, np, &sorted));
+        other = sorted == ha.p ? hb.p : ha.p;
+        KG_TRY((device_scan<uint32_t>(ctx, n_hits, HeadFlagU64{sorted}, CompactKeysU64{sorted, other}, d_cnt.p)));
+        KG_TRY(read_back(ctx, d_cnt.p, &n_uniq, 1));
+    }
+    const uint64_t *hits = other;  // unique hits grouped by read (sorted when the general path ran), n_uniq of them
+    hp->hits = hits;
+    st->n_unique_hits = n_uniq;
+    // the segment scan below carries two 32-bit counters in one word whose top two bits are the scan's status flags
+    if (n_uniq >= (1u << 31)) return ctx_fail(ctx, KOMBGPU_EINVAL, "%u distinct (read, unitig) hits exceed the 2^31 per-device limit", n_uniq);
+
+    // 2. reads with >= 2 unitigs -> segments; pairs per segment -> offsets
+    DevBuf<uint64_t> d_tot(ctx, 1);
+    KG_ALLOC(ctx, hp->seg_head, (size_t)n_uniq / 2 + 1);
+    KG_ALLOC(ctx, hp->seg_tail, (size_t)n_uniq / 2 + 1);
+    if (!d_tot) return ctx_fail(ctx, KOMBGPU_ENOMEM, "workspace");
+    KG_TRY((device_scan<uint64_t>(ctx, n_uniq, SegFlagIn{hits, n_uniq}, SegFlagOut{hp->seg_head.p, hp->seg_tail.p}, d_tot.p)));
+    uint64_t seg_tot = 0;
+    KG_TRY(read_back(ctx, d_tot.p, &seg_tot, 1));
+    hp->n_seg = (uint32_t)(seg_tot >> 32);
+    KG_ALLOC(ctx, hp->seg_base, (size_t)hp->n_seg + 1);
+    KG_TRY((device_scan<uint64_t>(ctx, hp->n_seg, SegPairsIn{hp->seg_head.p, hp->seg_tail.p}, SegPairsOut{hp->seg_base.p}, d_tot.p)));
+    KG_TRY(read_back(ctx, d_tot.p, &hp->n_pairs, 1));
+    st->n_pairs = hp->n_pairs;
+    return KOMBGPU_OK;
+}
+
+int pack_pairs(kombgpu_ctx *ctx, const uint32_t *u, const uint32_t *v, uint64_t n, uint32_t n_vertices, uint64_t *dst) {
+    DevBuf<uint32_t> info(ctx, 2);
+    if (!info) return ctx_fail(ctx, KOMBGPU_ENOMEM, "workspace");
+    KG_CUDA(ctx, cudaMemsetAsync(info.p, 0, 2 * sizeof(uint32_t), ctx->stream));
+    if (n) KG_LAUNCH(ctx, pack_pairs_kernel, min(grid_for(n, kThreads), 148u * 16u), kThreads, 0, u, v, n, n_vertices, dst, info.p);
+    uint32_t h_info[2] = {0, 0};
+    KG_TRY(read_back(ctx, info.p, h_info, 2));
+    if (h_info[1]) return ctx_fail(ctx, KOMBGPU_EINVAL, "edge endpoint >= n_vertices (%u)", n_vertices);
+    return KOMBGPU_OK;
+}
+
 int hits_to_edges(kombgpu_ctx *ctx, const uint32_t *read_key, const uint32_t *unitig, uint64_t n_hits, uint32_t n_vertices,
                   DevBuf<uint64_t> &edges, uint64_t *n_edges, kombgpu_stats *st, DevBuf<uint32_t> *mult, uint32_t *n_chunks) {
     DevBuf<uint64_t> pa, pb;
-    uint64_t *psorted = nullptr, n_pairs = 0;
-    EdgeSink sink{&edges, n_edges, mult, n_chunks};
-    KG_TRY(hits_to_sorted_pairs(ctx, read_key, unitig, n_hits, n_vertices, pa, pb, &psorted, &n_pairs, st, true, &sink));
-    if (sink.done) return KOMBGPU_OK;
+    uint64_t *psorted = nullptr;
+    {
+        HitPairs hp;
+        KG_TRY(count_hit_pairs(ctx, read_key, unitig, n_hits, n_vertices, &hp, st));
+        const uint64_t n_pairs = hp.n_pairs;
+        const int bn = bits_for(n_vertices > 0 ? n_vertices - 1 : 0);
+        if (const uint64_t chunk = pair_chunk(n_pairs)) {
+            // 3'. chunks of pairs, each emitted from its global pair index
+            EdgeSink sink{&edges, n_edges, mult, n_chunks};
+            return chunked_edges(ctx, n_pairs, chunk, bn, [&](uint64_t p0, uint64_t p1, uint64_t *dst) { return hp.emit(p0, p1, dst); },
+                                 &sink);
+        }
+        if (n_pairs >= (1ull << 32))
+            return ctx_fail(ctx, KOMBGPU_EINVAL, "%llu clique pairs exceed the 2^32 per-device limit", (unsigned long long)n_pairs);
+
+        // 3. emit all pairs, sort
+        KG_ALLOC(ctx, pa, n_pairs);
+        KG_ALLOC(ctx, pb, n_pairs);
+        psorted = pa.p;
+        if (n_pairs) {
+            KG_TRY(hp.emit(0, n_pairs, pa.p));
+            RadixPass passes[8];
+            const int np = plan_radix_passes(0, bn, 32, 32 + bn, passes);
+            KG_TRY(radix_sort_u64(ctx, pa.p, pb.p, n_pairs, passes, np, &psorted));
+        }
+    }   // the hits and segments are dead
     if (n_chunks) *n_chunks = 1;
-    return unique_edges(ctx, psorted, n_pairs, edges, n_edges, mult);
+    return unique_edges(ctx, psorted, st->n_pairs, edges, n_edges, mult);
 }
 
 int pairs_to_edges(kombgpu_ctx *ctx, const uint32_t *u, const uint32_t *v, uint64_t n_pairs, uint32_t n_vertices,
                    DevBuf<uint64_t> &edges, uint64_t *n_edges, DevBuf<uint32_t> *mult, uint32_t *n_chunks) {
     if (const uint64_t chunk = pair_chunk(n_pairs)) {
         // chunks of the input, packed and range-checked as the one-shot path does
-        DevBuf<uint32_t> info(ctx, 2);
-        if (!info) return ctx_fail(ctx, KOMBGPU_ENOMEM, "workspace");
-        KG_CUDA(ctx, cudaMemsetAsync(info.p, 0, 2 * sizeof(uint32_t), ctx->stream));
-        auto emit = [&](uint64_t p0, uint64_t p1, uint64_t *dst) -> int {
-            KG_LAUNCH(ctx, pack_pairs_kernel, min(grid_for(p1 - p0, kThreads), 148u * 16u), kThreads, 0, u + p0, v + p0, p1 - p0,
-                      n_vertices, dst, info.p);
-            uint32_t h_info[2] = {0, 0};
-            KG_TRY(read_back(ctx, info.p, h_info, 2));
-            if (h_info[1]) return ctx_fail(ctx, KOMBGPU_EINVAL, "edge endpoint >= n_vertices (%u)", n_vertices);
-            return KOMBGPU_OK;
-        };
+        auto emit = [&](uint64_t p0, uint64_t p1, uint64_t *dst) { return pack_pairs(ctx, u + p0, v + p0, p1 - p0, n_vertices, dst); };
         EdgeSink sink{&edges, n_edges, mult, n_chunks};
         return chunked_edges(ctx, n_pairs, chunk, bits_for(n_vertices > 0 ? n_vertices - 1 : 0), emit, &sink);
     }
@@ -852,29 +855,6 @@ int pairs_to_edges(kombgpu_ctx *ctx, const uint32_t *u, const uint32_t *v, uint6
     uint64_t *sorted = nullptr;
     KG_TRY(pairs_to_sorted_keys(ctx, u, v, n_pairs, n_vertices, ka, kb, &sorted));
     return unique_edges(ctx, sorted, n_pairs, edges, n_edges, mult);
-}
-
-// hits -> every clique pair as a canonical key (min << 32 | max), in emission order (not sorted, duplicates in)
-int hits_to_pairs(kombgpu_ctx *ctx, const uint32_t *read_key, const uint32_t *unitig, uint64_t n_hits, uint32_t n_vertices,
-                  DevBuf<uint64_t> &pairs, uint64_t *n_pairs, kombgpu_stats *st) {
-    DevBuf<uint64_t> unused;
-    uint64_t *p = nullptr;
-    return hits_to_sorted_pairs(ctx, read_key, unitig, n_hits, n_vertices, pairs, unused, &p, n_pairs, st, false);
-}
-
-// (u, v) pairs -> canonical keys (min << 32 | max), input order; ids are range-checked
-int pairs_to_keys(kombgpu_ctx *ctx, const uint32_t *u, const uint32_t *v, uint64_t n_pairs, uint32_t n_vertices, DevBuf<uint64_t> &keys) {
-    if (n_pairs >= (1ull << 32)) return ctx_fail(ctx, KOMBGPU_EINVAL, "n_pairs >= 2^32 is not supported on one device");
-    DevBuf<uint32_t> info(ctx, 2);
-    KG_ALLOC(ctx, keys, n_pairs);
-    if (!info) return ctx_fail(ctx, KOMBGPU_ENOMEM, "workspace");
-    KG_CUDA(ctx, cudaMemsetAsync(info.p, 0, 2 * sizeof(uint32_t), ctx->stream));
-    if (n_pairs)
-        KG_LAUNCH(ctx, pack_pairs_kernel, min(grid_for(n_pairs, kThreads), 148u * 16u), kThreads, 0, u, v, n_pairs, n_vertices, keys.p, info.p);
-    uint32_t h_info[2] = {0, 0};
-    KG_TRY(read_back(ctx, info.p, h_info, 2));
-    if (h_info[1]) return ctx_fail(ctx, KOMBGPU_EINVAL, "edge endpoint >= n_vertices (%u)", n_vertices);
-    return KOMBGPU_OK;
 }
 
 int row_starts(kombgpu_ctx *ctx, const uint64_t *keys, uint64_t count, uint32_t base, uint32_t n_rows, uint32_t lo_bound, uint32_t *start,

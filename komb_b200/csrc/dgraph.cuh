@@ -15,6 +15,7 @@ struct kombgpu_dist_graph {
     uint64_t n_fwd = 0;        // edges (u, v), u < v, whose u this rank owns: its slice of the canonical edge list
     uint64_t n_directed = 0;   // CSR entries of the local rows
     uint64_t n_edges_global = 0;
+    uint32_t build_rounds = 0;     // rounds the build emitted, routed and reduced the pairs in (1: one shot)
     uint64_t *edges = nullptr;     // [n_fwd]  (u << 32 | v), global ids, ascending
     uint32_t *mult = nullptr;      // [n_fwd]
     uint32_t *fwd_start = nullptr; // [n_local + 1]
@@ -45,7 +46,10 @@ int dist_build(kombgpu_comm *c, const uint32_t *a, const uint32_t *b, uint64_t c
                kombgpu_dist_graph *g);
 // send every key to the rank that owns its high word (hi / step); returns the keys this rank received, in the
 // symmetric heap (valid until the caller's sym_release).  kRebase: the high word arrives as hi - owner * step.
-int route_keys(kombgpu_comm *c, const uint64_t *keys, uint64_t n, uint32_t step, bool rebase, uint64_t **recv, uint64_t *n_recv);
+// local_rc: this rank has already failed with that code; it sends nothing, and every rank returns an error (the
+// failing rank its own code and message, the others the code of the first failing rank).
+int route_keys(kombgpu_comm *c, const uint64_t *keys, uint64_t n, uint32_t step, bool rebase, uint64_t **recv, uint64_t *n_recv,
+               int local_rc = KOMBGPU_OK);
 // ppeel.cu
 int dist_peel(kombgpu_dist_graph *g);
 // apeel.cu

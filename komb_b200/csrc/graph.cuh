@@ -51,9 +51,37 @@ int hits_to_edges(kombgpu_ctx *ctx, const uint32_t *read_key, const uint32_t *un
                   uint32_t *n_chunks = nullptr);
 int pairs_to_edges(kombgpu_ctx *ctx, const uint32_t *u, const uint32_t *v, uint64_t n_pairs, uint32_t n_vertices,
                    DevBuf<uint64_t> &edges, uint64_t *n_edges, DevBuf<uint32_t> *mult = nullptr, uint32_t *n_chunks = nullptr);
-int hits_to_pairs(kombgpu_ctx *ctx, const uint32_t *read_key, const uint32_t *unitig, uint64_t n_hits, uint32_t n_vertices,
-                  DevBuf<uint64_t> &pairs, uint64_t *n_pairs, kombgpu_stats *st);
-int pairs_to_keys(kombgpu_ctx *ctx, const uint32_t *u, const uint32_t *v, uint64_t n_pairs, uint32_t n_vertices, DevBuf<uint64_t> &keys);
+// Steps 1-2 of a build from hits: the unique hits grouped by read, the reads with >= 2 unitigs as segments and the
+// global index of every segment's first pair.  P is known before any pair exists; emit(p0, p1, dst) then writes the
+// canonical keys (min << 32 | max) of pairs [p0, p1) to dst[0, p1 - p0), in emission order (not sorted, duplicates in):
+// the whole list in one shot or one chunk of it (a chunk may start inside a read's clique).
+struct HitPairs {
+    kombgpu_ctx *ctx = nullptr;
+    DevBuf<uint64_t> ha, hb, hc, seg_base;
+    DevBuf<uint32_t> seg_head, seg_tail, tile_seg;
+    const uint64_t *hits = nullptr;   // unique hits grouped by read, inside ha / hb / hc
+    uint32_t n_seg = 0;
+    uint64_t n_pairs = 0;
+    int emit(uint64_t p0, uint64_t p1, uint64_t *dst);
+    void release();
+};
+int count_hit_pairs(kombgpu_ctx *ctx, const uint32_t *read_key, const uint32_t *unitig, uint64_t n_hits, uint32_t n_vertices,
+                    HitPairs *hp, kombgpu_stats *st);
+// (u, v) pairs -> canonical keys (min << 32 | max) in dst[0, n), input order; KOMBGPU_EINVAL when an id is >= n_vertices
+int pack_pairs(kombgpu_ctx *ctx, const uint32_t *u, const uint32_t *v, uint64_t n, uint32_t n_vertices, uint64_t *dst);
+
+// Pairs reduced a chunk at a time (build.cu, "chunked path"): the chunk size, and KOMBGPU_PAIR_CHUNK (0 when unset)
+constexpr uint64_t kPairChunk = (1ull << 30) - (1ull << 20);   // below 2^30: every chunk sorts with the single-read passes
+uint64_t pair_chunk_env();
+// the running edge list of a chunked build: sorted unique keys and how many pairs support each (saturating at 2^32 - 1)
+struct EdgeRun {
+    DevBuf<uint64_t> keys;
+    DevBuf<uint32_t> cnt;
+    uint64_t n = 0;
+};
+// one sorted chunk of pair keys (duplicates and loops in, n_c < 2^32) -> sorted unique (key, count) in cuniq / ccnt
+// (n_c entries of room each), merged into the running list.  KOMBGPU_EINVAL when the list would reach 2^32 edges.
+int merge_sorted_chunk(kombgpu_ctx *ctx, const uint64_t *sorted, uint64_t n_c, uint64_t *cuniq, uint32_t *ccnt, EdgeRun *run);
 // sorted canonical keys (duplicates and loops in) -> unique simple edges (+ optional multiplicities)
 int unique_edges(kombgpu_ctx *ctx, const uint64_t *keys, uint64_t count, DevBuf<uint64_t> &edges, uint64_t *n_edges,
                  DevBuf<uint32_t> *mult);

@@ -182,6 +182,12 @@ __global__ void __launch_bounds__(kThreads) low_words_kernel(const uint64_t *__r
     for (uint64_t i = (uint64_t)blockIdx.x * blockDim.x + threadIdx.x; i < n; i += (uint64_t)gridDim.x * blockDim.x) out[i] = (uint32_t)keys[i];
 }
 
+struct SymRewind {   // gives the symmetric heap back to a mark when the scope ends, on every return path
+    kombgpu_comm *c;
+    SymMark mark;
+    ~SymRewind() { sym_release(c, mark); }
+};
+
 struct EvTimer {   // CUDA-event split timer on the context's stream
     kombgpu_ctx *ctx;
     cudaEvent_t a = nullptr, b = nullptr;
@@ -226,26 +232,29 @@ int dist_peel_mode() {   // 0 log, 1 async, 2 auto, 3 replicated
     return 2;
 }
 
-int route_keys(kombgpu_comm *c, const uint64_t *keys, uint64_t n, uint32_t step, bool rebase, uint64_t **recv, uint64_t *n_recv) {
+int route_keys(kombgpu_comm *c, const uint64_t *keys, uint64_t n, uint32_t step, bool rebase, uint64_t **recv, uint64_t *n_recv,
+               int local_rc) {
     kombgpu_ctx *ctx = c->ctx;
     const int world = c->world;
     DevBuf<unsigned long long> d_counts(ctx, 2 * kMaxRanks);   // [counts | cursors]
     DevBuf<uint32_t> d_err(ctx, 1);
     if (!d_counts || !d_err) return ctx_fail(ctx, KOMBGPU_ENOMEM, "workspace");
-    KG_CUDA(ctx, cudaMemsetAsync(d_counts.p, 0, 2 * kMaxRanks * sizeof(unsigned long long), ctx->stream));
-    KG_CUDA(ctx, cudaMemsetAsync(d_err.p, 0, sizeof(uint32_t), ctx->stream));
     const uint32_t grid = min(grid_for(n, kRtTile), (uint32_t)ctx->sm_count * 8u);
-    if (n) KG_LAUNCH(ctx, route_count_kernel, grid, kRtThreads, 0, keys, n, step, world, d_counts.p, d_err.p);
     unsigned long long h_counts[kMaxRanks + 1] = {};
-    KG_TRY(read_back(ctx, d_counts.p, h_counts, kMaxRanks));
     uint32_t h_err = 0;
-    KG_TRY(read_back(ctx, d_err.p, &h_err, 1));
-    // a rank with bad input still takes part in the exchange (its peers are waiting), then everybody fails together
-    h_counts[world] = h_err;
+    if (local_rc == KOMBGPU_OK) {   // a rank that has failed already sends nothing and only reports its error
+        KG_CUDA(ctx, cudaMemsetAsync(d_counts.p, 0, 2 * kMaxRanks * sizeof(unsigned long long), ctx->stream));
+        KG_CUDA(ctx, cudaMemsetAsync(d_err.p, 0, sizeof(uint32_t), ctx->stream));
+        if (n) KG_LAUNCH(ctx, route_count_kernel, grid, kRtThreads, 0, keys, n, step, world, d_counts.p, d_err.p);
+        KG_TRY(read_back(ctx, d_counts.p, h_counts, kMaxRanks));
+        KG_TRY(read_back(ctx, d_err.p, &h_err, 1));
+    }
+    // a rank with bad input still takes part in the exchange (its peers are waiting), then everybody fails together:
+    // the error word is the rank's (negated) error code
+    h_counts[world] = local_rc != KOMBGPU_OK ? (unsigned long long)-local_rc : (h_err ? (unsigned long long)-KOMBGPU_EINVAL : 0ull);
     unsigned long long matrix[kMaxRanks * (kMaxRanks + 1)];   // matrix[q * (world + 1) + p] = keys rank q sends to rank p
     KG_TRY(comm_exchange(c, h_counts, world + 1, matrix));
     unsigned long long my_off[kMaxRanks] = {}, max_recv = 0, mine = 0;
-    bool any_err = false;
     for (int p = 0; p < world; ++p) {
         unsigned long long tot = 0;
         for (int q = 0; q < world; ++q) {
@@ -255,8 +264,13 @@ int route_keys(kombgpu_comm *c, const uint64_t *keys, uint64_t n, uint32_t step,
         if (tot > max_recv) max_recv = tot;
         if (p == c->rank) mine = tot;
     }
-    for (int q = 0; q < world; ++q) any_err = any_err || matrix[q * (world + 1) + world] != 0;
-    if (any_err) return ctx_fail(ctx, KOMBGPU_EINVAL, "a unitig id is outside [0, n_vertices_global) on some rank");
+    for (int q = 0; q < world; ++q) {
+        const unsigned long long e = matrix[q * (world + 1) + world];
+        if (!e) continue;
+        if (local_rc != KOMBGPU_OK) return local_rc;   // this rank's own message stands
+        if (h_err) return ctx_fail(ctx, KOMBGPU_EINVAL, "a unitig id is outside [0, n_vertices_global) on some rank");
+        return ctx_fail(ctx, -(int)e, "rank %d failed; the build stopped on every rank", q);
+    }
     if (max_recv >= (1ull << 32)) return ctx_fail(ctx, KOMBGPU_EINVAL, "%llu keys routed to one rank exceed the 2^32 per-device limit", max_recv);
     uint64_t *buf = nullptr;
     PeerPtrs<uint64_t> peers{};
@@ -291,65 +305,104 @@ int dist_build(kombgpu_comm *c, const uint32_t *a, const uint32_t *b, uint64_t c
     const int bn = bits_for(n_global > 0 ? n_global - 1 : 0);
     EvTimer total(ctx), split(ctx);
 
-    // 1. this rank's pairs
-    DevBuf<uint64_t> pairs;
-    uint64_t n_pairs = 0;
+    // 1. count this rank's pairs (hits: unique hits, segments and their pair offsets) without emitting them
+    HitPairs hp;
+    uint64_t n_pairs = count;
     int rc_local = KOMBGPU_OK;
     if (from_hits) {
         kombgpu_stats st{};
-        rc_local = hits_to_pairs(ctx, a, b, count, n_global, pairs, &n_pairs, &st);
+        rc_local = count_hit_pairs(ctx, a, b, count, n_global, &hp, &st);
+        n_pairs = hp.n_pairs;
         g->st.n_hits_local = count;
-    } else {
-        rc_local = pairs_to_keys(ctx, a, b, count, n_global, pairs);
-        n_pairs = count;
-    }
-    // a rank whose input is bad must not leave its peers waiting in the first exchange: it routes nothing and
-    // reports the error through the count exchange of route_keys
-    if (rc_local != KOMBGPU_OK) {
-        // poison: one key with an out-of-range owner makes every rank fail in route_keys
-        DevBuf<uint64_t> bad(ctx, 1);
-        if (bad) {
-            const uint64_t k = ~0ull;
-            cudaMemcpyAsync(bad.p, &k, sizeof(k), cudaMemcpyHostToDevice, ctx->stream);
-            uint64_t *r = nullptr, nr = 0;
-            const std::string msg = ctx->err;
-            route_keys(c, bad.p, 1, g->step, false, &r, &nr);
-            ctx->err = msg;
-        }
-        return rc_local;
     }
     g->st.n_pairs_local = n_pairs;
 
-    // 2. pairs -> owner of min(u, v); sort + unique there
-    const SymMark mark = sym_mark(c);
-    uint64_t *recv = nullptr, n_recv = 0;
-    KG_TRY(route_keys(c, pairs.p, n_pairs, g->step, false, &recv, &n_recv));
-    pairs.release();
-    g->st.n_pairs_received = n_recv;
-    g->st.ms_build_route = split.lap();
-    DevBuf<uint64_t> tmp, edges;
-    DevBuf<uint32_t> mult;
-    uint64_t n_fwd = 0;
-    {
-        KG_ALLOC(ctx, tmp, n_recv);
-        RadixPass passes[8];
-        const int np = plan_radix_passes(0, bn, 32, 32 + bn, passes);
-        uint64_t *sorted = recv;
-        KG_TRY(radix_sort_u64(ctx, recv, tmp.p, n_recv, passes, np, &sorted));
-        KG_TRY(unique_edges(ctx, sorted, n_recv, edges, &n_fwd, &mult));
+    // one decision for every rank: one shot while the pairs of all ranks stay below 2^32 (so does every owner's share),
+    // else R rounds of at most `chunk` pairs per rank (DESIGN.md §4).  A rank whose count failed reports its error here.
+    unsigned long long mine_p[2] = {rc_local == KOMBGPU_OK ? n_pairs : 0ull, (unsigned long long)-rc_local}, all_p[kMaxRanks * 2];
+    KG_TRY(comm_exchange(c, mine_p, 2, all_p));
+    uint64_t sum_p = 0, max_p = 0;
+    for (int q = 0; q < world; ++q) {
+        sum_p += all_p[q * 2];
+        max_p = all_p[q * 2] > max_p ? all_p[q * 2] : max_p;
+    }
+    if (rc_local != KOMBGPU_OK) return rc_local;
+    for (int q = 0; q < world; ++q)
+        if (all_p[q * 2 + 1]) return ctx_fail(ctx, -(int)all_p[q * 2 + 1], "rank %d failed; the build stopped on every rank", q);
+    uint64_t chunk = 0;   // 0: one shot
+    const uint64_t cap = pair_chunk_env();
+    if (cap && max_p > cap) chunk = min(cap, (uint64_t)(0xffffffffu / (uint32_t)world));   // world x chunk < 2^32: an owner's counts are 32-bit
+    else if (sum_p >= (1ull << 32)) chunk = kPairChunk / (uint64_t)world;   // an owner receives < 2^30 keys a round
+    const uint64_t per_round = chunk ? chunk : n_pairs;
+    const uint32_t rounds = chunk ? (uint32_t)((max_p + chunk - 1) / chunk) : 1u;
+    g->build_rounds = rounds;
+
+    // 2. every round: emit the next pairs, route them to the owner of min(u, v), sort there, then unique (one shot) or
+    //    reduce and merge into the running edge list.  From here on a rank that fails keeps taking part in the
+    //    exchanges, routes nothing and reports its error in the next route_keys, where every rank stops.
+    SymRewind heap{c, sym_mark(c)};   // each round's receive buffer is released once it is reduced; all of them on failure
+    if (chunk) {
+        // an owner receives at most world x chunk keys a round: one segment of that size up front, so a round that
+        // outgrows an earlier one does not stack another segment on the heap (same call on every rank: collective)
+        uint64_t *reserve = nullptr;
+        PeerPtrs<uint64_t> peers{};
+        KG_TRY(sym_alloc(c, (size_t)(world * chunk), &reserve, &peers));
+        sym_release(c, heap.mark);
+    }
+    DevBuf<uint64_t> edges, tmp;   // tmp: the sort's second buffer (in rounds also the reduced keys)
+    DevBuf<uint32_t> mult, ccnt;   // ccnt: the reduced keys' counts
+    // in rounds both are sized once for the largest receive, as the single-GPU chunk buffers are: no round reallocates
+    if (chunk && (!tmp.alloc(ctx, world * chunk) || !ccnt.alloc(ctx, world * chunk)))
+        rc_local = ctx_fail(ctx, KOMBGPU_ENOMEM, "device workspace for %llu routed pairs", (unsigned long long)(world * chunk));
+    EdgeRun run;
+    uint64_t n_fwd = 0, n_recv_total = 0;
+    for (uint32_t r = 0; r < rounds; ++r) {
+        const uint64_t p0 = min(n_pairs, (uint64_t)r * per_round), p1 = min(n_pairs, p0 + per_round);
+        DevBuf<uint64_t> pairs;
+        if (rc_local == KOMBGPU_OK) {
+            if (!pairs.alloc(ctx, p1 - p0)) rc_local = ctx_fail(ctx, KOMBGPU_ENOMEM, "device workspace for %llu pairs", (unsigned long long)(p1 - p0));
+            else rc_local = from_hits ? hp.emit(p0, p1, pairs.p) : pack_pairs(ctx, a + p0, b + p0, p1 - p0, n_global, pairs.p);
+        }
+        if (p1 >= n_pairs) hp.release();   // every pair of this rank is out: the hits and segments are dead
+        uint64_t *recv = nullptr, n_recv = 0;
+        KG_TRY(route_keys(c, pairs.p, rc_local == KOMBGPU_OK ? p1 - p0 : 0, g->step, false, &recv, &n_recv, rc_local));
+        pairs.release();
+        n_recv_total += n_recv;
+        g->st.ms_build_route += split.lap();
+        // route_keys succeeded, so no rank has failed so far
+        rc_local = [&]() -> int {
+            if (!chunk) KG_ALLOC(ctx, tmp, n_recv);
+            RadixPass passes[8];
+            const int np = plan_radix_passes(0, bn, 32, 32 + bn, passes);
+            uint64_t *sorted = recv;
+            KG_TRY(radix_sort_u64(ctx, recv, tmp.p, n_recv, passes, np, &sorted));
+            if (!chunk) return unique_edges(ctx, sorted, n_recv, edges, &n_fwd, &mult);
+            if (n_recv == 0) return KOMBGPU_OK;
+            return merge_sorted_chunk(ctx, sorted, n_recv, sorted == recv ? tmp.p : recv, ccnt.p, &run);
+        }();
+        sym_release(c, heap.mark);   // the receive buffer is dead (stream-ordered: later kernels of this stream come after its readers)
+        g->st.ms_build_sort += split.lap();
     }
     tmp.release();
-    sym_release(c, mark);   // the receive buffer is dead (stream-ordered: later kernels of this stream come after its readers)
+    ccnt.release();
+    if (chunk && rc_local == KOMBGPU_OK) {
+        if (!run.keys && !run.keys.alloc(ctx, 0)) rc_local = ctx_fail(ctx, KOMBGPU_ENOMEM, "workspace");
+        if (!run.cnt && !run.cnt.alloc(ctx, 0)) rc_local = ctx_fail(ctx, KOMBGPU_ENOMEM, "workspace");
+        edges = std::move(run.keys);
+        mult = std::move(run.cnt);
+        n_fwd = run.n;
+    }
+    g->st.n_pairs_received = n_recv_total;
     g->n_fwd = n_fwd;
     g->st.n_fwd_local = n_fwd;
-    g->st.ms_build_sort = split.lap();
 
     // 3. reversed copies -> owner of max(u, v) (high word rebased to the owner's range); stable sort by row there
     DevBuf<uint64_t> swapped;
-    KG_ALLOC(ctx, swapped, n_fwd);
-    if (n_fwd) KG_LAUNCH(ctx, swap_edges_kernel, min(grid_for(n_fwd, kThreads), 148u * 16u), kThreads, 0, edges.p, n_fwd, swapped.p);
+    if (rc_local == KOMBGPU_OK && !swapped.alloc(ctx, n_fwd)) rc_local = ctx_fail(ctx, KOMBGPU_ENOMEM, "device workspace for %llu edges", (unsigned long long)n_fwd);
+    if (rc_local == KOMBGPU_OK && n_fwd)
+        KG_LAUNCH(ctx, swap_edges_kernel, min(grid_for(n_fwd, kThreads), 148u * 16u), kThreads, 0, edges.p, n_fwd, swapped.p);
     uint64_t *back = nullptr, n_back = 0;
-    KG_TRY(route_keys(c, swapped.p, n_fwd, g->step, true, &back, &n_back));
+    KG_TRY(route_keys(c, swapped.p, rc_local == KOMBGPU_OK ? n_fwd : 0, g->step, true, &back, &n_back, rc_local));
     swapped.release();
     g->st.ms_build_route += split.lap();
     // 4. the local entries keyed by neighbour: (v << 32 | u - v_lo) for the forward edges, (w << 32 | u - v_lo) for what arrived;
@@ -413,7 +466,7 @@ int dist_build(kombgpu_comm *c, const uint32_t *a, const uint32_t *b, uint64_t c
     KG_TRY(read_back(ctx, max_deg.p, &h_max, 1));
     keys_a.release();
     keys_b.release();
-    sym_release(c, mark);
+    sym_release(c, heap.mark);
     g->st.ms_build_csr = split.lap();
 
     // global figures (also the barrier that ends the stage: every rank's rows are complete)

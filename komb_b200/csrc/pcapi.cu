@@ -4,6 +4,7 @@
 #include <new>
 
 #include "dgraph.cuh"
+#include "kombgpu_debug.h"
 
 using namespace kg;
 
@@ -173,6 +174,13 @@ int kombgpu_dist_graph_device_arrays(const kombgpu_dist_graph *g, const uint64_t
     if (degree) *degree = g->deg;
     if (coreness) *coreness = g->has_core ? g->core : nullptr;
     if (score) *score = g->has_score ? g->score : nullptr;
+    return KOMBGPU_OK;
+}
+
+// measurement aid (include/kombgpu_debug.h): how many rounds the build reduced its pairs in
+int kombgpu_debug_dist_build_rounds(const kombgpu_dist_graph *g, uint32_t *n_rounds) {
+    if (!g || !n_rounds) return KOMBGPU_EINVAL;
+    *n_rounds = g->build_rounds;
     return KOMBGPU_OK;
 }
 

@@ -121,6 +121,12 @@ class DistGraph:
         self._ctx._check(self._lib.kombgpu_dist_graph_stats(self._h, byref(st)))
         return st.as_dict()
 
+    def build_rounds(self) -> int:
+        """Rounds the build emitted, routed and reduced the clique pairs in: 1 on the one-shot path (kombgpu_debug.h)."""
+        n = c_uint32()
+        self._ctx._check(self._lib.kombgpu_debug_dist_build_rounds(self._h, byref(n)))
+        return n.value
+
     def summary(self) -> tuple[int, float]:
         mc, ms = c_int32(), c_double()
         self._ctx._check(self._lib.kombgpu_dist_graph_summary(self._h, byref(mc), byref(ms)))
