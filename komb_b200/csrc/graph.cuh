@@ -71,7 +71,7 @@ int count_hit_pairs(kombgpu_ctx *ctx, const uint32_t *read_key, const uint32_t *
 int pack_pairs(kombgpu_ctx *ctx, const uint32_t *u, const uint32_t *v, uint64_t n, uint32_t n_vertices, uint64_t *dst);
 
 // Pairs reduced a chunk at a time (build.cu, "chunked path"): the chunk size, and KOMBGPU_PAIR_CHUNK (0 when unset)
-constexpr uint64_t kPairChunk = (1ull << 30) - (1ull << 20);   // below 2^30: every chunk sorts with the single-read passes
+constexpr uint64_t kPairChunk = (1ull << 30) - (1ull << 20);   // bounds the memory of a chunk: its keys, sort buffer, counts
 uint64_t pair_chunk_env();
 // the running edge list of a chunked build: sorted unique keys and how many pairs support each (saturating at 2^32 - 1)
 struct EdgeRun {

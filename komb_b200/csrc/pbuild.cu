@@ -332,7 +332,7 @@ int dist_build(kombgpu_comm *c, const uint32_t *a, const uint32_t *b, uint64_t c
     uint64_t chunk = 0;   // 0: one shot
     const uint64_t cap = pair_chunk_env();
     if (cap && max_p > cap) chunk = min(cap, (uint64_t)(0xffffffffu / (uint32_t)world));   // world x chunk < 2^32: an owner's counts are 32-bit
-    else if (sum_p >= (1ull << 32)) chunk = kPairChunk / (uint64_t)world;   // an owner receives < 2^30 keys a round
+    else if (sum_p >= (1ull << 32)) chunk = kPairChunk / (uint64_t)world;   // an owner receives < 2^30 keys a round: bounds its buffers
     const uint64_t per_round = chunk ? chunk : n_pairs;
     const uint32_t rounds = chunk ? (uint32_t)((max_p + chunk - 1) / chunk) : 1u;
     g->build_rounds = rounds;

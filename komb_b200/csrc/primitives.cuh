@@ -1,9 +1,7 @@
 // primitives.cuh — device-wide building blocks used by the graph build and
-// CORE-A stages: a generic three-phase prefix scan (also used as stream
-// compaction) and an LSD radix sort of 64-bit keys.  All HBM-bound integer work.
+// CORE-A stages: a generic single-pass prefix scan (also used as stream
+// compaction) and an LSD radix sort of 64-bit keys (sort.cu).  All HBM-bound integer work.
 #pragma once
-
-#include <cstdlib>
 
 #include "common.cuh"
 
@@ -23,24 +21,6 @@ struct RadixPass {
 // fewest passes of at most 8 bits (equal widths), least significant first.
 int plan_radix_passes(int lo0, int hi0, int lo1, int hi1, RadixPass *out /* >= 8 entries */);
 
-#ifdef __CUDACC__
-// digit extraction shared by every sort kernel
-struct DigitSpec {
-    int shift, shift2, bits1;
-    uint32_t mask1, mask2, mask;   // mask = all digit bits
-    __host__ __device__ static DigitSpec of(const RadixPass &p) {
-        DigitSpec d;
-        d.shift = p.shift; d.shift2 = p.shift2; d.bits1 = p.bits;
-        d.mask1 = (1u << p.bits) - 1u; d.mask2 = (1u << p.bits2) - 1u;
-        d.mask = (1u << (p.bits + p.bits2)) - 1u;
-        return d;
-    }
-    __device__ __forceinline__ uint32_t operator()(uint64_t key) const {
-        return ((uint32_t)(key >> shift) & mask1) | (((uint32_t)(key >> shift2) & mask2) << bits1);
-    }
-};
-#endif
-
 // Stable LSD radix sort.  `a` holds the keys, `b` is scratch of the same size;
 // returns in *sorted whichever of the two holds the result.
 int radix_sort_u64(kombgpu_ctx *ctx, uint64_t *a, uint64_t *b, uint64_t n, const RadixPass *passes,
@@ -49,67 +29,11 @@ int radix_sort_u64(kombgpu_ctx *ctx, uint64_t *a, uint64_t *b, uint64_t n, const
 #ifdef __CUDACC__
 
 constexpr int kScanThreads = 512;
-constexpr int kScanItems = 16;
-constexpr int kScanTile = kScanThreads * kScanItems;
-
-// phase 1: per-tile sums of in(i)
-template <typename T, typename InFn>
-__global__ void __launch_bounds__(kScanThreads) scan_reduce_kernel(uint64_t n, InFn in, T *tile_sums) {
-    __shared__ T s_warp[kScanThreads / 32];
-    const uint64_t base = (uint64_t)blockIdx.x * kScanTile;
-    T acc = T(0);
-#pragma unroll 4
-    for (int j = 0; j < kScanItems; ++j) {
-        uint64_t i = base + (uint64_t)j * kScanThreads + threadIdx.x;
-        if (i < n) acc += in(i);
-    }
-    acc = warp_reduce_add(acc);
-    if (lane_id() == 0) s_warp[threadIdx.x >> 5] = acc;
-    __syncthreads();
-    if (threadIdx.x < 32) {
-        T v = threadIdx.x < kScanThreads / 32 ? s_warp[threadIdx.x] : T(0);
-        v = warp_reduce_add(v);
-        if (threadIdx.x == 0) tile_sums[blockIdx.x] = v;
-    }
-}
-
-// phase 2: one CTA turns tile sums into exclusive tile prefixes (+ grand total)
-template <typename T>
-__global__ void __launch_bounds__(1024) scan_tiles_kernel(T *tile_sums, uint32_t n_tiles, T *total) {
-    __shared__ T s_scan[33];
-    T carry = T(0);
-    for (uint32_t base = 0; base < n_tiles; base += 1024) {
-        uint32_t i = base + threadIdx.x;
-        T v = i < n_tiles ? tile_sums[i] : T(0);
-        T tot;
-        T ex = block_excl_scan_add<T, 1024>(v, s_scan, &tot);
-        if (i < n_tiles) tile_sums[i] = carry + ex;
-        carry += tot;
-    }
-    if (threadIdx.x == 0 && total) *total = carry;
-}
-
-// phase 3: out(i, exclusive_prefix_i, in(i))
-template <typename T, typename InFn, typename OutFn>
-__global__ void __launch_bounds__(kScanThreads) scan_downsweep_kernel(uint64_t n, InFn in, const T *tile_prefix, OutFn out) {
-    __shared__ T s_scan[kScanThreads / 32 + 1];
-    const uint64_t base = (uint64_t)blockIdx.x * kScanTile;
-    T carry = tile_prefix[blockIdx.x];
-    for (int j = 0; j < kScanItems; ++j) {
-        uint64_t i = base + (uint64_t)j * kScanThreads + threadIdx.x;
-        if (base + (uint64_t)j * kScanThreads >= n) break;  // uniform across the CTA
-        T v = i < n ? in(i) : T(0);
-        T tot;
-        T ex = block_excl_scan_add<T, kScanThreads>(v, s_scan, &tot);
-        if (i < n) out(i, carry + ex, v);
-        carry += tot;
-    }
-}
 
 // Single-pass scan (chained scan with decoupled look-back): every element's in(i) is evaluated ONCE (some of the
 // path's functors look back through a read or compare neighbouring keys) and every access stays coalesced (item j of
 // thread t is element base + j * threads + t).  Inside a tile: one warp scan per item, the 16 x 16 (item, warp)
-// totals scanned once by the CTA -- two barriers instead of the three per item of the downsweep kernel.  Tiles
+// totals scanned once by the CTA -- two barriers a tile, not three per item.  Tiles
 // take their index from a counter and learn the sum of all earlier tiles from 64-bit status words (2 flag bits +
 // 62-bit value: every sum on this path is far below 2^62), 32 predecessors per look-back step.
 constexpr uint64_t kScanFlagAgg = 1ull << 62, kScanFlagPrefix = 2ull << 62, kScanValueMask = (1ull << 62) - 1;
@@ -200,23 +124,12 @@ int device_scan(kombgpu_ctx *ctx, uint64_t n, InFn in, OutFn out, T *total_dev) 
         if (total_dev) KG_CUDA(ctx, cudaMemsetAsync(total_dev, 0, sizeof(T), ctx->stream));
         return KOMBGPU_OK;
     }
-    // KOMBGPU_SCAN=legacy: the three-kernel scan (reduce, tile prefixes, downsweep), kept for A/B runs
-    static const bool legacy = getenv("KOMBGPU_SCAN") != nullptr && getenv("KOMBGPU_SCAN")[0] == 'l';
-    if (!legacy) {
-        const uint32_t n_tiles = ceil_div_u64(n, (uint64_t)kScanThreads * ScanShape<T>::kItems);
-        DevBuf<uint64_t> status;   // [n_tiles status words | tile counter]
-        KG_ALLOC(ctx, status, (size_t)n_tiles + 1);
-        KG_CUDA(ctx, cudaMemsetAsync(status.p, 0, ((size_t)n_tiles + 1) * sizeof(uint64_t), ctx->stream));
-        KG_LAUNCH(ctx, (scan_onepass_kernel<T, InFn, OutFn>), n_tiles, kScanThreads, 0, n, in, out, status.p,
-                  reinterpret_cast<uint32_t *>(status.p + n_tiles), n_tiles, total_dev);
-        return KOMBGPU_OK;
-    }
-    uint32_t n_tiles = ceil_div_u64(n, kScanTile);
-    DevBuf<T> tiles;
-    KG_ALLOC(ctx, tiles, n_tiles);
-    KG_LAUNCH(ctx, (scan_reduce_kernel<T, InFn>), n_tiles, kScanThreads, 0, n, in, tiles.p);
-    KG_LAUNCH(ctx, (scan_tiles_kernel<T>), 1, 1024, 0, tiles.p, n_tiles, total_dev);
-    KG_LAUNCH(ctx, (scan_downsweep_kernel<T, InFn, OutFn>), n_tiles, kScanThreads, 0, n, in, tiles.p, out);
+    const uint32_t n_tiles = ceil_div_u64(n, (uint64_t)kScanThreads * ScanShape<T>::kItems);
+    DevBuf<uint64_t> status;   // [n_tiles status words | tile counter]
+    KG_ALLOC(ctx, status, (size_t)n_tiles + 1);
+    KG_CUDA(ctx, cudaMemsetAsync(status.p, 0, ((size_t)n_tiles + 1) * sizeof(uint64_t), ctx->stream));
+    KG_LAUNCH(ctx, (scan_onepass_kernel<T, InFn, OutFn>), n_tiles, kScanThreads, 0, n, in, out, status.p,
+              reinterpret_cast<uint32_t *>(status.p + n_tiles), n_tiles, total_dev);
     return KOMBGPU_OK;
 }
 

@@ -1,20 +1,14 @@
 // sort.cu — stable LSD radix sort of 64-bit keys (unitig pairs, swapped edges, CORE-A rank keys, and hits
 // when they do not arrive in read order).  Integer, HBM-bound.
 //
-// Default: single-read passes (radix_sweep_kernel, "onesweep"): one kernel histograms every pass's digit up
-// front, then each pass reads the keys once and writes them once; tiles learn their global offsets by a
-// decoupled look-back over per-tile status words.  The tile is staged in shared memory in digit order so
-// global stores are contiguous runs.  Measured on B200 (tools/sort_probe.py): 2.0 TB/s read+write per pass on
-// 33 M keys, 2.1 TB/s on 540 M, against 1.7 / 1.9 TB/s for the three-kernel passes (per-tile histogram, table
-// scan, scatter) that are kept for arrays of 2^30 keys and more and for A/B runs (KOMBGPU_SORT=legacy).
+// Single-read passes (radix_sweep_kernel, "onesweep"): one kernel histograms every pass's digit up front, then each
+// pass reads the keys once and writes them once; tiles learn their global offsets by a decoupled look-back over
+// per-tile status words.  The tile is staged in shared memory in digit order so global stores are contiguous runs.
+// One implementation serves every n < 2^32: only the width of the status words depends on n (see StatusWord).
 // What bounds a pass is instruction issue, not DRAM: ~130 thread-instructions per key, half of them the
-// ballot-per-digit-bit ranking (ncu: issue slots 50 % busy, ALU pipe 49 %, barrier stalls 44 % of samples, DRAM
-// 25 % of peak; profiles/r1/r1o_sweep_*).  MATCH.ANY ranks a key in one instruction but runs on the ADU pipe
-// and made every mix of the two slower (measured in round 1 with 0/2/4/8 items per thread; removed since).
-// Tile geometries measured in round 2 (33 M pair keys, 5 passes; profiles/r2/r2v_sort_geometries.log): 512 x 16 keys
-// 1.30 ms, 256 x 16 (4 CTAs/SM) 1.35, 256 x 16 (3) 1.85, 128 x 16 (8) 1.74, 256 x 8 (6) 1.61, 384 x 16 (2) 1.82.
-#include <cstdlib>
-
+// ballot-per-digit-bit ranking (profiles/r1/r1o_sweep_*).  MATCH.ANY ranks a key in one instruction but runs on the ADU
+// pipe and made every mix of the two slower (round 1).  Measurements of the passes and of the tile geometries that lost
+// to the one below are in DESIGN.md §4 "Sort".
 #include "kombgpu_debug.h"
 #include "primitives.cuh"
 
@@ -24,141 +18,25 @@ namespace {
 
 constexpr int kRsThreads = 512;
 constexpr int kRsItems = 8;
-constexpr int kRsTile = kRsThreads * kRsItems;  // 4096 keys per CTA
-constexpr int kRsWarps = kRsThreads / 32;
+constexpr int kRsTile = kRsThreads * kRsItems;  // 4096 keys per CTA of the histogram kernel
 constexpr int kRadix = 256;
+constexpr int kMaxPasses = 8;
 
-// table[d * n_tiles + tile] = number of keys of this tile whose digit is d
-__global__ void __launch_bounds__(kRsThreads) radix_hist_kernel(const uint64_t *__restrict__ keys, uint64_t n, DigitSpec dg,
-                                                                uint32_t *__restrict__ table, uint32_t n_tiles) {
-    const uint32_t mask = dg.mask;
-    __shared__ uint32_t s_hist[kRadix];
-    for (int d = threadIdx.x; d < kRadix; d += kRsThreads) s_hist[d] = 0;
-    __syncthreads();
-    const uint64_t base = (uint64_t)blockIdx.x * kRsTile;
-#pragma unroll
-    for (int j = 0; j < kRsItems; ++j) {
-        uint64_t i = base + (uint64_t)j * kRsThreads + threadIdx.x;
-        if (i < n) atomicAdd(&s_hist[dg(keys[i])], 1u);
+// digit extraction of one pass (RadixPass)
+struct DigitSpec {
+    int shift, shift2, bits1;
+    uint32_t mask1, mask2, mask;   // mask = all digit bits
+    __host__ __device__ static DigitSpec of(const RadixPass &p) {
+        DigitSpec d;
+        d.shift = p.shift; d.shift2 = p.shift2; d.bits1 = p.bits;
+        d.mask1 = (1u << p.bits) - 1u; d.mask2 = (1u << p.bits2) - 1u;
+        d.mask = (1u << (p.bits + p.bits2)) - 1u;
+        return d;
     }
-    __syncthreads();
-    for (int d = threadIdx.x; d <= (int)mask; d += kRsThreads) table[(uint64_t)d * n_tiles + blockIdx.x] = s_hist[d];
-}
-
-struct TableIn {
-    const uint32_t *t;
-    __device__ uint32_t operator()(uint64_t i) const { return t[i]; }
+    __device__ __forceinline__ uint32_t operator()(uint64_t key) const {
+        return ((uint32_t)(key >> shift) & mask1) | (((uint32_t)(key >> shift2) & mask2) << bits1);
+    }
 };
-struct TableOut {
-    uint32_t *t;
-    __device__ void operator()(uint64_t i, uint32_t prefix, uint32_t) const { t[i] = prefix; }
-};
-
-// dynamic shared memory layout of the scatter kernel
-struct ScatterSmem {
-    uint64_t keys[kRsTile];
-    uint32_t warp_cnt[kRsWarps][kRadix];
-    uint32_t digit_local[kRadix];   // first slot of digit d inside the staged tile
-    uint32_t digit_global[kRadix];  // global position of that slot minus digit_local
-    uint32_t scan_tmp[kRadix / 32 + 1];
-};
-
-__global__ void __launch_bounds__(kRsThreads) radix_scatter_kernel(const uint64_t *__restrict__ in, uint64_t *__restrict__ out,
-                                                                   uint64_t n, DigitSpec dg,
-                                                                   const uint32_t *__restrict__ table, uint32_t n_tiles) {
-    extern __shared__ __align__(16) unsigned char s_raw[];
-    ScatterSmem &s = *reinterpret_cast<ScatterSmem *>(s_raw);
-    const uint32_t mask = dg.mask;
-    const uint32_t warp = threadIdx.x >> 5, lane = lane_id();
-    const uint64_t tile_base = (uint64_t)blockIdx.x * kRsTile;
-    const uint32_t tile_count = (uint32_t)min((uint64_t)kRsTile, n - tile_base);
-
-    for (int i = threadIdx.x; i < kRsWarps * kRadix; i += kRsThreads) (&s.warp_cnt[0][0])[i] = 0;
-
-    // warp-striped load: item j of lane l is tile element warp*256 + j*32 + l,
-    // so (warp, j, lane) order is memory order and the sort stays stable.
-    uint64_t key[kRsItems];
-    uint32_t rank[kRsItems];
-    const uint32_t warp_base = warp * (32 * kRsItems);
-#pragma unroll
-    for (int j = 0; j < kRsItems; ++j) {
-        uint32_t e = warp_base + j * 32 + lane;
-        key[j] = e < tile_count ? in[tile_base + e] : 0;
-    }
-    __syncthreads();
-
-    // rank inside the warp.  Lanes with the same digit are found with one ballot per digit bit
-    // (__match_any_sync does it in one instruction, but MATCH runs on the ADU pipe at a few instructions per
-    // hundred cycles and made this kernel ADU-bound: profiles/r1g).  The group's leader takes the digit's running
-    // count with a shared-memory atomic; a warp issues those in j order, so earlier items get smaller bases and
-    // the sort stays stable without a warp-sync chain.
-#pragma unroll
-    for (int j = 0; j < kRsItems; ++j) {
-        const uint32_t e = warp_base + j * 32 + lane;
-        const bool valid = e < tile_count;
-        const uint32_t d = valid ? dg(key[j]) : 0u;
-        uint32_t same = __ballot_sync(kFullMask, valid);
-#pragma unroll
-        for (int b = 0; b < 8; ++b) {
-            if ((mask >> b) == 0) break;  // uniform: digits narrower than 8 bits need fewer ballots
-            const uint32_t vote = __ballot_sync(kFullMask, (d >> b) & 1u);
-            same &= ((d >> b) & 1u) ? vote : ~vote;
-        }
-        const uint32_t lead = valid ? (uint32_t)__ffs(same) - 1u : lane;
-        uint32_t base = 0;
-        if (valid && lead == lane) base = atomicAdd(&s.warp_cnt[warp][d], (uint32_t)__popc(same));
-        rank[j] = __popc(same & lanemask_lt()) + __shfl_sync(kFullMask, base, lead);
-    }
-    __syncthreads();
-
-    // per digit: exclusive prefix over warps, then over digits
-    uint32_t digit_total = 0;
-    if (threadIdx.x < kRadix) {
-        for (int w = 0; w < kRsWarps; ++w) {
-            uint32_t c = s.warp_cnt[w][threadIdx.x];
-            s.warp_cnt[w][threadIdx.x] = digit_total;
-            digit_total += c;
-        }
-    }
-    {
-        // exclusive scan of digit_total over the first 256 threads (8 warps)
-        uint32_t incl = warp_incl_scan_add(digit_total);
-        if (threadIdx.x < kRadix && lane == 31) s.scan_tmp[warp] = incl;
-        __syncthreads();
-        if (threadIdx.x < 32) {
-            uint32_t w = threadIdx.x < kRadix / 32 ? s.scan_tmp[threadIdx.x] : 0;
-            uint32_t wi = warp_incl_scan_add(w);
-            if (threadIdx.x < kRadix / 32) s.scan_tmp[threadIdx.x] = wi - w;
-        }
-        __syncthreads();
-        if (threadIdx.x < kRadix) {
-            uint32_t local = s.scan_tmp[warp] + incl - digit_total;
-            s.digit_local[threadIdx.x] = local;
-            uint32_t g = threadIdx.x <= mask ? table[(uint64_t)threadIdx.x * n_tiles + blockIdx.x] : 0;
-            s.digit_global[threadIdx.x] = g - local;
-        }
-    }
-    __syncthreads();
-
-    // stage the tile in digit order
-#pragma unroll
-    for (int j = 0; j < kRsItems; ++j) {
-        const uint32_t e = warp_base + j * 32 + lane;
-        if (e < tile_count) {
-            const uint32_t d = dg(key[j]);
-            s.keys[s.digit_local[d] + s.warp_cnt[warp][d] + rank[j]] = key[j];
-        }
-    }
-    __syncthreads();
-
-    // contiguous runs out to global memory
-    for (uint32_t i = threadIdx.x; i < tile_count; i += kRsThreads) {
-        const uint64_t k = s.keys[i];
-        const uint32_t d = dg(k);
-        out[(uint64_t)(s.digit_global[d] + i)] = k;
-    }
-}
-
 
 // ---------------------------------------------------------------------------
 // Single-read passes ("onesweep": Adinets & Merrill 2022).  One kernel up front
@@ -170,11 +48,27 @@ __global__ void __launch_bounds__(kRsThreads) radix_scatter_kernel(const uint64_
 // predecessors' words until it meets one marked (PREFIX | inclusive count)
 // (decoupled look-back); then it publishes its own PREFIX words.  In steady state a
 // walk ends after one or two hops, because predecessors started earlier.
-// Status words are 32 bit: 2 flag bits + a 30-bit count, so this path takes n < 2^30
-// keys; longer arrays use the three-kernel passes above.
 // ---------------------------------------------------------------------------
-constexpr uint32_t kFlagAgg = 1u << 30, kFlagPrefix = 2u << 30, kValueMask = (1u << 30) - 1u;
-constexpr int kMaxPasses = 8;
+
+// Look-back status word: 2 flag bits above a count.  uint32_t holds counts below 2^30, so it serves n < 2^30 keys;
+// longer arrays, where one digit's inclusive count can pass 2^30, take uint64_t (62-bit counts, the split of
+// scan_onepass_kernel's words).  Counts themselves stay below n < 2^32.
+template <typename W>
+struct StatusWord {
+    static constexpr int kShift = 8 * (int)sizeof(W) - 2;
+    static constexpr W kAgg = W(1) << kShift, kPrefix = W(2) << kShift, kValueMask = (W(1) << kShift) - 1;
+    // volatile accesses (other CTAs write these words during the launch), as width-specific inline asm
+    static __device__ __forceinline__ W load(const W *p) {
+        W w;
+        if constexpr (sizeof(W) == 4) asm volatile("ld.volatile.global.u32 %0, [%1];" : "=r"(w) : "l"(p) : "memory");
+        else asm volatile("ld.volatile.global.u64 %0, [%1];" : "=l"(w) : "l"(p) : "memory");
+        return w;
+    }
+    static __device__ __forceinline__ void store(W *p, W w) {
+        if constexpr (sizeof(W) == 4) asm volatile("st.volatile.global.u32 [%0], %1;" ::"l"(p), "r"(w) : "memory");
+        else asm volatile("st.volatile.global.u64 [%0], %1;" ::"l"(p), "l"(w) : "memory");
+    }
+};
 
 struct PassList {
     DigitSpec dg[kMaxPasses];
@@ -227,51 +121,52 @@ __global__ void __launch_bounds__(kRadix) radix_hist_scan_kernel(uint32_t *hist)
     h[threadIdx.x] = ex;
 }
 
-// tile geometry of the sweep kernel: kThreads x kItems keys per CTA, kMinBlocks CTAs per SM.  Measured on the 33 M-key
-// shape (6-pass sort): 512 x 16 keys 1.58 ms, 512 x 8 1.70 ms, 256 x 8 1.82 ms: the per-digit phases (prefix over warps,
-// look-back) are amortised over more keys.  KOMBGPU_SORT_TILE selects a geometry for A/B runs.
-template <int kThreads, int kItems>
-struct SweepSmemT {
-    uint64_t keys[kThreads * kItems];
-    uint32_t warp_cnt[kThreads / 32][kRadix];
+// Tile of the sweep kernel: 512 threads x 16 keys, 2 CTAs per SM.  The per-digit phases (prefix over warps, look-back)
+// are amortised over more keys than in the smaller tiles measured against it (DESIGN.md §4 "Sort").
+constexpr int kSweepThreads = 512, kSweepItems = 16, kSweepTile = kSweepThreads * kSweepItems, kSweepMinBlocks = 2;
+
+struct SweepSmem {
+    uint64_t keys[kSweepTile];
+    uint32_t warp_cnt[kSweepThreads / 32][kRadix];
     uint32_t digit_local[kRadix];   // first slot of digit d inside the staged tile
     uint32_t digit_global[kRadix];  // global position of that slot minus digit_local
     uint32_t digit_total[kRadix];
     uint32_t tile;
 };
 
-// kBits: digit width known at compile time (8), or 0 = read it from `mask`.
-template <int kBits, int kThreads, int kItems, int kMinBlocks>
-__global__ void __launch_bounds__(kThreads, kMinBlocks) radix_sweep_kernel(const uint64_t *__restrict__ in, uint64_t *__restrict__ out,
+// W: status word (StatusWord).  kBits: digit width known at compile time (8), or 0 = read it from `mask`.
+template <typename W, int kBits>
+__global__ void __launch_bounds__(kSweepThreads, kSweepMinBlocks) radix_sweep_kernel(const uint64_t *__restrict__ in, uint64_t *__restrict__ out,
                                                                     uint64_t n, DigitSpec dg,
                                                                     const uint32_t *__restrict__ digit_base,  // exclusive global histogram of this pass
-                                                                    uint32_t *status, uint32_t *tile_counter) {
-    constexpr int kTile = kThreads * kItems, kWarps = kThreads / 32;
+                                                                    W *status, uint32_t *tile_counter) {
+    using SW = StatusWord<W>;
+    constexpr int kWarps = kSweepThreads / 32;
     extern __shared__ __align__(16) unsigned char s_raw[];
-    SweepSmemT<kThreads, kItems> &s = *reinterpret_cast<SweepSmemT<kThreads, kItems> *>(s_raw);
+    SweepSmem &s = *reinterpret_cast<SweepSmem *>(s_raw);
     const uint32_t warp = threadIdx.x >> 5, lane = lane_id();
     const uint32_t mask = kBits ? (1u << kBits) - 1u : dg.mask;
     if (threadIdx.x == 0) s.tile = atomicAdd(tile_counter, 1u);
-    for (int i = threadIdx.x; i < kWarps * kRadix; i += kThreads) (&s.warp_cnt[0][0])[i] = 0;
+    for (int i = threadIdx.x; i < kWarps * kRadix; i += kSweepThreads) (&s.warp_cnt[0][0])[i] = 0;
     __syncthreads();
     const uint32_t tile = s.tile;
-    const uint64_t tile_base = (uint64_t)tile * kTile;
-    const uint32_t tile_count = (uint32_t)min((uint64_t)kTile, n - tile_base);
+    const uint64_t tile_base = (uint64_t)tile * kSweepTile;
+    const uint32_t tile_count = (uint32_t)min((uint64_t)kSweepTile, n - tile_base);
 
-    // warp-striped load: item j of lane l is tile element warp*32*kItems + j*32 + l, so (warp, j, lane) order is memory
-    // order and the sort stays stable
-    uint64_t key[kItems];
-    uint16_t rank[kItems];
-    const uint32_t warp_base = warp * (32 * kItems);
+    // warp-striped load: item j of lane l is tile element warp*32*kSweepItems + j*32 + l, so (warp, j, lane) order is
+    // memory order and the sort stays stable
+    uint64_t key[kSweepItems];
+    uint16_t rank[kSweepItems];
+    const uint32_t warp_base = warp * (32 * kSweepItems);
 #pragma unroll
-    for (int j = 0; j < kItems; ++j) {
+    for (int j = 0; j < kSweepItems; ++j) {
         const uint32_t e = warp_base + j * 32 + lane;
         key[j] = e < tile_count ? in[tile_base + e] : 0;
     }
     // rank inside the warp: lanes with the same digit are found with one ballot per digit bit; the group's leader takes
     // the digit's running count with a shared-memory atomic (issued in j order: stable)
 #pragma unroll
-    for (int j = 0; j < kItems; ++j) {
+    for (int j = 0; j < kSweepItems; ++j) {
         const uint32_t e = warp_base + j * 32 + lane;
         const bool valid = e < tile_count;
         const uint32_t d = valid ? dg(key[j]) : 0u;
@@ -291,7 +186,7 @@ __global__ void __launch_bounds__(kThreads, kMinBlocks) radix_sweep_kernel(const
     __syncthreads();
 
     // per digit: exclusive prefix over warps; publish the tile's count (the look-back starts from it)
-    for (uint32_t d = threadIdx.x; d < (uint32_t)kRadix; d += kThreads) {
+    for (uint32_t d = threadIdx.x; d < (uint32_t)kRadix; d += kSweepThreads) {
         uint32_t total = 0;
 #pragma unroll
         for (int w = 0; w < kWarps; ++w) {
@@ -300,10 +195,7 @@ __global__ void __launch_bounds__(kThreads, kMinBlocks) radix_sweep_kernel(const
             total += c;
         }
         s.digit_total[d] = total;
-        if (d <= mask) {
-            uint32_t *mine = status + (size_t)tile * kRadix + d;
-            asm volatile("st.volatile.global.u32 [%0], %1;" ::"l"(mine), "r"((tile == 0 ? kFlagPrefix : kFlagAgg) | total) : "memory");
-        }
+        if (d <= mask) SW::store(status + (size_t)tile * kRadix + d, (tile == 0 ? SW::kPrefix : SW::kAgg) | (W)total);
     }
     __syncthreads();
     if (warp == 0) {   // exclusive scan of the 256 digit totals: 8 per lane
@@ -318,58 +210,50 @@ __global__ void __launch_bounds__(kThreads, kMinBlocks) radix_sweep_kernel(const
 
     // stage the tile in digit order (the look-back follows, overlapping other CTAs' work)
 #pragma unroll
-    for (int j = 0; j < kItems; ++j) {
+    for (int j = 0; j < kSweepItems; ++j) {
         const uint32_t e = warp_base + j * 32 + lane;
         if (e < tile_count) {
             const uint32_t d = dg(key[j]);
             s.keys[s.digit_local[d] + s.warp_cnt[warp][d] + rank[j]] = key[j];
         }
     }
-    for (uint32_t d = threadIdx.x; d <= mask; d += kThreads) {
+    for (uint32_t d = threadIdx.x; d <= mask; d += kSweepThreads) {
         uint32_t excl = 0;
         if (tile > 0) {
             uint32_t p = tile - 1;
             uint32_t spins = 0;
             while (true) {
-                uint32_t w;
-                asm volatile("ld.volatile.global.u32 %0, [%1];" : "=r"(w) : "l"(status + (size_t)p * kRadix + d) : "memory");
-                if ((w >> 30) == 0) {             // predecessor has not ranked its keys yet
+                const W w = SW::load(status + (size_t)p * kRadix + d);
+                if ((w >> SW::kShift) == 0) {     // predecessor has not ranked its keys yet
                     if (++spins > (1u << 28)) __trap();
                     continue;
                 }
-                excl += w & kValueMask;
-                if (w & kFlagPrefix) break;        // tile 0 always publishes PREFIX: p never underflows
+                excl += (uint32_t)(w & SW::kValueMask);
+                if (w & SW::kPrefix) break;        // tile 0 always publishes PREFIX: p never underflows
                 --p;
             }
-            uint32_t *mine = status + (size_t)tile * kRadix + d;
-            asm volatile("st.volatile.global.u32 [%0], %1;" ::"l"(mine), "r"(kFlagPrefix | (excl + s.digit_total[d])) : "memory");
+            SW::store(status + (size_t)tile * kRadix + d, SW::kPrefix | (W)(excl + s.digit_total[d]));
         }
         s.digit_global[d] = digit_base[d] + excl - s.digit_local[d];
     }
     __syncthreads();
 
     // contiguous runs out to global memory
-    for (uint32_t i = threadIdx.x; i < tile_count; i += kThreads) {
+    for (uint32_t i = threadIdx.x; i < tile_count; i += kSweepThreads) {
         const uint64_t k = s.keys[i];
         const uint32_t d = dg(k);
         out[(uint64_t)(s.digit_global[d] + i)] = k;
     }
 }
 
-struct SweepGeom {
-    int threads, items;
-    size_t smem;
-    void (*k8)(const uint64_t *, uint64_t *, uint64_t, DigitSpec, const uint32_t *, uint32_t *, uint32_t *);
-    void (*k0)(const uint64_t *, uint64_t *, uint64_t, DigitSpec, const uint32_t *, uint32_t *, uint32_t *);
-};
-template <int kThreads, int kItems, int kMinBlocks>
-constexpr SweepGeom make_geom() {
-    return SweepGeom{kThreads, kItems, sizeof(SweepSmemT<kThreads, kItems>), radix_sweep_kernel<8, kThreads, kItems, kMinBlocks>,
-                     radix_sweep_kernel<0, kThreads, kItems, kMinBlocks>};
+template <typename W>
+int sweep_pass(kombgpu_ctx *ctx, const uint64_t *src, uint64_t *dst, uint64_t n, const RadixPass &pass, const DigitSpec &dg,
+               const uint32_t *digit_base, W *status, uint32_t *tile_counter) {
+    auto *kernel = pass.bits + pass.bits2 == 8 ? radix_sweep_kernel<W, 8> : radix_sweep_kernel<W, 0>;
+    KG_LAUNCH(ctx, kernel, ceil_div_u64(n, kSweepTile), kSweepThreads, sizeof(SweepSmem), src, dst, n, dg, digit_base, status,
+              tile_counter);
+    return KOMBGPU_OK;
 }
-const SweepGeom kGeoms[] = {make_geom<512, 16, 2>(), make_geom<256, 16, 4>(), make_geom<256, 16, 3>(), make_geom<128, 16, 8>(),
-                            make_geom<256, 8, 6>(), make_geom<384, 16, 2>()};
-constexpr int kNumGeoms = sizeof(kGeoms) / sizeof(kGeoms[0]);
 
 }  // namespace
 
@@ -396,56 +280,42 @@ int radix_sort_u64(kombgpu_ctx *ctx, uint64_t *a, uint64_t *b, uint64_t n, const
     *sorted = a;
     if (n < 2 || n_passes == 0) return KOMBGPU_OK;
     if (n >= (1ull << 32)) return ctx_fail(ctx, KOMBGPU_EINVAL, "radix_sort_u64: %llu keys exceed the 2^32 per-array limit", (unsigned long long)n);
-    const char *sort_env = getenv("KOMBGPU_SORT");   // "legacy": the three-kernel passes (kept for A/B measurements)
-    const bool legacy = n >= (1ull << 30) || n_passes > kMaxPasses || (sort_env && sort_env[0] == 'l');
+    if (n_passes > kMaxPasses) return ctx_fail(ctx, KOMBGPU_EINVAL, "radix_sort_u64: %d passes exceed %d", n_passes, kMaxPasses);
     if (!ctx->sort_attr_set) {   // function attributes are per device: once per context, not per process
-        KG_CUDA(ctx, cudaFuncSetAttribute(radix_scatter_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)sizeof(ScatterSmem)));
-        for (int g = 0; g < kNumGeoms; ++g) {
-            KG_CUDA(ctx, cudaFuncSetAttribute(kGeoms[g].k8, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)kGeoms[g].smem));
-            KG_CUDA(ctx, cudaFuncSetAttribute(kGeoms[g].k0, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)kGeoms[g].smem));
-        }
+        KG_CUDA(ctx, cudaFuncSetAttribute(radix_sweep_kernel<uint32_t, 8>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)sizeof(SweepSmem)));
+        KG_CUDA(ctx, cudaFuncSetAttribute(radix_sweep_kernel<uint32_t, 0>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)sizeof(SweepSmem)));
+        KG_CUDA(ctx, cudaFuncSetAttribute(radix_sweep_kernel<uint64_t, 8>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)sizeof(SweepSmem)));
+        KG_CUDA(ctx, cudaFuncSetAttribute(radix_sweep_kernel<uint64_t, 0>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)sizeof(SweepSmem)));
         ctx->sort_attr_set = true;
     }
-    const uint32_t n_tiles = ceil_div_u64(n, kRsTile);
+    // Workspace, in 32-bit words: [n_passes x 256 digit histograms | kMaxPasses tile counters | status words].  Below 2^30
+    // keys every pass has its own region of 32-bit words, all zeroed at once.  From 2^30 on the passes share one region
+    // of 64-bit words (n/4 bytes), zeroed again before each pass: one region per pass would cost up to 8 GiB.  The head
+    // has an even number of words, so the 64-bit words stay aligned.
+    const bool wide = n >= (1ull << 30);
+    const size_t region = (size_t)ceil_div_u64(n, kSweepTile) * kRadix;   // status words of one pass
+    const size_t head = (size_t)n_passes * kRadix + kMaxPasses;
+    const size_t words = head + (wide ? 2 * region : (size_t)n_passes * region);
+    DevBuf<uint32_t> ws;
+    KG_ALLOC(ctx, ws, words);
+    KG_CUDA(ctx, cudaMemsetAsync(ws.p, 0, words * sizeof(uint32_t), ctx->stream));
+    PassList pl{};
+    pl.n = n_passes;
+    for (int p = 0; p < n_passes; ++p) pl.dg[p] = DigitSpec::of(passes[p]);
     uint64_t *src = a, *dst = b;
-    if (!legacy) {
-        const char *tile_env = getenv("KOMBGPU_SORT_TILE");   // index into kGeoms (A/B runs)
-        int gi = tile_env ? atoi(tile_env) : 0;
-        if (gi < 0 || gi >= kNumGeoms) gi = 0;
-        const SweepGeom &geom = kGeoms[gi];
-        const uint32_t sw_tile = (uint32_t)(geom.threads * geom.items);
-        const uint32_t n_tiles = ceil_div_u64(n, sw_tile);
-        // [n_passes x 256 digit histograms | n_passes tile counters | n_passes x n_tiles x 256 status words]
-        const size_t head = (size_t)n_passes * kRadix + kMaxPasses;
-        DevBuf<uint32_t> ws;
-        KG_ALLOC(ctx, ws, head + (size_t)n_passes * n_tiles * kRadix);
-        KG_CUDA(ctx, cudaMemsetAsync(ws.p, 0, (head + (size_t)n_passes * n_tiles * kRadix) * sizeof(uint32_t), ctx->stream));
-        PassList pl{};
-        pl.n = n_passes;
-        for (int p = 0; p < n_passes; ++p) pl.dg[p] = DigitSpec::of(passes[p]);
-        const uint32_t hist_grid = min(ceil_div_u64(n, kRsTile), (uint32_t)ctx->sm_count * 4u);
-        KG_LAUNCH(ctx, radix_global_hist_kernel, hist_grid, kRsThreads, 0, src, n, pl, ws.p);
-        KG_LAUNCH(ctx, radix_hist_scan_kernel, n_passes, kRadix, 0, ws.p);
-        for (int p = 0; p < n_passes; ++p) {
-            const uint32_t *dbase = ws.p + (size_t)p * kRadix;
-            const bool w8 = passes[p].bits + passes[p].bits2 == 8;
-            uint32_t *status = ws.p + head + (size_t)p * n_tiles * kRadix, *counter = ws.p + (size_t)n_passes * kRadix + p;
-            (w8 ? geom.k8 : geom.k0)<<<n_tiles, geom.threads, geom.smem, ctx->stream>>>(src, dst, n, pl.dg[p], dbase, status, counter);
-            ctx->launches++;
-            KG_CUDA(ctx, cudaPeekAtLastError());
-            uint64_t *t = src; src = dst; dst = t;
-        }
-        *sorted = src;
-        return KOMBGPU_OK;
-    }
-    DevBuf<uint32_t> table;
-    KG_ALLOC(ctx, table, (size_t)kRadix * n_tiles);
+    const uint32_t hist_grid = min(ceil_div_u64(n, kRsTile), (uint32_t)ctx->sm_count * 4u);
+    KG_LAUNCH(ctx, radix_global_hist_kernel, hist_grid, kRsThreads, 0, src, n, pl, ws.p);
+    KG_LAUNCH(ctx, radix_hist_scan_kernel, n_passes, kRadix, 0, ws.p);
     for (int p = 0; p < n_passes; ++p) {
-        const DigitSpec dg = DigitSpec::of(passes[p]);
-        const uint64_t table_len = (uint64_t)(dg.mask + 1) * n_tiles;
-        KG_LAUNCH(ctx, radix_hist_kernel, n_tiles, kRsThreads, 0, src, n, dg, table.p, n_tiles);
-        KG_TRY((device_scan<uint32_t>(ctx, table_len, TableIn{table.p}, TableOut{table.p}, (uint32_t *)nullptr)));
-        KG_LAUNCH(ctx, radix_scatter_kernel, n_tiles, kRsThreads, sizeof(ScatterSmem), src, dst, n, dg, table.p, n_tiles);
+        const uint32_t *digit_base = ws.p + (size_t)p * kRadix;
+        uint32_t *counter = ws.p + (size_t)n_passes * kRadix + p;
+        if (wide) {
+            uint64_t *status = reinterpret_cast<uint64_t *>(ws.p + head);
+            if (p > 0) KG_CUDA(ctx, cudaMemsetAsync(status, 0, region * sizeof(uint64_t), ctx->stream));
+            KG_TRY(sweep_pass(ctx, src, dst, n, passes[p], pl.dg[p], digit_base, status, counter));
+        } else {
+            KG_TRY(sweep_pass(ctx, src, dst, n, passes[p], pl.dg[p], digit_base, ws.p + head + (size_t)p * region, counter));
+        }
         uint64_t *t = src; src = dst; dst = t;
     }
     *sorted = src;

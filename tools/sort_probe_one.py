@@ -1,8 +1,7 @@
-"""One sort of the 33M-pair shape (for ncu): sort_probe_one.py [sweep|legacy]"""
-import os, sys, ctypes
+"""One sort of the 33M-pair shape (for ncu): sort_probe_one.py"""
+import sys, ctypes
 from pathlib import Path
 sys.path.insert(0, str(Path(__file__).resolve().parents[1]))
-os.environ["KOMBGPU_SORT"] = sys.argv[1] if len(sys.argv) > 1 else "sweep"
 import komb_b200
 from komb_b200 import _lib
 lib = _lib.load(); ctx = komb_b200.Context(0)
