@@ -531,6 +531,25 @@ int kombgpu_dist_graph_device_arrays(const kombgpu_dist_graph *g, const uint64_t
 /* Global scalars of CombineCoreA::run: max coreness and max CORE-A score (every rank gets the same values). */
 int kombgpu_dist_graph_summary(const kombgpu_dist_graph *g, int32_t *max_coreness, double *max_score);
 
+/* The maximal core of the WHOLE partitioned graph and the trussness of its edges: what kombgpu_graph_max_core_truss
+ * computes on one GPU, with the same results bit for bit, on every rank.  Collective; needs kombgpu_dist_coreness
+ * (KOMBGPU_ESTATE otherwise, on every rank, before any rank waits for another).  Every rank pulls the coreness of
+ * the unitigs the other ranks own and their slices of the maximal core's edges, then computes the trussness of the
+ * whole maximal core itself: the maximal core has to fit one GPU and hold fewer than 2^32 edges (KOMBGPU_EINVAL on
+ * every rank otherwise); the whole graph need not.  When a rank fails, every rank returns an error.  Computed once
+ * per graph, cached; the results are held by every rank. */
+int kombgpu_dist_max_core_truss(kombgpu_dist_graph *g, uint32_t *n_core_vertices, uint64_t *n_core_edges,
+                                int32_t *max_trussness, uint32_t *n_truss_vertices);
+/* Local, not collective: the whole result on any rank, as kombgpu_graph_max_core_edges (original unitig ids, u < v,
+ * ascending, n_core_edges entries each) and kombgpu_graph_truss_vertices (ascending, n_truss_vertices entries). */
+int kombgpu_dist_max_core_edges(const kombgpu_dist_graph *g, uint32_t *u, uint32_t *v, int32_t *trussness);
+int kombgpu_dist_truss_vertices(const kombgpu_dist_graph *g, uint32_t *vids);
+/* The densest k-core of the WHOLE partitioned graph, as kombgpu_graph_densest_core (same level, sizes and density,
+ * same tie rule: equal density goes to the larger block) on every rank.  Collective; needs kombgpu_dist_coreness.
+ * The ranks sum their histograms of unitigs per coreness and of edges per min(core(u), core(v)). */
+int kombgpu_dist_densest_core(kombgpu_dist_graph *g, int32_t *k_star, uint32_t *n_vertices, uint64_t *n_edges,
+                              double *density);
+
 int kombgpu_abi_version(void);
 
 #ifdef __cplusplus

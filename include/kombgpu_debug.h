@@ -32,6 +32,11 @@ int kombgpu_debug_build_chunks(const kombgpu_graph *g, uint32_t *n_chunks);
  * 2^32 or, with KOMBGPU_PAIR_CHUNK=<pairs> set, when some rank's pairs exceed that many (the pairs per rank and round). */
 int kombgpu_debug_dist_build_rounds(const kombgpu_dist_graph *g, uint32_t *n_rounds);
 
+/* tools/dist_truss_probe.py: the CUDA-event split of this rank's last kombgpu_dist_max_core_truss -- the gather of the
+ * coreness, the selection of the maximal core with the gather of the edge slices, and the truss peel. */
+int kombgpu_debug_dist_truss_timing(const kombgpu_dist_graph *g, float *ms_core_gather, float *ms_slice_gather,
+                                    float *ms_truss);
+
 #ifdef __cplusplus
 }
 #endif

@@ -81,6 +81,7 @@ SIGNATURES = {
     "kombgpu_debug_peel_again": (c_int, [c_void_p]),
     "kombgpu_debug_build_chunks": (c_int, [c_void_p, POINTER(c_uint32)]),
     "kombgpu_debug_dist_build_rounds": (c_int, [c_void_p, POINTER(c_uint32)]),
+    "kombgpu_debug_dist_truss_timing": (c_int, [c_void_p, POINTER(c_float), POINTER(c_float), POINTER(c_float)]),
     "kombgpu_degree": (c_int, [c_void_p, c_void_p]),
     "kombgpu_coreness": (c_int, [c_void_p, c_void_p]),
     "kombgpu_corea": (c_int, [c_void_p, c_void_p, c_void_p, c_uint32, c_int, c_void_p]),
@@ -160,6 +161,10 @@ SIGNATURES = {
     "kombgpu_dist_graph_edges_csr": (c_int, [c_void_p, c_void_p, c_void_p]),
     "kombgpu_dist_graph_device_arrays": (c_int, [c_void_p] + [POINTER(c_void_p)] * 6),
     "kombgpu_dist_graph_summary": (c_int, [c_void_p, POINTER(c_int32), POINTER(c_double)]),
+    "kombgpu_dist_max_core_truss": (c_int, [c_void_p, POINTER(c_uint32), POINTER(c_uint64), POINTER(c_int32), POINTER(c_uint32)]),
+    "kombgpu_dist_max_core_edges": (c_int, [c_void_p, c_void_p, c_void_p, c_void_p]),
+    "kombgpu_dist_truss_vertices": (c_int, [c_void_p, c_void_p]),
+    "kombgpu_dist_densest_core": (c_int, [c_void_p, POINTER(c_int32), POINTER(c_uint32), POINTER(c_uint64), POINTER(c_double)]),
 }
 
 _lib = None

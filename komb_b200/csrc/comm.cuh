@@ -98,6 +98,27 @@ int comm_group_barrier(kombgpu_comm *c);
 // sum / max of one value over the ranks, via comm_exchange
 int comm_allreduce_sum(kombgpu_comm *c, unsigned long long v, unsigned long long *out);
 
+struct SymRewind {   // gives the symmetric heap back to a mark when the scope ends, on every return path
+    kombgpu_comm *c;
+    SymMark mark;
+    ~SymRewind() { sym_release(c, mark); }
+};
+
+struct EvTimer {   // CUDA-event split timer on the context's stream
+    kombgpu_ctx *ctx;
+    cudaEvent_t a = nullptr, b = nullptr;
+    explicit EvTimer(kombgpu_ctx *c) : ctx(c) { cudaEventCreate(&a); cudaEventCreate(&b); cudaEventRecord(a, ctx->stream); }
+    float lap() {
+        float ms = 0.f;
+        cudaEventRecord(b, ctx->stream);
+        cudaEventSynchronize(b);
+        cudaEventElapsedTime(&ms, a, b);
+        cudaEventRecord(a, ctx->stream);
+        return ms;
+    }
+    ~EvTimer() { cudaEventDestroy(a); cudaEventDestroy(b); }
+};
+
 template <typename T>
 int sym_alloc(kombgpu_comm *c, size_t count, T **local, PeerPtrs<T> *peers) {
     void *l = nullptr;

@@ -123,6 +123,32 @@ __global__ void __launch_bounds__(kThreads) block_member_kernel(const uint32_t *
 }
 
 }  // namespace
+
+int level_histogram(kombgpu_ctx *ctx, const int32_t *core, const uint64_t *edges, uint64_t count, uint32_t n_bins,
+                    unsigned long long *hist) {
+    if (count == 0) return KOMBGPU_OK;
+    const uint32_t grid = min(ceil_div_u64(count, kThreads), (uint32_t)ctx->sm_count * 8u);
+    if (edges) KG_LAUNCH(ctx, level_hist_kernel<true>, grid, kThreads, 0, core, edges, count, n_bins, hist);
+    else KG_LAUNCH(ctx, level_hist_kernel<false>, grid, kThreads, 0, core, (const uint64_t *)nullptr, count, n_bins, hist);
+    return KOMBGPU_OK;
+}
+
+DensestCore densest_level(const unsigned long long *hv, const unsigned long long *he, uint32_t n_bins, uint64_t n, uint64_t n_edges) {
+    DensestCore best{0, n, n_edges, n ? (double)n_edges / (double)n : 0.0};
+    if (!n || !n_edges) return best;
+    uint64_t v = 0, e = 0;
+    best.density = -1.0;
+    for (int64_t k = (int64_t)n_bins - 1; k >= 0; --k) {   // suffix sums over the levels, densest first
+        v += hv[k];
+        e += he[k];
+        if (v == 0) continue;
+        const double d = (double)e / (double)v;
+        // equal density: the larger block wins; an empty level leaves the block (and the reported k) as it is
+        if (d > best.density || (d == best.density && v > best.n_vertices)) best = DensestCore{(int32_t)k, v, e, d};
+    }
+    return best;
+}
+
 }  // namespace kg
 
 extern "C" int kombgpu_graph_densest_core(kombgpu_graph *g, int32_t *k_star, uint32_t *n_vertices, uint64_t *n_edges,
@@ -133,36 +159,21 @@ extern "C" int kombgpu_graph_densest_core(kombgpu_graph *g, int32_t *k_star, uin
     if (!g->has_core) return ctx_fail(ctx, KOMBGPU_ESTATE, "kombgpu_graph_densest_core needs kombgpu_coreness first");
     if (g->n_edges && !g->edges) return ctx_fail(ctx, KOMBGPU_ESTATE, "graph was adopted from a CSR: no canonical edge list");
     KG_CUDA(ctx, cudaSetDevice(ctx->device));
-    int32_t best_k = 0;
-    uint64_t best_v = g->n, best_e = g->n_edges;
-    double best_d = g->n ? (double)g->n_edges / (double)g->n : 0.0;
-    if (g->n && g->n_edges) {
-        const uint32_t n_bins = (uint32_t)g->st.max_coreness + 1;
+    const uint32_t n_bins = g->n && g->n_edges ? (uint32_t)g->st.max_coreness + 1 : 0u;
+    std::vector<unsigned long long> h(2 * (size_t)n_bins);
+    if (n_bins) {
         DevBuf<unsigned long long> hist;
         KG_ALLOC(ctx, hist, 2 * (size_t)n_bins);
         KG_CUDA(ctx, cudaMemsetAsync(hist.p, 0, 2 * (size_t)n_bins * sizeof(unsigned long long), ctx->stream));
-        const uint32_t cap = (uint32_t)ctx->sm_count * 8u;
-        KG_LAUNCH(ctx, level_hist_kernel<false>, min(ceil_div_u64(g->n, kThreads), cap), kThreads, 0, g->core, (const uint64_t *)nullptr,
-                  (uint64_t)g->n, n_bins, hist.p);
-        KG_LAUNCH(ctx, level_hist_kernel<true>, min(ceil_div_u64(g->n_edges, kThreads), cap), kThreads, 0, g->core, g->edges, g->n_edges,
-                  n_bins, hist.p + n_bins);
-        std::vector<unsigned long long> h(2 * (size_t)n_bins);
+        KG_TRY(level_histogram(ctx, g->core, nullptr, g->n, n_bins, hist.p));
+        KG_TRY(level_histogram(ctx, g->core, g->edges, g->n_edges, n_bins, hist.p + n_bins));
         KG_TRY(read_back(ctx, hist.p, h.data(), h.size()));
-        uint64_t v = 0, e = 0;
-        best_d = -1.0;
-        for (int64_t k = (int64_t)n_bins - 1; k >= 0; --k) {   // suffix sums over the levels, densest first
-            v += h[k];
-            e += h[n_bins + k];
-            if (v == 0) continue;
-            const double d = (double)e / (double)v;
-            // equal density: the larger block wins; an empty level leaves the block (and the reported k) as it is
-            if (d > best_d || (d == best_d && v > best_v)) { best_d = d; best_k = (int32_t)k; best_v = v; best_e = e; }
-        }
     }
-    if (k_star) *k_star = best_k;
-    if (n_vertices) *n_vertices = (uint32_t)best_v;
-    if (n_edges) *n_edges = best_e;
-    if (density) *density = best_d;
+    const DensestCore best = densest_level(h.data(), h.data() + n_bins, n_bins, g->n, g->n_edges);
+    if (k_star) *k_star = best.k;
+    if (n_vertices) *n_vertices = (uint32_t)best.n_vertices;
+    if (n_edges) *n_edges = best.n_edges;
+    if (density) *density = best.density;
     return KOMBGPU_OK;
 }
 

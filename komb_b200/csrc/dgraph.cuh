@@ -34,6 +34,10 @@ struct kombgpu_dist_graph {
     double *score = nullptr;       // [n_local] after CORE-A
     bool has_core = false, has_score = false;
     double max_score = 0.0;        // global
+    // the maximal core of the WHOLE graph and the trussness of its edges, the same on every rank (pcore.cu)
+    bool has_truss = false;
+    kg::MaxCoreTruss tr;
+    float ms_truss[3] = {0.f, 0.f, 0.f};   // CUDA-event times: coreness gather, selection + slice gather, truss peel
     kombgpu_dist_stats st{};
 };
 
@@ -61,6 +65,9 @@ int dist_peel_replicated(kombgpu_dist_graph *g);
 int dist_peel_mode();
 // pcorea.cu
 int dist_corea(kombgpu_dist_graph *g, int key_mode);
+// pcore.cu: the consumers of the finished coreness
+int dist_max_core_truss(kombgpu_dist_graph *g);
+int dist_densest_core(kombgpu_dist_graph *g, DensestCore *out);
 
 void dist_graph_release(kombgpu_dist_graph *g);
 

@@ -4,6 +4,19 @@
 
 #include "common.cuh"
 
+namespace kg {
+// the maximal core and the trussness of its edges (truss.cu), computed on demand
+struct MaxCoreTruss {
+    uint32_t n_core = 0, n_vertices = 0;
+    uint64_t m = 0;
+    int32_t tmax = 0;
+    uint32_t *core_vid = nullptr;   // [n_core] original ids of the maximal core, ascending
+    uint64_t *edges = nullptr;      // [m] induced edges, compact ids (a << 32 | b), canonical order
+    int32_t *truss = nullptr;       // [m]
+    uint32_t *vertices = nullptr;   // [n_vertices] original ids of the unitigs on edges of maximal trussness
+};
+}  // namespace kg
+
 struct kombgpu_graph {
     kombgpu_ctx *ctx = nullptr;
     uint32_t n = 0;            // vertices (hit unitigs)
@@ -20,15 +33,8 @@ struct kombgpu_graph {
     double max_score = 0.0;
     bool has_core = false, has_score = false;
     kombgpu_stats st{};
-    // maximal core + trussness of its edges (truss.cu), computed on demand
     bool has_truss = false;
-    uint32_t tr_n_core = 0, tr_n_vertices = 0;
-    uint64_t tr_m = 0;
-    int32_t tr_max = 0;
-    uint32_t *tr_core_vid = nullptr;   // [tr_n_core] original ids of the maximal core, ascending
-    uint64_t *tr_edges = nullptr;      // [tr_m] induced edges, compact ids (a << 32 | b), canonical order
-    int32_t *tr_truss = nullptr;       // [tr_m]
-    uint32_t *tr_vertices = nullptr;   // [tr_n_vertices] original ids of the unitigs on edges of maximal trussness
+    kg::MaxCoreTruss tr;
     // output files formatted on the device (format.cu): edgelist.txt, kcore.tsv, CoreA_anomaly.txt
     char *text[3] = {nullptr, nullptr, nullptr};
     uint64_t text_bytes[3] = {0, 0, 0};
@@ -110,6 +116,35 @@ int peel_coreness(kombgpu_graph *g);
 // stage 3 (corea.cu) — device pointers in, device score out; *max_score on host
 int corea_scores(kombgpu_ctx *ctx, const int32_t *core, const int32_t *deg, uint32_t n, int key_mode, double *score,
                  double *max_score_host);
+
+// the maximal core and its truss (truss.cu), in three steps the partitioned graph (pcore.cu) runs apart:
+// 1. sub_id[v] = compact id of v (~0 outside), core_vid = the original ids, for the n ids whose coreness is kmax
+int max_core_vertices(kombgpu_ctx *ctx, const int32_t *core, uint32_t n, int32_t kmax, DevBuf<uint32_t> &sub_id,
+                      DevBuf<uint32_t> &core_vid, uint32_t *n_core);
+// 2. the edges of a canonical list (or of a slice of it) with both ends in the core, relabelled; the relabelling is
+//    monotone, so the result stays canonical and sorted
+int max_core_edges(kombgpu_ctx *ctx, const uint64_t *edges, uint64_t count, const uint32_t *sub_id, DevBuf<uint64_t> &out,
+                   uint64_t *m);
+// 3. the trussness of every edge of the canonical sub-edge list (m < 2^32) and the unitigs on the edges of maximal
+//    trussness; on success sub_edges and core_vid move into *tr
+int sub_edges_truss(kombgpu_ctx *ctx, DevBuf<uint64_t> &sub_edges, uint64_t m, DevBuf<uint32_t> &core_vid, uint32_t n_core,
+                    MaxCoreTruss *tr);
+// the cached result to the host (u, v: original ids; any pointer may be NULL)
+int truss_edges_to_host(kombgpu_ctx *ctx, const MaxCoreTruss &tr, uint32_t *u, uint32_t *v, int32_t *trussness);
+int truss_vertices_to_host(kombgpu_ctx *ctx, const MaxCoreTruss &tr, uint32_t *vids);
+void truss_free(kombgpu_ctx *ctx, MaxCoreTruss *tr);
+
+// densest k-core (densest.cu): hist[core[v]] += 1 over `count` vertices (edges == NULL), or hist[min(core[u], core[v])]
+// += 1 over `count` edges of a canonical list; the k-core of the summed histograms with the largest density
+int level_histogram(kombgpu_ctx *ctx, const int32_t *core, const uint64_t *edges, uint64_t count, uint32_t n_bins,
+                    unsigned long long *hist);
+struct DensestCore {
+    int32_t k;
+    uint64_t n_vertices, n_edges;
+    double density;
+};
+// hv / he: histograms of n_bins levels over the n vertices and n_edges edges (unread when either count is 0)
+DensestCore densest_level(const unsigned long long *hv, const unsigned long long *he, uint32_t n_bins, uint64_t n, uint64_t n_edges);
 
 void graph_release(kombgpu_graph *g);
 void truss_release(kombgpu_graph *g);   // truss.cu

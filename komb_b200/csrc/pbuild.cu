@@ -182,27 +182,6 @@ __global__ void __launch_bounds__(kThreads) low_words_kernel(const uint64_t *__r
     for (uint64_t i = (uint64_t)blockIdx.x * blockDim.x + threadIdx.x; i < n; i += (uint64_t)gridDim.x * blockDim.x) out[i] = (uint32_t)keys[i];
 }
 
-struct SymRewind {   // gives the symmetric heap back to a mark when the scope ends, on every return path
-    kombgpu_comm *c;
-    SymMark mark;
-    ~SymRewind() { sym_release(c, mark); }
-};
-
-struct EvTimer {   // CUDA-event split timer on the context's stream
-    kombgpu_ctx *ctx;
-    cudaEvent_t a = nullptr, b = nullptr;
-    explicit EvTimer(kombgpu_ctx *c) : ctx(c) { cudaEventCreate(&a); cudaEventCreate(&b); cudaEventRecord(a, ctx->stream); }
-    float lap() {
-        float ms = 0.f;
-        cudaEventRecord(b, ctx->stream);
-        cudaEventSynchronize(b);
-        cudaEventElapsedTime(&ms, a, b);
-        cudaEventRecord(a, ctx->stream);
-        return ms;
-    }
-    ~EvTimer() { cudaEventDestroy(a); cudaEventDestroy(b); }
-};
-
 }  // namespace
 
 // KOMBGPU_DIST_PEEL = async | log | auto (default).  The asynchronous peel (apeel.cu) decrements a neighbour where it
@@ -506,6 +485,8 @@ void dist_graph_release(kombgpu_dist_graph *g) {
         if (p) ws_free(ctx, p);
     g->edges = nullptr; g->mult = nullptr; g->fwd_start = nullptr; g->nbr_ptr = nullptr; g->nbr = nullptr; g->row_ptr32 = nullptr; g->col = nullptr;
     g->deg = nullptr; g->core = nullptr; g->score = nullptr;
+    truss_free(ctx, &g->tr);
+    g->has_truss = false;
 }
 
 }  // namespace kg

@@ -1,0 +1,238 @@
+// pcore.cu — the consumers of the finished coreness on the partitioned graph: the maximal core with the trussness of
+// its edges (the reference's Kgraph::runTruss, truss.cu) and the densest k-core (densest.cu).
+//
+// Both need the coreness of unitigs other ranks own (the far end of an edge).  Every rank puts its coreness slice into
+// the symmetric heap and pulls the others' with plain device-to-device copies, as rpeel.cu pulls rows: 4 bytes per
+// unitig of the graph cross a link, once per call.
+//   truss    every rank selects the maximal core over all ids (max_coreness is global), filters and relabels ITS slice
+//            of the canonical edge list and pulls the other ranks' filtered slices.  The relabelling is monotone and the
+//            slices are in u-range order, so their concatenation is the canonical sorted edge list of the maximal core:
+//            no sort.  Every rank then runs the single-GPU truss on it (replicated, like rpeel.cu), so the maximal core
+//            has to fit one GPU and hold fewer than 2^32 edges; the whole graph need not.
+//   densest  every rank counts its unitigs per coreness and its forward edges per min(core(u), core(v)); the summed
+//            histograms go through the selection of the single-GPU densest core.
+// Every exchange carries each rank's status: a failure on one rank (allocation, CUDA) makes every rank return an error
+// at the next exchange, the failing rank its own and the others that of the first failing rank.
+#include <vector>
+
+#include "dgraph.cuh"
+#include "kombgpu_debug.h"
+
+namespace kg {
+namespace {
+
+// rank q owns ids [*lo, *lo + rows)
+uint32_t rows_of(const kombgpu_dist_graph *g, int q, uint64_t *lo) {
+    *lo = (uint64_t)q * g->step;
+    if (*lo >= g->n_global) return 0u;
+    const uint64_t hi = *lo + g->step < g->n_global ? *lo + g->step : g->n_global;
+    return (uint32_t)(hi - *lo);
+}
+
+int cuda_rc(kombgpu_ctx *ctx, cudaError_t e, const char *what) {
+    return e == cudaSuccess ? KOMBGPU_OK : ctx_fail(ctx, KOMBGPU_ECUDA, "%s: %s", what, cudaGetErrorString(e));
+}
+
+// comm_exchange of k words per rank (out[q * k + j]) that also carries every rank's status `rc`
+int exchange_rc(kombgpu_comm *c, int rc, const unsigned long long *vals, int k, unsigned long long *out) {
+    unsigned long long mine[kCtlWords], all[kMaxRanks * kCtlWords];
+    mine[0] = rc != KOMBGPU_OK ? (unsigned long long)-rc : 0ull;
+    for (int j = 0; j < k; ++j) mine[1 + j] = vals[j];
+    KG_TRY(comm_exchange(c, mine, k + 1, all));
+    for (int q = 0; q < c->world; ++q)
+        for (int j = 0; j < k; ++j) out[q * k + j] = all[q * (k + 1) + 1 + j];
+    if (rc != KOMBGPU_OK) return rc;   // this rank's own message stands
+    for (int q = 0; q < c->world; ++q)
+        if (all[q * (k + 1)]) return ctx_fail(c->ctx, -(int)all[q * (k + 1)], "rank %d failed; the call stopped on every rank", q);
+    return KOMBGPU_OK;
+}
+
+int barrier_rc(kombgpu_comm *c, int rc) { return exchange_rc(c, rc, nullptr, 0, nullptr); }
+
+// core_all[x] = coreness of unitig x, for every unitig of the graph
+int gather_coreness(kombgpu_dist_graph *g, DevBuf<int32_t> &core_all) {
+    kombgpu_comm *c = g->comm;
+    kombgpu_ctx *ctx = g->ctx;
+    SymRewind heap{c, sym_mark(c)};
+    int32_t *mine = nullptr;
+    PeerPtrs<int32_t> peers{};
+    KG_TRY(sym_alloc(c, (size_t)g->step, &mine, &peers));   // the same size on every rank
+    int rc = KOMBGPU_OK;
+    if (!core_all.alloc(ctx, g->n_global)) rc = ctx_fail(ctx, KOMBGPU_ENOMEM, "the coreness of %u unitigs", g->n_global);
+    if (rc == KOMBGPU_OK && g->n_local)
+        rc = cuda_rc(ctx, cudaMemcpyAsync(mine, g->core, (size_t)g->n_local * sizeof(int32_t), cudaMemcpyDeviceToDevice, ctx->stream),
+                     "coreness slice");
+    KG_TRY(barrier_rc(c, rc));   // every rank's slice is in place
+    for (int q = 0; q < c->world && rc == KOMBGPU_OK; ++q) {
+        uint64_t lo = 0;
+        const uint32_t rows = rows_of(g, q, &lo);
+        if (rows)
+            rc = cuda_rc(ctx, cudaMemcpyAsync(core_all.p + lo, peers.p[q], (size_t)rows * sizeof(int32_t), cudaMemcpyDeviceToDevice, ctx->stream),
+                         "coreness slice of a peer");
+    }
+    return barrier_rc(c, rc);   // everybody has read every slice: the buffer may go
+}
+
+}  // namespace
+
+int dist_max_core_truss(kombgpu_dist_graph *g) {
+    kombgpu_comm *c = g->comm;
+    kombgpu_ctx *ctx = g->ctx;
+    const int world = c->world;
+    truss_free(ctx, &g->tr);
+    g->has_truss = false;
+    EvTimer timer(ctx);
+
+    // 1. the coreness of every unitig, and with it the maximal core over all ids, relabelled in order
+    DevBuf<int32_t> core_all;
+    KG_TRY(gather_coreness(g, core_all));
+    g->ms_truss[0] = timer.lap();
+    DevBuf<uint32_t> sub_id, core_vid;
+    uint32_t n_core = 0;
+    int rc = max_core_vertices(ctx, core_all.p, g->n_global, g->st.max_coreness, sub_id, core_vid, &n_core);
+    core_all.release();
+    // 2. this rank's slice of the induced edges
+    DevBuf<uint64_t> slice;
+    uint64_t m_mine = 0;
+    if (rc == KOMBGPU_OK) rc = max_core_edges(ctx, g->edges, g->n_fwd, sub_id.p, slice, &m_mine);
+    sub_id.release();
+
+    // 3. every rank's slice, in rank order: the canonical sorted edge list of the maximal core
+    unsigned long long cnt = m_mine, all_cnt[kMaxRanks];
+    KG_TRY(exchange_rc(c, rc, &cnt, 1, all_cnt));
+    uint64_t off[kMaxRanks + 1] = {}, max_cnt = 0;
+    for (int q = 0; q < world; ++q) {
+        off[q + 1] = off[q] + all_cnt[q];
+        max_cnt = all_cnt[q] > max_cnt ? all_cnt[q] : max_cnt;
+    }
+    const uint64_t m = off[world];
+    if (m >= (1ull << 32))
+        return ctx_fail(ctx, KOMBGPU_EINVAL, "the maximal core has %llu edges: its truss is computed on one GPU and needs fewer than 2^32",
+                        (unsigned long long)m);
+    DevBuf<uint64_t> sub_edges;
+    {
+        SymRewind heap{c, sym_mark(c)};
+        uint64_t *mine = nullptr;
+        PeerPtrs<uint64_t> peers{};
+        KG_TRY(sym_alloc(c, (size_t)max_cnt, &mine, &peers));
+        if (m_mine)
+            rc = cuda_rc(ctx, cudaMemcpyAsync(mine, slice.p, m_mine * sizeof(uint64_t), cudaMemcpyDeviceToDevice, ctx->stream), "edge slice");
+        if (rc == KOMBGPU_OK && !sub_edges.alloc(ctx, m))
+            rc = ctx_fail(ctx, KOMBGPU_ENOMEM, "the %llu edges of the maximal core", (unsigned long long)m);
+        KG_TRY(barrier_rc(c, rc));   // every rank's slice is in place
+        slice.release();
+        for (int q = 0; q < world && rc == KOMBGPU_OK; ++q)
+            if (all_cnt[q])
+                rc = cuda_rc(ctx, cudaMemcpyAsync(sub_edges.p + off[q], peers.p[q], all_cnt[q] * sizeof(uint64_t), cudaMemcpyDeviceToDevice,
+                                                  ctx->stream), "edge slice of a peer");
+        KG_TRY(barrier_rc(c, rc));   // everybody has read every slice: the buffers may go
+    }
+    g->ms_truss[1] = timer.lap();
+
+    // 4. the truss of the whole maximal core, on every rank; one answer on every rank
+    rc = barrier_rc(c, sub_edges_truss(ctx, sub_edges, m, core_vid, n_core, &g->tr));
+    g->ms_truss[2] = timer.lap();
+    if (rc != KOMBGPU_OK) {
+        truss_free(ctx, &g->tr);
+        return rc;
+    }
+    g->has_truss = true;
+    return KOMBGPU_OK;
+}
+
+int dist_densest_core(kombgpu_dist_graph *g, DensestCore *out) {
+    kombgpu_comm *c = g->comm;
+    kombgpu_ctx *ctx = g->ctx;
+    const int world = c->world;
+    const uint64_t n = g->n_global, n_edges = g->n_edges_global;
+    const uint32_t n_bins = n && n_edges ? (uint32_t)g->st.max_coreness + 1 : 0u;   // the same on every rank
+    std::vector<unsigned long long> h(2 * (size_t)n_bins, 0ull);
+    if (n_bins) {
+        DevBuf<int32_t> core_all;
+        KG_TRY(gather_coreness(g, core_all));
+        SymRewind heap{c, sym_mark(c)};
+        unsigned long long *mine = nullptr;
+        PeerPtrs<unsigned long long> peers{};
+        KG_TRY(sym_alloc(c, 2 * (size_t)n_bins, &mine, &peers));
+        // unitigs per coreness over the local slice; forward edges per min(core(u), core(v)) over the local edges
+        int rc = cuda_rc(ctx, cudaMemsetAsync(mine, 0, 2 * (size_t)n_bins * sizeof(unsigned long long), ctx->stream), "histograms");
+        if (rc == KOMBGPU_OK) rc = level_histogram(ctx, g->core, nullptr, g->n_local, n_bins, mine);
+        if (rc == KOMBGPU_OK) rc = level_histogram(ctx, core_all.p, g->edges, g->n_fwd, n_bins, mine + n_bins);
+        KG_TRY(barrier_rc(c, rc));   // every rank's histograms are in place
+        core_all.release();
+        DevBuf<unsigned long long> all;
+        std::vector<unsigned long long> h_all((size_t)world * 2 * n_bins);
+        if (!all.alloc(ctx, h_all.size())) rc = ctx_fail(ctx, KOMBGPU_ENOMEM, "workspace");
+        for (int q = 0; q < world && rc == KOMBGPU_OK; ++q)
+            rc = cuda_rc(ctx, cudaMemcpyAsync(all.p + (size_t)q * 2 * n_bins, peers.p[q], 2 * (size_t)n_bins * sizeof(unsigned long long),
+                                              cudaMemcpyDeviceToDevice, ctx->stream), "histograms of a peer");
+        if (rc == KOMBGPU_OK) rc = read_back(ctx, all.p, h_all.data(), h_all.size());
+        KG_TRY(barrier_rc(c, rc));   // everybody has read every histogram: the buffer may go
+        for (int q = 0; q < world; ++q)
+            for (size_t i = 0; i < h.size(); ++i) h[i] += h_all[(size_t)q * 2 * n_bins + i];
+    }
+    *out = densest_level(h.data(), h.data() + n_bins, n_bins, n, n_edges);
+    return KOMBGPU_OK;
+}
+
+}  // namespace kg
+
+using namespace kg;
+
+extern "C" {
+
+int kombgpu_dist_max_core_truss(kombgpu_dist_graph *g, uint32_t *n_core_vertices, uint64_t *n_core_edges, int32_t *max_trussness,
+                                uint32_t *n_truss_vertices) {
+    if (!g) return KOMBGPU_EINVAL;
+    kombgpu_ctx *ctx = g->ctx;
+    if (!g->has_core) return ctx_fail(ctx, KOMBGPU_ESTATE, "kombgpu_dist_max_core_truss needs kombgpu_dist_coreness first");
+    KG_CUDA(ctx, cudaSetDevice(ctx->device));
+    if (!g->has_truss) KG_TRY(dist_max_core_truss(g));
+    if (n_core_vertices) *n_core_vertices = g->tr.n_core;
+    if (n_core_edges) *n_core_edges = g->tr.m;
+    if (max_trussness) *max_trussness = g->tr.tmax;
+    if (n_truss_vertices) *n_truss_vertices = g->tr.n_vertices;
+    return KOMBGPU_OK;
+}
+
+int kombgpu_dist_max_core_edges(const kombgpu_dist_graph *g, uint32_t *u, uint32_t *v, int32_t *trussness) {
+    if (!g) return KOMBGPU_EINVAL;
+    kombgpu_ctx *ctx = g->ctx;
+    if (!g->has_truss) return ctx_fail(ctx, KOMBGPU_ESTATE, "call kombgpu_dist_max_core_truss first");
+    KG_CUDA(ctx, cudaSetDevice(ctx->device));
+    return truss_edges_to_host(ctx, g->tr, u, v, trussness);
+}
+
+int kombgpu_dist_truss_vertices(const kombgpu_dist_graph *g, uint32_t *vids) {
+    if (!g) return KOMBGPU_EINVAL;
+    kombgpu_ctx *ctx = g->ctx;
+    if (!g->has_truss) return ctx_fail(ctx, KOMBGPU_ESTATE, "call kombgpu_dist_max_core_truss first");
+    KG_CUDA(ctx, cudaSetDevice(ctx->device));
+    return truss_vertices_to_host(ctx, g->tr, vids);
+}
+
+int kombgpu_dist_densest_core(kombgpu_dist_graph *g, int32_t *k_star, uint32_t *n_vertices, uint64_t *n_edges, double *density) {
+    if (!g) return KOMBGPU_EINVAL;
+    kombgpu_ctx *ctx = g->ctx;
+    if (!g->has_core) return ctx_fail(ctx, KOMBGPU_ESTATE, "kombgpu_dist_densest_core needs kombgpu_dist_coreness first");
+    KG_CUDA(ctx, cudaSetDevice(ctx->device));
+    DensestCore best{};
+    KG_TRY(dist_densest_core(g, &best));
+    if (k_star) *k_star = best.k;
+    if (n_vertices) *n_vertices = (uint32_t)best.n_vertices;
+    if (n_edges) *n_edges = best.n_edges;
+    if (density) *density = best.density;
+    return KOMBGPU_OK;
+}
+
+// measurement aid (include/kombgpu_debug.h): the CUDA-event split of the last kombgpu_dist_max_core_truss on this rank
+int kombgpu_debug_dist_truss_timing(const kombgpu_dist_graph *g, float *ms_core_gather, float *ms_slice_gather, float *ms_truss) {
+    if (!g) return KOMBGPU_EINVAL;
+    if (!g->has_truss) return ctx_fail(g->ctx, KOMBGPU_ESTATE, "call kombgpu_dist_max_core_truss first");
+    if (ms_core_gather) *ms_core_gather = g->ms_truss[0];
+    if (ms_slice_gather) *ms_slice_gather = g->ms_truss[1];
+    if (ms_truss) *ms_truss = g->ms_truss[2];
+    return KOMBGPU_OK;
+}
+
+}  // extern "C"

@@ -219,40 +219,45 @@ __global__ void __launch_bounds__(kThreads) sub_edges_original_kernel(const uint
 
 }  // namespace
 
-void truss_release(kombgpu_graph *g) {
-    kombgpu_ctx *ctx = g->ctx;
-    void *ptrs[] = {g->tr_core_vid, g->tr_edges, g->tr_truss, g->tr_vertices};
+void truss_free(kombgpu_ctx *ctx, MaxCoreTruss *tr) {
+    void *ptrs[] = {tr->core_vid, tr->edges, tr->truss, tr->vertices};
     for (void *p : ptrs)
         if (p) ws_free(ctx, p);
-    g->tr_core_vid = nullptr; g->tr_edges = nullptr; g->tr_truss = nullptr; g->tr_vertices = nullptr;
+    *tr = MaxCoreTruss{};
+}
+
+void truss_release(kombgpu_graph *g) {
+    truss_free(g->ctx, &g->tr);
     g->has_truss = false;
 }
 
-int max_core_truss(kombgpu_graph *g) {
-    kombgpu_ctx *ctx = g->ctx;
-    const uint32_t n = g->n;
-    const uint64_t E = g->n_edges;
-    truss_release(g);
-    const uint32_t cap = (uint32_t)ctx->sm_count * 8u;
-    const int32_t kmax = g->st.max_coreness;
-
-    // 1. the vertices of the maximal core, relabelled in order
-    DevBuf<uint32_t> sub_id, core_vid, d_cnt(ctx, 2);
+int max_core_vertices(kombgpu_ctx *ctx, const int32_t *core, uint32_t n, int32_t kmax, DevBuf<uint32_t> &sub_id,
+                      DevBuf<uint32_t> &core_vid, uint32_t *n_core) {
+    DevBuf<uint32_t> d_cnt(ctx, 1);
     KG_ALLOC(ctx, sub_id, n);
     KG_ALLOC(ctx, core_vid, n);
     if (!d_cnt) return ctx_fail(ctx, KOMBGPU_ENOMEM, "workspace");
-    KG_TRY((device_scan<uint32_t>(ctx, n, CoreFlagIn{g->core, kmax}, CoreFlagOut{sub_id.p, core_vid.p}, d_cnt.p)));
-    uint32_t n_core = 0;
-    KG_TRY(read_back(ctx, d_cnt.p, &n_core, 1));
+    KG_TRY((device_scan<uint32_t>(ctx, n, CoreFlagIn{core, kmax}, CoreFlagOut{sub_id.p, core_vid.p}, d_cnt.p)));
+    return read_back(ctx, d_cnt.p, n_core, 1);
+}
 
-    // 2. the induced edges (the relabelling is monotone: the list stays canonical and sorted)
-    DevBuf<uint64_t> sub_edges;
-    KG_ALLOC(ctx, sub_edges, E);
-    KG_TRY((device_scan<uint32_t>(ctx, E, SubEdgeFlagIn{g->edges, sub_id.p}, SubEdgeOut{g->edges, sub_id.p, sub_edges.p}, d_cnt.p)));
+int max_core_edges(kombgpu_ctx *ctx, const uint64_t *edges, uint64_t count, const uint32_t *sub_id, DevBuf<uint64_t> &out,
+                   uint64_t *m) {
+    DevBuf<uint32_t> d_cnt(ctx, 1);
+    KG_ALLOC(ctx, out, count);
+    if (!d_cnt) return ctx_fail(ctx, KOMBGPU_ENOMEM, "workspace");
+    KG_TRY((device_scan<uint32_t>(ctx, count, SubEdgeFlagIn{edges, sub_id}, SubEdgeOut{edges, sub_id, out.p}, d_cnt.p)));
     uint32_t m32 = 0;
     KG_TRY(read_back(ctx, d_cnt.p, &m32, 1));
-    const uint64_t m = m32;
-    sub_id.release();
+    *m = m32;
+    return KOMBGPU_OK;
+}
+
+int sub_edges_truss(kombgpu_ctx *ctx, DevBuf<uint64_t> &sub_edges, uint64_t m, DevBuf<uint32_t> &core_vid, uint32_t n_core,
+                    MaxCoreTruss *tr) {
+    const uint32_t cap = (uint32_t)ctx->sm_count * 8u;
+    DevBuf<uint32_t> d_cnt(ctx, 2);
+    if (!d_cnt) return ctx_fail(ctx, KOMBGPU_ENOMEM, "workspace");
 
     // 3. its CSR (rows sorted) and the entry -> edge id map
     kombgpu_graph sub;
@@ -328,15 +333,60 @@ int max_core_truss(kombgpu_graph *g) {
     rc = read_back(ctx, d_cnt.p, &n_tv, 1);
     if (rc != KOMBGPU_OK) return bail(rc);
     graph_release(&sub);
-    g->tr_n_core = n_core;
-    g->tr_m = m;
-    g->tr_max = tmax;
-    g->tr_n_vertices = n_tv;
-    g->tr_core_vid = core_vid.take();
-    g->tr_edges = sub_edges.take();
-    g->tr_truss = truss.take();
-    g->tr_vertices = tverts.take();
+    tr->n_core = n_core;
+    tr->m = m;
+    tr->tmax = tmax;
+    tr->n_vertices = n_tv;
+    tr->core_vid = core_vid.take();
+    tr->edges = sub_edges.take();
+    tr->truss = truss.take();
+    tr->vertices = tverts.take();
+    return KOMBGPU_OK;
+}
+
+int max_core_truss(kombgpu_graph *g) {
+    kombgpu_ctx *ctx = g->ctx;
+    truss_release(g);
+    // 1. the vertices of the maximal core, relabelled in order
+    DevBuf<uint32_t> sub_id, core_vid;
+    uint32_t n_core = 0;
+    KG_TRY(max_core_vertices(ctx, g->core, g->n, g->st.max_coreness, sub_id, core_vid, &n_core));
+    // 2. the induced edges
+    DevBuf<uint64_t> sub_edges;
+    uint64_t m = 0;
+    KG_TRY(max_core_edges(ctx, g->edges, g->n_edges, sub_id.p, sub_edges, &m));
+    sub_id.release();
+    // 3-5. their trussness
+    KG_TRY(sub_edges_truss(ctx, sub_edges, m, core_vid, n_core, &g->tr));
     g->has_truss = true;
+    return KOMBGPU_OK;
+}
+
+int truss_edges_to_host(kombgpu_ctx *ctx, const MaxCoreTruss &tr, uint32_t *u, uint32_t *v, int32_t *trussness) {
+    const uint64_t m = tr.m;
+    if (m == 0) return KOMBGPU_OK;
+    if (u || v) {
+        if (!u || !v) return ctx_fail(ctx, KOMBGPU_EINVAL, "u and v must be given together");
+        DevBuf<uint32_t> du, dv;
+        KG_ALLOC(ctx, du, m);
+        KG_ALLOC(ctx, dv, m);
+        KG_LAUNCH(ctx, sub_edges_original_kernel, grid_for(m, kThreads, (uint32_t)ctx->sm_count * 8u), kThreads, 0, tr.edges, m, tr.core_vid, du.p, dv.p);
+        KG_CUDA(ctx, cudaMemcpyAsync(u, du.p, m * sizeof(uint32_t), cudaMemcpyDeviceToHost, ctx->stream));
+        KG_CUDA(ctx, cudaMemcpyAsync(v, dv.p, m * sizeof(uint32_t), cudaMemcpyDeviceToHost, ctx->stream));
+        KG_CUDA(ctx, cudaStreamSynchronize(ctx->stream));
+    }
+    if (trussness) {
+        KG_CUDA(ctx, cudaMemcpyAsync(trussness, tr.truss, m * sizeof(int32_t), cudaMemcpyDeviceToHost, ctx->stream));
+        KG_CUDA(ctx, cudaStreamSynchronize(ctx->stream));
+    }
+    return KOMBGPU_OK;
+}
+
+int truss_vertices_to_host(kombgpu_ctx *ctx, const MaxCoreTruss &tr, uint32_t *vids) {
+    if (tr.n_vertices == 0) return KOMBGPU_OK;
+    if (!vids) return ctx_fail(ctx, KOMBGPU_EINVAL, "null argument");
+    KG_CUDA(ctx, cudaMemcpyAsync(vids, tr.vertices, (size_t)tr.n_vertices * sizeof(uint32_t), cudaMemcpyDeviceToHost, ctx->stream));
+    KG_CUDA(ctx, cudaStreamSynchronize(ctx->stream));
     return KOMBGPU_OK;
 }
 
@@ -354,10 +404,10 @@ int kombgpu_graph_max_core_truss(kombgpu_graph *g, uint32_t *n_core_vertices, ui
     if (g->n_edges && !g->edges) return ctx_fail(ctx, KOMBGPU_ESTATE, "graph was adopted from a CSR: no canonical edge list");
     KG_CUDA(ctx, cudaSetDevice(ctx->device));
     if (!g->has_truss) KG_TRY(max_core_truss(g));
-    if (n_core_vertices) *n_core_vertices = g->tr_n_core;
-    if (n_core_edges) *n_core_edges = g->tr_m;
-    if (max_trussness) *max_trussness = g->tr_max;
-    if (n_truss_vertices) *n_truss_vertices = g->tr_n_vertices;
+    if (n_core_vertices) *n_core_vertices = g->tr.n_core;
+    if (n_core_edges) *n_core_edges = g->tr.m;
+    if (max_trussness) *max_trussness = g->tr.tmax;
+    if (n_truss_vertices) *n_truss_vertices = g->tr.n_vertices;
     return KOMBGPU_OK;
 }
 
@@ -366,35 +416,15 @@ int kombgpu_graph_max_core_edges(const kombgpu_graph *g, uint32_t *u, uint32_t *
     kombgpu_ctx *ctx = g->ctx;
     if (!g->has_truss) return ctx_fail(ctx, KOMBGPU_ESTATE, "call kombgpu_graph_max_core_truss first");
     KG_CUDA(ctx, cudaSetDevice(ctx->device));
-    const uint64_t m = g->tr_m;
-    if (m == 0) return KOMBGPU_OK;
-    if (u || v) {
-        if (!u || !v) return ctx_fail(ctx, KOMBGPU_EINVAL, "u and v must be given together");
-        DevBuf<uint32_t> du, dv;
-        KG_ALLOC(ctx, du, m);
-        KG_ALLOC(ctx, dv, m);
-        KG_LAUNCH(ctx, sub_edges_original_kernel, grid_for(m, kThreads, (uint32_t)ctx->sm_count * 8u), kThreads, 0, g->tr_edges, m, g->tr_core_vid, du.p, dv.p);
-        KG_CUDA(ctx, cudaMemcpyAsync(u, du.p, m * sizeof(uint32_t), cudaMemcpyDeviceToHost, ctx->stream));
-        KG_CUDA(ctx, cudaMemcpyAsync(v, dv.p, m * sizeof(uint32_t), cudaMemcpyDeviceToHost, ctx->stream));
-        KG_CUDA(ctx, cudaStreamSynchronize(ctx->stream));
-    }
-    if (trussness) {
-        KG_CUDA(ctx, cudaMemcpyAsync(trussness, g->tr_truss, m * sizeof(int32_t), cudaMemcpyDeviceToHost, ctx->stream));
-        KG_CUDA(ctx, cudaStreamSynchronize(ctx->stream));
-    }
-    return KOMBGPU_OK;
+    return truss_edges_to_host(ctx, g->tr, u, v, trussness);
 }
 
 int kombgpu_graph_truss_vertices(const kombgpu_graph *g, uint32_t *vids) {
     if (!g) return KOMBGPU_EINVAL;
     kombgpu_ctx *ctx = g->ctx;
     if (!g->has_truss) return ctx_fail(ctx, KOMBGPU_ESTATE, "call kombgpu_graph_max_core_truss first");
-    if (g->tr_n_vertices == 0) return KOMBGPU_OK;
-    if (!vids) return ctx_fail(ctx, KOMBGPU_EINVAL, "null argument");
     KG_CUDA(ctx, cudaSetDevice(ctx->device));
-    KG_CUDA(ctx, cudaMemcpyAsync(vids, g->tr_vertices, (size_t)g->tr_n_vertices * sizeof(uint32_t), cudaMemcpyDeviceToHost, ctx->stream));
-    KG_CUDA(ctx, cudaStreamSynchronize(ctx->stream));
-    return KOMBGPU_OK;
+    return truss_vertices_to_host(ctx, g->tr, vids);
 }
 
 }  // extern "C"

@@ -10,7 +10,7 @@ from __future__ import annotations
 
 import ctypes
 import threading
-from ctypes import byref, c_double, c_int, c_int32, c_uint32, c_uint64, c_void_p
+from ctypes import byref, c_double, c_float, c_int, c_int32, c_uint32, c_uint64, c_void_p
 
 import numpy as np
 
@@ -131,6 +131,32 @@ class DistGraph:
         mc, ms = c_int32(), c_double()
         self._ctx._check(self._lib.kombgpu_dist_graph_summary(self._h, byref(mc), byref(ms)))
         return mc.value, ms.value
+
+    def max_core_truss(self) -> dict:
+        """Maximal core of the whole graph + trussness of its edges, the dict of Graph.max_core_truss on every rank
+        (kombgpu_dist_max_core_truss).  Collective."""
+        nc, mc, tm, nt = c_uint32(), c_uint64(), c_int32(), c_uint32()
+        self._ctx._check(self._lib.kombgpu_dist_max_core_truss(self._h, byref(nc), byref(mc), byref(tm), byref(nt)))
+        u, v, tr = np.empty(mc.value, np.uint32), np.empty(mc.value, np.uint32), np.empty(mc.value, np.int32)
+        self._ctx._check(self._lib.kombgpu_dist_max_core_edges(self._h, c_void_p(u.ctypes.data), c_void_p(v.ctypes.data),
+                                                               c_void_p(tr.ctypes.data)))
+        tv = np.empty(nt.value, np.uint32)
+        self._ctx._check(self._lib.kombgpu_dist_truss_vertices(self._h, c_void_p(tv.ctypes.data)))
+        return {"n_core_vertices": nc.value, "n_core_edges": mc.value, "max_trussness": tm.value, "u": u, "v": v, "trussness": tr,
+                "truss_vertices": tv}
+
+    def truss_timing(self) -> dict:
+        """CUDA-event split of this rank's last max_core_truss() in ms (measurement aid, include/kombgpu_debug.h)."""
+        a, b, c = c_float(), c_float(), c_float()
+        self._ctx._check(self._lib.kombgpu_debug_dist_truss_timing(self._h, byref(a), byref(b), byref(c)))
+        return {"ms_core_gather": a.value, "ms_slice_gather": b.value, "ms_truss": c.value}
+
+    def densest_core(self) -> dict:
+        """Densest k-core of the whole graph, the dict of Graph.densest_core on every rank (kombgpu_dist_densest_core).
+        Collective."""
+        k, nv, ne, d = c_int32(), c_uint32(), c_uint64(), c_double()
+        self._ctx._check(self._lib.kombgpu_dist_densest_core(self._h, byref(k), byref(nv), byref(ne), byref(d)))
+        return {"k": k.value, "n_vertices": nv.value, "n_edges": ne.value, "density": d.value}
 
     def results(self, out: dict | None = None) -> dict:
         """degree / coreness / score of the local unitigs [v_lo, v_lo + n_local) on the host."""
