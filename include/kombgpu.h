@@ -549,6 +549,20 @@ int kombgpu_dist_truss_vertices(const kombgpu_dist_graph *g, uint32_t *vids);
  * The ranks sum their histograms of unitigs per coreness and of edges per min(core(u), core(v)). */
 int kombgpu_dist_densest_core(kombgpu_dist_graph *g, int32_t *k_star, uint32_t *n_vertices, uint64_t *n_edges,
                               double *density);
+/* The densest BLOCK of the WHOLE partitioned graph, as kombgpu_graph_densest_block (the same passes, sizes, weight
+ * sum and density; with weights whose partial sums are exact, such as multiples of a power of two, bit for bit).
+ * `weight`: this rank's slice, n_local host doubles >= 0 for unitigs [v_lo, v_lo + n_local), or NULL (weights 0);
+ * use_scores != 0 for the graph's own CORE-A scores (needs kombgpu_dist_corea, KOMBGPU_ESTATE otherwise).  eps and
+ * use_scores must be the same on every rank.  member (optional): this rank's slice, n_local bytes.  The scalars are
+ * global: every rank gets the same values.  Collective; needs only the build; nothing is cached.  The passes are
+ * driven by the host: every rank marks its own unitigs, the ranks exchange what they removed (4 bytes per removed
+ * unitig cross a link) and every rank lowers the degrees of its own survivors.  The arguments are checked before the
+ * first pass: a bad one on any rank gives KOMBGPU_EINVAL there (an eps that differs between the ranks: on every rank)
+ * and an error on every other rank.  Any later failure on a rank also makes every rank return an error.  The graph and
+ * the communicator stay usable. */
+int kombgpu_dist_densest_block(kombgpu_dist_graph *g, const double *weight, int use_scores, double eps,
+                               uint32_t *n_vertices, uint64_t *n_edges, double *weight_sum, double *density,
+                               uint32_t *n_passes, uint8_t *member);
 
 int kombgpu_abi_version(void);
 

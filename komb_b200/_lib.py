@@ -165,6 +165,8 @@ SIGNATURES = {
     "kombgpu_dist_max_core_edges": (c_int, [c_void_p, c_void_p, c_void_p, c_void_p]),
     "kombgpu_dist_truss_vertices": (c_int, [c_void_p, c_void_p]),
     "kombgpu_dist_densest_core": (c_int, [c_void_p, POINTER(c_int32), POINTER(c_uint32), POINTER(c_uint64), POINTER(c_double)]),
+    "kombgpu_dist_densest_block": (c_int, [c_void_p, c_void_p, c_int, c_double, POINTER(c_uint32), POINTER(c_uint64), POINTER(c_double),
+                                           POINTER(c_double), POINTER(c_uint32), c_void_p]),
 }
 
 _lib = None

@@ -61,21 +61,47 @@ __global__ void __launch_bounds__(kThreads) level_hist_kernel(const int32_t *__r
 // survivor with priority <= 2 (1 + eps) density(S): the priorities sum to at most 2 f(S), so a pass removes at least an
 // eps / (1 + eps) share of the survivors (O(log n / eps) passes) and the best S seen is a 2 (1 + eps)-approximation,
 // against 2 for the serial order.  Ties need no rule: a pass is a set.
-constexpr uint32_t kUnset = 0xffffffffu;
 
-struct BlockPass {
-    unsigned long long removed, single, both;   // unitigs removed; entries towards survivors / towards unitigs removed in the same pass
-    double w_removed;
+// one warp per removed unitig: its survivors lose a neighbour
+__global__ void __launch_bounds__(kThreads) block_update_kernel(const uint64_t *__restrict__ row_ptr, const uint32_t *__restrict__ col,
+                                                                const uint32_t *__restrict__ list, uint32_t n_list,
+                                                                uint32_t t, const uint32_t *__restrict__ pass, int32_t *__restrict__ deg_s,
+                                                                BlockPass *__restrict__ st) {
+    block_update_warps(row_ptr, col, list, n_list, t, pass, deg_s, st);
+}
+
+// the single-GPU steps: every unitig is local, the list holds the removed ids
+struct GraphBlockSteps final : BlockSteps {
+    kombgpu_ctx *ctx;
+    const kombgpu_graph *g;
+    const double *w;
+    int32_t *deg_s;
+    uint32_t *pass, *list;
+    BlockPass *st;
+    GraphBlockSteps(kombgpu_ctx *c, const kombgpu_graph *gr, const double *wt, int32_t *d, uint32_t *p, uint32_t *l, BlockPass *s)
+        : ctx(c), g(gr), w(wt), deg_s(d), pass(p), list(l), st(s) {}
+    int mark(double thr, uint32_t t, BlockPass *h) override {
+        KG_CUDA(ctx, cudaMemsetAsync(st, 0, sizeof(BlockPass), ctx->stream));
+        KG_LAUNCH(ctx, block_mark_kernel, block_grid(ctx, g->n), kBlockThreads, 0, w, deg_s, g->n, thr, t, 0u, pass, list, st);
+        return read_back(ctx, st, h, 1);
+    }
+    int update(uint32_t t, BlockPass *h) override {
+        const uint32_t ugrid = min(ceil_div_u64(h->removed * 32u, kThreads), (uint32_t)ctx->sm_count * 16u);
+        KG_LAUNCH(ctx, block_update_kernel, ugrid, kThreads, 0, g->row_ptr, g->col, list, (uint32_t)h->removed, t, pass, deg_s, st);
+        return read_back(ctx, st, h, 1);
+    }
 };
 
-__global__ void __launch_bounds__(kThreads) block_mark_kernel(const double *__restrict__ w, const int32_t *__restrict__ deg_s, uint32_t n,
-                                                              double thr, uint32_t t, uint32_t *__restrict__ pass, uint32_t *__restrict__ list,
-                                                              BlockPass *__restrict__ st) {
+}  // namespace
+
+__global__ void __launch_bounds__(kBlockThreads) block_mark_kernel(const double *__restrict__ w, const int32_t *__restrict__ deg_s, uint32_t n,
+                                                                   double thr, uint32_t t, uint32_t id_base, uint32_t *__restrict__ pass,
+                                                                   uint32_t *__restrict__ list, BlockPass *__restrict__ st) {
     double wsum = 0.0;
     for (uint32_t base = blockIdx.x * blockDim.x; base < n; base += gridDim.x * blockDim.x) {
         const uint32_t i = base + threadIdx.x;
         bool take = false;
-        if (i < n && pass[i] == kUnset) {
+        if (i < n && pass[i] == kBlockUnset) {
             const double wi = w ? w[i] : 0.0;
             take = wi + (double)deg_s[i] <= thr;
             if (take) { pass[i] = t; wsum += wi; }
@@ -85,44 +111,70 @@ __global__ void __launch_bounds__(kThreads) block_mark_kernel(const double *__re
             uint32_t pos = 0;
             if (lane_id() == 0) pos = (uint32_t)atomicAdd(&st->removed, (unsigned long long)__popc(m));
             pos = __shfl_sync(kFullMask, pos, 0) + __popc(m & lanemask_lt());
-            if (take) list[pos] = i;
+            if (take) list[pos] = id_base + i;
         }
     }
     wsum = warp_reduce_add(wsum);
     if (lane_id() == 0 && wsum != 0.0) atomicAdd(&st->w_removed, wsum);
 }
 
-// one warp per removed unitig: its survivors lose a neighbour
-__global__ void __launch_bounds__(kThreads) block_update_kernel(const uint64_t *__restrict__ row_ptr, const uint32_t *__restrict__ col,
-                                                                const uint32_t *__restrict__ list, uint32_t n_list,
-                                                                uint32_t t, const uint32_t *__restrict__ pass, int32_t *__restrict__ deg_s,
-                                                                BlockPass *__restrict__ st) {
-    const uint32_t warp = (blockIdx.x * blockDim.x + threadIdx.x) >> 5, n_warps = (gridDim.x * blockDim.x) >> 5, lane = lane_id();
-    unsigned long long single = 0, both = 0;
-    for (uint32_t k = warp; k < n_list; k += n_warps) {
-        const uint32_t i = list[k];
-        const uint64_t lo = row_ptr[i], hi = row_ptr[i + 1];
-        for (uint64_t e = lo + lane; e < hi; e += 32) {
-            const uint32_t j = col[e];
-            const uint32_t pj = pass[j];
-            if (pj == kUnset) { atomicSub(&deg_s[j], 1); ++single; }
-            else if (pj == t) ++both;
-        }
-    }
-    single = warp_reduce_add(single);
-    both = warp_reduce_add(both);
-    if (lane == 0) {
-        if (single) atomicAdd(&st->single, single);
-        if (both) atomicAdd(&st->both, both);
-    }
-}
-
-__global__ void __launch_bounds__(kThreads) block_member_kernel(const uint32_t *__restrict__ pass, uint32_t n, uint32_t t_best,
-                                                                uint8_t *__restrict__ member) {
+__global__ void __launch_bounds__(kBlockThreads) block_member_kernel(const uint32_t *__restrict__ pass, uint32_t n, uint32_t t_best,
+                                                                     uint8_t *__restrict__ member) {
     for (uint32_t i = blockIdx.x * blockDim.x + threadIdx.x; i < n; i += gridDim.x * blockDim.x) member[i] = pass[i] >= t_best ? 1 : 0;
 }
 
-}  // namespace
+int block_weight_sum(kombgpu_ctx *ctx, const double *w, const int32_t *deg_s, uint32_t n, uint32_t *list, BlockPass *st, double *sum) {
+    *sum = 0.0;
+    if (!n) return KOMBGPU_OK;
+    DevBuf<uint32_t> scratch;
+    KG_ALLOC(ctx, scratch, n);
+    KG_CUDA(ctx, cudaMemsetAsync(st, 0, sizeof(BlockPass), ctx->stream));
+    KG_CUDA(ctx, cudaMemsetAsync(scratch.p, 0xff, (size_t)n * sizeof(uint32_t), ctx->stream));
+    KG_LAUNCH(ctx, block_mark_kernel, block_grid(ctx, n), kBlockThreads, 0, w, deg_s, n, 1e308, 0u, 0u, scratch.p, list, st);
+    BlockPass h{};
+    KG_TRY(read_back(ctx, st, &h, 1));
+    *sum = h.w_removed;
+    return KOMBGPU_OK;
+}
+
+int block_member(kombgpu_ctx *ctx, const uint32_t *pass, uint32_t n, uint32_t t_best, uint8_t *member) {
+    if (!member || !n) return KOMBGPU_OK;
+    DevBuf<uint8_t> member_dev;
+    KG_ALLOC(ctx, member_dev, n);
+    KG_LAUNCH(ctx, block_member_kernel, block_grid(ctx, n), kBlockThreads, 0, pass, n, t_best, member_dev.p);
+    KG_CUDA(ctx, cudaMemcpyAsync(member, member_dev.p, n, cudaMemcpyDeviceToHost, ctx->stream));
+    KG_CUDA(ctx, cudaStreamSynchronize(ctx->stream));
+    return KOMBGPU_OK;
+}
+
+int densest_block_passes(kombgpu_ctx *ctx, uint64_t n, uint64_t n_edges, double W, double eps, BlockSteps &steps, DensestBlock *out) {
+    uint64_t E = n_edges, N = n;
+    DensestBlock best{n, n_edges, W, n ? (W + (double)E) / (double)n : 0.0, 0u, 0u};
+    uint32_t t = 0;
+    while (N > 0) {
+        const double rho = (W + (double)E) / (double)N;
+        if (t == 0 || rho > best.density) best = DensestBlock{N, E, W, rho, 0u, t};
+        double thr = 2.0 * (1.0 + eps) * rho;
+        BlockPass h{};
+        for (int attempt = 0;; ++attempt) {
+            KG_TRY(steps.mark(thr, t, &h));
+            if (h.removed) break;
+            // the smallest priority is at most the mean, which is at most 2 rho; only rounding in the weight sums can leave a pass empty
+            if (attempt >= 60) return ctx_fail(ctx, KOMBGPU_EINTERNAL, "densest block: a pass removed nothing");
+            thr = thr * 1.0000001 + 1e-300;
+        }
+        KG_TRY(steps.update(t, &h));
+        N -= h.removed;
+        E -= h.single + h.both / 2;
+        W -= h.w_removed;
+        if (W < 0.0 || N == 0) W = 0.0;
+        ++t;
+        if (t == kBlockUnset - 1) return ctx_fail(ctx, KOMBGPU_EINTERNAL, "densest block: too many passes");
+    }
+    best.passes = t;
+    *out = best;
+    return KOMBGPU_OK;
+}
 
 int level_histogram(kombgpu_ctx *ctx, const int32_t *core, const uint64_t *edges, uint64_t count, uint32_t n_bins,
                     unsigned long long *hist) {
@@ -203,62 +255,22 @@ extern "C" int kombgpu_graph_densest_block(kombgpu_graph *g, const double *weigh
     DevBuf<uint32_t> pass, list;
     DevBuf<int32_t> deg_s;
     DevBuf<BlockPass> st(ctx, 1);
-    DevBuf<uint8_t> member_dev;
     KG_ALLOC(ctx, pass, n);
     KG_ALLOC(ctx, list, n);
     KG_ALLOC(ctx, deg_s, n);
     if (!st) return ctx_fail(ctx, KOMBGPU_ENOMEM, "workspace");
     KG_CUDA(ctx, cudaMemsetAsync(pass.p, 0xff, (size_t)(n ? n : 1) * sizeof(uint32_t), ctx->stream));
     if (n) KG_CUDA(ctx, cudaMemcpyAsync(deg_s.p, g->deg, (size_t)n * sizeof(int32_t), cudaMemcpyDeviceToDevice, ctx->stream));
-    const uint32_t grid = min(ceil_div_u64(n ? n : 1, kThreads), (uint32_t)ctx->sm_count * 8u);
-    if (use_scores && n) {   // W = sum of the scores: one marking pass over nobody would do; use the mark kernel's reduction on a scratch pass
-        KG_CUDA(ctx, cudaMemsetAsync(st.p, 0, sizeof(BlockPass), ctx->stream));
-        DevBuf<uint32_t> scratch;
-        KG_ALLOC(ctx, scratch, n);
-        KG_CUDA(ctx, cudaMemsetAsync(scratch.p, 0xff, (size_t)n * sizeof(uint32_t), ctx->stream));
-        KG_LAUNCH(ctx, block_mark_kernel, grid, kThreads, 0, w, deg_s.p, n, 1e308, 0u, scratch.p, list.p, st.p);
-        BlockPass h{};
-        KG_TRY(read_back(ctx, st.p, &h, 1));
-        W = h.w_removed;
-    }
-    uint64_t E = g->n_edges, N = n, best_e = E, best_n = n;
-    double best_w = W, best_d = n ? (W + (double)E) / (double)n : 0.0;
-    uint32_t t = 0, t_best = 0;
-    while (N > 0) {
-        const double rho = (W + (double)E) / (double)N;
-        if (t == 0 || rho > best_d) { best_d = rho; best_n = N; best_e = E; best_w = W; t_best = t; }
-        double thr = 2.0 * (1.0 + eps) * rho;
-        BlockPass h{};
-        for (int attempt = 0;; ++attempt) {
-            KG_CUDA(ctx, cudaMemsetAsync(st.p, 0, sizeof(BlockPass), ctx->stream));
-            KG_LAUNCH(ctx, block_mark_kernel, grid, kThreads, 0, w, deg_s.p, n, thr, t, pass.p, list.p, st.p);
-            KG_TRY(read_back(ctx, st.p, &h, 1));
-            if (h.removed) break;
-            // the smallest priority is at most the mean, which is at most 2 rho; only rounding in the weight sums can leave a pass empty
-            if (attempt >= 60) return ctx_fail(ctx, KOMBGPU_EINTERNAL, "densest block: a pass removed nothing");
-            thr = thr * 1.0000001 + 1e-300;
-        }
-        const uint32_t ugrid = min(ceil_div_u64((uint64_t)h.removed * 32u, kThreads), (uint32_t)ctx->sm_count * 16u);
-        KG_LAUNCH(ctx, block_update_kernel, ugrid, kThreads, 0, g->row_ptr, g->col, list.p, (uint32_t)h.removed, t, pass.p, deg_s.p, st.p);
-        KG_TRY(read_back(ctx, st.p, &h, 1));
-        N -= h.removed;
-        E -= h.single + h.both / 2;
-        W -= h.w_removed;
-        if (W < 0.0 || N == 0) W = 0.0;
-        ++t;
-        if (t == kUnset - 1) return ctx_fail(ctx, KOMBGPU_EINTERNAL, "densest block: too many passes");
-    }
-    if (member && n) {
-        KG_ALLOC(ctx, member_dev, n);
-        KG_LAUNCH(ctx, block_member_kernel, grid, kThreads, 0, pass.p, n, t_best, member_dev.p);
-        KG_CUDA(ctx, cudaMemcpyAsync(member, member_dev.p, n, cudaMemcpyDeviceToHost, ctx->stream));
-        KG_CUDA(ctx, cudaStreamSynchronize(ctx->stream));
-    }
+    if (use_scores) KG_TRY(block_weight_sum(ctx, w, deg_s.p, n, list.p, st.p, &W));
+    GraphBlockSteps steps(ctx, g, w, deg_s.p, pass.p, list.p, st.p);
+    DensestBlock best{};
+    KG_TRY(densest_block_passes(ctx, n, g->n_edges, W, eps, steps, &best));
+    KG_TRY(block_member(ctx, pass.p, n, best.t_best, member));
     g->st.kernel_launches += ctx->launches - launches0;
-    if (n_vertices) *n_vertices = (uint32_t)best_n;
-    if (n_edges) *n_edges = best_e;
-    if (weight_sum) *weight_sum = best_w;
-    if (density) *density = best_d;
-    if (n_passes) *n_passes = t;
+    if (n_vertices) *n_vertices = (uint32_t)best.n_vertices;
+    if (n_edges) *n_edges = best.n_edges;
+    if (weight_sum) *weight_sum = best.weight_sum;
+    if (density) *density = best.density;
+    if (n_passes) *n_passes = best.passes;
     return KOMBGPU_OK;
 }

@@ -68,6 +68,8 @@ int dist_corea(kombgpu_dist_graph *g, int key_mode);
 // pcore.cu: the consumers of the finished coreness
 int dist_max_core_truss(kombgpu_dist_graph *g);
 int dist_densest_core(kombgpu_dist_graph *g, DensestCore *out);
+// weight: this rank's slice (host, or NULL); member: this rank's slice (host, n_local bytes, or NULL)
+int dist_densest_block(kombgpu_dist_graph *g, const double *weight, int use_scores, double eps, DensestBlock *out, uint8_t *member);
 
 void dist_graph_release(kombgpu_dist_graph *g);
 

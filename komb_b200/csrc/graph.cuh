@@ -146,6 +146,75 @@ struct DensestCore {
 // hv / he: histograms of n_bins levels over the n vertices and n_edges edges (unread when either count is 0)
 DensestCore densest_level(const unsigned long long *hv, const unsigned long long *he, uint32_t n_bins, uint64_t n, uint64_t n_edges);
 
+// densest block (densest.cu): the bulk greedy peel, shared by the single-GPU graph and the partitioned one (pcore.cu).
+// pass[v] = the pass that removed v, kBlockUnset while v survives.
+constexpr int kBlockThreads = 256;
+constexpr uint32_t kBlockUnset = 0xffffffffu;
+struct BlockPass {
+    unsigned long long removed, single, both;   // unitigs removed; entries towards survivors / towards unitigs removed in the same pass
+    double w_removed;
+};
+// over the n unitigs of a slice: pass[i] = t for every survivor with w[i] + deg_s[i] <= thr (w NULL: weights 0); their ids
+// id_base + i go to list[st->removed ...], st->removed and st->w_removed count them
+__global__ void __launch_bounds__(kBlockThreads) block_mark_kernel(const double *__restrict__ w, const int32_t *__restrict__ deg_s, uint32_t n,
+                                                                   double thr, uint32_t t, uint32_t id_base, uint32_t *__restrict__ pass,
+                                                                   uint32_t *__restrict__ list, BlockPass *__restrict__ st);
+__global__ void __launch_bounds__(kBlockThreads) block_member_kernel(const uint32_t *__restrict__ pass, uint32_t n, uint32_t t_best,
+                                                                     uint8_t *__restrict__ member);
+inline uint32_t block_grid(const kombgpu_ctx *ctx, uint64_t n) {
+    const uint32_t g = ceil_div_u64(n ? n : 1, kBlockThreads), cap = (uint32_t)ctx->sm_count * 8u;
+    return g < cap ? g : cap;
+}
+// the sum of n weights on the device, by the mark kernel's reduction over a scratch pass map (list: n entries of room)
+int block_weight_sum(kombgpu_ctx *ctx, const double *w, const int32_t *deg_s, uint32_t n, uint32_t *list, BlockPass *st, double *sum);
+// pass[0, n) >= t_best to the host (n bytes)
+int block_member(kombgpu_ctx *ctx, const uint32_t *pass, uint32_t n, uint32_t t_best, uint8_t *member);
+
+// The two steps of one pass over the whole graph; densest_block_passes drives them.
+struct BlockSteps {
+    // pass t: remove every survivor with w(v) + deg_S(v) <= thr; h->removed and h->w_removed over the whole graph
+    virtual int mark(double thr, uint32_t t, BlockPass *h) = 0;
+    // the survivors lose their neighbours removed in pass t; h->single and h->both over the whole graph
+    virtual int update(uint32_t t, BlockPass *h) = 0;
+};
+struct DensestBlock {
+    uint64_t n_vertices, n_edges;
+    double weight_sum, density;
+    uint32_t passes, t_best;   // the block is {v : pass[v] >= t_best}
+};
+// the pass loop over a graph of n unitigs, n_edges edges and weight sum W: density and best block, threshold, the retry of
+// an empty pass, the clamp of W and the pass limit
+int densest_block_passes(kombgpu_ctx *ctx, uint64_t n, uint64_t n_edges, double W, double eps, BlockSteps &steps, DensestBlock *out);
+
+#ifdef __CUDACC__
+// one warp per removed unitig list[k]: it walks the unitig's neighbours nb[ptr[x] .. ptr[x + 1]) (ids into pass and deg_s).
+// A survivor loses a neighbour; st->single counts the entries towards survivors, st->both those towards unitigs removed
+// in the same pass t.
+template <typename Ptr>
+__device__ __forceinline__ void block_update_warps(const Ptr *__restrict__ ptr, const uint32_t *__restrict__ nb, const uint32_t *__restrict__ list,
+                                                   uint32_t n_list, uint32_t t, const uint32_t *__restrict__ pass, int32_t *__restrict__ deg_s,
+                                                   BlockPass *__restrict__ st) {
+    const uint32_t warp = (blockIdx.x * blockDim.x + threadIdx.x) >> 5, n_warps = (gridDim.x * blockDim.x) >> 5, lane = lane_id();
+    unsigned long long single = 0, both = 0;
+    for (uint32_t k = warp; k < n_list; k += n_warps) {
+        const uint32_t i = list[k];
+        const uint64_t lo = ptr[i], hi = ptr[i + 1];
+        for (uint64_t e = lo + lane; e < hi; e += 32) {
+            const uint32_t j = nb[e];
+            const uint32_t pj = pass[j];
+            if (pj == kBlockUnset) { atomicSub(&deg_s[j], 1); ++single; }
+            else if (pj == t) ++both;
+        }
+    }
+    single = warp_reduce_add(single);
+    both = warp_reduce_add(both);
+    if (lane == 0) {
+        if (single) atomicAdd(&st->single, single);
+        if (both) atomicAdd(&st->both, both);
+    }
+}
+#endif
+
 void graph_release(kombgpu_graph *g);
 void truss_release(kombgpu_graph *g);   // truss.cu
 void format_release(kombgpu_graph *g);  // format.cu

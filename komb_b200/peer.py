@@ -158,6 +158,23 @@ class DistGraph:
         self._ctx._check(self._lib.kombgpu_dist_densest_core(self._h, byref(k), byref(nv), byref(ne), byref(d)))
         return {"k": k.value, "n_vertices": nv.value, "n_edges": ne.value, "density": d.value}
 
+    def densest_block(self, weight=None, use_scores: bool = False, eps: float = 0.5) -> dict:
+        """Densest block of the whole graph by the bulk greedy peel, the dict of Graph.densest_block on every rank
+        (kombgpu_dist_densest_block).  `weight` and the returned `member` are this rank's slice: unitigs
+        [v_lo, v_lo + n_local).  Collective."""
+        st = self.stats()
+        n = st["n_local"]
+        wt = np.ascontiguousarray(weight, dtype=np.float64) if weight is not None else None
+        if wt is not None and wt.shape != (n,):
+            raise ValueError("weight must hold one value per unitig of this rank")
+        nv, ne, ws, d, np_ = c_uint32(), c_uint64(), c_double(), c_double(), c_uint32()
+        member = np.zeros(n, np.uint8)
+        self._ctx._check(self._lib.kombgpu_dist_densest_block(self._h, c_void_p(wt.ctypes.data) if wt is not None else None,
+                                                              int(bool(use_scores)), float(eps), byref(nv), byref(ne), byref(ws),
+                                                              byref(d), byref(np_), c_void_p(member.ctypes.data)))
+        return {"n_vertices": nv.value, "n_edges": ne.value, "weight_sum": ws.value, "density": d.value, "passes": np_.value,
+                "member": member.astype(bool), "v_lo": st["v_lo"]}
+
     def results(self, out: dict | None = None) -> dict:
         """degree / coreness / score of the local unitigs [v_lo, v_lo + n_local) on the host."""
         st = self.stats()
