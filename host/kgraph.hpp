@@ -125,7 +125,8 @@ class Kgraph {
     kombgpu_ctx *_ctx = nullptr;
     kombgpu_graph *_graph = nullptr;
     kombgpu_hits *_hits = nullptr;       // device-resident hits when the SAM text is tokenised on the GPU
-    bool _gpu_tokenise = true;           // KOMB_TOKENIZE=host keeps the host tokeniser (always used with several GPUs)
+    bool _gpu_tokenise = true;           // one GPU: kombgpu_sam_parse (KOMB_TOKENIZE=host keeps the host tokeniser)
+    bool _dist_tokenise = false;         // several GPUs: kombgpu_dist_sam_parse in runMulti (the same switch)
     bool _device_output = true;          // KOMB_OUTPUT=host formats the three files on the host (always without device hits)
     std::unique_ptr<PinnedArray<char>> _text[3];   // the files' bytes, formatted on the device
     uint64_t _text_bytes[3] = {0, 0, 0};
@@ -145,8 +146,11 @@ class Kgraph {
         std::vector<uint32_t> v;
         std::vector<int32_t> deg, core;
         std::vector<double> score;
+        std::vector<std::string> names;   // unitig names of [v_lo, v_lo + n_local) (partitioned SAM parse)
+        uint32_t n_unitigs = 0;
         int rc = KOMBGPU_OK;
         std::string err;
+        bool bad_input = false;           // malformed SAM: err is the parse's message, the same on every rank
     };
     std::vector<int> _devices;
     std::vector<RankOut> _ranks;
@@ -174,7 +178,9 @@ class Kgraph {
     Kgraph(uint32_t threads, uint64_t readlength, int device, int key_mode, std::vector<int> devices = {})
         : _threads(threads ? threads : 1), _readlength(readlength), _key_mode(key_mode), _device(device), _devices(std::move(devices)) {
         const char *tok_env = getenv("KOMB_TOKENIZE");
-        _gpu_tokenise = !multi() && !(tok_env && strcmp(tok_env, "host") == 0);
+        const bool host_tok = tok_env && strcmp(tok_env, "host") == 0;
+        _gpu_tokenise = !multi() && !host_tok;
+        _dist_tokenise = multi() && !host_tok;
         const char *out_env = getenv("KOMB_OUTPUT");
         _device_output = _gpu_tokenise && !(out_env && strcmp(out_env, "host") == 0);
         if (multi()) { timing_mark("start"); return; }   // every rank's thread creates its own context (runMulti)
@@ -212,7 +218,7 @@ class Kgraph {
     // Tokenise one SAM file; the mapped file must outlive `hits` (spans point into it).
     void readSAM(const std::string &samfile, MappedFile &file, HitTable &hits, bool /*fulgor: ignored like the reference*/) {
         if (!file.open(samfile)) fileNotFoundError(samfile);
-        if (_gpu_tokenise) { _sam_files.push_back(&file); return; }   // the bytes go to the device as they are (getEdgeInfo)
+        if (_gpu_tokenise || _dist_tokenise) { _sam_files.push_back(&file); return; }   // the bytes go to the device as they are
         try {
             tokenise_sam(file, (int)_threads, hits.tokens, samfile);
         } catch (const std::exception &e) {
@@ -226,6 +232,7 @@ class Kgraph {
     // mates' unitig sets per read (reference getEdgeInfo) needs no host work: equal keys get equal ids.
     void getEdgeInfo(HitTable &hits) {
         if (_gpu_tokenise) { tokeniseOnDevice(hits); return; }
+        if (_dist_tokenise) { timing_mark("map SAMs"); return; }   // every rank parses its slice of the text in runMulti
         timing_mark("tokenise SAMs");
         const size_t h = hits.tokens.keys.size();
         // ordered: ids follow first appearance, so the two mate files arrive as (at most) two runs of non-decreasing
@@ -290,14 +297,19 @@ class Kgraph {
         timing_mark("unitig names to the host");
     }
 
-    // The whole device phase over several GPUs: hits split by read range (a read's hits stay together), one host
-    // thread per rank; the ranks talk through peer memory inside libkombgpu (include/kombgpu.h, peer-memory path).
+    // The whole device phase over several GPUs, one host thread per rank; the ranks talk through peer memory inside
+    // libkombgpu (include/kombgpu.h, peer-memory path).  By default every rank parses its slice of the mapped SAM
+    // files and ends up with the hits of its own reads (kombgpu_dist_sam_parse); with KOMB_TOKENIZE=host the host's
+    // hits are split by read range (a read's hits stay together) and uploaded.
     void runMulti(HitTable &hits) {
         const int world = (int)_devices.size();
-        const uint32_t n = (uint32_t)hits.names.size();
+        uint32_t n = (uint32_t)hits.names.size();
         const size_t h = hits.read_key.size();
         uint32_t n_reads = 0;
         for (size_t i = 0; i < h; ++i) n_reads = std::max(n_reads, hits.read_key[i] + 1);
+        std::vector<const char *> texts;
+        std::vector<uint64_t> sizes;
+        for (const MappedFile *f : _sam_files) { texts.push_back(f->data); sizes.push_back(f->size); }
         _ranks.assign(world, RankOut());
         void *group_slot = nullptr;
         // phase 1: the contexts (seconds each on a cold driver, so in parallel); nobody enters a collective before all exist
@@ -337,7 +349,37 @@ class Kgraph {
                 };
                 int rc = kombgpu_comm_create_local(ctx, r, world, &group_slot, 0, &comm);
                 if (rc != KOMBGPU_OK) fail(rc, "kombgpu_comm_create_local");
-                if (rc == KOMBGPU_OK) {
+                if (rc == KOMBGPU_OK && _dist_tokenise) {
+                    kombgpu_dist_hits *dh = nullptr;
+                    rc = kombgpu_dist_sam_parse(comm, texts.data(), sizes.data(), (int)texts.size(), &dh);
+                    if (rc == KOMBGPU_EINVAL) { o.rc = rc; o.err = kombgpu_last_error(ctx); o.bad_input = true; }
+                    else if (rc != KOMBGPU_OK) fail(rc, "kombgpu_dist_sam_parse");
+                    if (rc == KOMBGPU_OK) {
+                        // the names of this rank's unitigs, as spans of the mapped files (kcore.tsv, the FASTA join)
+                        kombgpu_dist_hits_counts(dh, nullptr, nullptr, nullptr, &o.n_unitigs, nullptr);
+                        const uint64_t step = o.n_unitigs ? ((uint64_t)o.n_unitigs + world - 1) / world : 1;
+                        const uint64_t n_lo = std::min<uint64_t>(o.n_unitigs, step * r);
+                        const size_t nl = (size_t)(std::min<uint64_t>(o.n_unitigs, n_lo + step) - n_lo);
+                        std::vector<uint32_t> file(nl), len(nl);
+                        std::vector<uint64_t> off(nl);
+                        rc = kombgpu_dist_hits_names(dh, file.data(), off.data(), len.data());
+                        if (rc != KOMBGPU_OK) fail(rc, "kombgpu_dist_hits_names");
+                        o.names.resize(nl);
+                        for (size_t i = 0; rc == KOMBGPU_OK && i < nl; ++i) o.names[i].assign(texts[file[i]] + off[i], len[i]);
+                        if (r == 0 && getenv("KOMB_TIMING")) {
+                            float up = 0.f, parse = 0.f, intern = 0.f, route = 0.f;
+                            kombgpu_dist_hits_timing(dh, &up, &parse, &intern, &route, nullptr);
+                            fprintf(stderr, "[komb2 timing]   rank 0 partitioned tokeniser: upload %.3f ms, parse %.3f ms, intern %.3f ms, "
+                                    "route %.3f ms\n", up, parse, intern, route);
+                        }
+                    }
+                    // every rank reaches the build, which is collective: a rank whose names failed reports it there
+                    if (dh) {
+                        const int brc = kombgpu_dist_build_graph_hits(dh, &g);
+                        if (rc == KOMBGPU_OK && brc != KOMBGPU_OK) fail(rc = brc, "kombgpu_dist_build_graph_hits");
+                        kombgpu_dist_hits_destroy(dh);
+                    }
+                } else if (rc == KOMBGPU_OK) {
                     // this rank's reads: ids [lo, hi)
                     const uint32_t lo = (uint32_t)((uint64_t)n_reads * r / world), hi = (uint32_t)((uint64_t)n_reads * (r + 1) / world);
                     std::vector<uint32_t> rk, ut;
@@ -368,12 +410,23 @@ class Kgraph {
             });
         for (auto &t : th) t.join();
         if (keep_ctx) _ctx = ctxs[0];
+        if (_ranks[0].bad_input) {   // malformed SAM: the tokeniser's message (every rank has the same) and exit code
+            std::cerr << _ranks[0].err << std::endl;
+            exit(EXIT_FAILURE);
+        }
         for (int r = 0; r < world; ++r)
             if (_ranks[r].rc != KOMBGPU_OK) {
                 std::cerr << "komb2: rank " << r << " (device " << _devices[r] << "): " << _ranks[r].err << " (" << _ranks[r].rc << ")" << std::endl;
                 exit(EXIT_FAILURE);
             }
-        timing_mark("multi-GPU build + peel + CORE-A + results");
+        if (_dist_tokenise) {   // the ranks' name ranges, in rank order, are the names of vertices 0, 1, ...
+            n = _ranks[0].n_unitigs;
+            hits.names.clear();
+            hits.names.reserve(n);
+            for (RankOut &o : _ranks)
+                for (std::string &s : o.names) hits.names.push_back(std::move(s));
+        }
+        timing_mark(_dist_tokenise ? "multi-GPU SAM parse + build + peel + CORE-A + results" : "multi-GPU build + peel + CORE-A + results");
     }
 
     void generateGraph(HitTable &hits) {

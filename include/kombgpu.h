@@ -564,6 +564,40 @@ int kombgpu_dist_densest_block(kombgpu_dist_graph *g, const double *weight, int 
                                uint32_t *n_vertices, uint64_t *n_edges, double *weight_sum, double *density,
                                uint32_t *n_passes, uint8_t *member);
 
+/* SAM text -> hits over the ranks (kombgpu_sam_parse's token rules, unitig numbering and error messages).  Rank q
+ * uploads and parses only the lines that START in bytes [cut_q, cut_{q+1}) of every input, cut_q = the first line
+ * start at or after floor(size * q / world) (a line is never split; a slice may be empty).  Every string goes to the
+ * rank picked by a fixed-seed hash of its bytes, which interns it by its BYTES (a 64-bit collision rebuilds the table
+ * with another seed).  The unitig ids are those of kombgpu_sam_parse on the same inputs: names in order of their
+ * first occurrence, every @SQ record before every hit, each group in (input, byte offset) order, names with at least
+ * one hit only.  Read ids are unique over the ranks but do NOT follow first appearance: rank q's keys take ids
+ * [q * stride, q * stride + n), and all hits of a read, from both mates, end up on that rank (what
+ * kombgpu_dist_build_hits_dev needs).  A malformed line anywhere gives KOMBGPU_EINVAL on every rank with the message
+ * kombgpu_sam_parse gives (the earliest malformed line in (input, line) order); any other failure on one rank makes
+ * every rank return an error.  Limits: fewer than 2^30 lines in a rank's slices, 2^32 routed hits per rank, 2^32 - 1
+ * distinct names and keys per rank that interns them, and read ids below 2^32 (KOMBGPU_EINVAL otherwise).  The contexts
+ * and the communicator stay usable after an error. */
+typedef struct kombgpu_dist_hits kombgpu_dist_hits;
+/* Collective.  Every rank passes the same inputs (mate 1 first).  Within one process the pointers may be shared.
+ * Between processes, each process maps the files itself. */
+int kombgpu_dist_sam_parse(kombgpu_comm *comm, const char *const *texts, const uint64_t *sizes, int n_files,
+                           kombgpu_dist_hits **out);
+void kombgpu_dist_hits_destroy(kombgpu_dist_hits *h);
+/* this rank's hits after routing; global hits, reads, unitigs (= vertices), terminated lines; any pointer may be NULL */
+int kombgpu_dist_hits_counts(const kombgpu_dist_hits *h, uint64_t *n_hits_local, uint64_t *n_hits_global,
+                             uint32_t *n_reads_global, uint32_t *n_unitigs, uint64_t *n_lines_global);
+/* Names of the vertices [v_lo, v_lo + n_local) of the unitig-range partition (step = ceil(n / world), the same
+ * partition as kombgpu_dist_graph), as (input, offset inside that input, length); file may be NULL. */
+int kombgpu_dist_hits_names(const kombgpu_dist_hits *h, uint32_t *file, uint64_t *offset, uint32_t *len);
+/* this rank's routed hits to the host, n_hits_local each; either pointer may be NULL */
+int kombgpu_dist_hits_download(const kombgpu_dist_hits *h, uint32_t *read_key, uint32_t *unitig);
+int kombgpu_dist_hits_device_arrays(const kombgpu_dist_hits *h, const uint32_t **read_key_dev, const uint32_t **unitig_dev);
+/* CUDA-event times of the upload, the parse, the interning and the routing on this rank, and the hash seeds tried */
+int kombgpu_dist_hits_timing(const kombgpu_dist_hits *h, float *ms_upload, float *ms_parse, float *ms_intern,
+                             float *ms_route, int *hash_rounds);
+/* kombgpu_dist_build_hits_dev on the rank's routed hits, with n_vertices_global = n_unitigs.  Collective. */
+int kombgpu_dist_build_graph_hits(const kombgpu_dist_hits *h, kombgpu_dist_graph **out);
+
 int kombgpu_abi_version(void);
 
 #ifdef __cplusplus

@@ -167,6 +167,15 @@ SIGNATURES = {
     "kombgpu_dist_densest_core": (c_int, [c_void_p, POINTER(c_int32), POINTER(c_uint32), POINTER(c_uint64), POINTER(c_double)]),
     "kombgpu_dist_densest_block": (c_int, [c_void_p, c_void_p, c_int, c_double, POINTER(c_uint32), POINTER(c_uint64), POINTER(c_double),
                                            POINTER(c_double), POINTER(c_uint32), c_void_p]),
+    "kombgpu_dist_sam_parse": (c_int, [c_void_p, POINTER(c_char_p), POINTER(c_uint64), c_int, POINTER(c_void_p)]),
+    "kombgpu_dist_hits_destroy": (None, [c_void_p]),
+    "kombgpu_dist_hits_counts": (c_int, [c_void_p, POINTER(c_uint64), POINTER(c_uint64), POINTER(c_uint32), POINTER(c_uint32),
+                                         POINTER(c_uint64)]),
+    "kombgpu_dist_hits_names": (c_int, [c_void_p, c_void_p, c_void_p, c_void_p]),
+    "kombgpu_dist_hits_download": (c_int, [c_void_p, c_void_p, c_void_p]),
+    "kombgpu_dist_hits_device_arrays": (c_int, [c_void_p, POINTER(c_void_p), POINTER(c_void_p)]),
+    "kombgpu_dist_hits_timing": (c_int, [c_void_p, POINTER(c_float), POINTER(c_float), POINTER(c_float), POINTER(c_float), POINTER(c_int)]),
+    "kombgpu_dist_build_graph_hits": (c_int, [c_void_p, POINTER(c_void_p)]),
 }
 
 _lib = None

@@ -102,6 +102,13 @@ class DistGraph:
         return cls._build(comm._lib.kombgpu_dist_build_hits_dev, comm, read_key, unitig, n_global)
 
     @classmethod
+    def from_dist_hits(cls, hits: "DistHits") -> "DistGraph":
+        """The graph of the hits a DistHits routed to this rank, n_global = its n_unitigs.  Collective."""
+        h = c_void_p()
+        hits.comm.ctx._check(hits._lib.kombgpu_dist_build_graph_hits(hits._h, byref(h)))
+        return cls(hits.comm, h, keep=hits)
+
+    @classmethod
     def from_pairs(cls, comm: Comm, u, v, n_global: int) -> "DistGraph":
         """This rank's share of an edge list.  Collective."""
         return cls._build(comm._lib.kombgpu_dist_build_pairs_dev, comm, u, v, n_global)
@@ -218,6 +225,72 @@ class DistGraph:
     def close(self):
         if getattr(self, "_h", None):
             self._lib.kombgpu_dist_graph_destroy(self._h)
+            self._h = None
+
+    def __enter__(self):
+        return self
+
+    def __exit__(self, *exc):
+        self.close()
+
+
+class DistHits:
+    """kombgpu_dist_hits: SAM text parsed and interned over the ranks.  This rank holds the hits of its own reads
+    (global unitig ids, read ids unique over the ranks) and the names of the unitigs it owns."""
+
+    def __init__(self, comm: Comm, handle: c_void_p, texts):
+        self.comm = comm
+        self._ctx = comm.ctx
+        self._lib = comm._lib
+        self._h = handle
+        self._texts = texts
+
+    @classmethod
+    def parse(cls, comm: Comm, texts) -> "DistHits":
+        """SAM bytes of the mate files (mate 1 first), the same on every rank (kombgpu_dist_sam_parse).  Collective."""
+        texts = [bytes(t) for t in texts]
+        n = len(texts)
+        arr = (ctypes.c_char_p * max(n, 1))(*texts)
+        sizes = (c_uint64 * max(n, 1))(*[len(t) for t in texts])
+        h = c_void_p()
+        comm.ctx._check(comm._lib.kombgpu_dist_sam_parse(comm._h, arr, sizes, n, byref(h)))
+        return cls(comm, h, texts)
+
+    def counts(self) -> dict:
+        hl, hg, nr, nu, nl = c_uint64(), c_uint64(), c_uint32(), c_uint32(), c_uint64()
+        self._ctx._check(self._lib.kombgpu_dist_hits_counts(self._h, byref(hl), byref(hg), byref(nr), byref(nu), byref(nl)))
+        return {"n_hits_local": hl.value, "n_hits": hg.value, "n_reads": nr.value, "n_unitigs": nu.value, "n_lines": nl.value}
+
+    def local_range(self) -> tuple[int, int]:
+        """(v_lo, n_local) of this rank in the unitig-range partition (step = ceil(n_unitigs / world))."""
+        n = self.counts()["n_unitigs"]
+        step = -(-n // self.comm.world) if n else 1
+        lo = min(n, self.comm.rank * step)
+        return lo, min(n, lo + step) - lo
+
+    def names(self) -> list[bytes]:
+        """Names of the unitigs this rank owns, [v_lo, v_lo + n_local), cut out of the input bytes."""
+        _, n = self.local_range()
+        f, off, ln = np.empty(n, np.uint32), np.empty(n, np.uint64), np.empty(n, np.uint32)
+        self._ctx._check(self._lib.kombgpu_dist_hits_names(self._h, c_void_p(f.ctypes.data), c_void_p(off.ctypes.data),
+                                                           c_void_p(ln.ctypes.data)))
+        return [self._texts[int(f[i])][int(off[i]):int(off[i]) + int(ln[i])] for i in range(n)]
+
+    def hits(self) -> tuple[np.ndarray, np.ndarray]:
+        """This rank's routed hits (read id, unitig id) on the host."""
+        n = self.counts()["n_hits_local"]
+        rk, ut = np.empty(n, np.uint32), np.empty(n, np.uint32)
+        self._ctx._check(self._lib.kombgpu_dist_hits_download(self._h, c_void_p(rk.ctypes.data), c_void_p(ut.ctypes.data)))
+        return rk, ut
+
+    def timing(self) -> dict:
+        a, b, c, d, r = c_float(), c_float(), c_float(), c_float(), c_int()
+        self._ctx._check(self._lib.kombgpu_dist_hits_timing(self._h, byref(a), byref(b), byref(c), byref(d), byref(r)))
+        return {"ms_upload": a.value, "ms_parse": b.value, "ms_intern": c.value, "ms_route": d.value, "hash_rounds": r.value}
+
+    def close(self):
+        if getattr(self, "_h", None):
+            self._lib.kombgpu_dist_hits_destroy(self._h)
             self._h = None
 
     def __enter__(self):
