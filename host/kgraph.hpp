@@ -127,7 +127,8 @@ class Kgraph {
     kombgpu_hits *_hits = nullptr;       // device-resident hits when the SAM text is tokenised on the GPU
     bool _gpu_tokenise = true;           // one GPU: kombgpu_sam_parse (KOMB_TOKENIZE=host keeps the host tokeniser)
     bool _dist_tokenise = false;         // several GPUs: kombgpu_dist_sam_parse in runMulti (the same switch)
-    bool _device_output = true;          // KOMB_OUTPUT=host formats the three files on the host (always without device hits)
+    bool _device_output = true;          // KOMB_OUTPUT=host formats the three files on the host (always without device hits:
+                                         // KOMB_TOKENIZE=host)
     std::unique_ptr<PinnedArray<char>> _text[3];   // the files' bytes, formatted on the device
     uint64_t _text_bytes[3] = {0, 0, 0};
     std::vector<const MappedFile *> _sam_files;
@@ -146,18 +147,27 @@ class Kgraph {
         std::vector<uint32_t> v;
         std::vector<int32_t> deg, core;
         std::vector<double> score;
-        std::vector<std::string> names;   // unitig names of [v_lo, v_lo + n_local) (partitioned SAM parse)
+        std::vector<std::string> names;   // unitig names of [v_lo, v_lo + n_local) (partitioned SAM parse, host output or FASTA)
         uint32_t n_unitigs = 0;
+        std::unique_ptr<PinnedArray<char>> text[3];   // the rank's slices of the three files, formatted on its device
+        uint64_t text_bytes[3] = {0, 0, 0};
         int rc = KOMBGPU_OK;
         std::string err;
         bool bad_input = false;           // malformed SAM: err is the parse's message, the same on every rank
     };
     std::vector<int> _devices;
-    std::vector<RankOut> _ranks;
+    std::vector<RankOut> _ranks;         // holds page-locked text of the rank contexts: cleared before they are destroyed
+    std::vector<kombgpu_ctx *> _rank_ctxs;   // one per rank, alive until the files are written (rank 0's is _ctx)
     uint64_t _m_multi = 0;
     int32_t _max_core_multi = 0;
     double _max_score_multi = 0.0;
     bool multi() const { return _devices.size() > 1; }
+    void releaseRanks() {
+        _ranks.clear();
+        for (kombgpu_ctx *c : _rank_ctxs) kombgpu_ctx_destroy(c);
+        if (!_rank_ctxs.empty()) _ctx = nullptr;
+        _rank_ctxs.clear();
+    }
     std::unique_ptr<PinnedArray<int32_t>> _deg, _core;
     std::unique_ptr<PinnedArray<double>> _score;
     bool _fasta_anomalous = false, _fasta_truss = false;   // KOMB_UNITIG_FASTA
@@ -182,7 +192,7 @@ class Kgraph {
         _gpu_tokenise = !multi() && !host_tok;
         _dist_tokenise = multi() && !host_tok;
         const char *out_env = getenv("KOMB_OUTPUT");
-        _device_output = _gpu_tokenise && !(out_env && strcmp(out_env, "host") == 0);
+        _device_output = (_gpu_tokenise || _dist_tokenise) && !(out_env && strcmp(out_env, "host") == 0);
         if (multi()) { timing_mark("start"); return; }   // every rank's thread creates its own context (runMulti)
         // Creating the CUDA context costs seconds on a box without the persistence daemon (1.9 - 4.1 s measured on
         // the B200 boxes, against 0.75 s for everything else on a 2.5 M-hit SAM pair): do it on a helper thread
@@ -199,6 +209,7 @@ class Kgraph {
         if (_ctx_ready.valid()) _ctx_ready.wait();
         _efp.reset(); _ev.reset(); _deg.reset(); _core.reset(); _score.reset();  // pinned buffers go before the context
         for (auto &t : _text) t.reset();
+        releaseRanks();
         if (_graph) kombgpu_graph_destroy(_graph);
         if (_hits) kombgpu_hits_destroy(_hits);
         if (_ctx) kombgpu_ctx_destroy(_ctx);
@@ -300,7 +311,9 @@ class Kgraph {
     // The whole device phase over several GPUs, one host thread per rank; the ranks talk through peer memory inside
     // libkombgpu (include/kombgpu.h, peer-memory path).  By default every rank parses its slice of the mapped SAM
     // files and ends up with the hits of its own reads (kombgpu_dist_sam_parse); with KOMB_TOKENIZE=host the host's
-    // hits are split by read range (a read's hits stay together) and uploaded.
+    // hits are split by read range (a read's hits stay together) and uploaded.  By default every rank also formats
+    // its slices of the three files (kombgpu_dist_graph_format) into page-locked memory of its own context; the
+    // edge-list download runs under the peel and CORE-A.  The contexts live until the files are written.
     void runMulti(HitTable &hits) {
         const int world = (int)_devices.size();
         uint32_t n = (uint32_t)hits.names.size();
@@ -310,7 +323,8 @@ class Kgraph {
         std::vector<const char *> texts;
         std::vector<uint64_t> sizes;
         for (const MappedFile *f : _sam_files) { texts.push_back(f->data); sizes.push_back(f->size); }
-        _ranks.assign(world, RankOut());
+        _ranks.clear();
+        _ranks.resize(world);
         void *group_slot = nullptr;
         // phase 1: the contexts (seconds each on a cold driver, so in parallel); nobody enters a collective before all exist
         std::vector<kombgpu_ctx *> ctxs(world, nullptr);
@@ -334,7 +348,8 @@ class Kgraph {
             }
         }
         timing_mark("kombgpu_ctx_create (all devices)");
-        const bool keep_ctx = _fasta_anomalous;   // the unitig FASTA work runs on rank 0's device after the ranks are done
+        const bool device_output = _device_output;
+        const bool want_names = !device_output || _fasta_anomalous;   // the host writes kcore.tsv, or joins the unitig FASTA
         std::vector<std::thread> th;
         for (int r = 0; r < world; ++r)
             th.emplace_back([&, r]() {
@@ -342,42 +357,50 @@ class Kgraph {
                 kombgpu_ctx *ctx = ctxs[r];
                 kombgpu_comm *comm = nullptr;
                 kombgpu_dist_graph *g = nullptr;
+                kombgpu_dist_hits *dh = nullptr;   // kept until kcore.tsv is formatted: the names' bytes live in it
                 auto fail = [&](int rc, const char *what) {
                     o.rc = rc;
                     o.err = std::string(what) + ": " + kombgpu_last_error(ctx);
                     if (comm) kombgpu_comm_abort(comm);
                 };
+                // this rank's slice of one file: formatted, then downloaded on the copy stream (local, not collective)
+                auto format = [&](int which) {
+                    int frc = kombgpu_dist_graph_format(g, which, dh, &o.text_bytes[which]);
+                    if (frc != KOMBGPU_OK) { fail(frc, "kombgpu_dist_graph_format"); return frc; }
+                    o.text[which].reset(new PinnedArray<char>(ctx, o.text_bytes[which]));
+                    frc = kombgpu_dist_graph_format_fetch(g, which, o.text[which]->data(), 1);
+                    if (frc != KOMBGPU_OK) fail(frc, "kombgpu_dist_graph_format_fetch");
+                    return frc;
+                };
                 int rc = kombgpu_comm_create_local(ctx, r, world, &group_slot, 0, &comm);
                 if (rc != KOMBGPU_OK) fail(rc, "kombgpu_comm_create_local");
                 if (rc == KOMBGPU_OK && _dist_tokenise) {
-                    kombgpu_dist_hits *dh = nullptr;
                     rc = kombgpu_dist_sam_parse(comm, texts.data(), sizes.data(), (int)texts.size(), &dh);
                     if (rc == KOMBGPU_EINVAL) { o.rc = rc; o.err = kombgpu_last_error(ctx); o.bad_input = true; }
                     else if (rc != KOMBGPU_OK) fail(rc, "kombgpu_dist_sam_parse");
-                    if (rc == KOMBGPU_OK) {
+                    if (rc == KOMBGPU_OK) kombgpu_dist_hits_counts(dh, nullptr, nullptr, nullptr, &o.n_unitigs, nullptr);
+                    if (rc == KOMBGPU_OK && want_names) {
                         // the names of this rank's unitigs, as spans of the mapped files (kcore.tsv, the FASTA join)
-                        kombgpu_dist_hits_counts(dh, nullptr, nullptr, nullptr, &o.n_unitigs, nullptr);
                         const uint64_t step = o.n_unitigs ? ((uint64_t)o.n_unitigs + world - 1) / world : 1;
                         const uint64_t n_lo = std::min<uint64_t>(o.n_unitigs, step * r);
                         const size_t nl = (size_t)(std::min<uint64_t>(o.n_unitigs, n_lo + step) - n_lo);
                         std::vector<uint32_t> file(nl), len(nl);
                         std::vector<uint64_t> off(nl);
-                        rc = kombgpu_dist_hits_names(dh, file.data(), off.data(), len.data());
+                        if (nl) rc = kombgpu_dist_hits_names(dh, file.data(), off.data(), len.data());   // a rank may own no unitig
                         if (rc != KOMBGPU_OK) fail(rc, "kombgpu_dist_hits_names");
                         o.names.resize(nl);
                         for (size_t i = 0; rc == KOMBGPU_OK && i < nl; ++i) o.names[i].assign(texts[file[i]] + off[i], len[i]);
-                        if (r == 0 && getenv("KOMB_TIMING")) {
-                            float up = 0.f, parse = 0.f, intern = 0.f, route = 0.f;
-                            kombgpu_dist_hits_timing(dh, &up, &parse, &intern, &route, nullptr);
-                            fprintf(stderr, "[komb2 timing]   rank 0 partitioned tokeniser: upload %.3f ms, parse %.3f ms, intern %.3f ms, "
-                                    "route %.3f ms\n", up, parse, intern, route);
-                        }
+                    }
+                    if (rc == KOMBGPU_OK && r == 0 && getenv("KOMB_TIMING")) {
+                        float up = 0.f, parse = 0.f, intern = 0.f, route = 0.f;
+                        kombgpu_dist_hits_timing(dh, &up, &parse, &intern, &route, nullptr);
+                        fprintf(stderr, "[komb2 timing]   rank 0 partitioned tokeniser: upload %.3f ms, parse %.3f ms, intern %.3f ms, "
+                                "route %.3f ms\n", up, parse, intern, route);
                     }
                     // every rank reaches the build, which is collective: a rank whose names failed reports it there
                     if (dh) {
                         const int brc = kombgpu_dist_build_graph_hits(dh, &g);
                         if (rc == KOMBGPU_OK && brc != KOMBGPU_OK) fail(rc = brc, "kombgpu_dist_build_graph_hits");
-                        kombgpu_dist_hits_destroy(dh);
                     }
                 } else if (rc == KOMBGPU_OK) {
                     // this rank's reads: ids [lo, hi)
@@ -388,28 +411,44 @@ class Kgraph {
                     rc = kombgpu_dist_build_hits(comm, rk.data(), ut.data(), rk.size(), n, &g);
                     if (rc != KOMBGPU_OK) fail(rc, "kombgpu_dist_build_hits");
                 }
+                if (rc == KOMBGPU_OK && device_output) rc = format(KOMBGPU_FILE_EDGELIST);   // downloads under the peel and CORE-A
                 if (rc == KOMBGPU_OK && (rc = kombgpu_dist_coreness(g)) != KOMBGPU_OK) fail(rc, "kombgpu_dist_coreness");
                 if (rc == KOMBGPU_OK && (rc = kombgpu_dist_corea(g, _key_mode)) != KOMBGPU_OK) fail(rc, "kombgpu_dist_corea");
                 if (rc == KOMBGPU_OK) {
                     kombgpu_dist_stats st;
                     kombgpu_dist_graph_stats(g, &st);
                     o.v_lo = st.v_lo; o.n_local = st.n_local; o.n_fwd = st.n_fwd_local;
-                    o.fwd_ptr.resize((size_t)o.n_local + 1); o.v.resize(o.n_fwd);
-                    o.deg.resize(o.n_local); o.core.resize(o.n_local); o.score.resize(o.n_local);
-                    rc = kombgpu_dist_graph_results(g, o.deg.data(), o.core.data(), o.score.data());
-                    if (rc == KOMBGPU_OK) rc = kombgpu_dist_graph_edges_csr(g, o.fwd_ptr.data(), o.v.data());
-                    if (rc != KOMBGPU_OK) fail(rc, "kombgpu_dist_graph_results");
+                    if (device_output) {
+                        rc = format(KOMBGPU_FILE_KCORE);
+                        if (rc == KOMBGPU_OK) rc = format(KOMBGPU_FILE_COREA);
+                        if (rc == KOMBGPU_OK && _fasta_anomalous) {   // the anomalous unitigs are picked on the host from every score
+                            o.score.resize(o.n_local);
+                            if ((rc = kombgpu_dist_graph_results(g, nullptr, nullptr, o.score.data())) != KOMBGPU_OK) fail(rc, "kombgpu_dist_graph_results");
+                        }
+                    } else {
+                        o.fwd_ptr.resize((size_t)o.n_local + 1); o.v.resize(o.n_fwd);
+                        o.deg.resize(o.n_local); o.core.resize(o.n_local); o.score.resize(o.n_local);
+                        rc = kombgpu_dist_graph_results(g, o.deg.data(), o.core.data(), o.score.data());
+                        if (rc == KOMBGPU_OK) rc = kombgpu_dist_graph_edges_csr(g, o.fwd_ptr.data(), o.v.data());
+                        if (rc != KOMBGPU_OK) fail(rc, "kombgpu_dist_graph_results");
+                    }
                     if (r == 0) {
                         _m_multi = st.n_edges_global;
                         kombgpu_dist_graph_summary(g, &_max_core_multi, &_max_score_multi);
                     }
                 }
-                if (g) kombgpu_dist_graph_destroy(g);
+                if (dh) kombgpu_dist_hits_destroy(dh);
+                if (g) {
+                    // the downloads into the page-locked slices end before the graph's text goes
+                    const int wrc = device_output ? kombgpu_dist_graph_format_wait(g) : KOMBGPU_OK;
+                    if (rc == KOMBGPU_OK && wrc != KOMBGPU_OK) fail(rc = wrc, "kombgpu_dist_graph_format_wait");
+                    kombgpu_dist_graph_destroy(g);
+                }
                 if (comm) kombgpu_comm_destroy(comm);
-                if (ctx && !(r == 0 && keep_ctx)) kombgpu_ctx_destroy(ctx);
             });
         for (auto &t : th) t.join();
-        if (keep_ctx) _ctx = ctxs[0];
+        _rank_ctxs = ctxs;   // destroyed with the ranks' page-locked text, after the three files are written
+        _ctx = ctxs[0];      // the unitig FASTA work runs on rank 0's device after the ranks are done
         if (_ranks[0].bad_input) {   // malformed SAM: the tokeniser's message (every rank has the same) and exit code
             std::cerr << _ranks[0].err << std::endl;
             exit(EXIT_FAILURE);
@@ -426,7 +465,9 @@ class Kgraph {
             for (RankOut &o : _ranks)
                 for (std::string &s : o.names) hits.names.push_back(std::move(s));
         }
-        timing_mark(_dist_tokenise ? "multi-GPU SAM parse + build + peel + CORE-A + results" : "multi-GPU build + peel + CORE-A + results");
+        timing_mark(!_dist_tokenise ? "multi-GPU build + peel + CORE-A + results"
+                    : device_output ? "multi-GPU SAM parse + build + peel + CORE-A + format + download"
+                                    : "multi-GPU SAM parse + build + peel + CORE-A + results");
     }
 
     void generateGraph(HitTable &hits) {
@@ -448,9 +489,14 @@ class Kgraph {
         uint64_t m = 0;
         if (multi()) {
             // the ranks' slices of the canonical edge list, in rank order, ARE the sorted list
-            n = (uint32_t)hits.names.size();
+            for (const RankOut &o : _ranks) n += o.n_local;
             m = _m_multi;
-            for (const RankOut &o : _ranks) {
+            for (RankOut &o : _ranks) {
+                if (_device_output) {   // the slice's text, formatted on the rank's device
+                    if (o.text_bytes[0] && fwrite(o.text[0]->data(), 1, o.text_bytes[0], ef) != o.text_bytes[0]) fileNotFoundError(edgelist_file);
+                    o.text[0].reset();
+                    continue;
+                }
                 const uint64_t *fp = o.fwd_ptr.data();
                 write_row_blocks(ef, o.n_fwd, 24, (int)_threads, [&](char *p, size_t lo, size_t hi) {
                     size_t x = (size_t)(std::upper_bound(fp, fp + o.n_local + 1, (uint64_t)lo) - fp) - 1;
@@ -550,12 +596,19 @@ class Kgraph {
     void runCore(const std::string &dir, HitTable &hits) {
         const std::string kcore_file = dir + "/kcore.tsv";
         const uint32_t n = (uint32_t)hits.names.size();
-        if (_device_output && !multi()) {
+        if (_device_output) {
             FILE *kf = fopen(kcore_file.c_str(), "w+");
             if (kf == nullptr) fileNotFoundError(kcore_file);
-            if (fwrite(_text[1]->data(), 1, _text_bytes[1], kf) != _text_bytes[1]) fileNotFoundError(kcore_file);
+            if (multi()) {   // rank 0's slice starts with the header
+                for (RankOut &o : _ranks) {
+                    if (o.text_bytes[1] && fwrite(o.text[1]->data(), 1, o.text_bytes[1], kf) != o.text_bytes[1]) fileNotFoundError(kcore_file);
+                    o.text[1].reset();
+                }
+            } else {
+                if (fwrite(_text[1]->data(), 1, _text_bytes[1], kf) != _text_bytes[1]) fileNotFoundError(kcore_file);
+                _text[1].reset();
+            }
             fclose(kf);
-            _text[1].reset();
             timing_mark("write kcore.tsv");
             return;
         }
@@ -608,7 +661,10 @@ class Kgraph {
             const std::string anomaly_output = dir + "/CoreA_anomaly.txt";
             FILE *fp = fopen(anomaly_output.c_str(), "w+");
             if (fp == nullptr) fileNotFoundError(anomaly_output);
-            if (_device_output && !multi()) {
+            if (_device_output && multi()) {
+                for (const RankOut &o : _ranks)
+                    if (o.text_bytes[2] && fwrite(o.text[2]->data(), 1, o.text_bytes[2], fp) != o.text_bytes[2]) fileNotFoundError(anomaly_output);
+            } else if (_device_output) {
                 if (_text_bytes[2] && fwrite(_text[2]->data(), 1, _text_bytes[2], fp) != _text_bytes[2]) fileNotFoundError(anomaly_output);
             } else
             write_rows(fp, n, 64, (int)_threads, [&](char *p, size_t i) {
@@ -622,7 +678,7 @@ class Kgraph {
         if (_fasta_anomalous || _fasta_truss) writeUnitigFasta(dir, fasta_path, hits, score_all);
         _efp.reset(); _ev.reset(); _deg.reset(); _core.reset(); _score.reset();
         for (auto &t : _text) t.reset();
-        _ranks.clear();
+        releaseRanks();
         if (_graph) kombgpu_graph_destroy(_graph);
         _graph = nullptr;
         timing_mark("free pinned + graph");

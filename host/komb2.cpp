@@ -11,8 +11,9 @@
 //              (default "ref32" reproduces the reference's int32 wrap, quirk Q5);
 //              KOMB_TOKENIZE=host tokenises and interns the SAM text on the host (default: on the device,
 //              kombgpu_sam_parse with one GPU, kombgpu_dist_sam_parse over the ranks with KOMB_GPU_DEVICES);
-//              KOMB_OUTPUT=host formats the three files on the host (default with one GPU and device tokenisation:
-//              on the device, kombgpu_graph_format; with several GPUs always on the host); KOMB_TIMING=1 prints wall-clock marks;
+//              KOMB_OUTPUT=host formats the three files on the host (default with device tokenisation: on the device,
+//              kombgpu_graph_format with one GPU, each rank's slice with kombgpu_dist_graph_format with KOMB_GPU_DEVICES;
+//              with KOMB_TOKENIZE=host always on the host); KOMB_TIMING=1 prints wall-clock marks;
 //              KOMB_UNITIG_FASTA=anomalous, =truss or =anomalous,truss also writes the -u FASTA's records of the
 //              anomalous unitigs (CORE-A above the IQR fence q3 + 1.5 (q3 - q1)) to <outdir>/anomalous_unitigs.fasta and
 //              of the unitigs on the max-truss edges of the maximal core to <outdir>/truss_unitigs.fasta, indexed, joined

@@ -598,6 +598,19 @@ int kombgpu_dist_hits_timing(const kombgpu_dist_hits *h, float *ms_upload, float
 /* kombgpu_dist_build_hits_dev on the rank's routed hits, with n_vertices_global = n_unitigs.  Collective. */
 int kombgpu_dist_build_graph_hits(const kombgpu_dist_hits *h, kombgpu_dist_graph **out);
 
+/* This rank's slice of the output files, formatted on its device: the slices of ranks 0, 1, ... concatenate to
+ * exactly the bytes kombgpu_graph_format gives for the same graph on one GPU.  EDGELIST: the rank's slice of the
+ * canonical edge list (needs the build); KCORE: rows v_lo .. v_lo + n_local - 1, rank 0's slice starting with the
+ * header even when the graph is empty (needs kombgpu_dist_coreness and the kombgpu_dist_hits the graph was built
+ * from: the parse leaves every name's bytes on the rank that owns its vertex); COREA: the same rows (needs
+ * kombgpu_dist_corea).  Local, NOT collective: a rank formats and fetches when it likes and waits for no other.
+ * KOMBGPU_ESTATE for a file whose stage has not run, or a fetch before the format; KOMBGPU_EINVAL for `which` out of
+ * range or a KCORE names handle that is missing or belongs to another communicator or partition.  The text is
+ * cached in the graph until it is destroyed; fetch and wait work as kombgpu_graph_format_fetch / _wait. */
+int kombgpu_dist_graph_format(kombgpu_dist_graph *g, int which, const kombgpu_dist_hits *names, uint64_t *bytes);
+int kombgpu_dist_graph_format_fetch(kombgpu_dist_graph *g, int which, char *dst, int async);
+int kombgpu_dist_graph_format_wait(kombgpu_dist_graph *g);
+
 int kombgpu_abi_version(void);
 
 #ifdef __cplusplus

@@ -176,6 +176,9 @@ SIGNATURES = {
     "kombgpu_dist_hits_device_arrays": (c_int, [c_void_p, POINTER(c_void_p), POINTER(c_void_p)]),
     "kombgpu_dist_hits_timing": (c_int, [c_void_p, POINTER(c_float), POINTER(c_float), POINTER(c_float), POINTER(c_float), POINTER(c_int)]),
     "kombgpu_dist_build_graph_hits": (c_int, [c_void_p, POINTER(c_void_p)]),
+    "kombgpu_dist_graph_format": (c_int, [c_void_p, c_int, c_void_p, POINTER(c_uint64)]),
+    "kombgpu_dist_graph_format_fetch": (c_int, [c_void_p, c_int, c_void_p, c_int]),
+    "kombgpu_dist_graph_format_wait": (c_int, [c_void_p]),
 }
 
 _lib = None

@@ -1,5 +1,5 @@
 // dgraph.cuh — one rank's share of a unitig graph partitioned by unitig-id range over the ranks of a communicator
-// (SURVEY.md section 8(e)); stage entry points of the partitioned path (pbuild.cu, ppeel.cu, pcorea.cu).
+// (SURVEY.md section 8(e)); stage entry points of the partitioned path (pbuild.cu, ppeel.cu, pcorea.cu, format.cu).
 #pragma once
 
 #include "comm.cuh"
@@ -38,6 +38,9 @@ struct kombgpu_dist_graph {
     bool has_truss = false;
     kg::MaxCoreTruss tr;
     float ms_truss[3] = {0.f, 0.f, 0.f};   // CUDA-event times: coreness gather, selection + slice gather, truss peel
+    // this rank's slices of the three output files, formatted on the device (format.cu), cached until destroy
+    char *text[3] = {nullptr, nullptr, nullptr};
+    uint64_t text_bytes[3] = {0, 0, 0};
     kombgpu_dist_stats st{};
 };
 
@@ -70,6 +73,19 @@ int dist_max_core_truss(kombgpu_dist_graph *g);
 int dist_densest_core(kombgpu_dist_graph *g, DensestCore *out);
 // weight: this rank's slice (host, or NULL); member: this rank's slice (host, n_local bytes, or NULL)
 int dist_densest_block(kombgpu_dist_graph *g, const double *weight, int use_scores, double eps, DensestBlock *out, uint8_t *member);
+
+// psam.cu: the names of the vertices [v_lo, v_lo + n_local) a kombgpu_dist_hits holds on this rank's device:
+// name i is bytes[off[i] .. off[i] + len[i])
+struct DistNames {
+    const kombgpu_comm *comm;
+    uint32_t n_unitigs, v_lo, n_local;
+    const unsigned char *bytes;
+    const uint64_t *off;
+    const uint32_t *len;
+};
+int dist_hits_name_text(const kombgpu_dist_hits *h, DistNames *out);
+// format.cu
+void dist_format_release(kombgpu_dist_graph *g);
 
 void dist_graph_release(kombgpu_dist_graph *g);
 

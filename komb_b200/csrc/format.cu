@@ -5,7 +5,7 @@
 // "%d\t%f\n" (src/CombineCoreA.h:36-39).  Here one scan computes every row's length and hands each row its offset
 // in the file; the row is formatted in place by the thread that owns it, and the host receives the bytes of the file
 // and issues one write.  "%f" is glibc's: six decimals of the EXACT binary value, ties to even.
-#include "graph.cuh"
+#include "dgraph.cuh"
 #include "primitives.cuh"
 
 struct kombgpu_hits;
@@ -108,12 +108,13 @@ struct EdgeRowOut {
     }
 };
 
-// ---- kcore.tsv (rows; the header is copied in front)
+// ---- kcore.tsv (rows; the header is copied in front).  Row i is unitig id0 + i (id0: the first unitig of a rank's slice)
 struct KcoreRowLen {
     const uint32_t *name_len;
     const int32_t *core, *deg;
+    uint32_t id0;
     __device__ uint64_t operator()(uint64_t i) const {
-        return digits_u32((uint32_t)i) + name_len[i] + digits_i32(core[i]) + digits_i32(deg[i]) + 4u;
+        return digits_u32(id0 + (uint32_t)i) + name_len[i] + digits_i32(core[i]) + digits_i32(deg[i]) + 4u;
     }
 };
 struct KcoreRowOut {
@@ -123,8 +124,10 @@ struct KcoreRowOut {
     const int32_t *core, *deg;
     char *text;
     uint64_t base;
+    uint32_t id0;
     __device__ void operator()(uint64_t i, uint64_t at, uint64_t) const {
-        char *p = put_u32(text + base + at, (uint32_t)i, digits_u32((uint32_t)i));
+        const uint32_t id = id0 + (uint32_t)i;
+        char *p = put_u32(text + base + at, id, digits_u32(id));
         *p++ = '\t';
         const unsigned char *nm = names + name_off[i];
         const uint32_t nl = name_len[i];
@@ -138,25 +141,28 @@ struct KcoreRowOut {
     }
 };
 
-// ---- CoreA_anomaly.txt
+// ---- CoreA_anomaly.txt (row i is unitig id0 + i)
 struct ScoreRowLen {
     const double *score;
     uint32_t *err;
+    uint32_t id0;
     __device__ uint64_t operator()(uint64_t i) const {
         uint64_t q = 0;
         bool neg = false;
         if (!micro_units(score[i], &q, &neg)) { atomicExch(err, 1u); q = 0; neg = false; }
-        return digits_u32((uint32_t)i) + 1u + f6_len(q, neg) + 1u;
+        return digits_u32(id0 + (uint32_t)i) + 1u + f6_len(q, neg) + 1u;
     }
 };
 struct ScoreRowOut {
     const double *score;
     char *text;
+    uint32_t id0;
     __device__ void operator()(uint64_t i, uint64_t at, uint64_t) const {
         uint64_t q = 0;
         bool neg = false;
         if (!micro_units(score[i], &q, &neg)) { q = 0; neg = false; }
-        char *p = put_u32(text + at, (uint32_t)i, digits_u32((uint32_t)i));
+        const uint32_t id = id0 + (uint32_t)i;
+        char *p = put_u32(text + at, id, digits_u32(id));
         *p++ = '\t';
         p = put_f6(p, q, neg);
         *p = '\n';
@@ -185,19 +191,26 @@ int format_rows(kombgpu_ctx *ctx, uint64_t n_rows, LenFn len, OutFn (*make_out)(
     return KOMBGPU_OK;
 }
 
-struct KcoreArgs { const unsigned char *names; const uint64_t *off; const uint32_t *len; const int32_t *core, *deg; };
+// base: bytes in front of the rows (the header, or 0 in a slice that does not start the file)
+struct KcoreArgs { const unsigned char *names; const uint64_t *off; const uint32_t *len; const int32_t *core, *deg; uint64_t base; uint32_t id0; };
 EdgeRowOut make_edge_out(char *text, void *arg) { return EdgeRowOut{static_cast<const uint64_t *>(arg), text}; }
 KcoreRowOut make_kcore_out(char *text, void *arg) {
     const KcoreArgs *a = static_cast<const KcoreArgs *>(arg);
-    return KcoreRowOut{a->names, a->off, a->len, a->core, a->deg, text, kKcoreHeaderLen};
+    return KcoreRowOut{a->names, a->off, a->len, a->core, a->deg, text, a->base, a->id0};
 }
-ScoreRowOut make_score_out(char *text, void *arg) { return ScoreRowOut{static_cast<const double *>(arg), text}; }
+struct ScoreArgs { const double *score; uint32_t id0; };
+ScoreRowOut make_score_out(char *text, void *arg) {
+    const ScoreArgs *a = static_cast<const ScoreArgs *>(arg);
+    return ScoreRowOut{a->score, text, a->id0};
+}
 
-int format_scores(kombgpu_ctx *ctx, const double *score_dev, uint32_t n, char **text, uint64_t *bytes) {
+// the rows of unitigs id0 .. id0 + n - 1
+int format_scores(kombgpu_ctx *ctx, const double *score_dev, uint32_t n, uint32_t id0, char **text, uint64_t *bytes) {
     DevBuf<uint32_t> err(ctx, 1);
     if (!err) return ctx_fail(ctx, KOMBGPU_ENOMEM, "workspace");
     KG_CUDA(ctx, cudaMemsetAsync(err.p, 0, sizeof(uint32_t), ctx->stream));
-    KG_TRY(format_rows(ctx, n, ScoreRowLen{score_dev, err.p}, make_score_out, (void *)score_dev, 0, text, bytes));
+    ScoreArgs a{score_dev, id0};
+    KG_TRY(format_rows(ctx, n, ScoreRowLen{score_dev, err.p, id0}, make_score_out, &a, 0, text, bytes));
     uint32_t h_err = 0;
     KG_TRY(read_back(ctx, err.p, &h_err, 1));
     if (h_err) {
@@ -208,15 +221,39 @@ int format_scores(kombgpu_ctx *ctx, const double *score_dev, uint32_t n, char **
     return KOMBGPU_OK;
 }
 
-}  // namespace
+// the text of file `which` to the host: async != 0 on the copy stream, behind everything the compute stream has queued
+int fetch_text(kombgpu_ctx *ctx, const char *text, uint64_t bytes, char *dst, int async) {
+    if (!dst && bytes) return ctx_fail(ctx, KOMBGPU_EINVAL, "null destination");
+    KG_CUDA(ctx, cudaSetDevice(ctx->device));
+    if (!bytes) return KOMBGPU_OK;
+    if (async) {
+        // later compute on the stream overlaps the download
+        cudaEvent_t ev = nullptr;
+        KG_CUDA(ctx, cudaEventCreateWithFlags(&ev, cudaEventDisableTiming));
+        cudaError_t e = cudaEventRecord(ev, ctx->stream);
+        if (e == cudaSuccess) e = cudaStreamWaitEvent(ctx->copy_stream, ev, 0);
+        if (e == cudaSuccess) e = cudaMemcpyAsync(dst, text, bytes, cudaMemcpyDeviceToHost, ctx->copy_stream);
+        cudaEventDestroy(ev);
+        KG_CUDA(ctx, e);
+        return KOMBGPU_OK;
+    }
+    KG_CUDA(ctx, cudaMemcpyAsync(dst, text, bytes, cudaMemcpyDeviceToHost, ctx->stream));
+    KG_CUDA(ctx, cudaStreamSynchronize(ctx->stream));
+    return KOMBGPU_OK;
+}
 
-void format_release(kombgpu_graph *g) {
+void release_texts(kombgpu_ctx *ctx, char **text, uint64_t *text_bytes) {
     for (int w = 0; w < 3; ++w) {
-        if (g->text[w]) ws_free(g->ctx, g->text[w]);
-        g->text[w] = nullptr;
-        g->text_bytes[w] = 0;
+        if (text[w]) ws_free(ctx, text[w]);
+        text[w] = nullptr;
+        text_bytes[w] = 0;
     }
 }
+
+}  // namespace
+
+void format_release(kombgpu_graph *g) { release_texts(g->ctx, g->text, g->text_bytes); }
+void dist_format_release(kombgpu_dist_graph *g) { release_texts(g->ctx, g->text, g->text_bytes); }
 
 }  // namespace kg
 
@@ -245,11 +282,12 @@ int kombgpu_graph_format(kombgpu_graph *g, int which, const kombgpu_hits *names,
             return ctx_fail(ctx, KOMBGPU_EINVAL, "kcore.tsv needs the unitig names: the kombgpu_hits this graph was built from");
         a.core = g->core;
         a.deg = g->deg;
-        KG_TRY(format_rows(ctx, g->n, KcoreRowLen{a.len, a.core, a.deg}, make_kcore_out, &a, kKcoreHeaderLen, &text, &total));
+        a.base = kKcoreHeaderLen;
+        KG_TRY(format_rows(ctx, g->n, KcoreRowLen{a.len, a.core, a.deg, 0u}, make_kcore_out, &a, kKcoreHeaderLen, &text, &total));
         KG_CUDA(ctx, cudaMemcpyAsync(text, kKcoreHeader, kKcoreHeaderLen, cudaMemcpyHostToDevice, ctx->stream));
     } else {
         if (!g->has_score) return ctx_fail(ctx, KOMBGPU_ESTATE, "kombgpu_graph_corea has not run");
-        KG_TRY(format_scores(ctx, g->score, g->n, &text, &total));
+        KG_TRY(format_scores(ctx, g->score, g->n, 0u, &text, &total));
     }
     g->text[which] = text;
     g->text_bytes[which] = total;
@@ -262,23 +300,7 @@ int kombgpu_graph_format_fetch(kombgpu_graph *g, int which, char *dst, int async
     if (!g) return KOMBGPU_EINVAL;
     kombgpu_ctx *ctx = g->ctx;
     if (which < 0 || which > 2 || !g->text[which]) return ctx_fail(ctx, KOMBGPU_ESTATE, "kombgpu_graph_format has not run for this file");
-    if (!dst && g->text_bytes[which]) return ctx_fail(ctx, KOMBGPU_EINVAL, "null destination");
-    KG_CUDA(ctx, cudaSetDevice(ctx->device));
-    if (!g->text_bytes[which]) return KOMBGPU_OK;
-    if (async) {
-        // behind everything the compute stream has queued so far, on the copy stream: later compute overlaps the download
-        cudaEvent_t ev = nullptr;
-        KG_CUDA(ctx, cudaEventCreateWithFlags(&ev, cudaEventDisableTiming));
-        cudaError_t e = cudaEventRecord(ev, ctx->stream);
-        if (e == cudaSuccess) e = cudaStreamWaitEvent(ctx->copy_stream, ev, 0);
-        if (e == cudaSuccess) e = cudaMemcpyAsync(dst, g->text[which], g->text_bytes[which], cudaMemcpyDeviceToHost, ctx->copy_stream);
-        cudaEventDestroy(ev);
-        KG_CUDA(ctx, e);
-        return KOMBGPU_OK;
-    }
-    KG_CUDA(ctx, cudaMemcpyAsync(dst, g->text[which], g->text_bytes[which], cudaMemcpyDeviceToHost, ctx->stream));
-    KG_CUDA(ctx, cudaStreamSynchronize(ctx->stream));
-    return KOMBGPU_OK;
+    return fetch_text(ctx, g->text[which], g->text_bytes[which], dst, async);
 }
 
 int kombgpu_graph_format_wait(kombgpu_graph *g) {
@@ -297,7 +319,7 @@ int kombgpu_format_corea(kombgpu_ctx *ctx, const double *score, uint32_t n, char
     if (n) KG_CUDA(ctx, cudaMemcpyAsync(d.p, score, (size_t)n * sizeof(double), cudaMemcpyHostToDevice, ctx->stream));
     char *text = nullptr;
     uint64_t total = 0;
-    KG_TRY(format_scores(ctx, d.p, n, &text, &total));
+    KG_TRY(format_scores(ctx, d.p, n, 0u, &text, &total));
     DevBuf<char> hold;
     hold.ctx = ctx;
     hold.p = text;
@@ -307,6 +329,52 @@ int kombgpu_format_corea(kombgpu_ctx *ctx, const double *score, uint32_t n, char
         KG_CUDA(ctx, cudaMemcpyAsync(dst, text, total, cudaMemcpyDeviceToHost, ctx->stream));
         KG_CUDA(ctx, cudaStreamSynchronize(ctx->stream));
     }
+    return KOMBGPU_OK;
+}
+
+// ---- the partitioned graph: this rank's slice of each file (local, not collective)
+
+int kombgpu_dist_graph_format(kombgpu_dist_graph *g, int which, const kombgpu_dist_hits *names, uint64_t *bytes) {
+    if (!g) return KOMBGPU_EINVAL;
+    kombgpu_ctx *ctx = g->ctx;
+    if (!bytes || which < 0 || which > 2) return ctx_fail(ctx, KOMBGPU_EINVAL, "bad argument");
+    KG_CUDA(ctx, cudaSetDevice(ctx->device));
+    if (g->text[which]) { *bytes = g->text_bytes[which]; return KOMBGPU_OK; }
+    char *text = nullptr;
+    uint64_t total = 0;
+    if (which == KOMBGPU_FILE_EDGELIST) {
+        KG_TRY(format_rows(ctx, g->n_fwd, EdgeRowLen{g->edges}, make_edge_out, (void *)g->edges, 0, &text, &total));
+    } else if (which == KOMBGPU_FILE_KCORE) {
+        if (!g->has_core) return ctx_fail(ctx, KOMBGPU_ESTATE, "kombgpu_dist_coreness has not run");
+        DistNames nm{};
+        if (!names || dist_hits_name_text(names, &nm) != KOMBGPU_OK || nm.comm != g->comm || nm.n_unitigs != g->n_global || nm.v_lo != g->v_lo ||
+            nm.n_local != g->n_local)
+            return ctx_fail(ctx, KOMBGPU_EINVAL, "kcore.tsv needs the unitig names: the kombgpu_dist_hits this graph was built from");
+        // the header starts rank 0's slice, the file's first (even when the graph is empty)
+        const uint64_t head = g->comm->rank == 0 ? kKcoreHeaderLen : 0;
+        KcoreArgs a{nm.bytes, nm.off, nm.len, g->core, g->deg, head, g->v_lo};
+        KG_TRY(format_rows(ctx, g->n_local, KcoreRowLen{a.len, a.core, a.deg, g->v_lo}, make_kcore_out, &a, head, &text, &total));
+        if (head) KG_CUDA(ctx, cudaMemcpyAsync(text, kKcoreHeader, kKcoreHeaderLen, cudaMemcpyHostToDevice, ctx->stream));
+    } else {
+        if (!g->has_score) return ctx_fail(ctx, KOMBGPU_ESTATE, "kombgpu_dist_corea has not run");
+        KG_TRY(format_scores(ctx, g->score, g->n_local, g->v_lo, &text, &total));
+    }
+    g->text[which] = text;
+    g->text_bytes[which] = total;
+    *bytes = total;
+    return KOMBGPU_OK;
+}
+
+int kombgpu_dist_graph_format_fetch(kombgpu_dist_graph *g, int which, char *dst, int async) {
+    if (!g) return KOMBGPU_EINVAL;
+    if (which < 0 || which > 2 || !g->text[which]) return ctx_fail(g->ctx, KOMBGPU_ESTATE, "kombgpu_dist_graph_format has not run for this file");
+    return fetch_text(g->ctx, g->text[which], g->text_bytes[which], dst, async);
+}
+
+int kombgpu_dist_graph_format_wait(kombgpu_dist_graph *g) {
+    if (!g) return KOMBGPU_EINVAL;
+    KG_CUDA(g->ctx, cudaSetDevice(g->ctx->device));
+    KG_CUDA(g->ctx, cudaStreamSynchronize(g->ctx->copy_stream));
     return KOMBGPU_OK;
 }
 

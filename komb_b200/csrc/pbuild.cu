@@ -487,6 +487,7 @@ void dist_graph_release(kombgpu_dist_graph *g) {
     g->deg = nullptr; g->core = nullptr; g->score = nullptr;
     truss_free(ctx, &g->tr);
     g->has_truss = false;
+    dist_format_release(g);
 }
 
 }  // namespace kg

@@ -14,7 +14,8 @@
 //                    holds that byte.  A home sorts the keys it received; the ranks exchange their counts per (class,
 //                    input), so vid = global offset of the group + offset of the home in it + rank in the home's sort.
 //                    The vid goes back home -> owner -> sender; the home also stores (input, offset, length) of the
-//                    vid in the rank that owns the vid's range (kombgpu_dist_hits_names)
+//                    vid in the rank that owns the vid's range (kombgpu_dist_hits_names), and sends it the name's
+//                    bytes, which it still holds: the owner formats kcore.tsv rows from them (format.cu)
 //   5. routing       (read id << 32 | vid) of every hit goes to the owner of its read: route_keys (pbuild.cu)
 // Steps 2-4 send variable-length strings, which route_keys (fixed 64-bit keys) cannot carry: send_msgs below scans
 // the sizes once per destination and stores every message and its bytes into the destination's receive buffers
@@ -36,6 +37,8 @@ struct kombgpu_dist_hits {
     uint32_t *unitig = nullptr;     // [n_hits_local]
     uint64_t *name_key = nullptr;   // [n_local] input << 56 | offset inside that input, of vertex v_lo + i
     uint32_t *name_len = nullptr;   // [n_local]
+    unsigned char *name_bytes = nullptr;   // the bytes of the names of vertices [v_lo, v_lo + n_local), in no order
+    uint64_t *name_off = nullptr;          // [n_local] where the name of vertex v_lo + i starts in name_bytes
     float ms_upload = 0.f, ms_parse = 0.f, ms_intern = 0.f, ms_route = 0.f;
     int hash_rounds = 0;
 };
@@ -60,7 +63,7 @@ struct Msg {             // one item sent to a rank
 struct Inbox {
     Msg *msg = nullptr;
     unsigned char *bytes = nullptr;
-    uint64_t n = 0;
+    uint64_t n = 0, n_bytes = 0;
 };
 
 struct DestFlagIn {
@@ -217,10 +220,12 @@ __global__ void __launch_bounds__(kThreads) msg_keys_kernel(const Msg *__restric
 }
 
 // home: vid = rank of the key among the home's sorted keys + the offset of its (class, input) group; the vid goes to
-// the owner of the name, the name's span to the owner of the vid
+// the owner of the name, the name's span to the owner of the vid.  out / dest / src_off: the message that carries the
+// name's bytes (in this rank's text buffer) to the owner of the vid, idx = vid - owner * step
 __global__ void __launch_bounds__(kThreads) vid_kernel(const Msg *__restrict__ msg, uint64_t n, const uint64_t *__restrict__ sorted,
                                                        const unsigned long long *__restrict__ delta, int n_files, uint32_t step,
-                                                       PeerPtrs<uint32_t> vid_reply, PeerPtrs<uint64_t> name_key, PeerPtrs<uint32_t> name_len) {
+                                                       PeerPtrs<uint32_t> vid_reply, PeerPtrs<uint64_t> name_key, PeerPtrs<uint32_t> name_len,
+                                                       Slices sl, Msg *__restrict__ out, uint32_t *__restrict__ dest, uint64_t *__restrict__ src_off) {
     for (uint64_t i = (uint64_t)blockIdx.x * blockDim.x + threadIdx.x; i < n; i += (uint64_t)gridDim.x * blockDim.x) {
         const Msg m = msg[i];
         uint64_t lo = 0, hi = n;   // the keys are distinct: lower bound = rank
@@ -234,7 +239,16 @@ __global__ void __launch_bounds__(kThreads) vid_kernel(const Msg *__restrict__ m
         const uint32_t o = vid / step;
         name_key.p[o][vid - o * step] = m.key & ~kKeyClassHit;
         name_len.p[o][vid - o * step] = m.len;
+        const uint32_t f = (uint32_t)((m.key >> kKeyFileShift) & 63u);
+        out[i] = Msg{0ull, 0ull, m.len, vid - o * step, 0u, 0u};
+        dest[i] = o;
+        src_off[i] = sl.base[f] + (m.key & kKeyOffMask) - sl.cut_lo[f];
     }
+}
+
+// owner: where the name of each of its vertices starts in the received bytes
+__global__ void __launch_bounds__(kThreads) name_off_kernel(const Msg *__restrict__ msg, uint64_t n, uint64_t *__restrict__ name_off) {
+    for (uint64_t i = (uint64_t)blockIdx.x * blockDim.x + threadIdx.x; i < n; i += (uint64_t)gridDim.x * blockDim.x) name_off[msg[i].idx] = msg[i].off;
 }
 
 // owner: the vid of every received name goes into its sender's reply slot
@@ -321,7 +335,7 @@ int send_msgs(kombgpu_comm *c, int rc, const Msg *msg, const uint32_t *dest, uin
             nt += all[(size_t)q * (1 + 2 * world) + 1 + p];
             bt += all[(size_t)q * (1 + 2 * world) + 1 + world + p];
         }
-        if (p == rank) in->n = nt;
+        if (p == rank) { in->n = nt; in->n_bytes = bt; }
         max_n = nt > max_n ? nt : max_n;
         max_bytes = bt > max_bytes ? bt : max_bytes;
     }
@@ -639,9 +653,10 @@ int dist_sam_parse(kombgpu_comm *c, const char *const *texts, const uint64_t *si
         DevBuf<unsigned long long> d_delta;
         KG_ALLOC(ctx, d_delta, delta.size());
         KG_CUDA(ctx, cudaMemcpyAsync(d_delta.p, delta.data(), delta.size() * sizeof(unsigned long long), cudaMemcpyHostToDevice, ctx->stream));
+        KG_TRY(outbox(hin.n));
         if (hin.n)
             KG_LAUNCH(ctx, vid_kernel, grid_for(hin.n, kThreads, ctx->sm_count), kThreads, 0, hin.msg, hin.n, hsorted, d_delta.p, F, step, pvid, pkey,
-                      plen);
+                      plen, Slices{d_base.p, d_cut_lo.p, F}, out_msg.p, out_dest.p, out_off.p);
         return KOMBGPU_OK;
     }();
     KG_TRY(barrier(c, rc));
@@ -657,11 +672,23 @@ int dist_sam_parse(kombgpu_comm *c, const char *const *texts, const uint64_t *si
         return KOMBGPU_OK;
     }();
     KG_TRY(barrier(c, rc));
+    // home -> owner of the vid: the bytes of the name (a line is never split between slices, so the home holds them)
+    Inbox bin;
+    KG_TRY(send_msgs(c, KOMBGPU_OK, out_msg.p, out_dest.p, hin.n, text.p, out_off.p, &bin));
+    DevBuf<unsigned char> name_bytes;
+    DevBuf<uint64_t> name_off;
+    rc = [&]() -> int {
+        KG_ALLOC(ctx, name_bytes, bin.n_bytes);
+        KG_ALLOC(ctx, name_off, bin.n);
+        if (bin.n_bytes) KG_CUDA(ctx, cudaMemcpyAsync(name_bytes.p, bin.bytes, bin.n_bytes, cudaMemcpyDeviceToDevice, ctx->stream));
+        if (bin.n) KG_LAUNCH(ctx, name_off_kernel, grid_for(bin.n, kThreads, ctx->sm_count), kThreads, 0, bin.msg, bin.n, name_off.p);
+        return KOMBGPU_OK;
+    }();
     h->ms_intern = tm.lap();
 
     // ---- 5. (read id << 32 | vid) of every hit -> the owner of the read
     DevBuf<uint64_t> hit_keys;
-    rc = [&]() -> int {
+    if (rc == KOMBGPU_OK) rc = [&]() -> int {
         KG_ALLOC(ctx, hit_keys, n_hits);
         if (n_hits)
             KG_LAUNCH(ctx, hit_keys_kernel, grid_for(n_hits, kThreads, ctx->sm_count), kThreads, 0, key_ids.p, read_id, name_ids.p + n_sq, name_vid,
@@ -700,18 +727,26 @@ int dist_sam_parse(kombgpu_comm *c, const char *const *texts, const uint64_t *si
     h->unitig = unitig.take();
     h->name_key = name_key.take();
     h->name_len = name_len.take();
+    h->name_bytes = name_bytes.take();
+    h->name_off = name_off.take();
     return KOMBGPU_OK;
 }
 
 void dist_hits_release(kombgpu_dist_hits *h) {
     if (!h || !h->ctx) return;
-    void *ptrs[] = {h->read_key, h->unitig, h->name_key, h->name_len};
+    void *ptrs[] = {h->read_key, h->unitig, h->name_key, h->name_len, h->name_bytes, h->name_off};
     for (void *p : ptrs)
         if (p) ws_free(h->ctx, p);
-    h->read_key = nullptr; h->unitig = nullptr; h->name_key = nullptr; h->name_len = nullptr;
+    h->read_key = nullptr; h->unitig = nullptr; h->name_key = nullptr; h->name_len = nullptr; h->name_bytes = nullptr; h->name_off = nullptr;
 }
 
 }  // namespace
+
+int dist_hits_name_text(const kombgpu_dist_hits *h, DistNames *out) {
+    if (!h) return KOMBGPU_EINVAL;
+    *out = DistNames{h->comm, h->n_unitigs, h->v_lo, h->n_local, h->name_bytes, h->name_off, h->name_len};
+    return KOMBGPU_OK;
+}
 }  // namespace kg
 
 using namespace kg;

@@ -182,6 +182,18 @@ class DistGraph:
         return {"n_vertices": nv.value, "n_edges": ne.value, "weight_sum": ws.value, "density": d.value, "passes": np_.value,
                 "member": member.astype(bool), "v_lo": st["v_lo"]}
 
+    FILE_EDGELIST, FILE_KCORE, FILE_COREA = 0, 1, 2
+
+    def format(self, which: int, hits: "DistHits | None" = None) -> bytes:
+        """This rank's slice of edgelist.txt / kcore.tsv / CoreA_anomaly.txt, formatted on its device
+        (kombgpu_dist_graph_format): the slices of ranks 0, 1, ... concatenate to Graph.format on one GPU.  kcore.tsv
+        takes the unitig names from the DistHits the graph was built from.  Local, not collective."""
+        n = c_uint64()
+        self._ctx._check(self._lib.kombgpu_dist_graph_format(self._h, int(which), hits._h if hits is not None else None, byref(n)))
+        buf = ctypes.create_string_buffer(max(n.value, 1))
+        self._ctx._check(self._lib.kombgpu_dist_graph_format_fetch(self._h, int(which), buf, 0))
+        return buf.raw[:n.value]
+
     def results(self, out: dict | None = None) -> dict:
         """degree / coreness / score of the local unitigs [v_lo, v_lo + n_local) on the host."""
         st = self.stats()
