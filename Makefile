@@ -7,7 +7,7 @@ ARCH      := -gencode arch=compute_100a,code=sm_100a
 NVCCFLAGS := -O3 -std=c++17 -lineinfo $(ARCH) -Xcompiler -fPIC,-Wall,-Wno-unused-function -Iinclude -Ikomb_b200/csrc
 CSRC      := komb_b200/csrc
 OBJDIR    := build/obj
-CU        := $(CSRC)/capi.cu $(CSRC)/build.cu $(CSRC)/sort.cu $(CSRC)/peel.cu $(CSRC)/corea.cu $(CSRC)/dist.cu $(CSRC)/densest.cu $(CSRC)/comm.cu $(CSRC)/pbuild.cu $(CSRC)/ppeel.cu $(CSRC)/apeel.cu $(CSRC)/rpeel.cu $(CSRC)/pcore.cu $(CSRC)/pcapi.cu $(CSRC)/truss.cu $(CSRC)/sam.cu $(CSRC)/format.cu $(CSRC)/fasta.cu $(CSRC)/psam.cu
+CU        := $(CSRC)/capi.cu $(CSRC)/build.cu $(CSRC)/sort.cu $(CSRC)/peel.cu $(CSRC)/corea.cu $(CSRC)/dist.cu $(CSRC)/densest.cu $(CSRC)/comm.cu $(CSRC)/pbuild.cu $(CSRC)/ppeel.cu $(CSRC)/apeel.cu $(CSRC)/rpeel.cu $(CSRC)/pcore.cu $(CSRC)/pcapi.cu $(CSRC)/truss.cu $(CSRC)/sam.cu $(CSRC)/format.cu $(CSRC)/fasta.cu $(CSRC)/psam.cu $(CSRC)/pfasta.cu
 OBJ       := $(patsubst $(CSRC)/%.cu,$(OBJDIR)/%.o,$(CU))
 HDR       := include/kombgpu.h $(wildcard $(CSRC)/*.cuh)
 

@@ -12,7 +12,8 @@
 //   runCore            :455-484               degree / coreness (kombgpu_graph_results) -> kcore.tsv
 //   anomalyDetection   :637-648               CORE-A scores (kombgpu_graph_results) -> CoreA_anomaly.txt
 //                       (CombineCoreA::run, src/CombineCoreA.h:16-43); with KOMB_UNITIG_FASTA also the
-//                                             records of the anomalous / max-truss unitigs (writeUnitigFasta)
+//                                             records of the anomalous / max-truss unitigs (writeUnitigFasta; over
+//                                             several GPUs each rank extracts its slice in runMulti)
 // Errors follow the reference: a message on stderr and exit(EXIT_FAILURE)
 // (src/graph.cpp:58-61).
 #pragma once
@@ -147,10 +148,14 @@ class Kgraph {
         std::vector<uint32_t> v;
         std::vector<int32_t> deg, core;
         std::vector<double> score;
-        std::vector<std::string> names;   // unitig names of [v_lo, v_lo + n_local) (partitioned SAM parse, host output or FASTA)
+        std::vector<std::string> names;   // unitig names of [v_lo, v_lo + n_local) (partitioned SAM parse with host output)
         uint32_t n_unitigs = 0;
         std::unique_ptr<PinnedArray<char>> text[3];   // the rank's slices of the three files, formatted on its device
         uint64_t text_bytes[3] = {0, 0, 0};
+        std::unique_ptr<PinnedArray<char>> fasta;     // the rank's slice of anomalous_unitigs.fasta
+        uint64_t fasta_bytes = 0;
+        std::string fasta_err;            // malformed FASTA or a selected unitig without a record: reported after the three files
+        bool fasta_bad_file = false;      // ... and which of the two (the message is the same on every rank)
         int rc = KOMBGPU_OK;
         std::string err;
         bool bad_input = false;           // malformed SAM: err is the parse's message, the same on every rank
@@ -171,6 +176,9 @@ class Kgraph {
     std::unique_ptr<PinnedArray<int32_t>> _deg, _core;
     std::unique_ptr<PinnedArray<double>> _score;
     bool _fasta_anomalous = false, _fasta_truss = false;   // KOMB_UNITIG_FASTA
+    std::string _fasta_path;                                // the -u FASTA
+    MappedFile _fasta_file;                                 // several GPUs: mapped once, every rank reads its slice
+    bool _fasta_unopened = false;                           // ... could not be mapped: reported where one GPU reports it
 
     // exit() must not run CUDA's teardown under a context that is still being created
     void settleDevice() { if (_ctx_ready.valid()) _ctx_ready.wait(); }
@@ -349,7 +357,11 @@ class Kgraph {
         }
         timing_mark("kombgpu_ctx_create (all devices)");
         const bool device_output = _device_output;
-        const bool want_names = !device_output || _fasta_anomalous;   // the host writes kcore.tsv, or joins the unitig FASTA
+        const bool want_names = !device_output;   // the host writes kcore.tsv
+        // anomalous_unitigs.fasta: every rank indexes its slice of the mapped -u file, joins its unitigs' names, picks
+        // them by the fence over every rank's scores and extracts its slice of the output (kombgpu_dist_fasta_*)
+        if (_fasta_anomalous) _fasta_unopened = !_fasta_file.open(_fasta_path);
+        const bool fasta = _fasta_anomalous && !_fasta_unopened;
         std::vector<std::thread> th;
         for (int r = 0; r < world; ++r)
             th.emplace_back([&, r]() {
@@ -421,10 +433,6 @@ class Kgraph {
                     if (device_output) {
                         rc = format(KOMBGPU_FILE_KCORE);
                         if (rc == KOMBGPU_OK) rc = format(KOMBGPU_FILE_COREA);
-                        if (rc == KOMBGPU_OK && _fasta_anomalous) {   // the anomalous unitigs are picked on the host from every score
-                            o.score.resize(o.n_local);
-                            if ((rc = kombgpu_dist_graph_results(g, nullptr, nullptr, o.score.data())) != KOMBGPU_OK) fail(rc, "kombgpu_dist_graph_results");
-                        }
                     } else {
                         o.fwd_ptr.resize((size_t)o.n_local + 1); o.v.resize(o.n_fwd);
                         o.deg.resize(o.n_local); o.core.resize(o.n_local); o.score.resize(o.n_local);
@@ -437,6 +445,7 @@ class Kgraph {
                         kombgpu_dist_graph_summary(g, &_max_core_multi, &_max_score_multi);
                     }
                 }
+                if (rc == KOMBGPU_OK && fasta) rc = anomalousFastaSlice(o, ctx, comm, g, dh, hits, fail);
                 if (dh) kombgpu_dist_hits_destroy(dh);
                 if (g) {
                     // the downloads into the page-locked slices end before the graph's text goes
@@ -448,7 +457,7 @@ class Kgraph {
             });
         for (auto &t : th) t.join();
         _rank_ctxs = ctxs;   // destroyed with the ranks' page-locked text, after the three files are written
-        _ctx = ctxs[0];      // the unitig FASTA work runs on rank 0's device after the ranks are done
+        _ctx = ctxs[0];
         if (_ranks[0].bad_input) {   // malformed SAM: the tokeniser's message (every rank has the same) and exit code
             std::cerr << _ranks[0].err << std::endl;
             exit(EXIT_FAILURE);
@@ -640,20 +649,17 @@ class Kgraph {
 
     void anomalyDetection(const std::string &dir, bool weight, const std::string &fasta_path, const HitTable &hits) {
         uint32_t n = 0;
-        std::vector<double> score_all;
         int32_t max_core = 0;
         double max_score = 0.0;
         if (multi()) {
             for (const RankOut &o : _ranks) n += o.n_local;
-            score_all.resize(n);
-            for (const RankOut &o : _ranks) std::copy(o.score.begin(), o.score.end(), score_all.begin() + o.v_lo);
             max_core = _max_core_multi;
             max_score = _max_score_multi;
         } else {
             kombgpu_graph_counts(_graph, &n, nullptr);
             kombgpu_graph_summary(_graph, &max_core, &max_score);
         }
-        const double *score = multi() ? score_all.data() : (_score ? _score->data() : nullptr);  // fetched by readEdgeList / runMulti
+        const double *score = _score ? _score->data() : nullptr;  // one GPU, host output: fetched by readEdgeList
         const double dense_ratio = (double)(max_core / 2);  // integer division, like CombineCoreA.h:24
         fprintf(stdout, "Dense Ratio: %f\n", n ? dense_ratio : 0.0);
         if (weight) {
@@ -666,6 +672,13 @@ class Kgraph {
                     if (o.text_bytes[2] && fwrite(o.text[2]->data(), 1, o.text_bytes[2], fp) != o.text_bytes[2]) fileNotFoundError(anomaly_output);
             } else if (_device_output) {
                 if (_text_bytes[2] && fwrite(_text[2]->data(), 1, _text_bytes[2], fp) != _text_bytes[2]) fileNotFoundError(anomaly_output);
+            } else if (multi()) {   // every rank's scores, fetched by runMulti
+                for (const RankOut &o : _ranks)
+                    write_rows(fp, o.n_local, 64, (int)_threads, [&](char *p, size_t i) {
+                        p = put_u64(p, o.v_lo + i); *p++ = '\t';
+                        p += snprintf(p, 48, "%f\n", o.score[i]);
+                        return p;
+                    });
             } else
             write_rows(fp, n, 64, (int)_threads, [&](char *p, size_t i) {
                 p = put_u64(p, i); *p++ = '\t';
@@ -675,7 +688,8 @@ class Kgraph {
             fclose(fp);
             timing_mark("write CoreA_anomaly.txt");
         }
-        if (_fasta_anomalous || _fasta_truss) writeUnitigFasta(dir, fasta_path, hits, score_all);
+        if (multi() && _fasta_anomalous) writeRankFasta(dir, fasta_path);
+        else if (_fasta_anomalous || _fasta_truss) writeUnitigFasta(dir, fasta_path, hits);
         _efp.reset(); _ev.reset(); _deg.reset(); _core.reset(); _score.reset();
         for (auto &t : _text) t.reset();
         releaseRanks();
@@ -684,14 +698,75 @@ class Kgraph {
         timing_mark("free pinned + graph");
     }
 
-    // KOMB_UNITIG_FASTA: which unitig FASTA files anomalyDetection writes (with several GPUs, rank 0's context is kept
-    // for them)
-    void setUnitigFasta(bool anomalous, bool truss) { _fasta_anomalous = anomalous; _fasta_truss = truss; }
+    // KOMB_UNITIG_FASTA: which unitig FASTA files anomalyDetection writes, from the -u file
+    void setUnitigFasta(bool anomalous, bool truss, const std::string &path) {
+        _fasta_anomalous = anomalous;
+        _fasta_truss = truss;
+        _fasta_path = path;
+    }
 
-    // <dir>/anomalous_unitigs.fasta (IQR fence, whisker 1.5, on this run's CORE-A scores) and <dir>/truss_unitigs.fasta
-    // (the unitigs on the edges of maximal trussness in the maximal core, the file the reference's runTruss writes):
-    // the records of the -u FASTA, indexed, joined by name and copied out on the device.
-    void writeUnitigFasta(const std::string &dir, const std::string &fasta_path, const HitTable &hits, const std::vector<double> &score_all) {
+    // One rank's part of anomalous_unitigs.fasta (runMulti, after CORE-A; every call but the fetch is collective).  A
+    // malformed file or a selected unitig without a record is kept in o.fasta_err and reported after the three files.
+    template <typename Fail>
+    int anomalousFastaSlice(RankOut &o, kombgpu_ctx *ctx, kombgpu_comm *comm, kombgpu_dist_graph *g, kombgpu_dist_hits *dh,
+                            const HitTable &hits, Fail &fail) {
+        kombgpu_dist_fasta *fa = nullptr;
+        int rc = kombgpu_dist_fasta_load(comm, _fasta_file.data, _fasta_file.size, &fa);
+        if (rc == KOMBGPU_EINVAL) { o.fasta_err = kombgpu_last_error(ctx); o.fasta_bad_file = true; return KOMBGPU_OK; }
+        if (rc != KOMBGPU_OK) { fail(rc, "kombgpu_dist_fasta_load"); return rc; }
+        uint32_t n_missing = 0;
+        if (dh) {
+            rc = kombgpu_dist_fasta_join_hits(fa, dh, &n_missing);
+        } else {   // the host tokeniser's names of this rank's unitigs
+            std::vector<uint64_t> off((size_t)o.n_local + 1, 0);
+            std::string bytes;
+            for (uint32_t i = 0; i < o.n_local; ++i) {
+                bytes += hits.names[o.v_lo + i];
+                off[i + 1] = bytes.size();
+            }
+            rc = kombgpu_dist_fasta_join_names(fa, bytes.data(), off.data(), o.n_local, &n_missing);
+        }
+        if (rc != KOMBGPU_OK) fail(rc, "kombgpu_dist_fasta_join");
+        std::vector<uint8_t> mask(o.n_local, 0);
+        if (rc == KOMBGPU_OK && (rc = kombgpu_dist_anomalous(g, 1.5, nullptr, nullptr, nullptr, nullptr, mask.data())) != KOMBGPU_OK)
+            fail(rc, "kombgpu_dist_anomalous");
+        if (rc == KOMBGPU_OK) {
+            rc = kombgpu_dist_fasta_extract(fa, mask.data(), o.n_local, &o.fasta_bytes);
+            if (rc == KOMBGPU_EINVAL) {
+                o.fasta_err = kombgpu_last_error(ctx);
+                rc = KOMBGPU_OK;
+            } else if (rc != KOMBGPU_OK) {
+                fail(rc, "kombgpu_dist_fasta_extract");
+            } else {
+                o.fasta.reset(new PinnedArray<char>(ctx, o.fasta_bytes));
+                if ((rc = kombgpu_dist_fasta_extract_fetch(fa, o.fasta->data())) != KOMBGPU_OK) fail(rc, "kombgpu_dist_fasta_extract_fetch");
+            }
+        }
+        kombgpu_dist_fasta_destroy(fa);
+        return rc;
+    }
+
+    // anomalous_unitigs.fasta from several GPUs: the ranks' slices in rank order, or the error one GPU reports here
+    void writeRankFasta(const std::string &dir, const std::string &fasta_path) {
+        if (_fasta_unopened) fileNotFoundError(fasta_path);
+        const RankOut &r0 = _ranks[0];
+        if (!r0.fasta_err.empty()) {   // the same message on every rank
+            std::cerr << "komb2: " << (r0.fasta_bad_file ? fasta_path : std::string("anomalous_unitigs.fasta")) << ": " << r0.fasta_err << std::endl;
+            exit(EXIT_FAILURE);
+        }
+        const std::string path = dir + "/anomalous_unitigs.fasta";
+        FILE *f = fopen(path.c_str(), "w");
+        if (f == nullptr) fileNotFoundError(path);
+        for (const RankOut &o : _ranks)
+            if (o.fasta_bytes && fwrite(o.fasta->data(), 1, o.fasta_bytes, f) != o.fasta_bytes) fileNotFoundError(path);
+        fclose(f);
+        timing_mark("unitig FASTA files");
+    }
+
+    // One GPU: <dir>/anomalous_unitigs.fasta (IQR fence, whisker 1.5, on this run's CORE-A scores) and
+    // <dir>/truss_unitigs.fasta (the unitigs on the edges of maximal trussness in the maximal core, the file the
+    // reference's runTruss writes): the records of the -u FASTA, indexed, joined by name and copied out on the device.
+    void writeUnitigFasta(const std::string &dir, const std::string &fasta_path, const HitTable &hits) {
         MappedFile file;
         if (!file.open(fasta_path)) fileNotFoundError(fasta_path);
         kombgpu_fasta *fa = nullptr;
@@ -713,8 +788,8 @@ class Kgraph {
             rc = kombgpu_fasta_join_names(fa, bytes.data(), off.data(), (uint32_t)hits.names.size(), &n_missing);
         }
         if (rc != KOMBGPU_OK) gpuError("kombgpu_fasta_join", rc);
-        uint32_t n = (uint32_t)score_all.size();
-        if (!multi()) kombgpu_graph_counts(_graph, &n, nullptr);
+        uint32_t n = 0;
+        kombgpu_graph_counts(_graph, &n, nullptr);
         std::vector<uint8_t> mask(n, 0);
         auto write = [&](const char *name) {
             const std::string path = dir + "/" + name;
@@ -733,12 +808,11 @@ class Kgraph {
             fclose(f);
         };
         if (_fasta_anomalous) {
-            rc = multi() ? kombgpu_anomalous(_ctx, score_all.data(), n, 1.5, nullptr, nullptr, nullptr, nullptr, mask.data())
-                         : kombgpu_graph_anomalous(_graph, 1.5, nullptr, nullptr, nullptr, nullptr, mask.data());
+            rc = kombgpu_graph_anomalous(_graph, 1.5, nullptr, nullptr, nullptr, nullptr, mask.data());
             if (rc != KOMBGPU_OK) gpuError("kombgpu_anomalous", rc);
             write("anomalous_unitigs.fasta");
         }
-        if (_fasta_truss) {   // single GPU only: the partitioned graph has no truss (komb2.cpp refuses the combination)
+        if (_fasta_truss) {   // single GPU only (komb2.cpp refuses the combination with several GPUs)
             uint32_t n_truss = 0;
             if ((rc = kombgpu_graph_max_core_truss(_graph, nullptr, nullptr, nullptr, &n_truss)) != KOMBGPU_OK) gpuError("kombgpu_graph_max_core_truss", rc);
             std::vector<uint32_t> vids(n_truss);

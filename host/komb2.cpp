@@ -78,7 +78,7 @@ int main(int argc, const char **argv) {
     }
 
     komb::Kgraph kg((uint32_t)opt.threads, (uint64_t)opt.readlen, device, key_mode, devices);
-    kg.setUnitigFasta(fasta_anomalous, fasta_truss);
+    kg.setUnitigFasta(fasta_anomalous, fasta_truss, opt.input_unitigs);
     komb::HitTable hits;
     komb::MappedFile sam1, sam2;  // the hit table points into these until the ids exist
     auto begin_komb = std::chrono::steady_clock::now();

@@ -611,6 +611,42 @@ int kombgpu_dist_graph_format(kombgpu_dist_graph *g, int which, const kombgpu_di
 int kombgpu_dist_graph_format_fetch(kombgpu_dist_graph *g, int which, char *dst, int async);
 int kombgpu_dist_graph_format_wait(kombgpu_dist_graph *g);
 
+/* The unitig FASTA over the ranks: the rules of the single-GPU "unitig FASTA" section above (records, names, join, fence,
+ * extraction), with the same results and the same error messages (record numbers, byte offsets and vertex ids are
+ * global).  Rank q uploads and indexes only bytes [cut_q, cut_{q+1}) of the file, cut_q = the first record start at or
+ * after floor(size * q / world) (cut_0 = 0: bytes before the first record lie in rank 0's slice; a record is never split;
+ * a slice may be empty).  Record names and vertex names meet on the rank a fixed-seed hash of their bytes picks, so no
+ * GPU holds the whole file, all names or all scores, and nothing of their size passes through the host.  The
+ * extraction slices of ranks 0, 1, ... concatenate to exactly the bytes kombgpu_fasta_extract gives on one GPU for the
+ * same file, names and mask.  Every call but _counts, _extract_fetch and _timing is collective.  A malformed file, a
+ * selected vertex without a record or a bad argument on one rank gives an error on every rank (KOMBGPU_EINVAL with the
+ * single-GPU message where one GPU would give it); the contexts, the communicator and the graph stay usable. */
+typedef struct kombgpu_dist_fasta kombgpu_dist_fasta;
+/* Every rank passes the same bytes of one FASTA file (within one process the pointer may be shared). */
+int kombgpu_dist_fasta_load(kombgpu_comm *comm, const char *text, uint64_t size, kombgpu_dist_fasta **out);
+void kombgpu_dist_fasta_destroy(kombgpu_dist_fasta *fa);
+/* records in this rank's slice, records of the file, first global record id and byte range of the slice; any may be NULL */
+int kombgpu_dist_fasta_counts(const kombgpu_dist_fasta *fa, uint32_t *n_records_local, uint32_t *n_records_global,
+                              uint32_t *rec_lo, uint64_t *byte_lo, uint64_t *byte_hi);
+/* vertex -> record for this rank's vertices: the names of the kombgpu_dist_hits the graph was built from (its unitigs
+ * [v_lo, v_lo + n_local)), or a packed host table of n_local names (n_local + 1 offsets, as kombgpu_fasta_join_names);
+ * the ranks' vertices follow one another in rank order.  *n_missing: vertices without a record over ALL ranks. */
+int kombgpu_dist_fasta_join_hits(kombgpu_dist_fasta *fa, const kombgpu_dist_hits *names, uint32_t *n_missing);
+int kombgpu_dist_fasta_join_names(kombgpu_dist_fasta *fa, const char *bytes, const uint64_t *offsets, uint32_t n_local,
+                                  uint32_t *n_missing);
+/* mask: this rank's n_local host bytes (of its last join).  *bytes: size of THIS rank's slice of the output, which only
+ * the rank holding the file's last record ends with the '\n' an unterminated selected last record gets. */
+int kombgpu_dist_fasta_extract(kombgpu_dist_fasta *fa, const uint8_t *mask, uint32_t n_local, uint64_t *bytes);
+int kombgpu_dist_fasta_extract_fetch(kombgpu_dist_fasta *fa, char *dst);   /* local */
+/* CUDA-event times on this rank (they include the waits for the other ranks) and the kernels it launched */
+int kombgpu_dist_fasta_timing(const kombgpu_dist_fasta *fa, float *ms_upload, float *ms_index, float *ms_join,
+                              float *ms_extract, uint64_t *kernel_launches);
+/* The IQR fence on CORE-A over the scores of ALL ranks (needs kombgpu_dist_corea, KOMBGPU_ESTATE otherwise): q1, q3,
+ * fence and n_selected are global and bit-equal to kombgpu_graph_anomalous on one GPU; member (optional) is this rank's
+ * n_local bytes.  A radix select over the ranks finds the order statistics: no score crosses a link.  Collective. */
+int kombgpu_dist_anomalous(kombgpu_dist_graph *g, double whisker, double *q1, double *q3, double *fence,
+                           uint32_t *n_selected, uint8_t *member);
+
 int kombgpu_abi_version(void);
 
 #ifdef __cplusplus

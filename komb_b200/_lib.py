@@ -179,6 +179,18 @@ SIGNATURES = {
     "kombgpu_dist_graph_format": (c_int, [c_void_p, c_int, c_void_p, POINTER(c_uint64)]),
     "kombgpu_dist_graph_format_fetch": (c_int, [c_void_p, c_int, c_void_p, c_int]),
     "kombgpu_dist_graph_format_wait": (c_int, [c_void_p]),
+    "kombgpu_dist_fasta_load": (c_int, [c_void_p, c_char_p, c_uint64, POINTER(c_void_p)]),
+    "kombgpu_dist_fasta_destroy": (None, [c_void_p]),
+    "kombgpu_dist_fasta_counts": (c_int, [c_void_p, POINTER(c_uint32), POINTER(c_uint32), POINTER(c_uint32), POINTER(c_uint64),
+                                          POINTER(c_uint64)]),
+    "kombgpu_dist_fasta_join_hits": (c_int, [c_void_p, c_void_p, POINTER(c_uint32)]),
+    "kombgpu_dist_fasta_join_names": (c_int, [c_void_p, c_char_p, c_void_p, c_uint32, POINTER(c_uint32)]),
+    "kombgpu_dist_fasta_extract": (c_int, [c_void_p, c_void_p, c_uint32, POINTER(c_uint64)]),
+    "kombgpu_dist_fasta_extract_fetch": (c_int, [c_void_p, c_void_p]),
+    "kombgpu_dist_fasta_timing": (c_int, [c_void_p, POINTER(c_float), POINTER(c_float), POINTER(c_float), POINTER(c_float),
+                                          POINTER(c_uint64)]),
+    "kombgpu_dist_anomalous": (c_int, [c_void_p, c_double, POINTER(c_double), POINTER(c_double), POINTER(c_double), POINTER(c_uint32),
+                                       c_void_p]),
 }
 
 _lib = None

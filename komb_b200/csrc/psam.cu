@@ -17,8 +17,8 @@
 //                    vid in the rank that owns the vid's range (kombgpu_dist_hits_names), and sends it the name's
 //                    bytes, which it still holds: the owner formats kcore.tsv rows from them (format.cu)
 //   5. routing       (read id << 32 | vid) of every hit goes to the owner of its read: route_keys (pbuild.cu)
-// Steps 2-4 send variable-length strings, which route_keys (fixed 64-bit keys) cannot carry: send_msgs below scans
-// the sizes once per destination and stores every message and its bytes into the destination's receive buffers
+// Steps 2-4 send variable-length strings, which route_keys (fixed 64-bit keys) cannot carry: send_msgs (pmsg.cuh)
+// scans the sizes once per destination and stores every message and its bytes into the destination's receive buffers
 // (symmetric heap, peer memory), sized by an exchanged count matrix as in route_keys.  A reply is one store into the
 // sender's reply array at the index the message carries.
 #include <cstring>
@@ -26,6 +26,7 @@
 #include <vector>
 
 #include "dgraph.cuh"
+#include "pmsg.cuh"
 #include "sam.cuh"
 
 struct kombgpu_dist_hits {
@@ -50,70 +51,7 @@ constexpr uint64_t kOwnerSeed = 0x2545f4914f6cdd1dull;   // picks a string's own
 constexpr int kKeyFileShift = 56;                        // occurrence key: class << 63 | input << 56 | offset
 constexpr uint64_t kKeyOffMask = (1ull << kKeyFileShift) - 1;
 constexpr uint64_t kKeyClassHit = 1ull << 63;
-
-struct Msg {             // one item sent to a rank
-    uint64_t key;        // occurrence key (names)
-    uint64_t off;        // where its bytes start in the receiver's byte buffer
-    uint32_t len;        // length of its string
-    uint32_t idx;        // the sender's index of the item: where a reply goes
-    uint32_t rank;       // the sender
-    uint32_t flag;       // the name has a hit on the sender
-};
-
-struct Inbox {
-    Msg *msg = nullptr;
-    unsigned char *bytes = nullptr;
-    uint64_t n = 0, n_bytes = 0;
-};
-
-struct DestFlagIn {
-    const uint32_t *dest;
-    uint32_t d;
-    __device__ uint32_t operator()(uint64_t i) const { return dest[i] == d ? 1u : 0u; }
-};
-struct DestSlotOut {
-    uint32_t *slot;
-    __device__ void operator()(uint64_t i, uint32_t prefix, uint32_t flag) const {
-        if (flag) slot[i] = prefix;
-    }
-};
-struct DestBytesIn {
-    const uint32_t *dest;
-    const Msg *msg;
-    uint32_t d;
-    __device__ uint64_t operator()(uint64_t i) const { return dest[i] == d ? (uint64_t)msg[i].len : 0ull; }
-};
-struct DestBytesOut {
-    const uint32_t *dest;
-    uint32_t d;
-    uint64_t *boff;
-    __device__ void operator()(uint64_t i, uint64_t prefix, uint64_t) const {
-        if (dest[i] == d) boff[i] = prefix;
-    }
-};
-
-struct SendBase {   // where this rank's run starts in every destination's buffers
-    unsigned long long slot[kMaxRanks], byte[kMaxRanks];
-};
-
-// one warp per message: lane 0 stores the message, the lanes store its bytes
-__global__ void __launch_bounds__(kThreads) send_kernel(const Msg *__restrict__ msg, const uint32_t *__restrict__ dest,
-                                                        const uint32_t *__restrict__ slot, const uint64_t *__restrict__ boff,
-                                                        const unsigned char *__restrict__ text, const uint64_t *__restrict__ src_off, uint64_t n,
-                                                        SendBase base, PeerPtrs<Msg> dmsg, PeerPtrs<unsigned char> dbytes) {
-    const uint64_t warps = (uint64_t)gridDim.x * (blockDim.x >> 5);
-    for (uint64_t i = ((uint64_t)blockIdx.x * blockDim.x + threadIdx.x) >> 5; i < n; i += warps) {
-        const uint32_t d = dest[i];
-        Msg m = msg[i];
-        if (src_off) {
-            m.off = base.byte[d] + boff[i];
-            const unsigned char *s = text + src_off[i];
-            unsigned char *t = dbytes.p[d] + m.off;
-            for (uint32_t k = lane_id(); k < m.len; k += 32) t[k] = s[k];
-        }
-        if (lane_id() == 0) dmsg.p[d][base.slot[d] + slot[i]] = m;
-    }
-}
+constexpr const char *kStage = "the SAM parse";   // named in the error of a rank whose peer failed
 
 // the received strings as items to intern
 __global__ void __launch_bounds__(kThreads) inbox_items_kernel(const Msg *__restrict__ msg, uint64_t n, const unsigned char *__restrict__ bytes,
@@ -276,103 +214,13 @@ __global__ void __launch_bounds__(kThreads) split_hits_kernel(const uint64_t *__
     }
 }
 
-// All-gather of mine.size() words per rank (any number: exchanges of kCtlWords words each).  Word 0 is the rank's
-// status: when a rank has failed, every rank returns an error (the failing rank its own).
-int gather_words(kombgpu_comm *c, int rc_local, std::vector<unsigned long long> &mine, std::vector<unsigned long long> &all) {
-    const int k = (int)mine.size(), world = c->world;
-    mine[0] = rc_local != KOMBGPU_OK ? (unsigned long long)-rc_local : 0ull;
-    all.assign((size_t)world * k, 0ull);
-    unsigned long long part[kMaxRanks * kCtlWords];
-    for (int j0 = 0; j0 < k; j0 += kCtlWords) {
-        const int kk = k - j0 < kCtlWords ? k - j0 : kCtlWords;
-        KG_TRY(comm_exchange(c, mine.data() + j0, kk, part));
-        for (int q = 0; q < world; ++q)
-            for (int j = 0; j < kk; ++j) all[(size_t)q * k + j0 + j] = part[q * kk + j];
-    }
-    if (rc_local != KOMBGPU_OK) return rc_local;
-    for (int q = 0; q < world; ++q)
-        if (all[(size_t)q * k]) return ctx_fail(c->ctx, -(int)all[(size_t)q * k], "rank %d failed; the SAM parse stopped on every rank", q);
-    return KOMBGPU_OK;
-}
-
-int barrier(kombgpu_comm *c, int rc_local) {
-    std::vector<unsigned long long> mine(1), all;
-    return gather_words(c, rc_local, mine, all);
-}
-
-// Collective: message i (and, with src_off, the string text[src_off[i] .. + len)) goes to rank dest[i].  The messages
-// a rank receives arrive in sender order, each sender's in its own order; they live in the symmetric heap.
-int send_msgs(kombgpu_comm *c, int rc, const Msg *msg, const uint32_t *dest, uint64_t n, const unsigned char *text, const uint64_t *src_off,
-              Inbox *in) {
-    kombgpu_ctx *ctx = c->ctx;
-    const int world = c->world, rank = c->rank;
-    std::vector<unsigned long long> mine(1 + 2 * (size_t)world, 0ull), all;
-    DevBuf<uint32_t> slot, d_cnt;
-    DevBuf<uint64_t> boff, d_bytes;
-    if (rc == KOMBGPU_OK) rc = [&]() -> int {
-        KG_ALLOC(ctx, slot, n);
-        KG_ALLOC(ctx, boff, n);
-        KG_ALLOC(ctx, d_cnt, world);
-        KG_ALLOC(ctx, d_bytes, world);
-        for (int d = 0; d < world; ++d) {   // one size scan per destination: the messages' slots, the strings' offsets
-            KG_TRY((device_scan<uint32_t>(ctx, n, DestFlagIn{dest, (uint32_t)d}, DestSlotOut{slot.p}, d_cnt.p + d)));
-            if (src_off) KG_TRY((device_scan<uint64_t>(ctx, n, DestBytesIn{dest, msg, (uint32_t)d}, DestBytesOut{dest, (uint32_t)d, boff.p}, d_bytes.p + d)));
-        }
-        std::vector<uint32_t> cnt(world);
-        std::vector<uint64_t> bytes(world, 0);
-        KG_TRY(read_back(ctx, d_cnt.p, cnt.data(), world));
-        if (src_off) KG_TRY(read_back(ctx, d_bytes.p, bytes.data(), world));
-        for (int d = 0; d < world; ++d) { mine[1 + d] = cnt[d]; mine[1 + world + d] = bytes[d]; }
-        return KOMBGPU_OK;
-    }();
-    KG_TRY(gather_words(c, rc, mine, all));
-    SendBase base{};
-    unsigned long long max_n = 0, max_bytes = 0;
-    for (int p = 0; p < world; ++p) {
-        unsigned long long nt = 0, bt = 0;
-        for (int q = 0; q < world; ++q) {
-            if (q == rank) { base.slot[p] = nt; base.byte[p] = bt; }
-            nt += all[(size_t)q * (1 + 2 * world) + 1 + p];
-            bt += all[(size_t)q * (1 + 2 * world) + 1 + world + p];
-        }
-        if (p == rank) { in->n = nt; in->n_bytes = bt; }
-        max_n = nt > max_n ? nt : max_n;
-        max_bytes = bt > max_bytes ? bt : max_bytes;
-    }
-    if (max_n >= 0xffffffffull) return ctx_fail(ctx, KOMBGPU_EINVAL, "%llu strings sent to one rank exceed its 2^32 - 1 limit", max_n);
-    PeerPtrs<Msg> pmsg{};
-    PeerPtrs<unsigned char> pbytes{};
-    KG_TRY(sym_alloc(c, (size_t)max_n, &in->msg, &pmsg));
-    KG_TRY(sym_alloc(c, (size_t)max_bytes, &in->bytes, &pbytes));
-    if (n) rc = [&]() -> int {
-        KG_LAUNCH(ctx, send_kernel, grid_for(n * 32, kThreads, ctx->sm_count), kThreads, 0, msg, dest, slot.p, boff.p, text, src_off, n, base,
-                  pmsg, pbytes);
-        return KOMBGPU_OK;
-    }();
-    return barrier(c, rc);   // everything every rank stored has landed
-}
-
-// cut[q * n_files + f] = the first line start at or after floor(size_f * q / world); cut[world * n_files + f] = size_f
-void slice_cuts(const char *const *texts, const uint64_t *sizes, int n_files, int world, std::vector<uint64_t> &cut) {
-    cut.assign((size_t)(world + 1) * n_files, 0);
-    for (int f = 0; f < n_files; ++f)
-        for (int q = 1; q <= world; ++q) {
-            uint64_t x = q == world ? sizes[f] : (uint64_t)((unsigned __int128)sizes[f] * (unsigned)q / (unsigned)world);
-            if (x > 0 && x < sizes[f] && texts[f][x - 1] != '\n') {
-                const void *nl = memchr(texts[f] + x, '\n', sizes[f] - x);
-                x = nl ? (uint64_t)(static_cast<const char *>(nl) - texts[f]) + 1 : sizes[f];
-            }
-            cut[(size_t)q * n_files + f] = x;
-        }
-}
-
 int dist_sam_parse(kombgpu_comm *c, const char *const *texts, const uint64_t *sizes, int n_files, kombgpu_dist_hits *h) {
     kombgpu_ctx *ctx = c->ctx;
     const int world = c->world, rank = c->rank, F = n_files;
     SymRewind heap{c, sym_mark(c)};
     EvTimer tm(ctx);
     std::vector<uint64_t> cut;
-    slice_cuts(texts, sizes, F, world, cut);
+    slice_cuts(texts, sizes, F, world, 0, cut);
     std::vector<uint64_t> base(F, 0), cut_lo(F), len(F);
     uint64_t total = 0;
     for (int f = 0; f < F; ++f) {
@@ -455,7 +303,7 @@ int dist_sam_parse(kombgpu_comm *c, const char *const *texts, const uint64_t *si
             mine[1] = ~0ull;
         }
         for (int f = 0; f < F; ++f) mine[2 + f] = n_lines[f + 1];
-        KG_TRY(gather_words(c, rc, mine, all));
+        KG_TRY(gather_words(c, rc, mine, all, kStage));
         const size_t k = 2 + (size_t)F;
         int best_q = -1;
         for (int q = 0; q < world; ++q) {   // (input, rank, line) order = (input, line) order
@@ -529,7 +377,7 @@ int dist_sam_parse(kombgpu_comm *c, const char *const *texts, const uint64_t *si
         return KOMBGPU_OK;
     }();
     Inbox kin;
-    KG_TRY(send_msgs(c, rc, out_msg.p, out_dest.p, n_kd, text.p, out_off.p, &kin));
+    KG_TRY(send_msgs(c, rc, out_msg.p, out_dest.p, n_kd, text.p, out_off.p, &kin, kStage));
     DevBuf<uint32_t> kin_ids, kin_first;
     uint32_t n_owned_keys = 0;
     rc = [&]() -> int {
@@ -543,7 +391,7 @@ int dist_sam_parse(kombgpu_comm *c, const char *const *texts, const uint64_t *si
     uint32_t *read_id = nullptr;   // [distinct local key] its global id (symmetric heap, until the end)
     {
         std::vector<unsigned long long> mine = {0ull, n_owned_keys, n_kd, n_nd}, all;
-        KG_TRY(gather_words(c, rc, mine, all));
+        KG_TRY(gather_words(c, rc, mine, all, kStage));
         unsigned long long max_keys = 1, max_kd = 1, sum = 0;
         for (int q = 0; q < world; ++q) {
             max_keys = all[q * 4 + 1] > max_keys ? all[q * 4 + 1] : max_keys;
@@ -561,7 +409,7 @@ int dist_sam_parse(kombgpu_comm *c, const char *const *texts, const uint64_t *si
             if (kin.n) KG_LAUNCH(ctx, reply_kernel, grid_for(kin.n, kThreads, ctx->sm_count), kThreads, 0, kin.msg, kin.n, kin_ids.p, (uint32_t)rank * stride, preply);
             return KOMBGPU_OK;
         }();
-        KG_TRY(barrier(c, rc));
+        KG_TRY(barrier(c, rc, kStage));
         kin_ids.release();
         kin_first.release();
         key_first.release();
@@ -577,7 +425,7 @@ int dist_sam_parse(kombgpu_comm *c, const char *const *texts, const uint64_t *si
         return KOMBGPU_OK;
     }();
     Inbox nin;
-    KG_TRY(send_msgs(c, rc, out_msg.p, out_dest.p, n_nd, text.p, out_off.p, &nin));
+    KG_TRY(send_msgs(c, rc, out_msg.p, out_dest.p, n_nd, text.p, out_off.p, &nin, kStage));
     DevBuf<uint32_t> nin_ids, nin_first, nhit, nlen;
     DevBuf<unsigned long long> nmin;
     uint32_t n_owned_names = 0, n_hit_names = 0;
@@ -603,7 +451,7 @@ int dist_sam_parse(kombgpu_comm *c, const char *const *texts, const uint64_t *si
         return read_back(ctx, d_n.p, &n_hit_names, 1);
     }();
     Inbox hin;
-    KG_TRY(send_msgs(c, rc, out_msg.p, out_dest.p, n_hit_names, nullptr, nullptr, &hin));
+    KG_TRY(send_msgs(c, rc, out_msg.p, out_dest.p, n_hit_names, nullptr, nullptr, &hin, kStage));
     // home: sort the keys it received, count them per (class, input)
     const int G = 2 * F;
     DevBuf<uint64_t> hkeys, htmp;
@@ -625,7 +473,7 @@ int dist_sam_parse(kombgpu_comm *c, const char *const *texts, const uint64_t *si
         return KOMBGPU_OK;
     }();
     mine[1] = n_owned_names;
-    KG_TRY(gather_words(c, rc, mine, all));
+    KG_TRY(gather_words(c, rc, mine, all, kStage));
     const size_t k = 2 + (size_t)G;
     std::vector<unsigned long long> delta(G ? G : 1, 0);
     unsigned long long n_unitigs = 0, max_owned = 1;
@@ -659,7 +507,7 @@ int dist_sam_parse(kombgpu_comm *c, const char *const *texts, const uint64_t *si
                       plen, Slices{d_base.p, d_cut_lo.p, F}, out_msg.p, out_dest.p, out_off.p);
         return KOMBGPU_OK;
     }();
-    KG_TRY(barrier(c, rc));
+    KG_TRY(barrier(c, rc, kStage));
     hkeys.release();
     htmp.release();
     // owner -> sender: the vid of every name it sent
@@ -671,10 +519,10 @@ int dist_sam_parse(kombgpu_comm *c, const char *const *texts, const uint64_t *si
             KG_LAUNCH(ctx, name_reply_kernel, grid_for(nin.n, kThreads, ctx->sm_count), kThreads, 0, nin.msg, nin.n, nin_ids.p, vid_reply, pname_vid);
         return KOMBGPU_OK;
     }();
-    KG_TRY(barrier(c, rc));
+    KG_TRY(barrier(c, rc, kStage));
     // home -> owner of the vid: the bytes of the name (a line is never split between slices, so the home holds them)
     Inbox bin;
-    KG_TRY(send_msgs(c, KOMBGPU_OK, out_msg.p, out_dest.p, hin.n, text.p, out_off.p, &bin));
+    KG_TRY(send_msgs(c, KOMBGPU_OK, out_msg.p, out_dest.p, hin.n, text.p, out_off.p, &bin, kStage));
     DevBuf<unsigned char> name_bytes;
     DevBuf<uint64_t> name_off;
     rc = [&]() -> int {
@@ -717,7 +565,7 @@ int dist_sam_parse(kombgpu_comm *c, const char *const *texts, const uint64_t *si
     }();
     {
         std::vector<unsigned long long> m2 = {0ull, n_recv}, a2;   // also the barrier after which the heap is reused
-        KG_TRY(gather_words(c, rc, m2, a2));
+        KG_TRY(gather_words(c, rc, m2, a2, kStage));
         h->n_hits_global = 0;
         for (int q = 0; q < world; ++q) h->n_hits_global += a2[q * 2 + 1];
     }

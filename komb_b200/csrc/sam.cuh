@@ -10,14 +10,7 @@
 namespace kg {
 namespace {
 
-constexpr int kThreads = 256;
 enum : uint8_t { kLineSkip = 0, kLineHit = 1, kLineSq = 2 };
-
-inline uint32_t grid_for(uint64_t n, int per_block, int sms) {
-    const uint64_t g = (n + per_block - 1) / per_block;
-    const uint64_t cap = (uint64_t)sms * 16u;
-    return (uint32_t)(g < 1 ? 1 : (g > cap ? cap : g));
-}
 
 __device__ __forceinline__ uint32_t newlines_in(uint4 w) {
     const uint32_t nl = 0x0a0a0a0au;

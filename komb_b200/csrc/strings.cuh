@@ -31,4 +31,14 @@ __device__ __forceinline__ uint64_t hash_span(const unsigned char *__restrict__ 
 
 #endif  // __CUDACC__
 
+namespace {
+// launch geometry of the text kernels: grid-stride loops over at most 16 blocks per SM
+constexpr int kThreads = 256;
+inline uint32_t grid_for(uint64_t n, int per_block, int sms) {
+    const uint64_t g = (n + per_block - 1) / per_block;
+    const uint64_t cap = (uint64_t)sms * 16u;
+    return (uint32_t)(g < 1 ? 1 : (g > cap ? cap : g));
+}
+}  // namespace
+
 }  // namespace kg

@@ -194,6 +194,18 @@ class DistGraph:
         self._ctx._check(self._lib.kombgpu_dist_graph_format_fetch(self._h, int(which), buf, 0))
         return buf.raw[:n.value]
 
+    def anomalous(self, whisker: float = 1.5) -> dict:
+        """IQR fence on the CORE-A scores of all ranks, the dict of Graph.anomalous on every rank
+        (kombgpu_dist_anomalous; needs corea() first).  `member` is this rank's slice: unitigs [v_lo, v_lo + n_local).
+        Collective."""
+        st = self.stats()
+        member = np.zeros(st["n_local"], np.uint8)
+        q1, q3, fence, ns = c_double(), c_double(), c_double(), c_uint32()
+        self._ctx._check(self._lib.kombgpu_dist_anomalous(self._h, float(whisker), byref(q1), byref(q3), byref(fence), byref(ns),
+                                                          c_void_p(member.ctypes.data)))
+        return {"q1": q1.value, "q3": q3.value, "fence": fence.value, "n_selected": ns.value, "member": member.astype(bool),
+                "v_lo": st["v_lo"]}
+
     def results(self, out: dict | None = None) -> dict:
         """degree / coreness / score of the local unitigs [v_lo, v_lo + n_local) on the host."""
         st = self.stats()
@@ -303,6 +315,72 @@ class DistHits:
     def close(self):
         if getattr(self, "_h", None):
             self._lib.kombgpu_dist_hits_destroy(self._h)
+            self._h = None
+
+    def __enter__(self):
+        return self
+
+    def __exit__(self, *exc):
+        self.close()
+
+
+class DistFasta:
+    """kombgpu_dist_fasta: a FASTA file indexed over the ranks, each holding its slice of the records; the mirror of
+    Fasta.  join() and extract() work on this rank's vertices, and the extraction slices of ranks 0, 1, ... concatenate
+    to Fasta.extract on one GPU."""
+
+    def __init__(self, comm: Comm, handle: c_void_p):
+        self.comm = comm
+        self._ctx = comm.ctx
+        self._lib = comm._lib
+        self._h = handle
+
+    @classmethod
+    def load(cls, comm: Comm, text: bytes) -> "DistFasta":
+        """The bytes of one FASTA file, the same on every rank (kombgpu_dist_fasta_load).  Collective."""
+        text = bytes(text)
+        h = c_void_p()
+        comm.ctx._check(comm._lib.kombgpu_dist_fasta_load(comm._h, text, len(text), byref(h)))
+        return cls(comm, h)
+
+    def counts(self) -> dict:
+        nl, ng, rl, bl, bh = c_uint32(), c_uint32(), c_uint32(), c_uint64(), c_uint64()
+        self._ctx._check(self._lib.kombgpu_dist_fasta_counts(self._h, byref(nl), byref(ng), byref(rl), byref(bl), byref(bh)))
+        return {"n_records_local": nl.value, "n_records": ng.value, "rec_lo": rl.value, "byte_lo": bl.value, "byte_hi": bh.value}
+
+    def join(self, hits: "DistHits | None" = None, names=None) -> int:
+        """vertex -> record by name for this rank's vertices: the names `hits` holds for the unitigs this rank owns, or a
+        host list of this rank's names (bytes).  Returns the vertices without a record over all ranks.  Collective."""
+        if (hits is None) == (names is None):
+            raise ValueError("pass exactly one of hits= and names=")
+        miss = c_uint32()
+        if hits is not None:
+            self._ctx._check(self._lib.kombgpu_dist_fasta_join_hits(self._h, hits._h, byref(miss)))
+        else:
+            names = [bytes(x) for x in names]
+            off = np.zeros(len(names) + 1, np.uint64)
+            np.cumsum([len(x) for x in names], out=off[1:])
+            self._ctx._check(self._lib.kombgpu_dist_fasta_join_names(self._h, b"".join(names), c_void_p(off.ctypes.data), len(names),
+                                                                     byref(miss)))
+        return miss.value
+
+    def extract(self, mask) -> bytes:
+        """This rank's slice of the records of the selected vertices; `mask` covers this rank's vertices.  Collective."""
+        m = np.ascontiguousarray(np.asarray(mask).astype(bool).astype(np.uint8))
+        n = c_uint64()
+        self._ctx._check(self._lib.kombgpu_dist_fasta_extract(self._h, c_void_p(m.ctypes.data), m.shape[0], byref(n)))
+        buf = ctypes.create_string_buffer(max(n.value, 1))
+        self._ctx._check(self._lib.kombgpu_dist_fasta_extract_fetch(self._h, buf))
+        return buf.raw[:n.value]
+
+    def timing(self) -> dict:
+        up, ix, jn, ex, l = c_float(), c_float(), c_float(), c_float(), c_uint64()
+        self._ctx._check(self._lib.kombgpu_dist_fasta_timing(self._h, byref(up), byref(ix), byref(jn), byref(ex), byref(l)))
+        return {"ms_upload": up.value, "ms_index": ix.value, "ms_join": jn.value, "ms_extract": ex.value, "kernel_launches": l.value}
+
+    def close(self):
+        if getattr(self, "_h", None):
+            self._lib.kombgpu_dist_fasta_destroy(self._h)
             self._h = None
 
     def __enter__(self):
