@@ -10,6 +10,7 @@
 //   readEdgeList       :395-453               writes edgelist.txt (simple edges, quirk Q7), prints
 //                                             GraphInfo, calls runCore
 //   runCore            :455-484               degree / coreness (kombgpu_graph_results) -> kcore.tsv
+//                                             with KOMB_ONION=1 also onion.tsv (writeOnion)
 //   anomalyDetection   :637-648               CORE-A scores (kombgpu_graph_results) -> CoreA_anomaly.txt
 //                       (CombineCoreA::run, src/CombineCoreA.h:16-43); with KOMB_UNITIG_FASTA also the
 //                                             records of the anomalous / max-truss unitigs (writeUnitigFasta; over
@@ -175,6 +176,7 @@ class Kgraph {
     }
     std::unique_ptr<PinnedArray<int32_t>> _deg, _core;
     std::unique_ptr<PinnedArray<double>> _score;
+    bool _onion = false;                                    // KOMB_ONION=1: onion.tsv after kcore.tsv
     bool _fasta_anomalous = false, _fasta_truss = false;   // KOMB_UNITIG_FASTA
     std::string _fasta_path;                                // the -u FASTA
     MappedFile _fasta_file;                                 // several GPUs: mapped once, every rank reads its slice
@@ -619,6 +621,7 @@ class Kgraph {
             }
             fclose(kf);
             timing_mark("write kcore.tsv");
+            if (_onion) writeOnion(dir, hits);
             return;
         }
         // fetched by readEdgeList (one GPU) or runMulti (every rank's slice)
@@ -645,6 +648,40 @@ class Kgraph {
         });
         fclose(kcf);
         timing_mark("write kcore.tsv");
+        if (_onion) writeOnion(dir, hits, core);
+    }
+
+    // <dir>/onion.tsv (KOMB_ONION=1, one GPU): the kcore.tsv row with every unitig's onion layer in the fourth column.
+    // Formatted on the device with the other files, else on the host from the layers and the coreness (`core`).
+    void writeOnion(const std::string &dir, const HitTable &hits, const int32_t *core = nullptr) {
+        const std::string path = dir + "/onion.tsv";
+        uint32_t n = 0;
+        kombgpu_graph_counts(_graph, &n, nullptr);
+        std::vector<uint32_t> layer(core ? n : 0);
+        int rc = kombgpu_graph_onion(_graph, core ? layer.data() : nullptr, nullptr);
+        if (rc != KOMBGPU_OK) gpuError("kombgpu_graph_onion", rc);
+        FILE *f = fopen(path.c_str(), "w");
+        if (f == nullptr) fileNotFoundError(path);
+        if (!core) {
+            uint64_t bytes = 0;
+            if ((rc = kombgpu_graph_format(_graph, KOMBGPU_FILE_ONION, _hits, &bytes)) != KOMBGPU_OK) gpuError("kombgpu_graph_format", rc);
+            PinnedArray<char> text(_ctx, bytes);
+            if ((rc = kombgpu_graph_format_fetch(_graph, KOMBGPU_FILE_ONION, text.data(), 0)) != KOMBGPU_OK) gpuError("kombgpu_graph_format_fetch", rc);
+            if (bytes && fwrite(text.data(), 1, bytes, f) != bytes) fileNotFoundError(path);
+        } else {
+            fprintf(f, "#VID\tName\tCoreness\tLayer\n");
+            size_t max_name = 0;
+            for (auto &s : hits.names) max_name = std::max(max_name, s.size());
+            write_rows(f, n, max_name + 40, (int)_threads, [&](char *p, size_t i) {
+                p = put_u64(p, i); *p++ = '\t';
+                memcpy(p, hits.names[i].data(), hits.names[i].size()); p += hits.names[i].size(); *p++ = '\t';
+                p = put_u64(p, (uint64_t)core[i]); *p++ = '\t';
+                p = put_u64(p, layer[i]); *p++ = '\n';
+                return p;
+            });
+        }
+        fclose(f);
+        timing_mark("write onion.tsv");
     }
 
     void anomalyDetection(const std::string &dir, bool weight, const std::string &fasta_path, const HitTable &hits) {
@@ -697,6 +734,8 @@ class Kgraph {
         _graph = nullptr;
         timing_mark("free pinned + graph");
     }
+
+    void setOnion(bool on) { _onion = on; }
 
     // KOMB_UNITIG_FASTA: which unitig FASTA files anomalyDetection writes, from the -u file
     void setUnitigFasta(bool anomalous, bool truss, const std::string &path) {

@@ -19,6 +19,9 @@
 //              of the unitigs on the max-truss edges of the maximal core to <outdir>/truss_unitigs.fasta, indexed, joined
 //              and copied on the device (truss needs one GPU: not with KOMB_GPU_DEVICES).  Unset, the FASTA is only
 //              opened, as the reference does.
+//              KOMB_ONION=1 also writes <outdir>/onion.tsv after kcore.tsv: every unitig's onion layer (the layers of a
+//              synchronous k-core peel, kombgpu_graph_onion) as "#VID\tName\tCoreness\tLayer" rows, formatted where the
+//              other files are (one GPU only: not with KOMB_GPU_DEVICES).
 #include <omp.h>
 
 #include <chrono>
@@ -77,8 +80,23 @@ int main(int argc, const char **argv) {
         }
     }
 
+    bool onion = false;
+    if (const char *on = getenv("KOMB_ONION")) {
+        if (strcmp(on, "1") == 0) onion = true;
+        else if (on[0] && strcmp(on, "0") != 0) {
+            fprintf(stderr, "komb2: KOMB_ONION=%s: expected 1 (write onion.tsv) or 0\n", on);
+            return EXIT_FAILURE;
+        }
+        if (onion && devices.size() > 1) {
+            fprintf(stderr, "komb2: KOMB_ONION=1: onion.tsv needs one GPU (the graph partitioned over KOMB_GPU_DEVICES has no onion "
+                            "layers)\n");
+            return EXIT_FAILURE;
+        }
+    }
+
     komb::Kgraph kg((uint32_t)opt.threads, (uint64_t)opt.readlen, device, key_mode, devices);
     kg.setUnitigFasta(fasta_anomalous, fasta_truss, opt.input_unitigs);
+    kg.setOnion(onion);
     komb::HitTable hits;
     komb::MappedFile sam1, sam2;  // the hit table points into these until the ids exist
     auto begin_komb = std::chrono::steady_clock::now();

@@ -226,13 +226,26 @@ int kombgpu_graph_summary(const kombgpu_graph *g, int32_t *max_coreness, double 
  * edge-list download) overlaps it; kombgpu_graph_format_wait ends the asynchronous copies.  KCORE needs the
  * coreness and the kombgpu_hits the graph was built from (the names live in its copy of the SAM text); COREA
  * needs the scores.  The host issues one write per file. */
-enum { KOMBGPU_FILE_EDGELIST = 0, KOMBGPU_FILE_KCORE = 1, KOMBGPU_FILE_COREA = 2 };
+enum { KOMBGPU_FILE_EDGELIST = 0, KOMBGPU_FILE_KCORE = 1, KOMBGPU_FILE_COREA = 2, KOMBGPU_FILE_ONION = 3 };
 int kombgpu_graph_format(kombgpu_graph *g, int which, const kombgpu_hits *names, uint64_t *bytes);
 int kombgpu_graph_format_fetch(kombgpu_graph *g, int which, char *dst, int async);
 int kombgpu_graph_format_wait(kombgpu_graph *g);
 /* CoreA_anomaly.txt from a host array of scores (finite, |score| < 2^43): *bytes = size of the text; it is
  * copied to dst when it fits `capacity` (else KOMBGPU_EINVAL, *bytes still set). */
 int kombgpu_format_corea(kombgpu_ctx *ctx, const double *score, uint32_t n, char *dst, uint64_t capacity, uint64_t *bytes);
+
+/* ---- onion layers -------------------------------------------------------------------------------------------
+ *
+ * The onion decomposition (Hebert-Dufresne, Grochow & Allard, Sci. Rep. 6:31708, 2016; networkx.onion_layers): every
+ * k-shell split into the layers of a synchronous peel.  Degree-0 vertices, when there are any, form layer 1.  Then,
+ * starting at k = 1: k = max(k, smallest remaining degree); the next layer is every remaining vertex whose degree
+ * among the remaining vertices is <= k; they are removed at once.  The level k a vertex leaves at is its coreness.
+ * layer[n] (1-based; may be NULL) and *n_layers (the largest layer, 0 for an empty graph; may be NULL).  Needs only
+ * the CSR, so it works on every graph (not kombgpu_coreness); computed once per graph and cached with it.
+ * KOMBGPU_FILE_ONION formats onion.tsv: "#VID\tName\tCoreness\tLayer\n" + "%d\t%s\t%d\t%u\n" per unitig, the
+ * kcore.tsv row with the layer in the fourth column; it needs this call and the kombgpu_hits that supply the names,
+ * as KCORE does. */
+int kombgpu_graph_onion(kombgpu_graph *g, uint32_t *layer, uint32_t *n_layers);
 
 /* ---- whole path + introspection --------------------------------------------- */
 

@@ -37,6 +37,12 @@ int kombgpu_debug_dist_build_rounds(const kombgpu_dist_graph *g, uint32_t *n_rou
 int kombgpu_debug_dist_truss_timing(const kombgpu_dist_graph *g, float *ms_core_gather, float *ms_slice_gather,
                                     float *ms_truss);
 
+/* tools/onion_probe.py: run the onion decomposition again on a graph that already holds it, and what the last run
+ * measured: the kernel's CUDA-event time, the non-empty levels, the steps between grid barriers (scans, thin runs
+ * and wide layers) and the layers CTA 0 ran alone.  KOMBGPU_ESTATE before kombgpu_graph_onion.  Any pointer may be NULL. */
+int kombgpu_debug_onion_again(kombgpu_graph *g);
+int kombgpu_debug_onion_timing(const kombgpu_graph *g, float *ms_kernel, uint32_t *levels, uint32_t *steps, uint32_t *thin_layers);
+
 #ifdef __cplusplus
 }
 #endif

@@ -96,6 +96,9 @@ SIGNATURES = {
     "kombgpu_graph_max_core_truss": (c_int, [c_void_p, POINTER(c_uint32), POINTER(c_uint64), POINTER(c_int32), POINTER(c_uint32)]),
     "kombgpu_graph_max_core_edges": (c_int, [c_void_p, c_void_p, c_void_p, c_void_p]),
     "kombgpu_graph_truss_vertices": (c_int, [c_void_p, c_void_p]),
+    "kombgpu_graph_onion": (c_int, [c_void_p, c_void_p, POINTER(c_uint32)]),
+    "kombgpu_debug_onion_again": (c_int, [c_void_p]),
+    "kombgpu_debug_onion_timing": (c_int, [c_void_p, POINTER(c_float), POINTER(c_uint32), POINTER(c_uint32), POINTER(c_uint32)]),
     "kombgpu_graph_results": (c_int, [c_void_p, c_int, c_void_p, c_void_p, c_void_p, c_void_p, c_void_p]),
     "kombgpu_graph_stats": (c_int, [c_void_p, POINTER(Stats)]),
     "kombgpu_graph_device_arrays": (c_int, [c_void_p] + [POINTER(c_void_p)] * 6),

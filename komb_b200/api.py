@@ -459,11 +459,11 @@ class Graph:
     def analyse(self, key_mode: int = KEY_REF32):
         self._ctx._check(self._lib.kombgpu_graph_analyse(self._h, int(key_mode)))
 
-    FILE_EDGELIST, FILE_KCORE, FILE_COREA = 0, 1, 2
+    FILE_EDGELIST, FILE_KCORE, FILE_COREA, FILE_ONION = 0, 1, 2, 3
 
     def format(self, which: int, hits: "Hits | None" = None) -> bytes:
-        """The bytes of edgelist.txt / kcore.tsv / CoreA_anomaly.txt, formatted on the device (kombgpu_graph_format);
-        kcore.tsv takes the unitig names from the Hits the graph was built from."""
+        """The bytes of edgelist.txt / kcore.tsv / CoreA_anomaly.txt / onion.tsv, formatted on the device
+        (kombgpu_graph_format); kcore.tsv and onion.tsv take the unitig names from the Hits the graph was built from."""
         n = c_uint64()
         self._ctx._check(self._lib.kombgpu_graph_format(self._h, int(which), hits._h if hits is not None else None, byref(n)))
         buf = ctypes.create_string_buffer(max(n.value, 1))
@@ -506,6 +506,23 @@ class Graph:
         self._ctx._check(self._lib.kombgpu_graph_truss_vertices(self._h, _ptr(tv)))
         return {"n_core_vertices": nc.value, "n_core_edges": mc.value, "max_trussness": tm.value, "u": u, "v": v, "trussness": tr,
                 "truss_vertices": tv}
+
+    def onion(self, again: bool = False) -> dict:
+        """Onion layers (kombgpu_graph_onion; networkx.onion_layers): the 1-based layer of every vertex and the number of
+        layers.  `again=True` (measurement aid, include/kombgpu_debug.h) runs the decomposition once more."""
+        n, _ = self.counts()
+        if again:
+            self._ctx._check(self._lib.kombgpu_debug_onion_again(self._h))
+        layer, nl = np.empty(n, np.uint32), c_uint32()
+        self._ctx._check(self._lib.kombgpu_graph_onion(self._h, _ptr(layer), byref(nl)))
+        return {"layer": layer, "n_layers": nl.value}
+
+    def onion_timing(self) -> dict:
+        """What the last onion run measured (measurement aid, include/kombgpu_debug.h): kernel time from CUDA events,
+        non-empty levels, steps between grid barriers, layers run by one CTA."""
+        ms, lv, steps, thin = ctypes.c_float(), c_uint32(), c_uint32(), c_uint32()
+        self._ctx._check(self._lib.kombgpu_debug_onion_timing(self._h, byref(ms), byref(lv), byref(steps), byref(thin)))
+        return {"ms_kernel": ms.value, "levels": lv.value, "steps": steps.value, "thin_layers": thin.value}
 
     def anomalous(self, whisker: float = 1.5) -> dict:
         """IQR fence on the graph's own CORE-A scores (kombgpu_graph_anomalous; needs corea() first)."""

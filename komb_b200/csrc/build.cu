@@ -1021,6 +1021,7 @@ void graph_release(kombgpu_graph *g) {
     if (!g || !g->ctx) return;
     kombgpu_ctx *ctx = g->ctx;
     truss_release(g);
+    onion_release(g);
     format_release(g);
     if (g->edges) ws_free(ctx, g->edges);
     if (g->fwd_start) ws_free(ctx, g->fwd_start);

@@ -1,4 +1,4 @@
-// format.cu — the three output files formatted on the device (SURVEY.md section 8, row N2).
+// format.cu — the three output files formatted on the device (SURVEY.md section 8, row N2), and onion.tsv.
 //
 // The reference writes its files with one fprintf per row: edgelist.txt "%d\t%d\n" (src/graph.cpp:423-426),
 // kcore.tsv "#VID\tName\tCoreness\tDegree\n" + "%d\t%s\t%d\t%d\n" (src/graph.cpp:467-475) and CoreA_anomaly.txt
@@ -141,6 +141,39 @@ struct KcoreRowOut {
     }
 };
 
+// ---- onion.tsv: the kcore.tsv row with the layer in the fourth column
+constexpr char kOnionHeader[] = "#VID\tName\tCoreness\tLayer\n";
+constexpr uint64_t kOnionHeaderLen = sizeof(kOnionHeader) - 1;
+struct OnionRowLen {
+    const uint32_t *name_len;
+    const int32_t *core;
+    const uint32_t *layer;
+    __device__ uint64_t operator()(uint64_t i) const {
+        return digits_u32((uint32_t)i) + name_len[i] + digits_i32(core[i]) + digits_u32(layer[i]) + 4u;
+    }
+};
+struct OnionRowOut {
+    const unsigned char *names;
+    const uint64_t *name_off;
+    const uint32_t *name_len;
+    const int32_t *core;
+    const uint32_t *layer;
+    char *text;
+    __device__ void operator()(uint64_t i, uint64_t at, uint64_t) const {
+        char *p = put_u32(text + kOnionHeaderLen + at, (uint32_t)i, digits_u32((uint32_t)i));
+        *p++ = '\t';
+        const unsigned char *nm = names + name_off[i];
+        const uint32_t nl = name_len[i];
+        for (uint32_t k = 0; k < nl; ++k) p[k] = (char)nm[k];
+        p += nl;
+        *p++ = '\t';
+        p = put_i32(p, core[i]);
+        *p++ = '\t';
+        p = put_u32(p, layer[i], digits_u32(layer[i]));
+        *p = '\n';
+    }
+};
+
 // ---- CoreA_anomaly.txt (row i is unitig id0 + i)
 struct ScoreRowLen {
     const double *score;
@@ -198,6 +231,11 @@ KcoreRowOut make_kcore_out(char *text, void *arg) {
     const KcoreArgs *a = static_cast<const KcoreArgs *>(arg);
     return KcoreRowOut{a->names, a->off, a->len, a->core, a->deg, text, a->base, a->id0};
 }
+struct OnionArgs { const unsigned char *names; const uint64_t *off; const uint32_t *len; const int32_t *core; const uint32_t *layer; };
+OnionRowOut make_onion_out(char *text, void *arg) {
+    const OnionArgs *a = static_cast<const OnionArgs *>(arg);
+    return OnionRowOut{a->names, a->off, a->len, a->core, a->layer, text};
+}
 struct ScoreArgs { const double *score; uint32_t id0; };
 ScoreRowOut make_score_out(char *text, void *arg) {
     const ScoreArgs *a = static_cast<const ScoreArgs *>(arg);
@@ -242,8 +280,8 @@ int fetch_text(kombgpu_ctx *ctx, const char *text, uint64_t bytes, char *dst, in
     return KOMBGPU_OK;
 }
 
-void release_texts(kombgpu_ctx *ctx, char **text, uint64_t *text_bytes) {
-    for (int w = 0; w < 3; ++w) {
+void release_texts(kombgpu_ctx *ctx, char **text, uint64_t *text_bytes, int n_files) {
+    for (int w = 0; w < n_files; ++w) {
         if (text[w]) ws_free(ctx, text[w]);
         text[w] = nullptr;
         text_bytes[w] = 0;
@@ -252,8 +290,8 @@ void release_texts(kombgpu_ctx *ctx, char **text, uint64_t *text_bytes) {
 
 }  // namespace
 
-void format_release(kombgpu_graph *g) { release_texts(g->ctx, g->text, g->text_bytes); }
-void dist_format_release(kombgpu_dist_graph *g) { release_texts(g->ctx, g->text, g->text_bytes); }
+void format_release(kombgpu_graph *g) { release_texts(g->ctx, g->text, g->text_bytes, 4); }
+void dist_format_release(kombgpu_dist_graph *g) { release_texts(g->ctx, g->text, g->text_bytes, 3); }
 
 }  // namespace kg
 
@@ -264,7 +302,7 @@ extern "C" {
 int kombgpu_graph_format(kombgpu_graph *g, int which, const kombgpu_hits *names, uint64_t *bytes) {
     if (!g) return KOMBGPU_EINVAL;
     kombgpu_ctx *ctx = g->ctx;
-    if (!bytes || which < 0 || which > 2) return ctx_fail(ctx, KOMBGPU_EINVAL, "bad argument");
+    if (!bytes || which < 0 || which > KOMBGPU_FILE_ONION) return ctx_fail(ctx, KOMBGPU_EINVAL, "bad argument");
     KG_CUDA(ctx, cudaSetDevice(ctx->device));
     if (g->text[which]) { *bytes = g->text_bytes[which]; return KOMBGPU_OK; }
     const uint64_t launches0 = ctx->launches;
@@ -285,6 +323,17 @@ int kombgpu_graph_format(kombgpu_graph *g, int which, const kombgpu_hits *names,
         a.base = kKcoreHeaderLen;
         KG_TRY(format_rows(ctx, g->n, KcoreRowLen{a.len, a.core, a.deg, 0u}, make_kcore_out, &a, kKcoreHeaderLen, &text, &total));
         KG_CUDA(ctx, cudaMemcpyAsync(text, kKcoreHeader, kKcoreHeaderLen, cudaMemcpyHostToDevice, ctx->stream));
+    } else if (which == KOMBGPU_FILE_ONION) {
+        if (!g->has_onion) return ctx_fail(ctx, KOMBGPU_ESTATE, "kombgpu_graph_onion has not run");
+        kombgpu_ctx *hctx = nullptr;
+        OnionArgs a{};
+        uint32_t n_names = 0;
+        if (!names || hits_name_spans(names, &hctx, &a.names, &a.off, &a.len, &n_names) != KOMBGPU_OK || hctx != ctx || n_names != g->n)
+            return ctx_fail(ctx, KOMBGPU_EINVAL, "onion.tsv needs the unitig names: the kombgpu_hits this graph was built from");
+        a.core = g->onion_core;
+        a.layer = g->onion_layer;
+        KG_TRY(format_rows(ctx, g->n, OnionRowLen{a.len, a.core, a.layer}, make_onion_out, &a, kOnionHeaderLen, &text, &total));
+        KG_CUDA(ctx, cudaMemcpyAsync(text, kOnionHeader, kOnionHeaderLen, cudaMemcpyHostToDevice, ctx->stream));
     } else {
         if (!g->has_score) return ctx_fail(ctx, KOMBGPU_ESTATE, "kombgpu_graph_corea has not run");
         KG_TRY(format_scores(ctx, g->score, g->n, 0u, &text, &total));
@@ -299,7 +348,7 @@ int kombgpu_graph_format(kombgpu_graph *g, int which, const kombgpu_hits *names,
 int kombgpu_graph_format_fetch(kombgpu_graph *g, int which, char *dst, int async) {
     if (!g) return KOMBGPU_EINVAL;
     kombgpu_ctx *ctx = g->ctx;
-    if (which < 0 || which > 2 || !g->text[which]) return ctx_fail(ctx, KOMBGPU_ESTATE, "kombgpu_graph_format has not run for this file");
+    if (which < 0 || which > KOMBGPU_FILE_ONION || !g->text[which]) return ctx_fail(ctx, KOMBGPU_ESTATE, "kombgpu_graph_format has not run for this file");
     return fetch_text(ctx, g->text[which], g->text_bytes[which], dst, async);
 }
 

@@ -15,6 +15,11 @@ struct MaxCoreTruss {
     int32_t *truss = nullptr;       // [m]
     uint32_t *vertices = nullptr;   // [n_vertices] original ids of the unitigs on edges of maximal trussness
 };
+// what the last onion run measured (onion.cu; kombgpu_debug_onion_timing)
+struct OnionInfo {
+    float ms_kernel = 0.f;
+    uint32_t levels = 0, steps = 0, thin_layers = 0;
+};
 }  // namespace kg
 
 struct kombgpu_graph {
@@ -35,9 +40,15 @@ struct kombgpu_graph {
     kombgpu_stats st{};
     bool has_truss = false;
     kg::MaxCoreTruss tr;
-    // output files formatted on the device (format.cu): edgelist.txt, kcore.tsv, CoreA_anomaly.txt
-    char *text[3] = {nullptr, nullptr, nullptr};
-    uint64_t text_bytes[3] = {0, 0, 0};
+    // onion layers (onion.cu), computed on demand
+    bool has_onion = false;
+    uint32_t *onion_layer = nullptr;   // [n] 1-based layer of every vertex
+    int32_t *onion_core = nullptr;     // [n] the level each vertex left at: its coreness (onion.tsv's third column)
+    uint32_t onion_n_layers = 0;
+    kg::OnionInfo onion_info;
+    // output files formatted on the device (format.cu): edgelist.txt, kcore.tsv, CoreA_anomaly.txt, onion.tsv
+    char *text[4] = {nullptr, nullptr, nullptr, nullptr};
+    uint64_t text_bytes[4] = {0, 0, 0, 0};
 };
 
 namespace kg {
@@ -112,6 +123,10 @@ int adopt_csr(kombgpu_ctx *ctx, const uint64_t *row_ptr, const uint32_t *col, ui
 
 // stage 2 (peel.cu)
 int peel_coreness(kombgpu_graph *g);
+
+// onion layers (onion.cu): layer[] and the number of layers into the graph's cache
+int onion_layers(kombgpu_graph *g);
+void onion_release(kombgpu_graph *g);
 
 // stage 3 (corea.cu) — device pointers in, device score out; *max_score on host
 int corea_scores(kombgpu_ctx *ctx, const int32_t *core, const int32_t *deg, uint32_t n, int key_mode, double *score,
