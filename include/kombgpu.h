@@ -616,13 +616,26 @@ int kombgpu_dist_build_graph_hits(const kombgpu_dist_hits *h, kombgpu_dist_graph
  * canonical edge list (needs the build); KCORE: rows v_lo .. v_lo + n_local - 1, rank 0's slice starting with the
  * header even when the graph is empty (needs kombgpu_dist_coreness and the kombgpu_dist_hits the graph was built
  * from: the parse leaves every name's bytes on the rank that owns its vertex); COREA: the same rows (needs
- * kombgpu_dist_corea).  Local, NOT collective: a rank formats and fetches when it likes and waits for no other.
- * KOMBGPU_ESTATE for a file whose stage has not run, or a fetch before the format; KOMBGPU_EINVAL for `which` out of
- * range or a KCORE names handle that is missing or belongs to another communicator or partition.  The text is
- * cached in the graph until it is destroyed; fetch and wait work as kombgpu_graph_format_fetch / _wait. */
+ * kombgpu_dist_corea); ONION: the same rows of onion.tsv, rank 0's slice starting with its header even when the graph
+ * is empty (needs kombgpu_dist_onion and the names as KCORE does; a names handle that is missing or foreign is
+ * KOMBGPU_EINVAL before the onion's state is looked at).  Local, NOT collective: a rank formats and fetches when it
+ * likes and waits for no other.  KOMBGPU_ESTATE for a file whose stage has not run, or a fetch before the format;
+ * KOMBGPU_EINVAL for `which` out of range or a KCORE / ONION names handle that is missing or belongs to another
+ * communicator or partition.  The text is cached in the graph until it is destroyed; fetch and wait work as
+ * kombgpu_graph_format_fetch / _wait. */
 int kombgpu_dist_graph_format(kombgpu_dist_graph *g, int which, const kombgpu_dist_hits *names, uint64_t *bytes);
 int kombgpu_dist_graph_format_fetch(kombgpu_dist_graph *g, int which, char *dst, int async);
 int kombgpu_dist_graph_format_wait(kombgpu_dist_graph *g);
+
+/* Onion layers over the ranks: the rules of kombgpu_graph_onion, computed by a peel whose steps are exactly the layers
+ * (one meeting of all ranks per layer).  layer: this rank's slice, n_local entries for unitigs [v_lo, v_lo + n_local),
+ * or NULL; *n_layers (may be NULL): the number of layers of the whole graph, the same on every rank.  The slices of
+ * ranks 0, 1, ... concatenate to exactly what kombgpu_graph_onion gives on one GPU for the same graph.  Needs only the
+ * build, whichever layout it left.  The first call is collective; the result (and the coreness each unitig left at,
+ * for onion.tsv) is cached in the graph until it is destroyed, and later calls are local.  A broken invariant gives
+ * KOMBGPU_EINTERNAL on every rank; any other failure on one rank makes every rank return an error; the contexts, the
+ * communicator and the graph stay usable. */
+int kombgpu_dist_onion(kombgpu_dist_graph *g, uint32_t *layer, uint32_t *n_layers);
 
 /* The unitig FASTA over the ranks: the rules of the single-GPU "unitig FASTA" section above (records, names, join, fence,
  * extraction), with the same results and the same error messages (record numbers, byte offsets and vertex ids are

@@ -43,6 +43,15 @@ int kombgpu_debug_dist_truss_timing(const kombgpu_dist_graph *g, float *ms_core_
 int kombgpu_debug_onion_again(kombgpu_graph *g);
 int kombgpu_debug_onion_timing(const kombgpu_graph *g, float *ms_kernel, uint32_t *levels, uint32_t *steps, uint32_t *thin_layers);
 
+/* tools/dist_onion_probe.py: run the partitioned onion again on a graph that already holds it (collective), and what
+ * this rank's last run measured: the kernel's CUDA-event time (in the one-device emulation, the grid that holds every
+ * rank), the non-empty levels, the meetings of all ranks, the walk steps this rank ran on one CTA, and the time of the
+ * by-neighbour layout built from rows (0 when the build left that layout).  KOMBGPU_ESTATE before kombgpu_dist_onion.
+ * Any pointer may be NULL. */
+int kombgpu_debug_dist_onion_again(kombgpu_dist_graph *g);
+int kombgpu_debug_dist_onion_timing(const kombgpu_dist_graph *g, float *ms_kernel, uint32_t *levels, uint32_t *meetings,
+                                    uint32_t *solo_steps, float *ms_transpose);
+
 #ifdef __cplusplus
 }
 #endif

@@ -99,6 +99,9 @@ SIGNATURES = {
     "kombgpu_graph_onion": (c_int, [c_void_p, c_void_p, POINTER(c_uint32)]),
     "kombgpu_debug_onion_again": (c_int, [c_void_p]),
     "kombgpu_debug_onion_timing": (c_int, [c_void_p, POINTER(c_float), POINTER(c_uint32), POINTER(c_uint32), POINTER(c_uint32)]),
+    "kombgpu_debug_dist_onion_again": (c_int, [c_void_p]),
+    "kombgpu_debug_dist_onion_timing": (c_int, [c_void_p, POINTER(c_float), POINTER(c_uint32), POINTER(c_uint32), POINTER(c_uint32),
+                                                POINTER(c_float)]),
     "kombgpu_graph_results": (c_int, [c_void_p, c_int, c_void_p, c_void_p, c_void_p, c_void_p, c_void_p]),
     "kombgpu_graph_stats": (c_int, [c_void_p, POINTER(Stats)]),
     "kombgpu_graph_device_arrays": (c_int, [c_void_p] + [POINTER(c_void_p)] * 6),
@@ -182,6 +185,7 @@ SIGNATURES = {
     "kombgpu_dist_graph_format": (c_int, [c_void_p, c_int, c_void_p, POINTER(c_uint64)]),
     "kombgpu_dist_graph_format_fetch": (c_int, [c_void_p, c_int, c_void_p, c_int]),
     "kombgpu_dist_graph_format_wait": (c_int, [c_void_p]),
+    "kombgpu_dist_onion": (c_int, [c_void_p, c_void_p, POINTER(c_uint32)]),
     "kombgpu_dist_fasta_load": (c_int, [c_void_p, c_char_p, c_uint64, POINTER(c_void_p)]),
     "kombgpu_dist_fasta_destroy": (None, [c_void_p]),
     "kombgpu_dist_fasta_counts": (c_int, [c_void_p, POINTER(c_uint32), POINTER(c_uint32), POINTER(c_uint32), POINTER(c_uint64),

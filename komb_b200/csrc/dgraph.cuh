@@ -5,6 +5,14 @@
 #include "comm.cuh"
 #include "graph.cuh"
 
+namespace kg {
+// what the last partitioned onion run measured (ponion.cu; kombgpu_debug_dist_onion_timing)
+struct DistOnionInfo {
+    float ms_kernel = 0.f, ms_transpose = 0.f;   // ms_transpose: the by-neighbour layout built from rows (0 when the build left it)
+    uint32_t levels = 0, meetings = 0, solo_steps = 0;
+};
+}  // namespace kg
+
 // Sizes and device timings of one rank's share (kombgpu_dist_graph_stats)
 struct kombgpu_dist_graph {
     kombgpu_comm *comm = nullptr;
@@ -38,9 +46,16 @@ struct kombgpu_dist_graph {
     bool has_truss = false;
     kg::MaxCoreTruss tr;
     float ms_truss[3] = {0.f, 0.f, 0.f};   // CUDA-event times: coreness gather, selection + slice gather, truss peel
-    // this rank's slices of the three output files, formatted on the device (format.cu), cached until destroy
-    char *text[3] = {nullptr, nullptr, nullptr};
-    uint64_t text_bytes[3] = {0, 0, 0};
+    // onion layers of this rank's unitigs (ponion.cu), computed on demand and cached until destroy
+    bool has_onion = false;
+    uint32_t *onion_layer = nullptr;   // [n_local] 1-based layer, numbered over the whole graph
+    int32_t *onion_core = nullptr;     // [n_local] the level each unitig left at (its coreness)
+    uint32_t onion_n_layers = 0;       // global
+    kg::DistOnionInfo onion_info;
+    // this rank's slices of the output files (edgelist.txt, kcore.tsv, CoreA_anomaly.txt, onion.tsv), formatted on the
+    // device (format.cu), cached until destroy
+    char *text[4] = {nullptr, nullptr, nullptr, nullptr};
+    uint64_t text_bytes[4] = {0, 0, 0, 0};
     kombgpu_dist_stats st{};
 };
 
@@ -63,12 +78,21 @@ int dist_peel(kombgpu_dist_graph *g);
 int dist_peel_async(kombgpu_dist_graph *g);
 // rpeel.cu
 int dist_peel_replicated(kombgpu_dist_graph *g);
+// ponion.cu: onion layers over the ranks (collective); the cached result is freed by dist_onion_release
+int dist_onion(kombgpu_dist_graph *g);
+void dist_onion_release(kombgpu_dist_graph *g);
+// pbuild.cu: the by-neighbour layout (nbr_ptr / nbr, as a build for the log-based peel leaves it) of a build that holds
+// rows: their transpose, built locally
+int dist_rows_to_nbr(kombgpu_dist_graph *g, DevBuf<uint32_t> &nbr_ptr, DevBuf<uint32_t> &nbr);
 // which peel a build prepares for (pbuild.cu): KOMBGPU_DIST_PEEL = log (ranks meet once per cascade generation, ppeel.cu),
 // async (apeel.cu), replicated (rpeel.cu) or auto (default: by the shape of the graph).  0 log, 1 async, 2 auto, 3 replicated.
 int dist_peel_mode();
 // pcorea.cu
 int dist_corea(kombgpu_dist_graph *g, int key_mode);
-// pcore.cu: the consumers of the finished coreness
+// pcore.cu: comm_exchange of k words per rank (out[q * k + j]) that also carries every rank's status rc: a rank that
+// failed returns its own code, the others fail with the code of the first failing rank
+int exchange_rc(kombgpu_comm *c, int rc, const unsigned long long *vals, int k, unsigned long long *out);
+// the consumers of the finished coreness
 int dist_max_core_truss(kombgpu_dist_graph *g);
 int dist_densest_core(kombgpu_dist_graph *g, DensestCore *out);
 // weight: this rank's slice (host, or NULL); member: this rank's slice (host, n_local bytes, or NULL)

@@ -148,8 +148,9 @@ struct OnionRowLen {
     const uint32_t *name_len;
     const int32_t *core;
     const uint32_t *layer;
+    uint32_t id0;
     __device__ uint64_t operator()(uint64_t i) const {
-        return digits_u32((uint32_t)i) + name_len[i] + digits_i32(core[i]) + digits_u32(layer[i]) + 4u;
+        return digits_u32(id0 + (uint32_t)i) + name_len[i] + digits_i32(core[i]) + digits_u32(layer[i]) + 4u;
     }
 };
 struct OnionRowOut {
@@ -159,8 +160,11 @@ struct OnionRowOut {
     const int32_t *core;
     const uint32_t *layer;
     char *text;
+    uint64_t base;
+    uint32_t id0;
     __device__ void operator()(uint64_t i, uint64_t at, uint64_t) const {
-        char *p = put_u32(text + kOnionHeaderLen + at, (uint32_t)i, digits_u32((uint32_t)i));
+        const uint32_t id = id0 + (uint32_t)i;
+        char *p = put_u32(text + base + at, id, digits_u32(id));
         *p++ = '\t';
         const unsigned char *nm = names + name_off[i];
         const uint32_t nl = name_len[i];
@@ -231,10 +235,18 @@ KcoreRowOut make_kcore_out(char *text, void *arg) {
     const KcoreArgs *a = static_cast<const KcoreArgs *>(arg);
     return KcoreRowOut{a->names, a->off, a->len, a->core, a->deg, text, a->base, a->id0};
 }
-struct OnionArgs { const unsigned char *names; const uint64_t *off; const uint32_t *len; const int32_t *core; const uint32_t *layer; };
+struct OnionArgs {
+    const unsigned char *names;
+    const uint64_t *off;
+    const uint32_t *len;
+    const int32_t *core;
+    const uint32_t *layer;
+    uint64_t base;
+    uint32_t id0;
+};
 OnionRowOut make_onion_out(char *text, void *arg) {
     const OnionArgs *a = static_cast<const OnionArgs *>(arg);
-    return OnionRowOut{a->names, a->off, a->len, a->core, a->layer, text};
+    return OnionRowOut{a->names, a->off, a->len, a->core, a->layer, text, a->base, a->id0};
 }
 struct ScoreArgs { const double *score; uint32_t id0; };
 ScoreRowOut make_score_out(char *text, void *arg) {
@@ -291,7 +303,7 @@ void release_texts(kombgpu_ctx *ctx, char **text, uint64_t *text_bytes, int n_fi
 }  // namespace
 
 void format_release(kombgpu_graph *g) { release_texts(g->ctx, g->text, g->text_bytes, 4); }
-void dist_format_release(kombgpu_dist_graph *g) { release_texts(g->ctx, g->text, g->text_bytes, 3); }
+void dist_format_release(kombgpu_dist_graph *g) { release_texts(g->ctx, g->text, g->text_bytes, 4); }
 
 }  // namespace kg
 
@@ -332,7 +344,8 @@ int kombgpu_graph_format(kombgpu_graph *g, int which, const kombgpu_hits *names,
             return ctx_fail(ctx, KOMBGPU_EINVAL, "onion.tsv needs the unitig names: the kombgpu_hits this graph was built from");
         a.core = g->onion_core;
         a.layer = g->onion_layer;
-        KG_TRY(format_rows(ctx, g->n, OnionRowLen{a.len, a.core, a.layer}, make_onion_out, &a, kOnionHeaderLen, &text, &total));
+        a.base = kOnionHeaderLen;
+        KG_TRY(format_rows(ctx, g->n, OnionRowLen{a.len, a.core, a.layer, 0u}, make_onion_out, &a, kOnionHeaderLen, &text, &total));
         KG_CUDA(ctx, cudaMemcpyAsync(text, kOnionHeader, kOnionHeaderLen, cudaMemcpyHostToDevice, ctx->stream));
     } else {
         if (!g->has_score) return ctx_fail(ctx, KOMBGPU_ESTATE, "kombgpu_graph_corea has not run");
@@ -386,7 +399,7 @@ int kombgpu_format_corea(kombgpu_ctx *ctx, const double *score, uint32_t n, char
 int kombgpu_dist_graph_format(kombgpu_dist_graph *g, int which, const kombgpu_dist_hits *names, uint64_t *bytes) {
     if (!g) return KOMBGPU_EINVAL;
     kombgpu_ctx *ctx = g->ctx;
-    if (!bytes || which < 0 || which > 2) return ctx_fail(ctx, KOMBGPU_EINVAL, "bad argument");
+    if (!bytes || which < 0 || which > KOMBGPU_FILE_ONION) return ctx_fail(ctx, KOMBGPU_EINVAL, "bad argument");
     KG_CUDA(ctx, cudaSetDevice(ctx->device));
     if (g->text[which]) { *bytes = g->text_bytes[which]; return KOMBGPU_OK; }
     char *text = nullptr;
@@ -404,6 +417,17 @@ int kombgpu_dist_graph_format(kombgpu_dist_graph *g, int which, const kombgpu_di
         KcoreArgs a{nm.bytes, nm.off, nm.len, g->core, g->deg, head, g->v_lo};
         KG_TRY(format_rows(ctx, g->n_local, KcoreRowLen{a.len, a.core, a.deg, g->v_lo}, make_kcore_out, &a, head, &text, &total));
         if (head) KG_CUDA(ctx, cudaMemcpyAsync(text, kKcoreHeader, kKcoreHeaderLen, cudaMemcpyHostToDevice, ctx->stream));
+    } else if (which == KOMBGPU_FILE_ONION) {
+        // the names are checked before the state: a call without the graph's own names is wrong whenever it comes
+        DistNames nm{};
+        if (!names || dist_hits_name_text(names, &nm) != KOMBGPU_OK || nm.comm != g->comm || nm.n_unitigs != g->n_global || nm.v_lo != g->v_lo ||
+            nm.n_local != g->n_local)
+            return ctx_fail(ctx, KOMBGPU_EINVAL, "onion.tsv needs the unitig names: the kombgpu_dist_hits this graph was built from");
+        if (!g->has_onion) return ctx_fail(ctx, KOMBGPU_ESTATE, "kombgpu_dist_onion has not run");
+        const uint64_t head = g->comm->rank == 0 ? kOnionHeaderLen : 0;
+        OnionArgs a{nm.bytes, nm.off, nm.len, g->onion_core, g->onion_layer, head, g->v_lo};
+        KG_TRY(format_rows(ctx, g->n_local, OnionRowLen{a.len, a.core, a.layer, g->v_lo}, make_onion_out, &a, head, &text, &total));
+        if (head) KG_CUDA(ctx, cudaMemcpyAsync(text, kOnionHeader, kOnionHeaderLen, cudaMemcpyHostToDevice, ctx->stream));
     } else {
         if (!g->has_score) return ctx_fail(ctx, KOMBGPU_ESTATE, "kombgpu_dist_corea has not run");
         KG_TRY(format_scores(ctx, g->score, g->n_local, g->v_lo, &text, &total));
@@ -416,7 +440,7 @@ int kombgpu_dist_graph_format(kombgpu_dist_graph *g, int which, const kombgpu_di
 
 int kombgpu_dist_graph_format_fetch(kombgpu_dist_graph *g, int which, char *dst, int async) {
     if (!g) return KOMBGPU_EINVAL;
-    if (which < 0 || which > 2 || !g->text[which]) return ctx_fail(g->ctx, KOMBGPU_ESTATE, "kombgpu_dist_graph_format has not run for this file");
+    if (which < 0 || which > KOMBGPU_FILE_ONION || !g->text[which]) return ctx_fail(g->ctx, KOMBGPU_ESTATE, "kombgpu_dist_graph_format has not run for this file");
     return fetch_text(g->ctx, g->text[which], g->text_bytes[which], dst, async);
 }
 

@@ -182,6 +182,19 @@ __global__ void __launch_bounds__(kThreads) low_words_kernel(const uint64_t *__r
     for (uint64_t i = (uint64_t)blockIdx.x * blockDim.x + threadIdx.x; i < n; i += (uint64_t)gridDim.x * blockDim.x) out[i] = (uint32_t)keys[i];
 }
 
+// key (col[e] << 32 | u) for every entry e of local row u: the rows keyed by neighbour
+__global__ void __launch_bounds__(kThreads) row_keys_kernel(const uint32_t *__restrict__ row_ptr, const uint32_t *__restrict__ col, uint32_t n_local,
+                                                            uint64_t n, uint64_t *__restrict__ keys) {
+    for (uint64_t i = (uint64_t)blockIdx.x * blockDim.x + threadIdx.x; i < n; i += (uint64_t)gridDim.x * blockDim.x) {
+        uint32_t lo = 0, hi = n_local;   // the last row that starts at or before i
+        while (hi - lo > 1) {
+            const uint32_t mid = (lo + hi) >> 1;
+            if (row_ptr[mid] <= i) lo = mid; else hi = mid;
+        }
+        keys[i] = ((uint64_t)col[i] << 32) | lo;
+    }
+}
+
 }  // namespace
 
 // KOMBGPU_DIST_PEEL = async | log | auto (default).  The asynchronous peel (apeel.cu) decrements a neighbour where it
@@ -477,6 +490,32 @@ int dist_build(kombgpu_comm *c, const uint32_t *a, const uint32_t *b, uint64_t c
     return KOMBGPU_OK;
 }
 
+int dist_rows_to_nbr(kombgpu_dist_graph *g, DevBuf<uint32_t> &nbr_ptr, DevBuf<uint32_t> &nbr) {
+    kombgpu_ctx *ctx = g->ctx;
+    const uint64_t n_dir = g->n_directed;
+    const uint32_t n_local = g->n_local, n_global = g->n_global;
+    DevBuf<uint64_t> keys_a, keys_b;
+    DevBuf<uint32_t> d_err(ctx, 1);
+    if (!d_err) return ctx_fail(ctx, KOMBGPU_ENOMEM, "workspace");
+    KG_ALLOC(ctx, keys_a, n_dir);
+    KG_ALLOC(ctx, keys_b, n_dir);
+    KG_CUDA(ctx, cudaMemsetAsync(d_err.p, 0, sizeof(uint32_t), ctx->stream));
+    if (n_dir) KG_LAUNCH(ctx, row_keys_kernel, min(grid_for(n_dir, kThreads), 148u * 16u), kThreads, 0, g->row_ptr32, g->col, n_local, n_dir, keys_a.p);
+    // the sort, the row starts and the low words of dist_build's by-neighbour layout
+    uint64_t *nsorted = keys_a.p;
+    RadixPass passes[8];
+    const int np = plan_radix_passes(32, 32 + bits_for(n_global > 0 ? n_global - 1 : 0), 0, 0, passes);
+    KG_TRY(radix_sort_u64(ctx, keys_a.p, keys_b.p, n_dir, passes, np, &nsorted));
+    KG_ALLOC(ctx, nbr_ptr, (size_t)n_global + 1);
+    KG_ALLOC(ctx, nbr, n_dir);
+    KG_TRY(row_starts(ctx, nsorted, n_dir, 0u, n_global, n_local ? n_local : 1u, nbr_ptr.p, d_err.p));
+    if (n_dir) KG_LAUNCH(ctx, low_words_kernel, min(grid_for(n_dir, kThreads), 148u * 16u), kThreads, 0, nsorted, n_dir, nbr.p);
+    uint32_t h_err = 0;
+    KG_TRY(read_back(ctx, d_err.p, &h_err, 1));
+    if (h_err) return ctx_fail(ctx, KOMBGPU_EINTERNAL, "the rows hold an entry outside the graph");
+    return KOMBGPU_OK;
+}
+
 void dist_graph_release(kombgpu_dist_graph *g) {
     if (!g || !g->ctx) return;
     kombgpu_ctx *ctx = g->ctx;
@@ -487,6 +526,7 @@ void dist_graph_release(kombgpu_dist_graph *g) {
     g->deg = nullptr; g->core = nullptr; g->score = nullptr;
     truss_free(ctx, &g->tr);
     g->has_truss = false;
+    dist_onion_release(g);
     dist_format_release(g);
 }
 

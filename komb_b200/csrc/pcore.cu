@@ -40,6 +40,8 @@ int cuda_rc(kombgpu_ctx *ctx, cudaError_t e, const char *what) {
     return e == cudaSuccess ? KOMBGPU_OK : ctx_fail(ctx, KOMBGPU_ECUDA, "%s: %s", what, cudaGetErrorString(e));
 }
 
+}  // namespace
+
 // comm_exchange of k words per rank (out[q * k + j]) that also carries every rank's status `rc`
 int exchange_rc(kombgpu_comm *c, int rc, const unsigned long long *vals, int k, unsigned long long *out) {
     unsigned long long mine[kCtlWords], all[kMaxRanks * kCtlWords];
@@ -53,6 +55,8 @@ int exchange_rc(kombgpu_comm *c, int rc, const unsigned long long *vals, int k, 
         if (all[q * (k + 1)]) return ctx_fail(c->ctx, -(int)all[q * (k + 1)], "rank %d failed; the call stopped on every rank", q);
     return KOMBGPU_OK;
 }
+
+namespace {
 
 int barrier_rc(kombgpu_comm *c, int rc) { return exchange_rc(c, rc, nullptr, 0, nullptr); }
 

@@ -182,12 +182,32 @@ class DistGraph:
         return {"n_vertices": nv.value, "n_edges": ne.value, "weight_sum": ws.value, "density": d.value, "passes": np_.value,
                 "member": member.astype(bool), "v_lo": st["v_lo"]}
 
-    FILE_EDGELIST, FILE_KCORE, FILE_COREA = 0, 1, 2
+    def onion(self, again: bool = False) -> dict:
+        """Onion layers over the ranks (kombgpu_dist_onion): `layer` is this rank's slice, the 1-based layer of unitigs
+        [v_lo, v_lo + n_local); the slices of ranks 0, 1, ... concatenate to Graph.onion()["layer"] on one GPU, and
+        `n_layers` is the number of layers of the whole graph.  The first call is collective and the result is cached;
+        again=True runs it again (collective; measurement aid)."""
+        n = self.stats()["n_local"]
+        if again:
+            self._ctx._check(self._lib.kombgpu_debug_dist_onion_again(self._h))
+        layer, nl = np.empty(n, np.uint32), c_uint32()
+        self._ctx._check(self._lib.kombgpu_dist_onion(self._h, c_void_p(layer.ctypes.data) if n else None, byref(nl)))
+        return {"layer": layer, "n_layers": nl.value, "v_lo": self.stats()["v_lo"]}
+
+    def onion_timing(self) -> dict:
+        """What this rank's last onion run measured (measurement aid, include/kombgpu_debug.h): kernel time from CUDA
+        events, non-empty levels, meetings of all ranks, walk steps run on one CTA, and the time of the by-neighbour
+        layout built from rows (0.0 when the build left that layout)."""
+        ms, lv, mt, so, tr = c_float(), c_uint32(), c_uint32(), c_uint32(), c_float()
+        self._ctx._check(self._lib.kombgpu_debug_dist_onion_timing(self._h, byref(ms), byref(lv), byref(mt), byref(so), byref(tr)))
+        return {"ms_kernel": ms.value, "levels": lv.value, "meetings": mt.value, "solo_steps": so.value, "ms_transpose": tr.value}
+
+    FILE_EDGELIST, FILE_KCORE, FILE_COREA, FILE_ONION = 0, 1, 2, 3
 
     def format(self, which: int, hits: "DistHits | None" = None) -> bytes:
-        """This rank's slice of edgelist.txt / kcore.tsv / CoreA_anomaly.txt, formatted on its device
+        """This rank's slice of edgelist.txt / kcore.tsv / CoreA_anomaly.txt / onion.tsv, formatted on its device
         (kombgpu_dist_graph_format): the slices of ranks 0, 1, ... concatenate to Graph.format on one GPU.  kcore.tsv
-        takes the unitig names from the DistHits the graph was built from.  Local, not collective."""
+        and onion.tsv take the unitig names from the DistHits the graph was built from.  Local, not collective."""
         n = c_uint64()
         self._ctx._check(self._lib.kombgpu_dist_graph_format(self._h, int(which), hits._h if hits is not None else None, byref(n)))
         buf = ctypes.create_string_buffer(max(n.value, 1))
