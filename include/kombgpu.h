@@ -522,8 +522,11 @@ int kombgpu_dist_build_hits(kombgpu_comm *comm, const uint32_t *read_key, const 
                             uint32_t n_vertices_global, kombgpu_dist_graph **out);
 int kombgpu_dist_build_pairs(kombgpu_comm *comm, const uint32_t *u, const uint32_t *v, uint64_t n_pairs,
                              uint32_t n_vertices_global, kombgpu_dist_graph **out);
-int kombgpu_dist_coreness(kombgpu_dist_graph *g);               /* igraph_coreness over all ranks */
-int kombgpu_dist_corea(kombgpu_dist_graph *g, int key_mode);    /* CoreA::getAnomalyScore over all ranks */
+/* igraph_coreness and CoreA::getAnomalyScore over all ranks.  Collective.  A key_mode other than KOMBGPU_KEY_REF32 /
+ * KOMBGPU_KEY_EXACT64 on any rank gives KOMBGPU_EINVAL on every rank.  When one rank fails, every rank returns an
+ * error (the failing rank its own) and the contexts and the communicator stay usable. */
+int kombgpu_dist_coreness(kombgpu_dist_graph *g);
+int kombgpu_dist_corea(kombgpu_dist_graph *g, int key_mode);
 void kombgpu_dist_graph_destroy(kombgpu_dist_graph *g);
 
 int kombgpu_dist_graph_stats(const kombgpu_dist_graph *g, kombgpu_dist_stats *out);

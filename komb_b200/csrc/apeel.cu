@@ -27,9 +27,8 @@
 // Ranks that share one device (tests) run inside ONE grid, a group of CTAs per rank.
 #include <cstdio>
 #include <cstdlib>
-#include <vector>
 
-#include "dgraph.cuh"
+#include "prank.cuh"
 
 namespace kg {
 namespace {
@@ -42,7 +41,6 @@ constexpr uint32_t kASlice = 256;             // rows longer than this are cut i
 constexpr int kAScanItems = 8;
 constexpr unsigned long long kAEmpty = ~0ull;
 constexpr unsigned long long kASliceFlag = 1ull << 63;   // entry = flag | piece << 32 | local id ; else k << 32 | local id
-constexpr unsigned long long kAWatchdogNs = 20ull * 1000000000ull;
 constexpr int kALvlProf = 48;
 
 enum : uint32_t { kPhMin = 1, kPhScan = 2, kPhGo = 3, kPhExit = 4 };
@@ -66,7 +64,7 @@ struct AState {   // local to a rank
     uint32_t alive_cnt[2];
     uint32_t n_alive, alive_src;               // parameters of the current phase: list length, list index (2 = identity)
     int32_t local_min, cur_k, prev_k, max_core;
-    uint32_t levels, error;                    // error: 1 watchdog (workers), 2 watchdog (peers), 5 pool overflow
+    uint32_t levels, error;                    // error: kErr*
     uint32_t lvl_ns[kALvlProf], lvl_pushed[kALvlProf];   // first levels: time from GO to the end of the level, entries this rank processed
     int32_t lvl_k[kALvlProf];
 };
@@ -87,27 +85,6 @@ struct ARank {
     AState *st;
 };
 
-__device__ __forceinline__ unsigned long long a_ld_sys(const unsigned long long *p) {
-    unsigned long long v;
-    asm volatile("ld.relaxed.sys.global.u64 %0, [%1];" : "=l"(v) : "l"(p) : "memory");
-    return v;
-}
-__device__ __forceinline__ void a_st_sys(unsigned long long *p, unsigned long long v) {
-    asm volatile("st.relaxed.sys.global.u64 [%0], %1;" ::"l"(p), "l"(v) : "memory");
-}
-__device__ __forceinline__ unsigned long long a_ld_acq(const unsigned long long *p) {
-    unsigned long long v;
-    asm volatile("ld.acquire.gpu.global.u64 %0, [%1];" : "=l"(v) : "l"(p) : "memory");
-    return v;
-}
-__device__ __forceinline__ void a_st_rel(unsigned long long *p, unsigned long long v) {
-    asm volatile("st.release.gpu.global.u64 [%0], %1;" ::"l"(p), "l"(v) : "memory");
-}
-__device__ __forceinline__ unsigned long long a_ns() {
-    unsigned long long t;
-    asm volatile("mov.u64 %0, %%globaltimer;" : "=l"(t));
-    return t;
-}
 // ---- worker side ------------------------------------------------------------------------------------------------
 
 // decrement the neighbours col[lo, hi) of a unitig peeled at level k (whole warp)
@@ -148,8 +125,8 @@ __device__ __forceinline__ void a_walk(const ARank &R, AState *st, uint32_t lo, 
         for (int t = 0; t < kAU; ++t) {
             if (old[t] == k + 1) {   // this decrement took the unitig to level k: it is peeled now, by its owner
                 const unsigned long long tk = atomicAdd_system(&R.ctl_peer[own[t]]->q_tail, 1ull);
-                if (tk < R.pool_cap) a_st_sys(R.pool_peer[own[t]] + tk, ((unsigned long long)(uint32_t)k << 32) | li[t]);
-                else atomicCAS(&st->error, 0u, 5u);
+                if (tk < R.pool_cap) st_relaxed_sys(R.pool_peer[own[t]] + tk, ((unsigned long long)(uint32_t)k << 32) | li[t]);
+                else atomicCAS(&st->error, 0u, (uint32_t)kErrFull);
                 n_push += own[t] != (uint32_t)R.rank;
                 n_own += own[t] == (uint32_t)R.rank;
             }
@@ -186,7 +163,7 @@ __device__ __forceinline__ void a_process(const ARank &R, AState *st, unsigned l
     const bool use_map = R.dead_peer[R.rank] != nullptr &&
                          *(volatile unsigned long long *)&R.ctl_peer[R.rank]->q_tail > ticket + kABacklog;
     const uint32_t v = (uint32_t)entry;
-    if (v >= R.n_local) { atomicCAS(&st->error, 0u, 4u); return; }
+    if (v >= R.n_local) { atomicCAS(&st->error, 0u, (uint32_t)kErrBadEntry); return; }
     const uint32_t row_lo = R.row_ptr[v], row_hi = R.row_ptr[v + 1];
     if (entry & kASliceFlag) {
         const uint32_t piece = (uint32_t)(entry >> 32) & 0x1fffffu;
@@ -210,8 +187,8 @@ __device__ __forceinline__ void a_process(const ARank &R, AState *st, unsigned l
         }
         pos = __shfl_sync(kFullMask, pos, 0);
         for (uint32_t j = lane; j < n_extra; j += 32u) {
-            if (pos + j < R.pool_cap) a_st_sys(R.pool_peer[R.rank] + pos + j, kASliceFlag | ((unsigned long long)(j + 1u) << 32) | v);
-            else atomicCAS(&st->error, 0u, 5u);
+            if (pos + j < R.pool_cap) st_relaxed_sys(R.pool_peer[R.rank] + pos + j, kASliceFlag | ((unsigned long long)(j + 1u) << 32) | v);
+            else atomicCAS(&st->error, 0u, (uint32_t)kErrFull);
         }
         hi = row_lo + kASlice;
     }
@@ -273,8 +250,8 @@ __device__ __forceinline__ void a_phase_scan(const ARank &R, AState *st, uint32_
 #pragma unroll
         for (int j = 0; j < kAScanItems; ++j) {
             if (flag[j] == 1u) {
-                if (fpos < R.pool_cap) a_st_sys(pool + fpos, ((unsigned long long)(uint32_t)k << 32) | v[j]);
-                else atomicCAS(&st->error, 0u, 5u);
+                if (fpos < R.pool_cap) st_relaxed_sys(pool + fpos, ((unsigned long long)(uint32_t)k << 32) | v[j]);
+                else atomicCAS(&st->error, 0u, (uint32_t)kErrFull);
                 ++fpos;
             } else if (flag[j]) {
                 R.alive[dst][spos++] = v[j];
@@ -301,17 +278,17 @@ __device__ void a_worker(const ARank &R, uint32_t wcta, uint32_t n_wctas, uint32
         if (lane == 0) t = atomicAdd(&st->q_head, 1ull);
         t = __shfl_sync(kFullMask, t, 0);
         unsigned long long entry = kAEmpty;
-        unsigned long long t0 = a_ns();
+        unsigned long long t0 = pglobal_ns();
         uint32_t spins = 0;
         while (true) {
             if (armed && t < R.pool_cap) {
-                entry = a_ld_sys(pool + t);
+                entry = ld_relaxed_sys(pool + t);
                 // a slice only exists once its unitig's level was released; a unitig carries its level
                 if (entry != kAEmpty && ((entry & kASliceFlag) || (int32_t)((entry >> 32) & 0x7fffffffu) == go_k)) break;
             }
             unsigned long long pw = *(volatile unsigned long long *)&st->phase_word;
             if ((pw >> 40) != seen) {
-                pw = a_ld_acq(&st->phase_word);   // the phase's parameters were written before the word
+                pw = ld_acq_gpu(&st->phase_word);   // the phase's parameters were written before the word
                 const uint32_t type = (uint32_t)(pw >> 32) & 0xffu;
                 if (type == kPhExit) return;
                 if (type == kPhGo) {
@@ -330,12 +307,12 @@ __device__ void a_worker(const ARank &R, uint32_t wcta, uint32_t n_wctas, uint32
                     }
                 }
                 seen = pw >> 40;
-                t0 = a_ns();   // the peel is moving: the watchdog measures silence, not the length of the peel
+                t0 = pglobal_ns();   // the peel is moving: the watchdog measures silence, not the length of the peel
                 continue;
             }
             if ((++spins & 1023u) == 0) {
                 if (*(volatile uint32_t *)&st->error) return;
-                if (a_ns() - t0 > kAWatchdogNs) { atomicCAS(&st->error, 0u, 1u); return; }
+                if (pglobal_ns() - t0 > kPeelWatchdogNs) { atomicCAS(&st->error, 0u, (uint32_t)kErrBarrier); return; }
             }
         }
         a_process(R, st, entry, t);
@@ -347,16 +324,16 @@ __device__ void a_worker(const ARank &R, uint32_t wcta, uint32_t n_wctas, uint32
 __device__ __forceinline__ bool a_issue_and_wait(const ARank &R, AState *st, unsigned long long &seq, uint32_t type, int32_t k,
                                                  unsigned long long &phases_run, bool wait) {
     ++seq;
-    if (lane_id() == 0) a_st_rel(&st->phase_word, (seq << 40) | ((unsigned long long)type << 32) | (unsigned long long)(uint32_t)k);
+    if (lane_id() == 0) st_rel_gpu(&st->phase_word, (seq << 40) | ((unsigned long long)type << 32) | (unsigned long long)(uint32_t)k);
     if (!wait) return true;
     ++phases_run;
     const unsigned long long want = phases_run * (unsigned long long)(R.ctas - 1u);
     bool ok = true;
     if (lane_id() == 0) {
-        const unsigned long long t0 = a_ns();
+        const unsigned long long t0 = pglobal_ns();
         uint32_t spins = 0;
-        while (a_ld_acq(&st->phase_done) < want) {
-            if ((++spins & 1023u) == 0 && (*(volatile uint32_t *)&st->error || a_ns() - t0 > kAWatchdogNs)) { ok = false; break; }
+        while (ld_acq_gpu(&st->phase_done) < want) {
+            if ((++spins & 1023u) == 0 && (*(volatile uint32_t *)&st->error || pglobal_ns() - t0 > kPeelWatchdogNs)) { ok = false; break; }
         }
     }
     return __shfl_sync(kFullMask, ok ? 1 : 0, 0) != 0;
@@ -372,10 +349,10 @@ __device__ void a_manager(const ARank &R) {
     int32_t prev_k = -1;
     bool level_active = false;                // this rank processed entries in the level that just ended
     uint32_t n_alive = R.n_local, src = 2u;   // 2: every local unitig
-    unsigned long long tp = a_ns();
+    unsigned long long tp = pglobal_ns();
 #define KG_APROF(slot)                                \
     if (lane == 0) {                                  \
-        const unsigned long long now_ = a_ns();       \
+        const unsigned long long now_ = pglobal_ns();       \
         st->prof_ns[slot] += now_ - tp;               \
         tp = now_;                                    \
     }
@@ -404,22 +381,22 @@ __device__ void a_manager(const ARank &R) {
         lmin = __shfl_sync(kFullMask, lmin, 0);
         // bit 31: this rank peeled something in the level that just ended (a level named by a stale bound can be empty everywhere)
         const unsigned long long active_bit = level_active ? 0x80000000ull : 0ull;
-        if (has_peer) a_st_sys(&R.ctl_peer[lane]->min_next[R.rank], (epoch << 32) | active_bit | (unsigned long long)(uint32_t)lmin);
+        if (has_peer) st_relaxed_sys(&R.ctl_peer[lane]->min_next[R.rank], (epoch << 32) | active_bit | (unsigned long long)(uint32_t)lmin);
         int32_t gmin = INT32_MAX;
         bool any_active = false;
         {
-            const unsigned long long t0 = a_ns();
+            const unsigned long long t0 = pglobal_ns();
             uint32_t spins = 0;
             bool bad = false;
             unsigned long long w = 0;
             if (has_peer) {
-                while (((w = a_ld_sys(&mine->min_next[lane])) >> 32) != epoch) {
-                    if ((++spins & 1023u) == 0 && (*(volatile uint32_t *)&st->error || a_ns() - t0 > kAWatchdogNs)) { bad = true; break; }
+                while (((w = ld_relaxed_sys(&mine->min_next[lane])) >> 32) != epoch) {
+                    if ((++spins & 1023u) == 0 && (*(volatile uint32_t *)&st->error || pglobal_ns() - t0 > kPeelWatchdogNs)) { bad = true; break; }
                 }
                 gmin = (int32_t)((uint32_t)w & 0x7fffffffu);
                 any_active = ((uint32_t)w & 0x80000000u) != 0;
             }
-            if (__ballot_sync(kFullMask, bad)) { if (lane == 0) atomicCAS(&st->error, 0u, 2u); failed = true; break; }
+            if (__ballot_sync(kFullMask, bad)) { if (lane == 0) atomicCAS(&st->error, 0u, (uint32_t)kErrPeers); failed = true; break; }
             gmin = warp_reduce_min(gmin);
             any_active = __any_sync(kFullMask, any_active);
         }
@@ -446,46 +423,46 @@ __device__ void a_manager(const ARank &R) {
         prev_k = k;
         KG_APROF(2);
         // ---- nobody decrements before every rank's scan is complete
-        if (has_peer) a_st_sys(&R.ctl_peer[lane]->scan_seen[R.rank], epoch);
+        if (has_peer) st_relaxed_sys(&R.ctl_peer[lane]->scan_seen[R.rank], epoch);
         {
-            const unsigned long long t0 = a_ns();
+            const unsigned long long t0 = pglobal_ns();
             uint32_t spins = 0;
             bool bad = false;
             if (has_peer) {
-                while (a_ld_sys(&mine->scan_seen[lane]) != epoch) {
-                    if ((++spins & 1023u) == 0 && (*(volatile uint32_t *)&st->error || a_ns() - t0 > kAWatchdogNs)) { bad = true; break; }
+                while (ld_relaxed_sys(&mine->scan_seen[lane]) != epoch) {
+                    if ((++spins & 1023u) == 0 && (*(volatile uint32_t *)&st->error || pglobal_ns() - t0 > kPeelWatchdogNs)) { bad = true; break; }
                 }
             }
-            if (__ballot_sync(kFullMask, bad)) { if (lane == 0) atomicCAS(&st->error, 0u, 2u); failed = true; break; }
+            if (__ballot_sync(kFullMask, bad)) { if (lane == 0) atomicCAS(&st->error, 0u, (uint32_t)kErrPeers); failed = true; break; }
         }
         KG_APROF(3);
         a_issue_and_wait(R, st, seq, kPhGo, k, phases_run, false);
-        unsigned long long done_before = lane == 0 ? a_ld_sys(&mine->q_done) : 0ull;
+        unsigned long long done_before = lane == 0 ? ld_relaxed_sys(&mine->q_done) : 0ull;
         done_before = __shfl_sync(kFullMask, done_before, 0);
         // ---- the end of the level: every rank idle at one instant
         {
-            const unsigned long long t0 = a_ns();
+            const unsigned long long t0 = pglobal_ns();
             uint32_t spins = 0;
             while (true) {
                 unsigned long long d1 = 0, t1 = 0, t2 = 0;
                 if (has_peer) {
-                    d1 = a_ld_sys(&R.ctl_peer[lane]->q_done);    // done first: done <= tail at any instant
-                    t1 = a_ld_sys(&R.ctl_peer[lane]->q_tail);
+                    d1 = ld_relaxed_sys(&R.ctl_peer[lane]->q_done);    // done first: done <= tail at any instant
+                    t1 = ld_relaxed_sys(&R.ctl_peer[lane]->q_tail);
                 }
                 if (__all_sync(kFullMask, d1 == t1)) {
-                    if (has_peer) t2 = a_ld_sys(&R.ctl_peer[lane]->q_tail);
+                    if (has_peer) t2 = ld_relaxed_sys(&R.ctl_peer[lane]->q_tail);
                     if (__all_sync(kFullMask, t2 == t1)) break;
                 }
                 if ((++spins & 255u) == 0) {
-                    const bool bad = *(volatile uint32_t *)&st->error || a_ns() - t0 > kAWatchdogNs;
-                    if (__any_sync(kFullMask, bad)) { if (lane == 0) atomicCAS(&st->error, 0u, 2u); failed = true; break; }
+                    const bool bad = *(volatile uint32_t *)&st->error || pglobal_ns() - t0 > kPeelWatchdogNs;
+                    if (__any_sync(kFullMask, bad)) { if (lane == 0) atomicCAS(&st->error, 0u, (uint32_t)kErrPeers); failed = true; break; }
                 }
             }
-            unsigned long long done_after = lane == 0 ? a_ld_sys(&mine->q_done) : 0ull;
+            unsigned long long done_after = lane == 0 ? ld_relaxed_sys(&mine->q_done) : 0ull;
             done_after = __shfl_sync(kFullMask, done_after, 0);
             level_active = done_after != done_before;
             if (lane == 0 && epoch <= (unsigned long long)kALvlProf) {
-                st->lvl_ns[epoch - 1] = (uint32_t)(a_ns() - t0);
+                st->lvl_ns[epoch - 1] = (uint32_t)(pglobal_ns() - t0);
                 st->lvl_k[epoch - 1] = k;
                 st->lvl_pushed[epoch - 1] = (uint32_t)(done_after - done_before);
             }
@@ -514,129 +491,82 @@ __global__ void __launch_bounds__(kAThreads, 2) apeel_kernel(const ARank *ranks,
 
 }  // namespace
 
-int dist_peel_async(kombgpu_dist_graph *g) {
+int dist_peel_async(kombgpu_dist_graph *g, int rc) {
     kombgpu_comm *c = g->comm;
     kombgpu_ctx *ctx = g->ctx;
     const int world = c->world;
     const uint32_t n_local = g->n_local;
     if (!g->row_ptr32) return ctx_fail(ctx, KOMBGPU_ESTATE, "the asynchronous peel needs the rank's rows (built with the async layout)");
-    cudaEvent_t ev0 = nullptr, ev1 = nullptr;
-    KG_CUDA(ctx, cudaEventCreate(&ev0));
-    KG_CUDA(ctx, cudaEventCreate(&ev1));
-    KG_CUDA(ctx, cudaEventRecord(ev0, ctx->stream));
-    if (!g->core) {
-        g->core = static_cast<int32_t *>(ws_alloc(ctx, (n_local ? n_local : 1) * sizeof(int32_t)));
-        if (!g->core) return ctx_fail(ctx, KOMBGPU_ENOMEM, "coreness array");
-    }
-    KG_CUDA(ctx, cudaMemsetAsync(g->core, 0, (size_t)(n_local ? n_local : 1) * sizeof(int32_t), ctx->stream));
 
-    // symmetric: working degrees, pool, control block.  The pool holds every local unitig once plus the slices of long rows;
-    // all ranks size it alike (the symmetric heap hands out the same sequence of buffers everywhere).
+    // symmetric: working degrees, pool, control block, map of peeled unitigs (one byte per unitig of the graph on every
+    // rank).  The pool holds every local unitig once plus the slices of long rows; all ranks size it alike (the symmetric
+    // heap hands out the same sequence of buffers everywhere).
     unsigned long long mine_sz[1] = {(unsigned long long)n_local + g->n_directed / kASlice + 64ull}, all_sz[kMaxRanks];
-    KG_TRY(comm_exchange(c, mine_sz, 1, all_sz));
+    KG_TRY(exchange_rc(c, rc, mine_sz, 1, all_sz));
     unsigned long long cap64 = 0;
     for (int q = 0; q < world; ++q) cap64 = all_sz[q] > cap64 ? all_sz[q] : cap64;
-    if (cap64 >= 0xffffffffull) return ctx_fail(ctx, KOMBGPU_EINVAL, "partition too large for the peel's pool");
-    const SymMark mark = sym_mark(c);
+    if (cap64 >= 0xffffffffull) return ctx_fail(ctx, KOMBGPU_EINVAL, "partition too large for the peel's pool");   // on every rank
+    SymRewind heap{c, sym_mark(c)};
     int32_t *work = nullptr;
     unsigned long long *pool = nullptr;
     ACtl *ctl = nullptr;
+    uint8_t *dead = nullptr;
     PeerPtrs<int32_t> work_peers{};
     PeerPtrs<unsigned long long> pool_peers{};
     PeerPtrs<ACtl> ctl_peers{};
-    KG_TRY(sym_alloc(c, (size_t)g->step, &work, &work_peers));
-    KG_TRY(sym_alloc(c, (size_t)cap64, &pool, &pool_peers));
-    KG_TRY(sym_alloc(c, 1, &ctl, &ctl_peers));
-    // maps of peeled unitigs (one byte per unitig of the graph on every rank; KOMBGPU_APEEL_DEADMAP=0 turns them off)
-    uint8_t *dead = nullptr;
     PeerPtrs<uint8_t> dead_peers{};
-    const char *dm_env = getenv("KOMBGPU_APEEL_DEADMAP");
-    if (!(dm_env && dm_env[0] == '0')) {
-        KG_TRY(sym_alloc(c, (size_t)g->n_global, &dead, &dead_peers));
-        KG_CUDA(ctx, cudaMemsetAsync(dead, 0, (size_t)(g->n_global ? g->n_global : 1), ctx->stream));
-    }
-    KG_CUDA(ctx, cudaMemsetAsync(ctl, 0, sizeof(ACtl), ctx->stream));
-    KG_CUDA(ctx, cudaMemsetAsync(pool, 0xff, (size_t)cap64 * sizeof(unsigned long long), ctx->stream));
-    if (n_local) KG_CUDA(ctx, cudaMemcpyAsync(work, g->deg, (size_t)n_local * sizeof(int32_t), cudaMemcpyDeviceToDevice, ctx->stream));
+    rc = first_rc(rc, sym_alloc(c, (size_t)g->step, &work, &work_peers));
+    rc = first_rc(rc, sym_alloc(c, (size_t)cap64, &pool, &pool_peers));
+    rc = first_rc(rc, sym_alloc(c, 1, &ctl, &ctl_peers));
+    rc = first_rc(rc, sym_alloc(c, (size_t)g->n_global, &dead, &dead_peers));
 
     DevBuf<uint32_t> alive_a, alive_b;
-    DevBuf<AState> state(ctx, 1);
-    DevBuf<ARank> desc(ctx, kMaxRanks);
-    KG_ALLOC(ctx, alive_a, n_local);
-    KG_ALLOC(ctx, alive_b, n_local);
-    if (!state || !desc) return ctx_fail(ctx, KOMBGPU_ENOMEM, "workspace");
-    KG_CUDA(ctx, cudaMemsetAsync(state.p, 0, sizeof(AState), ctx->stream));
-
-    int per_sm = 0;
-    KG_CUDA(ctx, cudaOccupancyMaxActiveBlocksPerMultiprocessor(&per_sm, apeel_kernel, kAThreads, 0));
-    if (per_sm < 1) return ctx_fail(ctx, KOMBGPU_ECUDA, "asynchronous peel kernel does not fit on an SM");
-    const int resident = per_sm * ctx->sm_count;
-    const uint32_t ctas_per_rank = c->same_device ? (uint32_t)(resident / world) : (uint32_t)resident;
-    if (ctas_per_rank < 2) return ctx_fail(ctx, KOMBGPU_EINVAL, "too many ranks on one device");
-
+    DevBuf<AState> state;
+    DevBuf<ARank> desc;
+    uint32_t ctas_per_rank = 0;
     ARank R{};
-    R.n_local = n_local; R.v_lo = g->v_lo; R.n_global = g->n_global; R.step = g->step; R.world = world; R.rank = c->rank;
-    R.ctas = ctas_per_rank;
-    R.row_ptr = g->row_ptr32; R.col = g->col; R.core = g->core;
-    R.alive[0] = alive_a.p; R.alive[1] = alive_b.p;
-    R.pool_cap = (uint32_t)cap64;
-    for (int q = 0; q < world; ++q) {
-        R.deg_peer[q] = work_peers.p[q];
-        R.pool_peer[q] = pool_peers.p[q];
-        R.ctl_peer[q] = ctl_peers.p[q];
-        R.dead_peer[q] = dead_peers.p[q];
-    }
-    R.st = state.p;
-
-    // every rank's degrees, pool and control words are initialised before anyone reaches into them
-    unsigned long long token = 1, tokens[kMaxRanks];
-    KG_TRY(comm_exchange(c, &token, 1, tokens));
-
-    cudaError_t le = cudaSuccess;
-    if (!c->same_device) {
-        KG_CUDA(ctx, cudaMemcpyAsync(desc.p, &R, sizeof(R), cudaMemcpyHostToDevice, ctx->stream));
-        const ARank *dp = desc.p;
-        uint32_t cpr = ctas_per_rank;
-        void *args[] = {(void *)&dp, (void *)&cpr};
-        le = cudaLaunchCooperativeKernel((void *)apeel_kernel, dim3(ctas_per_rank), dim3(kAThreads), args, 0, ctx->stream);
-        ctx->launches++;
-        if (le == cudaSuccess) le = cudaStreamSynchronize(ctx->stream);
-    } else {
-        // emulation: one cooperative grid holds every rank (a group of CTAs each); rank 0's thread launches it
-        LocalGroup *grp = c->group;
-        grp->slot[c->rank] = &R;
-        KG_TRY(comm_group_barrier(c));
-        if (c->rank == 0) {
-            std::vector<ARank> all(world);
-            for (int q = 0; q < world; ++q) all[q] = *static_cast<ARank *>(grp->slot[q]);
-            le = cudaMemcpyAsync(desc.p, all.data(), sizeof(ARank) * world, cudaMemcpyHostToDevice, ctx->stream);
-            const ARank *dp = desc.p;
-            uint32_t cpr = ctas_per_rank;
-            void *args[] = {(void *)&dp, (void *)&cpr};
-            if (le == cudaSuccess)
-                le = cudaLaunchCooperativeKernel((void *)apeel_kernel, dim3(ctas_per_rank * world), dim3(kAThreads), args, 0, ctx->stream);
-            ctx->launches++;
-            if (le == cudaSuccess) le = cudaStreamSynchronize(ctx->stream);
-            grp->slot_rc = le == cudaSuccess ? 0 : 1;
+    if (rc == KOMBGPU_OK) rc = [&]() -> int {
+        KG_CUDA(ctx, cudaMemsetAsync(g->core, 0, (size_t)(n_local ? n_local : 1) * sizeof(int32_t), ctx->stream));
+        KG_CUDA(ctx, cudaMemsetAsync(dead, 0, (size_t)(g->n_global ? g->n_global : 1), ctx->stream));
+        KG_CUDA(ctx, cudaMemsetAsync(ctl, 0, sizeof(ACtl), ctx->stream));
+        KG_CUDA(ctx, cudaMemsetAsync(pool, 0xff, (size_t)cap64 * sizeof(unsigned long long), ctx->stream));
+        if (n_local) KG_CUDA(ctx, cudaMemcpyAsync(work, g->deg, (size_t)n_local * sizeof(int32_t), cudaMemcpyDeviceToDevice, ctx->stream));
+        KG_ALLOC(ctx, alive_a, n_local);
+        KG_ALLOC(ctx, alive_b, n_local);
+        KG_ALLOC(ctx, state, 1);
+        KG_ALLOC(ctx, desc, kMaxRanks);
+        KG_CUDA(ctx, cudaMemsetAsync(state.p, 0, sizeof(AState), ctx->stream));
+        KG_TRY(rank_ctas(ctx, c, apeel_kernel, kAThreads, 2, &ctas_per_rank));   // CTA 0 manages, the others work
+        R.n_local = n_local; R.v_lo = g->v_lo; R.n_global = g->n_global; R.step = g->step; R.world = world; R.rank = c->rank;
+        R.ctas = ctas_per_rank;
+        R.row_ptr = g->row_ptr32; R.col = g->col; R.core = g->core;
+        R.alive[0] = alive_a.p; R.alive[1] = alive_b.p;
+        R.pool_cap = (uint32_t)cap64;
+        for (int q = 0; q < world; ++q) {
+            R.deg_peer[q] = work_peers.p[q];
+            R.pool_peer[q] = pool_peers.p[q];
+            R.ctl_peer[q] = ctl_peers.p[q];
+            R.dead_peer[q] = dead_peers.p[q];
         }
-        KG_TRY(comm_group_barrier(c));
-        if (grp->slot_rc) le = cudaErrorLaunchFailure;
-        KG_TRY(comm_group_barrier(c));
-    }
-    if (le != cudaSuccess) return ctx_fail(ctx, KOMBGPU_ECUDA, "asynchronous peel kernel: %s", cudaGetErrorString(le));
+        R.st = state.p;
+        return KOMBGPU_OK;
+    }();
+    // every rank's degrees, pool and control words are initialised before anyone reaches into them
+    KG_TRY(barrier_rc(c, rc));
 
+    const cudaError_t le = launch_ranks(c, apeel_kernel, kAThreads, ctas_per_rank, R, desc.p, nullptr);
+    if (le != cudaSuccess) rc = ctx_fail(ctx, KOMBGPU_ECUDA, "asynchronous peel kernel: %s", cudaGetErrorString(le));
     AState fin{};
-    KG_TRY(read_back(ctx, state.p, &fin, 1));
     ACtl fin_ctl{};
-    KG_TRY(read_back(ctx, ctl, &fin_ctl, 1));
-    // global figures; also: nobody releases its pool while a peer may still be writing
+    if (rc == KOMBGPU_OK) rc = read_back(ctx, state.p, &fin, 1);
+    if (rc == KOMBGPU_OK) rc = read_back(ctx, ctl, &fin_ctl, 1);
+    // global figures; also: nobody gives back its pool (at return) while a peer may still be writing
     const unsigned long long peeled_here = fin_ctl.q_done - fin.n_slices;
     unsigned long long mine[3] = {fin.error, peeled_here, (unsigned long long)(uint32_t)fin.max_core}, all[kMaxRanks * 3];
-    KG_TRY(comm_exchange(c, mine, 3, all));
-    sym_release(c, mark);
+    KG_TRY(exchange_rc(c, rc, mine, 3, all));
     uint64_t peeled = 0;
     for (int q = 0; q < world; ++q) {
-        if (all[q * 3]) return ctx_fail(ctx, KOMBGPU_EINTERNAL, "asynchronous peel: rank %d reports error %llu (1/2 watchdog, 4 bad entry, 5 pool overflow)", q, all[q * 3]);
+        if (all[q * 3]) return ctx_fail(ctx, KOMBGPU_EINTERNAL, "asynchronous peel: rank %d reports error %llu (%s)", q, all[q * 3], rank_error_text(all[q * 3]));
         peeled += all[q * 3 + 1];
     }
     if (peeled != g->n_global) return ctx_fail(ctx, KOMBGPU_EINTERNAL, "asynchronous peel ended with %llu of %u unitigs peeled", (unsigned long long)peeled, g->n_global);
@@ -647,7 +577,6 @@ int dist_peel_async(kombgpu_dist_graph *g) {
     g->st.peel_async = 1;
     g->st.n_messages_sent = fin.n_remote_push;               // unitigs this rank discovered for other ranks (pushed into their pools)
     g->st.n_messages_recv = fin_ctl.q_tail - fin.n_own_push;   // unitigs other ranks pushed into this rank's pool
-    g->has_core = true;
     if (getenv("KOMBGPU_DEBUG"))
         fprintf(stderr, "[kombgpu] rank %d apeel: levels %u ctas %u | manager ms: min pass %.3f min exchange %.3f scan pass %.3f scan exchange %.3f "
                 "levels (go -> over) %.3f | peeled here %llu, slices %llu, entries visited %llu, remote decrements %llu, remote pushes %llu\n",
@@ -658,11 +587,6 @@ int dist_peel_async(kombgpu_dist_graph *g) {
         for (uint32_t i = 0; i < fin.levels && i < (uint32_t)kALvlProf; ++i) fprintf(stderr, " %d:%.0f/%u", fin.lvl_k[i], fin.lvl_ns[i] * 1e-3, fin.lvl_pushed[i]);
         fprintf(stderr, "\n");
     }
-    KG_CUDA(ctx, cudaEventRecord(ev1, ctx->stream));
-    KG_CUDA(ctx, cudaEventSynchronize(ev1));
-    cudaEventElapsedTime(&g->st.ms_peel, ev0, ev1);
-    cudaEventDestroy(ev0);
-    cudaEventDestroy(ev1);
     return KOMBGPU_OK;
 }
 

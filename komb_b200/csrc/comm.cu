@@ -233,6 +233,19 @@ int comm_exchange(kombgpu_comm *c, const unsigned long long *vals, int k, unsign
     return KOMBGPU_OK;
 }
 
+int exchange_rc(kombgpu_comm *c, int rc, const unsigned long long *vals, int k, unsigned long long *out) {
+    unsigned long long mine[kCtlWords], all[kMaxRanks * kCtlWords];
+    mine[0] = rc != KOMBGPU_OK ? (unsigned long long)-rc : 0ull;
+    for (int j = 0; j < k; ++j) mine[1 + j] = vals[j];
+    KG_TRY(comm_exchange(c, mine, k + 1, all));
+    for (int q = 0; q < c->world; ++q)
+        for (int j = 0; j < k; ++j) out[q * k + j] = all[q * (k + 1) + 1 + j];
+    if (rc != KOMBGPU_OK) return rc;   // this rank's own message stands
+    for (int q = 0; q < c->world; ++q)
+        if (all[q * (k + 1)]) return ctx_fail(c->ctx, -(int)all[q * (k + 1)], "rank %d failed; the call stopped on every rank", q);
+    return KOMBGPU_OK;
+}
+
 int comm_group_barrier(kombgpu_comm *c) {
     if (!c->group) return KOMBGPU_OK;
     if (group_barrier(c->group) != KOMBGPU_OK) return ctx_fail(c->ctx, KOMBGPU_ESTATE, "a rank of the local group failed");

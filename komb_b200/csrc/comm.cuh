@@ -47,8 +47,9 @@ struct LocalGroup {
     std::vector<unsigned char> blob;   // world x bytes_per_rank of the all-gather in flight
     bool broken = false;               // a rank failed: every waiter gives up
     int refs = 0;
-    // same-device emulation: what the ranks hand to the one thread that launches a kernel for all of them (ppeel.cu)
-    void *slot[kMaxRanks] = {};
+    // same-device emulation: the descriptors the ranks hand to the one thread that launches a persistent rank kernel
+    // for all of them (launch_ranks in prank.cuh, for ppeel.cu, apeel.cu and ponion.cu)
+    const void *slot[kMaxRanks] = {};
     int slot_rc = 0;
 };
 
@@ -91,6 +92,13 @@ void sym_release(kombgpu_comm *c, SymMark m);
 
 // all-gather of k <= kCtlWords words per rank + barrier, ordered on the context's stream; out[q * k + j] on the host
 int comm_exchange(kombgpu_comm *c, const unsigned long long *vals, int k, unsigned long long *out);
+// comm_exchange of k < kCtlWords words per rank that also carries every rank's status rc: a rank that failed returns
+// its own code, the others fail with the code of the first failing rank.  The collectives of the partitioned path meet
+// through these two, and a rank that failed locally keeps making the same calls as its peers up to the next one.
+int exchange_rc(kombgpu_comm *c, int rc, const unsigned long long *vals, int k, unsigned long long *out);
+inline int barrier_rc(kombgpu_comm *c, int rc) { return exchange_rc(c, rc, nullptr, 0, nullptr); }
+// a status that collects the steps every rank makes whatever failed before (sym_alloc): the first failure stands
+inline int first_rc(int rc, int next) { return rc != KOMBGPU_OK ? rc : next; }
 // host-side bootstrap all-gather (slow path: setup only)
 int comm_bootstrap_allgather(kombgpu_comm *c, const void *send, void *recv, size_t bytes_per_rank);
 // host barrier of the ranks of one process (same-device emulation only)

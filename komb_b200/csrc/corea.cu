@@ -448,72 +448,73 @@ int dist_corea(kombgpu_dist_graph *g, int key_mode) {
     kombgpu_ctx *ctx = g->ctx;
     const int world = c->world;
     const uint32_t n_local = g->n_local, n = g->n_global;
-    if (key_mode != KOMBGPU_KEY_REF32 && key_mode != KOMBGPU_KEY_EXACT64)
-        return ctx_fail(ctx, KOMBGPU_EINVAL, "unknown CORE-A key mode %d", key_mode);
-    cudaEvent_t ev0 = nullptr, ev1 = nullptr;
-    KG_CUDA(ctx, cudaEventCreate(&ev0));
-    KG_CUDA(ctx, cudaEventCreate(&ev1));
-    KG_CUDA(ctx, cudaEventRecord(ev0, ctx->stream));
-    if (!g->score) {
-        g->score = static_cast<double *>(ws_alloc(ctx, (n_local ? n_local : 1) * sizeof(double)));
-        if (!g->score) return ctx_fail(ctx, KOMBGPU_ENOMEM, "score array");
-    }
+    EvTimer timer(ctx);
+    SymRewind heap{c, sym_mark(c)};
     const uint32_t cap = (uint32_t)ctx->sm_count * 8u;
     const uint32_t max_deg = (uint32_t)g->st.max_degree, max_core = (uint32_t)(g->st.max_coreness > 0 ? g->st.max_coreness : 0);
-    const SymMark mark = sym_mark(c);
+    // a bad mode on one rank is an error on every rank, at the first exchange
+    int rc = key_mode == KOMBGPU_KEY_REF32 || key_mode == KOMBGPU_KEY_EXACT64 ? KOMBGPU_OK
+                                                                              : ctx_fail(ctx, KOMBGPU_EINVAL, "unknown CORE-A key mode %d", key_mode);
 
     // ---- degree ranks: sum of the ranks' histograms -> LUT
-    const uint32_t n_bins = max_deg + 1;
+    const uint32_t n_bins = max_deg + 1;   // the largest degree of the graph: the same on every rank
     uint32_t *hist = nullptr;
     PeerPtrs<uint32_t> hist_peers{};
-    KG_TRY(sym_alloc(c, (size_t)n_bins, &hist, &hist_peers));
-    KG_CUDA(ctx, cudaMemsetAsync(hist, 0, (size_t)n_bins * sizeof(uint32_t), ctx->stream));
-    if (n_local) KG_LAUNCH(ctx, degree_hist_kernel, grid_for(n_local, kThreads * 8, cap), kThreads, 0, g->deg, n_local, n_bins, hist);
-
-    // ---- local key order (same kernels as the single-GPU path, keys built with the GLOBAL n)
+    rc = first_rc(rc, sym_alloc(c, (size_t)n_bins, &hist, &hist_peers));
     DevBuf<uint64_t> ka, kb;
-    KG_ALLOC(ctx, ka, n_local);
-    KG_ALLOC(ctx, kb, n_local);
-    uint64_t *sorted = ka.p;
-    RadixPass passes[8];
+    uint64_t *sorted = nullptr;
     int wide = 0;
-    if (n_local) {
-        if (key_mode == KOMBGPU_KEY_REF32) {
-            KG_LAUNCH(ctx, pack_rank_keys_kernel, grid_for(n_local, kThreads, cap), kThreads, 0, g->core, g->deg, n_local, n, 0, 0, ka.p);
-            int np = plan_radix_passes(32, 64, 0, 0, passes);
-            KG_TRY(radix_sort_u64(ctx, ka.p, kb.p, n_local, passes, np, &sorted));
-        } else {
-            int cb, db;
-            exact_pair_bits(max_core, max_deg, n, &cb, &db);
-            if (db + cb <= 32) {
-                KG_LAUNCH(ctx, pack_rank_keys_kernel, grid_for(n_local, kThreads, cap), kThreads, 0, g->core, g->deg, n_local, n, 1, db, ka.p);
-                int np = plan_radix_passes(32, 32 + db + cb, 0, 0, passes);
+    DevBuf<uint32_t> head_pos, cls, d_classes;
+    uint32_t n_classes = 0;
+    if (rc == KOMBGPU_OK) rc = [&]() -> int {
+        if (!g->score) {
+            g->score = static_cast<double *>(ws_alloc(ctx, (n_local ? n_local : 1) * sizeof(double)));
+            if (!g->score) return ctx_fail(ctx, KOMBGPU_ENOMEM, "score array");
+        }
+        KG_CUDA(ctx, cudaMemsetAsync(hist, 0, (size_t)n_bins * sizeof(uint32_t), ctx->stream));
+        if (n_local) KG_LAUNCH(ctx, degree_hist_kernel, grid_for(n_local, kThreads * 8, cap), kThreads, 0, g->deg, n_local, n_bins, hist);
+
+        // ---- local key order (same kernels as the single-GPU path, keys built with the GLOBAL n)
+        KG_ALLOC(ctx, ka, n_local);
+        KG_ALLOC(ctx, kb, n_local);
+        sorted = ka.p;
+        RadixPass passes[8];
+        if (n_local) {
+            if (key_mode == KOMBGPU_KEY_REF32) {
+                KG_LAUNCH(ctx, pack_rank_keys_kernel, grid_for(n_local, kThreads, cap), kThreads, 0, g->core, g->deg, n_local, n, 0, 0, ka.p);
+                int np = plan_radix_passes(32, 64, 0, 0, passes);
                 KG_TRY(radix_sort_u64(ctx, ka.p, kb.p, n_local, passes, np, &sorted));
             } else {
-                wide = 1;
-                KG_LAUNCH(ctx, pack_rank_keys_kernel, grid_for(n_local, kThreads, cap), kThreads, 0, g->core, g->deg, n_local, n, 2, 0, ka.p);
-                int np = plan_radix_passes(32, 32 + db, 0, 0, passes);
-                KG_TRY(radix_sort_u64(ctx, ka.p, kb.p, n_local, passes, np, &sorted));
-                uint64_t *other = sorted == ka.p ? kb.p : ka.p;
-                KG_LAUNCH(ctx, rekey_by_core_kernel, grid_for(n_local, kThreads, cap), kThreads, 0, g->core, g->deg, n_local, n, sorted);
-                np = plan_radix_passes(32, 32 + cb, 0, 0, passes);
-                uint64_t *sorted2 = sorted;
-                KG_TRY(radix_sort_u64(ctx, sorted, other, n_local, passes, np, &sorted2));
-                sorted = sorted2;
+                int cb, db;
+                exact_pair_bits(max_core, max_deg, n, &cb, &db);
+                if (db + cb <= 32) {
+                    KG_LAUNCH(ctx, pack_rank_keys_kernel, grid_for(n_local, kThreads, cap), kThreads, 0, g->core, g->deg, n_local, n, 1, db, ka.p);
+                    int np = plan_radix_passes(32, 32 + db + cb, 0, 0, passes);
+                    KG_TRY(radix_sort_u64(ctx, ka.p, kb.p, n_local, passes, np, &sorted));
+                } else {
+                    wide = 1;
+                    KG_LAUNCH(ctx, pack_rank_keys_kernel, grid_for(n_local, kThreads, cap), kThreads, 0, g->core, g->deg, n_local, n, 2, 0, ka.p);
+                    int np = plan_radix_passes(32, 32 + db, 0, 0, passes);
+                    KG_TRY(radix_sort_u64(ctx, ka.p, kb.p, n_local, passes, np, &sorted));
+                    uint64_t *other = sorted == ka.p ? kb.p : ka.p;
+                    KG_LAUNCH(ctx, rekey_by_core_kernel, grid_for(n_local, kThreads, cap), kThreads, 0, g->core, g->deg, n_local, n, sorted);
+                    np = plan_radix_passes(32, 32 + cb, 0, 0, passes);
+                    uint64_t *sorted2 = sorted;
+                    KG_TRY(radix_sort_u64(ctx, sorted, other, n_local, passes, np, &sorted2));
+                    sorted = sorted2;
+                }
             }
         }
-    }
-    DevBuf<uint32_t> head_pos, cls, d_classes(ctx, 1);
-    KG_ALLOC(ctx, head_pos, n_local);
-    KG_ALLOC(ctx, cls, n_local);
-    if (!d_classes) return ctx_fail(ctx, KOMBGPU_ENOMEM, "workspace");
-    KG_TRY((device_scan<uint32_t>(ctx, n_local, ClassFlagIn{sorted, g->core, g->deg, n, wide}, ClassFlagOut{head_pos.p, cls.p}, d_classes.p)));
-    uint32_t n_classes = 0;
-    KG_TRY(read_back(ctx, d_classes.p, &n_classes, 1));
+        KG_ALLOC(ctx, head_pos, n_local);
+        KG_ALLOC(ctx, cls, n_local);
+        KG_ALLOC(ctx, d_classes, 1);
+        KG_TRY((device_scan<uint32_t>(ctx, n_local, ClassFlagIn{sorted, g->core, g->deg, n, wide}, ClassFlagOut{head_pos.p, cls.p}, d_classes.p)));
+        return read_back(ctx, d_classes.p, &n_classes, 1);
+    }();
 
     // ---- publish the list of distinct keys; meet; rank the local classes against every rank's list
     unsigned long long mine[2] = {n_classes, n_local}, all[kMaxRanks * 2];
-    KG_TRY(comm_exchange(c, mine, 2, all));   // also: every rank's histogram is complete
+    KG_TRY(exchange_rc(c, rc, mine, 2, all));   // also: every rank's histogram is complete
     uint32_t max_classes = 1;
     ClassLists L{};
     for (int q = 0; q < world; ++q) {
@@ -525,42 +526,40 @@ int dist_corea(kombgpu_dist_graph *g, int key_mode) {
     uint32_t *dhead = nullptr;
     PeerPtrs<uint64_t> dkey_peers{};
     PeerPtrs<uint32_t> dhead_peers{};
-    KG_TRY(sym_alloc(c, (size_t)max_classes, &dkey, &dkey_peers));
-    KG_TRY(sym_alloc(c, (size_t)max_classes, &dhead, &dhead_peers));
-    if (n_classes)
-        KG_LAUNCH(ctx, class_keys_kernel, grid_for(n_classes, kThreads, cap), kThreads, 0, sorted, head_pos.p, n_classes, g->core, g->deg, n,
-                  key_mode, dkey, dhead);
+    rc = sym_alloc(c, (size_t)max_classes, &dkey, &dkey_peers);
+    rc = first_rc(rc, sym_alloc(c, (size_t)max_classes, &dhead, &dhead_peers));
     DevBuf<uint32_t> hist_total;
     DevBuf<double> lut, class_rank;
-    KG_ALLOC(ctx, hist_total, n_bins);
-    KG_ALLOC(ctx, lut, n_bins);
-    KG_ALLOC(ctx, class_rank, n_classes);
-    KG_LAUNCH(ctx, sum_peer_hist_kernel, grid_for(n_bins, kThreads, cap), kThreads, 0, hist_peers, world, n_bins, hist_total.p);
-    KG_TRY((device_scan<uint32_t>(ctx, n_bins, HistIn{hist_total.p}, RankLutOut{lut.p, n}, (uint32_t *)nullptr)));
-    unsigned long long token = 1, tokens[kMaxRanks];
-    KG_TRY(comm_exchange(c, &token, 1, tokens));   // every rank's list is in place
-    for (int q = 0; q < world; ++q) { L.key[q] = dkey_peers.p[q]; L.head[q] = dhead_peers.p[q]; }
-    if (n_classes)
-        KG_LAUNCH(ctx, class_rank_kernel, grid_for(n_classes, kThreads, cap), kThreads, 0, L, world, c->rank, n, class_rank.p);
-    DevBuf<unsigned long long> max_bits(ctx, 1);
-    if (!max_bits) return ctx_fail(ctx, KOMBGPU_ENOMEM, "workspace");
-    KG_CUDA(ctx, cudaMemsetAsync(max_bits.p, 0, sizeof(unsigned long long), ctx->stream));
-    if (n_local)
-        KG_LAUNCH(ctx, dist_score_kernel, grid_for(n_local, kThreads, cap), kThreads, 0, sorted, cls.p, class_rank.p, g->deg, lut.p, n_local,
-                  g->score, max_bits.p);
+    if (rc == KOMBGPU_OK) rc = [&]() -> int {
+        if (n_classes)
+            KG_LAUNCH(ctx, class_keys_kernel, grid_for(n_classes, kThreads, cap), kThreads, 0, sorted, head_pos.p, n_classes, g->core, g->deg, n,
+                      key_mode, dkey, dhead);
+        KG_ALLOC(ctx, hist_total, n_bins);
+        KG_ALLOC(ctx, lut, n_bins);
+        KG_ALLOC(ctx, class_rank, n_classes);
+        KG_LAUNCH(ctx, sum_peer_hist_kernel, grid_for(n_bins, kThreads, cap), kThreads, 0, hist_peers, world, n_bins, hist_total.p);
+        return device_scan<uint32_t>(ctx, n_bins, HistIn{hist_total.p}, RankLutOut{lut.p, n}, (uint32_t *)nullptr);
+    }();
+    KG_TRY(barrier_rc(c, rc));   // every rank's list is in place
     unsigned long long h_bits = 0, all_bits[kMaxRanks];
-    KG_TRY(read_back(ctx, max_bits.p, &h_bits, 1));
-    KG_TRY(comm_exchange(c, &h_bits, 1, all_bits));   // also: nobody releases lists a peer is still reading
-    sym_release(c, mark);
+    DevBuf<unsigned long long> max_bits;
+    rc = [&]() -> int {
+        for (int q = 0; q < world; ++q) { L.key[q] = dkey_peers.p[q]; L.head[q] = dhead_peers.p[q]; }
+        if (n_classes)
+            KG_LAUNCH(ctx, class_rank_kernel, grid_for(n_classes, kThreads, cap), kThreads, 0, L, world, c->rank, n, class_rank.p);
+        KG_ALLOC(ctx, max_bits, 1);
+        KG_CUDA(ctx, cudaMemsetAsync(max_bits.p, 0, sizeof(unsigned long long), ctx->stream));
+        if (n_local)
+            KG_LAUNCH(ctx, dist_score_kernel, grid_for(n_local, kThreads, cap), kThreads, 0, sorted, cls.p, class_rank.p, g->deg, lut.p, n_local,
+                      g->score, max_bits.p);
+        return read_back(ctx, max_bits.p, &h_bits, 1);
+    }();
+    KG_TRY(exchange_rc(c, rc, &h_bits, 1, all_bits));   // also: nobody gives back lists (at return) a peer is still reading
     unsigned long long gmax = 0;
     for (int q = 0; q < world; ++q) gmax = all_bits[q] > gmax ? all_bits[q] : gmax;
     memcpy(&g->max_score, &gmax, sizeof(double));
     g->has_score = true;
-    KG_CUDA(ctx, cudaEventRecord(ev1, ctx->stream));
-    KG_CUDA(ctx, cudaEventSynchronize(ev1));
-    cudaEventElapsedTime(&g->st.ms_corea, ev0, ev1);
-    cudaEventDestroy(ev0);
-    cudaEventDestroy(ev1);
+    g->st.ms_corea = timer.lap();
     return KOMBGPU_OK;
 }
 

@@ -72,12 +72,11 @@ int dist_build(kombgpu_comm *c, const uint32_t *a, const uint32_t *b, uint64_t c
 // failing rank its own code and message, the others the code of the first failing rank).
 int route_keys(kombgpu_comm *c, const uint64_t *keys, uint64_t n, uint32_t step, bool rebase, uint64_t **recv, uint64_t *n_recv,
                int local_rc = KOMBGPU_OK);
-// ppeel.cu
-int dist_peel(kombgpu_dist_graph *g);
-// apeel.cu
-int dist_peel_async(kombgpu_dist_graph *g);
-// rpeel.cu
-int dist_peel_replicated(kombgpu_dist_graph *g);
+// the peels kombgpu_dist_coreness (pcapi.cu) picks from, into g->core: ppeel.cu, apeel.cu, rpeel.cu.  rc: this rank's
+// status so far; a rank that has failed still makes every collective call, and every rank returns an error.
+int dist_peel(kombgpu_dist_graph *g, int rc);
+int dist_peel_async(kombgpu_dist_graph *g, int rc);
+int dist_peel_replicated(kombgpu_dist_graph *g, int rc);
 // ponion.cu: onion layers over the ranks (collective); the cached result is freed by dist_onion_release
 int dist_onion(kombgpu_dist_graph *g);
 void dist_onion_release(kombgpu_dist_graph *g);
@@ -89,9 +88,6 @@ int dist_rows_to_nbr(kombgpu_dist_graph *g, DevBuf<uint32_t> &nbr_ptr, DevBuf<ui
 int dist_peel_mode();
 // pcorea.cu
 int dist_corea(kombgpu_dist_graph *g, int key_mode);
-// pcore.cu: comm_exchange of k words per rank (out[q * k + j]) that also carries every rank's status rc: a rank that
-// failed returns its own code, the others fail with the code of the first failing rank
-int exchange_rc(kombgpu_comm *c, int rc, const unsigned long long *vals, int k, unsigned long long *out);
 // the consumers of the finished coreness
 int dist_max_core_truss(kombgpu_dist_graph *g);
 int dist_densest_core(kombgpu_dist_graph *g, DensestCore *out);

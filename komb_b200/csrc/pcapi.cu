@@ -94,8 +94,19 @@ int kombgpu_dist_coreness(kombgpu_dist_graph *g) {
     if (!g) return KOMBGPU_EINVAL;
     KG_CUDA(g->ctx, cudaSetDevice(g->ctx->device));
     if (g->has_core) return KOMBGPU_OK;
+    kombgpu_ctx *ctx = g->ctx;
+    EvTimer timer(ctx);
+    int rc = KOMBGPU_OK;
+    if (!g->core) {
+        g->core = static_cast<int32_t *>(ws_alloc(ctx, (g->n_local ? g->n_local : 1) * sizeof(int32_t)));
+        if (!g->core) rc = ctx_fail(ctx, KOMBGPU_ENOMEM, "coreness array");
+    }
     // what the build prepared for (KOMBGPU_DIST_PEEL, or the shape of the graph)
-    return g->peel_choice == 2 ? dist_peel_replicated(g) : (g->peel_choice == 1 ? dist_peel_async(g) : dist_peel(g));
+    rc = g->peel_choice == 2 ? dist_peel_replicated(g, rc) : (g->peel_choice == 1 ? dist_peel_async(g, rc) : dist_peel(g, rc));
+    if (rc != KOMBGPU_OK) return rc;
+    g->st.ms_peel = timer.lap();
+    g->has_core = true;
+    return KOMBGPU_OK;
 }
 
 int kombgpu_dist_corea(kombgpu_dist_graph *g, int key_mode) {

@@ -40,26 +40,6 @@ int cuda_rc(kombgpu_ctx *ctx, cudaError_t e, const char *what) {
     return e == cudaSuccess ? KOMBGPU_OK : ctx_fail(ctx, KOMBGPU_ECUDA, "%s: %s", what, cudaGetErrorString(e));
 }
 
-}  // namespace
-
-// comm_exchange of k words per rank (out[q * k + j]) that also carries every rank's status `rc`
-int exchange_rc(kombgpu_comm *c, int rc, const unsigned long long *vals, int k, unsigned long long *out) {
-    unsigned long long mine[kCtlWords], all[kMaxRanks * kCtlWords];
-    mine[0] = rc != KOMBGPU_OK ? (unsigned long long)-rc : 0ull;
-    for (int j = 0; j < k; ++j) mine[1 + j] = vals[j];
-    KG_TRY(comm_exchange(c, mine, k + 1, all));
-    for (int q = 0; q < c->world; ++q)
-        for (int j = 0; j < k; ++j) out[q * k + j] = all[q * (k + 1) + 1 + j];
-    if (rc != KOMBGPU_OK) return rc;   // this rank's own message stands
-    for (int q = 0; q < c->world; ++q)
-        if (all[q * (k + 1)]) return ctx_fail(c->ctx, -(int)all[q * (k + 1)], "rank %d failed; the call stopped on every rank", q);
-    return KOMBGPU_OK;
-}
-
-namespace {
-
-int barrier_rc(kombgpu_comm *c, int rc) { return exchange_rc(c, rc, nullptr, 0, nullptr); }
-
 // core_all[x] = coreness of unitig x, for every unitig of the graph
 int gather_coreness(kombgpu_dist_graph *g, DevBuf<int32_t> &core_all) {
     kombgpu_comm *c = g->comm;

@@ -25,7 +25,6 @@
 #include <cstdio>
 #include <cstdlib>
 #include <cstring>
-#include <vector>
 
 #include "kombgpu_debug.h"
 #include "prank.cuh"
@@ -46,7 +45,6 @@ constexpr int kOPlanRing = 256;
 constexpr uint32_t kOPlanSync = 64;
 
 enum : uint32_t { kPlanWalk = 1, kPlanFull = 2, kPlanDone = 4 };   // the next step: a walk (else a scan), on all CTAs, or none
-enum : uint32_t { kErrBarrier = 1, kErrPeers = 2, kErrBadEntry = 4, kErrFull = 5 };
 
 // control words, one block per rank in symmetric memory: w[t & 1][src][i] is written by rank src at step t
 //   0: length of src's log   1: smallest surviving degree at src (scan steps)
@@ -99,28 +97,6 @@ struct OShared {
     unsigned long long src_lo[kMaxRanks], src_cnt[kMaxRanks];
     uint32_t bcast;
 };
-
-// every CTA learns the plan CTA 0 released for step t
-__device__ __forceinline__ uint32_t wait_plan(unsigned long long *word, uint32_t t, ORankState *st, uint32_t *s_bcast) {
-    if (threadIdx.x == 0) {
-        const unsigned long long t0 = pglobal_ns();
-        uint32_t spins = 0, res = 0;
-        while (true) {
-            const unsigned long long w = ld_acq_gpu(word);
-            if ((uint32_t)(w >> 8) == t) { res = (uint32_t)(w & 0xffu); break; }
-            if ((++spins & 4095u) == 0 && (*(volatile uint32_t *)&st->error || pglobal_ns() - t0 > kPeelWatchdogNs)) {
-                atomicCAS(&st->error, 0u, (uint32_t)kErrBarrier);
-                res = kPlanDone;
-                break;
-            }
-        }
-        *s_bcast = res;
-    }
-    __syncthreads();
-    const uint32_t r = *s_bcast;
-    __syncthreads();
-    return r;
-}
 
 // The lanes with found set took a degree from k + 1 to k: they log their unitig into layer lnext with coreness k.
 // Called by whole warps; one atomic on the log length per warp.
@@ -455,7 +431,7 @@ __global__ void __launch_bounds__(kOThreads, 2) ponion_kernel(const ORank *ranks
             rank_barrier(st, R.ctas, bar_gen, false);
         }
         if (leader_cta && warp == 0) meet(R, st, t, walk, k, lnum, !full, peer_log_hi, published);
-        flags = wait_plan(&st->plan[t % kOPlanRing], t, st, &sh.bcast);
+        flags = wait_plan<kPlanDone>(&st->plan[t % kOPlanRing], t, st, &sh.bcast);
         k = __ldcg(&st->plan_k[t % kOPlanRing]);
         lnum = __ldcg(&st->plan_layer[t % kOPlanRing]);
         if (*(volatile uint32_t *)&st->error) break;
@@ -489,10 +465,11 @@ int dist_onion(kombgpu_dist_graph *g) {
     PeerPtrs<OnionCtl> ctl_peers{};
     // every unitig of the graph is walked once on each rank: sum of ceil(len / kOSliceLen) over the long lists
     const uint64_t slice_cap64 = 2 * g->n_directed / kOSliceLen + 1;
-    int per_sm = 0;
     uint32_t ctas_per_rank = 0;
     ORank R{};
-    const int rc = [&]() -> int {
+    int rc = sym_alloc(c, (size_t)world * log_cap, &logs, &logs_peers);
+    rc = first_rc(rc, sym_alloc(c, 1, &ctl, &ctl_peers));
+    if (rc == KOMBGPU_OK) rc = [&]() -> int {
         const uint32_t *nbr_ptr = g->nbr_ptr, *nbr = g->nbr;
         if (!nbr_ptr) {
             // the build laid out rows for the asynchronous or replicated peel: the onion walks their transpose
@@ -503,8 +480,6 @@ int dist_onion(kombgpu_dist_graph *g) {
             nbr = t_nbr.p;
         }
         if (slice_cap64 >= 0xffffffffull) return ctx_fail(ctx, KOMBGPU_EINVAL, "partition too large for the onion's slice list");
-        KG_TRY(sym_alloc(c, (size_t)world * log_cap, &logs, &logs_peers));
-        KG_TRY(sym_alloc(c, 1, &ctl, &ctl_peers));
         KG_CUDA(ctx, cudaMemsetAsync(ctl, 0, sizeof(OnionCtl), ctx->stream));
         KG_CUDA(ctx, cudaMemsetAsync(logs, 0xff, (size_t)world * log_cap * sizeof(uint32_t), ctx->stream));   // kLogEmpty
         KG_ALLOC(ctx, layer, n_local);
@@ -521,11 +496,7 @@ int dist_onion(kombgpu_dist_graph *g) {
         ORankState init{};
         init.local_min = INT32_MAX;
         KG_CUDA(ctx, cudaMemcpyAsync(state.p, &init, sizeof(init), cudaMemcpyHostToDevice, ctx->stream));
-        KG_CUDA(ctx, cudaOccupancyMaxActiveBlocksPerMultiprocessor(&per_sm, ponion_kernel, kOThreads, 0));
-        if (per_sm < 1) return ctx_fail(ctx, KOMBGPU_ECUDA, "partitioned onion kernel does not fit on an SM");
-        const int resident = per_sm * ctx->sm_count;
-        ctas_per_rank = c->same_device ? (uint32_t)(resident / world) : (uint32_t)resident;
-        if (ctas_per_rank < 1) return ctx_fail(ctx, KOMBGPU_EINVAL, "too many ranks on one device");
+        KG_TRY(rank_ctas(ctx, c, ponion_kernel, kOThreads, 1, &ctas_per_rank));
         R.n_local = n_local; R.v_lo = g->v_lo; R.n_global = g->n_global; R.world = world; R.rank = c->rank; R.ctas = ctas_per_rank;
         R.nbr_ptr = nbr_ptr; R.nbr = nbr; R.deg = work.p; R.core = core.p; R.layer = layer.p;
         R.alive[0] = alive_a.p; R.alive[1] = alive_b.p;
@@ -541,52 +512,17 @@ int dist_onion(kombgpu_dist_graph *g) {
         KG_CUDA(ctx, cudaStreamSynchronize(ctx->stream));   // the control words are cleared before any peer publishes
         return KOMBGPU_OK;
     }();
-    KG_TRY(exchange_rc(c, rc, nullptr, 0, nullptr));
+    KG_TRY(barrier_rc(c, rc));
 
-    cudaEvent_t ev0 = nullptr, ev1 = nullptr;
-    cudaError_t le = cudaEventCreate(&ev0);
-    if (le == cudaSuccess) le = cudaEventCreate(&ev1);
-    auto launch = [&](const ORank *dp, uint32_t grid) -> cudaError_t {
-        uint32_t cpr = ctas_per_rank;
-        void *args[] = {(void *)&dp, (void *)&cpr};
-        cudaError_t e = cudaEventRecord(ev0, ctx->stream);
-        if (e == cudaSuccess) e = cudaLaunchCooperativeKernel((void *)ponion_kernel, dim3(grid), dim3(kOThreads), args, 0, ctx->stream);
-        ctx->launches++;
-        if (e == cudaSuccess) e = cudaEventRecord(ev1, ctx->stream);
-        if (e == cudaSuccess) e = cudaEventSynchronize(ev1);
-        if (e == cudaSuccess) e = cudaEventElapsedTime(&info.ms_kernel, ev0, ev1);
-        return e;
-    };
-    if (!c->same_device) {
-        if (le == cudaSuccess) le = cudaMemcpyAsync(desc.p, &R, sizeof(R), cudaMemcpyHostToDevice, ctx->stream);
-        if (le == cudaSuccess) le = launch(desc.p, ctas_per_rank);
-    } else {
-        // emulation: one cooperative grid holds every rank (a group of CTAs each); rank 0's thread launches it
-        LocalGroup *grp = c->group;
-        grp->slot[c->rank] = &R;
-        KG_TRY(comm_group_barrier(c));
-        if (c->rank == 0) {
-            std::vector<ORank> all(world);
-            for (int q = 0; q < world; ++q) all[q] = *static_cast<ORank *>(grp->slot[q]);
-            if (le == cudaSuccess) le = cudaMemcpyAsync(desc.p, all.data(), sizeof(ORank) * world, cudaMemcpyHostToDevice, ctx->stream);
-            if (le == cudaSuccess) le = launch(desc.p, ctas_per_rank * world);
-            grp->slot_rc = le == cudaSuccess ? 0 : 1;
-        }
-        KG_TRY(comm_group_barrier(c));
-        if (grp->slot_rc) le = cudaErrorLaunchFailure;
-        KG_TRY(comm_group_barrier(c));   // slot_rc was read by everyone before the next use
-    }
-    if (ev0) cudaEventDestroy(ev0);
-    if (ev1) cudaEventDestroy(ev1);
-
+    const cudaError_t le = launch_ranks(c, ponion_kernel, kOThreads, ctas_per_rank, R, desc.p, &info.ms_kernel);
+    if (le != cudaSuccess) rc = ctx_fail(ctx, KOMBGPU_ECUDA, "partitioned onion kernel: %s", cudaGetErrorString(le));
     ORankState fin{};
-    int rc_fin = le == cudaSuccess ? KOMBGPU_OK : ctx_fail(ctx, KOMBGPU_ECUDA, "partitioned onion kernel: %s", cudaGetErrorString(le));
-    if (rc_fin == KOMBGPU_OK) rc_fin = read_back(ctx, state.p, &fin, 1);
+    if (rc == KOMBGPU_OK) rc = read_back(ctx, state.p, &fin, 1);
     // global figures; also: nobody gives back its logs (at return) while a peer may still be writing
     uint32_t ms_bits = 0;
     memcpy(&ms_bits, &info.ms_kernel, sizeof(ms_bits));
     unsigned long long mine[5] = {fin.error, fin.log_cnt, fin.n_layers, fin.meetings, ms_bits}, all[kMaxRanks * 5];
-    KG_TRY(exchange_rc(c, rc_fin, mine, 5, all));
+    KG_TRY(exchange_rc(c, rc, mine, 5, all));
     if (c->same_device) {
         // every rank ran inside rank 0's launch, which its events timed
         ms_bits = (uint32_t)all[4];
@@ -594,7 +530,7 @@ int dist_onion(kombgpu_dist_graph *g) {
     }
     uint64_t placed = 0;
     for (int q = 0; q < world; ++q) {
-        if (all[q * 5]) return ctx_fail(ctx, KOMBGPU_EINTERNAL, "partitioned onion: rank %d reports error %llu (1/2 watchdog, 4 bad log entry, 5 list full)", q, all[q * 5]);
+        if (all[q * 5]) return ctx_fail(ctx, KOMBGPU_EINTERNAL, "partitioned onion: rank %d reports error %llu (%s)", q, all[q * 5], rank_error_text(all[q * 5]));
         placed += all[q * 5 + 1];
         if (all[q * 5 + 2] != fin.n_layers || all[q * 5 + 3] != fin.meetings)
             return ctx_fail(ctx, KOMBGPU_EINTERNAL, "partitioned onion: rank %d ended at layer %llu after %llu meetings, rank %d at %u after %u", q,

@@ -34,7 +34,6 @@
 
 #include <cstdio>
 #include <cstdlib>
-#include <vector>
 
 #include "prank.cuh"
 
@@ -78,7 +77,7 @@ struct PRankState {
     int32_t local_min;
     int32_t max_core;
     uint32_t levels, subrounds, solo_subrounds;
-    uint32_t error;                             // 1 watchdog (CTAs), 2 watchdog (peers), 4 bad log entry, 5 list overflow
+    uint32_t error;                             // kErr*
     // where the leader thread's time goes (ns): 0 scan + barrier, 1 plan A, 2 publish copy (+ barrier), 3 wait for the
     // peers, 4 exchange, 5 walk (+ barrier), 6 full publishes, 7 full walks
     unsigned long long prof_ns[8];
@@ -104,28 +103,6 @@ struct PRank {
     PRankState *st;
 };
 
-// every CTA learns what the leader decided for sub-round t
-__device__ __forceinline__ uint32_t wait_plan(unsigned long long *word, uint32_t t, PRankState *st, uint32_t *s_bcast) {
-    if (threadIdx.x == 0) {
-        const unsigned long long t0 = pglobal_ns();
-        uint32_t spins = 0, res = 0;
-        while (true) {
-            const unsigned long long w = ld_acq_gpu(word);
-            if ((uint32_t)(w >> 8) == t) { res = (uint32_t)(w & 0xffu); break; }
-            if ((++spins & 4095u) == 0 && (*(volatile uint32_t *)&st->error || pglobal_ns() - t0 > kPeelWatchdogNs)) {
-                atomicCAS(&st->error, 0u, 1u);
-                res = kFlagDone;
-                break;
-            }
-        }
-        *s_bcast = res;
-    }
-    __syncthreads();
-    const uint32_t r = *s_bcast;
-    __syncthreads();
-    return r;
-}
-
 // discoveries of a CTA are collected in shared memory and appended to the rank's log with ONE atomic per flush
 struct Stage {
     uint32_t n;
@@ -145,7 +122,7 @@ __device__ __forceinline__ void stage_flush(const PRank &R, PRankState *st, Stag
         uint32_t *log = R.log_local[R.rank];
         for (uint32_t i = threadIdx.x; i < n; i += kPThreads) {
             if (base + i < R.log_cap) log[base + i] = sg.ids[i];
-            else atomicCAS(&st->error, 0u, 5u);
+            else atomicCAS(&st->error, 0u, (uint32_t)kErrFull);
         }
         __syncthreads();
         if (threadIdx.x == 0) sg.n = 0;
@@ -169,7 +146,7 @@ __device__ __forceinline__ void discover(const PRank &R, PRankState *st, Stage &
         } else {
             const uint32_t at = atomicAdd(&st->log_cnt, 1u);
             if (at < R.log_cap) R.log_local[R.rank][at] = R.v_lo + loc;
-            else atomicCAS(&st->error, 0u, 5u);
+            else atomicCAS(&st->error, 0u, (uint32_t)kErrFull);
         }
     }
 }
@@ -258,7 +235,7 @@ __device__ __forceinline__ void walk_stage(const PRank &R, PRankState *st, Stage
             while (off >= sg.src_cnt[q]) { off -= sg.src_cnt[q]; ++q; }   // which source's log (i < total_new: q stays < world)
             const uint32_t x = log_read(&R.log_local[q][sg.src_lo[q] + off], st);
             if (x >= R.n_global) {
-                atomicCAS(&st->error, 0u, 4u);
+                atomicCAS(&st->error, 0u, (uint32_t)kErrBadEntry);
             } else {
                 first = R.nbr_ptr[x];
                 len = R.nbr_ptr[x + 1] - first;
@@ -275,7 +252,7 @@ __device__ __forceinline__ void walk_stage(const PRank &R, PRankState *st, Stage
             for (uint32_t s = 0; s < n_cut; ++s) {
                 const uint32_t l = min(kSliceLen, len - s * kSliceLen);
                 if (pos + s < R.slice_cap) R.slices[nxt][pos + s] = ((uint64_t)(first + s * kSliceLen) << 12) | (uint64_t)(l - 1u);
-                else atomicCAS(&st->error, 0u, 5u);
+                else atomicCAS(&st->error, 0u, (uint32_t)kErrFull);
             }
             if (n_cut) len = 0;
         }
@@ -329,7 +306,7 @@ __device__ __forceinline__ void scan_stage(const PRank &R, PRankState *st, uint3
         for (int j = 0; j < kScanItems; ++j) {
             if (flag[j] == 1u) {
                 if (fpos < R.log_cap) log[fpos] = R.v_lo + v[j];
-                else atomicCAS(&st->error, 0u, 5u);
+                else atomicCAS(&st->error, 0u, (uint32_t)kErrFull);
                 ++fpos;
             } else if (flag[j]) {
                 alive_dst[spos++] = v[j];
@@ -400,7 +377,7 @@ __device__ __forceinline__ void leader_exchange(const PRank &R, PRankState *st, 
     if (lane == 0) st->prof_ns[3] += pglobal_ns() - t_wait;
     if (__ballot_sync(kFullMask, failed)) {
         if (lane == 0) {
-            atomicCAS(&st->error, 0u, 2u);
+            atomicCAS(&st->error, 0u, (uint32_t)kErrPeers);
             st_rel_gpu(&st->plan_b[t % kPlanRing], ((unsigned long long)t << 8) | kFlagDone);
         }
         return;
@@ -497,7 +474,7 @@ __global__ void __launch_bounds__(kPThreads, 2) ppeel_kernel(const PRank *ranks,
             const uint32_t mode = (R.world > 1 && fresh > kSoloCopy) ? kCopyFull : 0u;
             st_rel_gpu(&st->plan_a[t % kPlanRing], ((unsigned long long)t << 8) | mode);
         }
-        const uint32_t mode_a = wait_plan(&st->plan_a[t % kPlanRing], t, st, &s_bcast);
+        const uint32_t mode_a = wait_plan<kFlagDone>(&st->plan_a[t % kPlanRing], t, st, &s_bcast);
         if (mode_a & kFlagDone) break;   // watchdog
         KG_PROF(1);
         // ---- publish
@@ -509,7 +486,7 @@ __global__ void __launch_bounds__(kPThreads, 2) ppeel_kernel(const PRank *ranks,
         KG_PROF(2);
         // ---- exchange (a short publish is done by the leader warp itself)
         if (leader_cta && warp == 0) leader_exchange(R, st, t, cur, k, scan, !(mode_a & kCopyFull), peer_log_hi, published);
-        const uint32_t flags = wait_plan(&st->plan_b[t % kPlanRing], t, st, &s_bcast);
+        const uint32_t flags = wait_plan<kFlagDone>(&st->plan_b[t % kPlanRing], t, st, &s_bcast);
         KG_PROF(4);
         // ---- walk
         if (!(flags & kFlagLevelOver)) {
@@ -530,7 +507,7 @@ __global__ void __launch_bounds__(kPThreads, 2) ppeel_kernel(const PRank *ranks,
         KG_PROF(5);
         if ((flags & kFlagDone) || *(volatile uint32_t *)&st->error) break;
         ++t;
-        if (t >= (1u << 24) - 2u) { if (tid == 0) atomicCAS(&st->error, 0u, 1u); break; }
+        if (t >= (1u << 24) - 2u) { if (tid == 0) atomicCAS(&st->error, 0u, (uint32_t)kErrBarrier); break; }
         if (flags & kFlagLevelOver) {
             k = __ldcg(&st->k_next[(t - 1u) % kPlanRing]);
             scan = true;
@@ -543,120 +520,76 @@ __global__ void __launch_bounds__(kPThreads, 2) ppeel_kernel(const PRank *ranks,
 
 }  // namespace
 
-int dist_peel(kombgpu_dist_graph *g) {
+int dist_peel(kombgpu_dist_graph *g, int rc) {
     kombgpu_comm *c = g->comm;
     kombgpu_ctx *ctx = g->ctx;
     const int world = c->world;
     const uint32_t n_local = g->n_local;
-    cudaEvent_t ev0 = nullptr, ev1 = nullptr;
-    KG_CUDA(ctx, cudaEventCreate(&ev0));
-    KG_CUDA(ctx, cudaEventCreate(&ev1));
-    KG_CUDA(ctx, cudaEventRecord(ev0, ctx->stream));
-    if (!g->core) {
-        g->core = static_cast<int32_t *>(ws_alloc(ctx, (n_local ? n_local : 1) * sizeof(int32_t)));
-        if (!g->core) return ctx_fail(ctx, KOMBGPU_ENOMEM, "coreness array");
-    }
-    KG_CUDA(ctx, cudaMemsetAsync(g->core, 0, (size_t)(n_local ? n_local : 1) * sizeof(int32_t), ctx->stream));
 
     // symmetric: one log per rank (every rank holds a copy of every rank's log) + the control words
     const uint32_t log_cap = g->step;   // the largest n_local
-    const SymMark mark = sym_mark(c);
+    SymRewind heap{c, sym_mark(c)};
     uint32_t *logs = nullptr;
     PeerPtrs<uint32_t> logs_peers{};
     PeelCtl *ctl = nullptr;
     PeerPtrs<PeelCtl> ctl_peers{};
-    KG_TRY(sym_alloc(c, (size_t)world * log_cap, &logs, &logs_peers));
-    KG_TRY(sym_alloc(c, 1, &ctl, &ctl_peers));
-    KG_CUDA(ctx, cudaMemsetAsync(ctl, 0, sizeof(PeelCtl), ctx->stream));
-    KG_CUDA(ctx, cudaMemsetAsync(logs, 0xff, (size_t)world * log_cap * sizeof(uint32_t), ctx->stream));   // kLogEmpty
+    rc = first_rc(rc, sym_alloc(c, (size_t)world * log_cap, &logs, &logs_peers));
+    rc = first_rc(rc, sym_alloc(c, 1, &ctl, &ctl_peers));
 
     // per-rank lists and state
     DevBuf<int32_t> work;
     DevBuf<uint32_t> alive_a, alive_b;
     DevBuf<uint64_t> slices_a, slices_b;
-    DevBuf<PRankState> state(ctx, 1);
-    DevBuf<PRank> desc(ctx, kMaxRanks);
-    // every unitig of the graph is walked once here, its list cut into ceil(len / kSliceLen) slices when it is long
-    const uint64_t slice_cap64 = g->n_directed / kSliceLen + (uint64_t)g->n_global / 64 + 1024;
-    if (slice_cap64 >= 0xffffffffull) return ctx_fail(ctx, KOMBGPU_EINVAL, "partition too large for the slice list");
-    KG_ALLOC(ctx, work, n_local);
-    KG_ALLOC(ctx, alive_a, n_local);
-    KG_ALLOC(ctx, alive_b, n_local);
-    KG_ALLOC(ctx, slices_a, slice_cap64);
-    KG_ALLOC(ctx, slices_b, slice_cap64);
-    if (!state || !desc) return ctx_fail(ctx, KOMBGPU_ENOMEM, "workspace");
-    KG_CUDA(ctx, cudaMemcpyAsync(work.p, g->deg, (size_t)n_local * sizeof(int32_t), cudaMemcpyDeviceToDevice, ctx->stream));
-    PRankState init{};
-    init.local_min = INT32_MAX;
-    KG_CUDA(ctx, cudaMemcpyAsync(state.p, &init, sizeof(init), cudaMemcpyHostToDevice, ctx->stream));
-
-    int per_sm = 0;
-    KG_CUDA(ctx, cudaOccupancyMaxActiveBlocksPerMultiprocessor(&per_sm, ppeel_kernel, kPThreads, 0));
-    if (per_sm < 1) return ctx_fail(ctx, KOMBGPU_ECUDA, "partitioned peel kernel does not fit on an SM");
-    const int resident = per_sm * ctx->sm_count;
-    const uint32_t ctas_per_rank = c->same_device ? (uint32_t)(resident / world) : (uint32_t)resident;
-    if (ctas_per_rank < 1) return ctx_fail(ctx, KOMBGPU_EINVAL, "too many ranks on one device");
-
+    DevBuf<PRankState> state;
+    DevBuf<PRank> desc;
+    uint32_t ctas_per_rank = 0;
     PRank R{};
-    R.n_local = n_local; R.v_lo = g->v_lo; R.n_global = g->n_global; R.world = world; R.rank = c->rank; R.ctas = ctas_per_rank;
-    R.nbr_ptr = g->nbr_ptr; R.nbr = g->nbr; R.deg = work.p; R.core = g->core;
-    R.alive[0] = alive_a.p; R.alive[1] = alive_b.p;
-    R.slices[0] = slices_a.p; R.slices[1] = slices_b.p; R.slice_cap = (uint32_t)slice_cap64;
-    R.log_cap = log_cap;
-    R.ctl_local = ctl;
-    for (int q = 0; q < world; ++q) {
-        R.ctl_peer[q] = ctl_peers.p[q];
-        R.log_local[q] = logs + (size_t)q * log_cap;                         // my copy of rank q's log
-        R.log_peer[q] = logs_peers.p[q] + (size_t)c->rank * log_cap;        // rank q's copy of my log
-    }
-    R.st = state.p;
-
-    // every rank's control words are cleared before anyone publishes into them
-    unsigned long long token = 1, tokens[kMaxRanks];
-    KG_TRY(comm_exchange(c, &token, 1, tokens));
-
-    cudaError_t le = cudaSuccess;
-    if (!c->same_device) {
-        KG_CUDA(ctx, cudaMemcpyAsync(desc.p, &R, sizeof(R), cudaMemcpyHostToDevice, ctx->stream));
-        const PRank *dp = desc.p;
-        uint32_t cpr = ctas_per_rank;
-        void *args[] = {(void *)&dp, (void *)&cpr};
-        le = cudaLaunchCooperativeKernel((void *)ppeel_kernel, dim3(ctas_per_rank), dim3(kPThreads), args, 0, ctx->stream);
-        ctx->launches++;
-        if (le == cudaSuccess) le = cudaStreamSynchronize(ctx->stream);
-    } else {
-        // emulation: one cooperative grid holds every rank (a group of CTAs each); rank 0's thread launches it
-        LocalGroup *grp = c->group;
-        grp->slot[c->rank] = &R;
-        KG_TRY(comm_group_barrier(c));
-        if (c->rank == 0) {
-            std::vector<PRank> all(world);
-            for (int q = 0; q < world; ++q) all[q] = *static_cast<PRank *>(grp->slot[q]);
-            le = cudaMemcpyAsync(desc.p, all.data(), sizeof(PRank) * world, cudaMemcpyHostToDevice, ctx->stream);
-            const PRank *dp = desc.p;
-            uint32_t cpr = ctas_per_rank;
-            void *args[] = {(void *)&dp, (void *)&cpr};
-            if (le == cudaSuccess)
-                le = cudaLaunchCooperativeKernel((void *)ppeel_kernel, dim3(ctas_per_rank * world), dim3(kPThreads), args, 0, ctx->stream);
-            ctx->launches++;
-            if (le == cudaSuccess) le = cudaStreamSynchronize(ctx->stream);
-            grp->slot_rc = le == cudaSuccess ? 0 : 1;
+    if (rc == KOMBGPU_OK) rc = [&]() -> int {
+        KG_CUDA(ctx, cudaMemsetAsync(g->core, 0, (size_t)(n_local ? n_local : 1) * sizeof(int32_t), ctx->stream));
+        KG_CUDA(ctx, cudaMemsetAsync(ctl, 0, sizeof(PeelCtl), ctx->stream));
+        KG_CUDA(ctx, cudaMemsetAsync(logs, 0xff, (size_t)world * log_cap * sizeof(uint32_t), ctx->stream));   // kLogEmpty
+        // every unitig of the graph is walked once here, its list cut into ceil(len / kSliceLen) slices when it is long
+        const uint64_t slice_cap64 = g->n_directed / kSliceLen + (uint64_t)g->n_global / 64 + 1024;
+        if (slice_cap64 >= 0xffffffffull) return ctx_fail(ctx, KOMBGPU_EINVAL, "partition too large for the slice list");
+        KG_ALLOC(ctx, work, n_local);
+        KG_ALLOC(ctx, alive_a, n_local);
+        KG_ALLOC(ctx, alive_b, n_local);
+        KG_ALLOC(ctx, slices_a, slice_cap64);
+        KG_ALLOC(ctx, slices_b, slice_cap64);
+        KG_ALLOC(ctx, state, 1);
+        KG_ALLOC(ctx, desc, kMaxRanks);
+        KG_CUDA(ctx, cudaMemcpyAsync(work.p, g->deg, (size_t)n_local * sizeof(int32_t), cudaMemcpyDeviceToDevice, ctx->stream));
+        PRankState init{};
+        init.local_min = INT32_MAX;
+        KG_CUDA(ctx, cudaMemcpyAsync(state.p, &init, sizeof(init), cudaMemcpyHostToDevice, ctx->stream));
+        KG_TRY(rank_ctas(ctx, c, ppeel_kernel, kPThreads, 1, &ctas_per_rank));
+        R.n_local = n_local; R.v_lo = g->v_lo; R.n_global = g->n_global; R.world = world; R.rank = c->rank; R.ctas = ctas_per_rank;
+        R.nbr_ptr = g->nbr_ptr; R.nbr = g->nbr; R.deg = work.p; R.core = g->core;
+        R.alive[0] = alive_a.p; R.alive[1] = alive_b.p;
+        R.slices[0] = slices_a.p; R.slices[1] = slices_b.p; R.slice_cap = (uint32_t)slice_cap64;
+        R.log_cap = log_cap;
+        R.ctl_local = ctl;
+        for (int q = 0; q < world; ++q) {
+            R.ctl_peer[q] = ctl_peers.p[q];
+            R.log_local[q] = logs + (size_t)q * log_cap;                         // my copy of rank q's log
+            R.log_peer[q] = logs_peers.p[q] + (size_t)c->rank * log_cap;        // rank q's copy of my log
         }
-        KG_TRY(comm_group_barrier(c));
-        if (grp->slot_rc) le = cudaErrorLaunchFailure;
-        KG_TRY(comm_group_barrier(c));   // slot_rc was read by everyone before the next use
-    }
-    if (le != cudaSuccess) return ctx_fail(ctx, KOMBGPU_ECUDA, "partitioned peel kernel: %s", cudaGetErrorString(le));
+        R.st = state.p;
+        return KOMBGPU_OK;
+    }();
+    // every rank's control words are cleared before anyone publishes into them
+    KG_TRY(barrier_rc(c, rc));
 
+    const cudaError_t le = launch_ranks(c, ppeel_kernel, kPThreads, ctas_per_rank, R, desc.p, nullptr);
+    if (le != cudaSuccess) rc = ctx_fail(ctx, KOMBGPU_ECUDA, "partitioned peel kernel: %s", cudaGetErrorString(le));
     PRankState fin{};
-    KG_TRY(read_back(ctx, state.p, &fin, 1));
-    // global figures; also: nobody releases its logs while a peer may still be writing
+    if (rc == KOMBGPU_OK) rc = read_back(ctx, state.p, &fin, 1);
+    // global figures; also: nobody gives back its logs (at return) while a peer may still be writing
     unsigned long long mine[3] = {fin.error, fin.log_cnt, (unsigned long long)(uint32_t)fin.max_core}, all[kMaxRanks * 3];
-    KG_TRY(comm_exchange(c, mine, 3, all));
-    sym_release(c, mark);
+    KG_TRY(exchange_rc(c, rc, mine, 3, all));
     uint64_t peeled = 0;
     for (int q = 0; q < world; ++q) {
-        if (all[q * 3]) return ctx_fail(ctx, KOMBGPU_EINTERNAL, "partitioned peel: rank %d reports error %llu (1/2 watchdog, 4 bad log entry, 5 list overflow)", q, all[q * 3]);
+        if (all[q * 3]) return ctx_fail(ctx, KOMBGPU_EINTERNAL, "partitioned peel: rank %d reports error %llu (%s)", q, all[q * 3], rank_error_text(all[q * 3]));
         peeled += all[q * 3 + 1];
     }
     if (peeled != g->n_global) return ctx_fail(ctx, KOMBGPU_EINTERNAL, "partitioned peel ended with %llu of %u unitigs peeled", (unsigned long long)peeled, g->n_global);
@@ -666,18 +599,12 @@ int dist_peel(kombgpu_dist_graph *g) {
     g->st.peel_solo_subrounds = fin.solo_subrounds;
     g->st.n_messages_sent = (uint64_t)fin.log_cnt * (uint64_t)(world - 1);   // ids copied to peers
     g->st.n_messages_recv = peeled - fin.log_cnt;
-    g->has_core = true;
     if (getenv("KOMBGPU_DEBUG"))
         fprintf(stderr, "[kombgpu] rank %d ppeel: levels %u subrounds %u (solo walks %u; full copies %u, full walks %u) ctas %u | leader ms: scan %.3f planA %.3f "
                 "publish %.3f (full %.3f) exchange %.3f (wait peers %.3f) walk %.3f (full %.3f) | peeled here %u, entries visited %llu\n",
                 c->rank, fin.levels, fin.subrounds, fin.solo_subrounds, fin.full_copy, fin.full_walk, ctas_per_rank, fin.prof_ns[0] * 1e-6,
                 fin.prof_ns[1] * 1e-6, fin.prof_ns[2] * 1e-6, fin.prof_ns[6] * 1e-6, fin.prof_ns[4] * 1e-6, fin.prof_ns[3] * 1e-6,
                 fin.prof_ns[5] * 1e-6, fin.prof_ns[7] * 1e-6, fin.log_cnt, fin.n_visited);
-    KG_CUDA(ctx, cudaEventRecord(ev1, ctx->stream));
-    KG_CUDA(ctx, cudaEventSynchronize(ev1));
-    cudaEventElapsedTime(&g->st.ms_peel, ev0, ev1);
-    cudaEventDestroy(ev0);
-    cudaEventDestroy(ev1);
     return KOMBGPU_OK;
 }
 

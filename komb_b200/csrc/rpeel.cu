@@ -26,21 +26,16 @@ __global__ void __launch_bounds__(kThreads) place_rows_kernel(const uint32_t *__
 
 }  // namespace
 
-int dist_peel_replicated(kombgpu_dist_graph *g) {
+int dist_peel_replicated(kombgpu_dist_graph *g, int rc) {
     kombgpu_comm *c = g->comm;
     kombgpu_ctx *ctx = g->ctx;
     const int world = c->world;
     const uint32_t n_local = g->n_local, n_global = g->n_global;
     if (!g->row_ptr32) return ctx_fail(ctx, KOMBGPU_ESTATE, "the replicated peel needs the rank's rows");
-    cudaEvent_t ev0 = nullptr, ev1 = nullptr;
-    KG_CUDA(ctx, cudaEventCreate(&ev0));
-    KG_CUDA(ctx, cudaEventCreate(&ev1));
-    KG_CUDA(ctx, cudaEventRecord(ev0, ctx->stream));
-    const uint64_t launches0 = ctx->launches;
 
     // every rank's share of the adjacency
     unsigned long long mine = g->n_directed, all_dir[kMaxRanks];
-    KG_TRY(comm_exchange(c, &mine, 1, all_dir));
+    KG_TRY(exchange_rc(c, rc, &mine, 1, all_dir));
     uint64_t total = 0, max_dir = 0, off[kMaxRanks + 1] = {};
     for (int q = 0; q < world; ++q) {
         off[q] = total;
@@ -48,18 +43,20 @@ int dist_peel_replicated(kombgpu_dist_graph *g) {
         max_dir = all_dir[q] > max_dir ? all_dir[q] : max_dir;
     }
     off[world] = total;
-    if (total >= (1ull << 32)) return ctx_fail(ctx, KOMBGPU_EINVAL, "graph too large for the replicated peel");
+    if (total >= (1ull << 32)) return ctx_fail(ctx, KOMBGPU_EINVAL, "graph too large for the replicated peel");   // on every rank
 
     // the rows go into the symmetric heap, where the peers can read them
-    const SymMark mark = sym_mark(c);
+    SymRewind heap{c, sym_mark(c)};
     uint32_t *col_sym = nullptr, *rp_sym = nullptr;
     PeerPtrs<uint32_t> col_peers{}, rp_peers{};
-    KG_TRY(sym_alloc(c, (size_t)max_dir, &col_sym, &col_peers));
-    KG_TRY(sym_alloc(c, (size_t)g->step + 1, &rp_sym, &rp_peers));
-    if (g->n_directed) KG_CUDA(ctx, cudaMemcpyAsync(col_sym, g->col, g->n_directed * sizeof(uint32_t), cudaMemcpyDeviceToDevice, ctx->stream));
-    KG_CUDA(ctx, cudaMemcpyAsync(rp_sym, g->row_ptr32, ((size_t)n_local + 1) * sizeof(uint32_t), cudaMemcpyDeviceToDevice, ctx->stream));
-    unsigned long long token = 1, tokens[kMaxRanks];
-    KG_TRY(comm_exchange(c, &token, 1, tokens));   // every rank's rows are in place
+    rc = sym_alloc(c, (size_t)max_dir, &col_sym, &col_peers);
+    rc = first_rc(rc, sym_alloc(c, (size_t)g->step + 1, &rp_sym, &rp_peers));
+    if (rc == KOMBGPU_OK) rc = [&]() -> int {
+        if (g->n_directed) KG_CUDA(ctx, cudaMemcpyAsync(col_sym, g->col, g->n_directed * sizeof(uint32_t), cudaMemcpyDeviceToDevice, ctx->stream));
+        KG_CUDA(ctx, cudaMemcpyAsync(rp_sym, g->row_ptr32, ((size_t)n_local + 1) * sizeof(uint32_t), cudaMemcpyDeviceToDevice, ctx->stream));
+        return KOMBGPU_OK;
+    }();
+    KG_TRY(barrier_rc(c, rc));   // every rank's rows are in place
 
     kombgpu_graph whole;
     whole.ctx = ctx;
@@ -67,37 +64,33 @@ int dist_peel_replicated(kombgpu_dist_graph *g) {
     whole.n_edges = total / 2;
     whole.st.max_coreness = -1;
     auto fail = [&](int rc) { graph_release(&whole); return rc; };
-    whole.row_ptr = static_cast<uint64_t *>(ws_alloc(ctx, ((size_t)n_global + 1) * sizeof(uint64_t)));
-    whole.col = static_cast<uint32_t *>(ws_alloc(ctx, (size_t)(total ? total : 1) * sizeof(uint32_t)));
-    whole.deg = static_cast<int32_t *>(ws_alloc(ctx, (size_t)(n_global ? n_global : 1) * sizeof(int32_t)));
-    if (!whole.row_ptr || !whole.col || !whole.deg) return fail(ctx_fail(ctx, KOMBGPU_ENOMEM, "the whole graph's CSR"));
-    for (int q = 0; q < world; ++q) {
-        const uint64_t lo = (uint64_t)q * g->step;
-        const uint32_t rows_q = lo < n_global ? (uint32_t)((lo + g->step < n_global ? lo + g->step : n_global) - lo) : 0u;
-        if (all_dir[q]) {
-            const cudaError_t e = cudaMemcpyAsync(whole.col + off[q], col_peers.p[q], all_dir[q] * sizeof(uint32_t), cudaMemcpyDeviceToDevice, ctx->stream);
-            if (e != cudaSuccess) return fail(ctx_fail(ctx, KOMBGPU_ECUDA, "copy of rank %d's rows: %s", q, cudaGetErrorString(e)));
+    rc = [&]() -> int {
+        whole.row_ptr = static_cast<uint64_t *>(ws_alloc(ctx, ((size_t)n_global + 1) * sizeof(uint64_t)));
+        whole.col = static_cast<uint32_t *>(ws_alloc(ctx, (size_t)(total ? total : 1) * sizeof(uint32_t)));
+        whole.deg = static_cast<int32_t *>(ws_alloc(ctx, (size_t)(n_global ? n_global : 1) * sizeof(int32_t)));
+        if (!whole.row_ptr || !whole.col || !whole.deg) return ctx_fail(ctx, KOMBGPU_ENOMEM, "the whole graph's CSR");
+        for (int q = 0; q < world; ++q) {
+            const uint64_t lo = (uint64_t)q * g->step;
+            const uint32_t rows_q = lo < n_global ? (uint32_t)((lo + g->step < n_global ? lo + g->step : n_global) - lo) : 0u;
+            if (all_dir[q]) {
+                const cudaError_t e = cudaMemcpyAsync(whole.col + off[q], col_peers.p[q], all_dir[q] * sizeof(uint32_t), cudaMemcpyDeviceToDevice, ctx->stream);
+                if (e != cudaSuccess) return ctx_fail(ctx, KOMBGPU_ECUDA, "copy of rank %d's rows: %s", q, cudaGetErrorString(e));
+            }
+            if (lo <= n_global && (rows_q || lo == n_global)) {
+                place_rows_kernel<<<min(ceil_div_u64((uint64_t)rows_q + 1, kThreads), 148u * 8u), kThreads, 0, ctx->stream>>>(
+                    rp_peers.p[q], rows_q, off[q], whole.row_ptr + lo, whole.deg + (lo < n_global ? lo : 0));
+                ctx->launches++;
+            }
         }
-        if (lo <= n_global && (rows_q || lo == n_global)) {
-            place_rows_kernel<<<min(ceil_div_u64((uint64_t)rows_q + 1, kThreads), 148u * 8u), kThreads, 0, ctx->stream>>>(
-                rp_peers.p[q], rows_q, off[q], whole.row_ptr + lo, whole.deg + (lo < n_global ? lo : 0));
-            ctx->launches++;
-        }
-    }
-    {
         const cudaError_t e = cudaPeekAtLastError();
-        if (e != cudaSuccess) return fail(ctx_fail(ctx, KOMBGPU_ECUDA, "place_rows_kernel: %s", cudaGetErrorString(e)));
-    }
-    int rc = comm_exchange(c, &token, 1, tokens);   // everybody has read everybody's rows: the symmetric buffers may go
-    sym_release(c, mark);
+        if (e != cudaSuccess) return ctx_fail(ctx, KOMBGPU_ECUDA, "place_rows_kernel: %s", cudaGetErrorString(e));
+        return KOMBGPU_OK;
+    }();
+    rc = barrier_rc(c, rc);   // everybody has read everybody's rows: the symmetric buffers may go
     if (rc != KOMBGPU_OK) return fail(rc);
 
     rc = peel_coreness(&whole);
     if (rc != KOMBGPU_OK) return fail(rc);
-    if (!g->core) {
-        g->core = static_cast<int32_t *>(ws_alloc(ctx, (n_local ? n_local : 1) * sizeof(int32_t)));
-        if (!g->core) return fail(ctx_fail(ctx, KOMBGPU_ENOMEM, "coreness array"));
-    }
     if (n_local) {
         const cudaError_t e = cudaMemcpyAsync(g->core, whole.core + g->v_lo, (size_t)n_local * sizeof(int32_t), cudaMemcpyDeviceToDevice, ctx->stream);
         if (e != cudaSuccess) return fail(ctx_fail(ctx, KOMBGPU_ECUDA, "coreness slice: %s", cudaGetErrorString(e)));
@@ -109,15 +102,8 @@ int dist_peel_replicated(kombgpu_dist_graph *g) {
     g->st.n_messages_sent = 0;
     g->st.n_messages_recv = total - g->n_directed;   // adjacency entries pulled from the peers
     g->st.peel_async = 2;
-    g->has_core = true;
     KG_CUDA(ctx, cudaStreamSynchronize(ctx->stream));
     graph_release(&whole);
-    (void)launches0;
-    KG_CUDA(ctx, cudaEventRecord(ev1, ctx->stream));
-    KG_CUDA(ctx, cudaEventSynchronize(ev1));
-    cudaEventElapsedTime(&g->st.ms_peel, ev0, ev1);
-    cudaEventDestroy(ev0);
-    cudaEventDestroy(ev1);
     return KOMBGPU_OK;
 }
 

@@ -150,6 +150,41 @@ def test_peer_path_bad_input_fails_on_every_rank():
     assert run_local(2, body) == [-1, -1]
 
 
+@pytest.mark.parametrize("world", [2, 3])
+def test_peer_path_bad_corea_mode_fails_on_every_rank(oracle_mod, world):
+    """A CORE-A key mode that only rank 1 gets wrong is KOMBGPU_EINVAL on every rank; then CORE-A runs again on the same
+    graph and gives the exact scores (the communicator and its symmetric heap are usable after the failure)."""
+    import torch
+    import komb_b200
+    from komb_b200._lib import EINVAL
+    from komb_b200.peer import DistGraph, run_local
+    key = oracle_mod.KEY_REF32
+
+    def body(comm):
+        _, n, a, b = _share("hits_small", comm.rank, comm.world)
+        dev = torch.device("cuda", comm.ctx.device)
+        ta = torch.from_numpy(a.view(np.int32).copy()).to(dev)
+        tb = torch.from_numpy(b.view(np.int32).copy()).to(dev)
+        torch.cuda.synchronize(dev)
+        with DistGraph.from_hits(comm, ta, tb, n) as g:
+            g.coreness()
+            code = 0
+            try:
+                g.corea(7 if comm.rank == 1 else key)
+            except komb_b200.KombGpuError as e:
+                code = e.code
+            g.corea(key)
+            return code, g.results()
+
+    out = run_local(world, body)
+    assert [code for code, _ in out] == [EINVAL] * world
+    _, _, deg, core = _expected(oracle_mod, "hits_small")
+    parts = sorted((r for _, r in out), key=lambda r: r["v_lo"])
+    assert np.array_equal(np.concatenate([r["degree"] for r in parts]), deg)
+    assert np.array_equal(np.concatenate([r["coreness"] for r in parts]), core)
+    oracle_mod.check_corea(np.concatenate([r["score"] for r in parts]), core, deg, key)
+
+
 @pytest.mark.parametrize("peel", ["async", "log", "replicated"])
 @pytest.mark.parametrize("case", ["hits_mid", "rmat", "ramp", "hubs"])
 def test_peer_path_one_gpu_per_rank_threads(oracle_mod, monkeypatch, case, peel):
