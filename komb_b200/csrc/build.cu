@@ -8,9 +8,8 @@
 //   all i<j pairs of every set         src/graph.cpp:332-347       segment scan + load-balanced pair emission
 //   dedup / igraph_simplify            src/graph.cpp:342-347,438   sort + adjacent-unique of (min, max)
 //   igraph_create adjacency index      src/graph.cpp:418           boundary detection + scan -> CSR
-// No atomics are needed anywhere in this stage: every count falls out of run
-// boundaries in sorted arrays, so the result (including the order inside each
-// CSR row) is deterministic.
+// Every count falls out of run boundaries in sorted arrays, except the CSR's per-vertex count of back neighbours, an
+// integer sum of atomic increments; so the result (including the order inside each CSR row) is deterministic.
 #include <cstdlib>
 
 #include "graph.cuh"
@@ -393,32 +392,51 @@ __global__ void __launch_bounds__(kThreads) swap_pack_kernel(const uint64_t *__r
 // only the neighbourhood of its own id range; an edge list may leave whole id ranges without edges) is recorded and
 // filled by a whole CTA in a second kernel, so one thread never writes millions of entries.
 // *err (optional) is raised when a key lies outside [base, base + n_rows) or its low word is >= lo_bound.
+// kCountLo: the same read also counts every key's low word, lo_count[lo] += 1 (the caller guarantees lo < lo_bound).
 constexpr int64_t kGapShort = 32;
 struct RowGap {
     uint32_t lo, hi, val;   // start[lo .. hi] = val
 };
+template <bool kCountLo>
 __global__ void __launch_bounds__(kThreads) row_bounds_kernel(const uint64_t *__restrict__ keys, uint64_t count, uint32_t base,
                                                               uint32_t n_rows, uint32_t lo_bound, uint32_t *__restrict__ start,
-                                                              RowGap *__restrict__ gaps, uint32_t *__restrict__ n_gaps, uint32_t *__restrict__ err) {
-    for (uint64_t i = (uint64_t)blockIdx.x * blockDim.x + threadIdx.x; i <= count; i += (uint64_t)gridDim.x * blockDim.x) {
-        int64_t cur = (int64_t)n_rows, prev = -1;
-        if (i < count) {
-            const uint64_t k = keys[i];
-            cur = (int64_t)(uint32_t)(k >> 32) - (int64_t)base;
-            if (cur < 0 || cur >= (int64_t)n_rows || (uint32_t)k >= lo_bound) {
-                if (err) atomicExch(err, 2u);
-                cur = (int64_t)n_rows;
+                                                              RowGap *__restrict__ gaps, uint32_t *__restrict__ n_gaps, uint32_t *__restrict__ err,
+                                                              uint32_t *__restrict__ lo_count) {
+    // the counting pass reads the whole edge list: kLoads keys per thread in flight before any is used
+    constexpr int kLoads = kCountLo ? 4 : 1;
+    const uint64_t stride = (uint64_t)gridDim.x * blockDim.x;
+    for (uint64_t i0 = (uint64_t)blockIdx.x * blockDim.x + threadIdx.x; i0 <= count; i0 += stride * kLoads) {
+        uint64_t key[kLoads], key_prev[kLoads];
+#pragma unroll
+        for (int j = 0; j < kLoads; ++j) {
+            const uint64_t i = i0 + j * stride;
+            key[j] = i < count ? keys[i] : 0;
+            key_prev[j] = i > 0 && i <= count ? keys[i - 1] : 0;
+        }
+#pragma unroll
+        for (int j = 0; j < kLoads; ++j) {
+            const uint64_t i = i0 + j * stride;
+            if (i > count) break;
+            int64_t cur = (int64_t)n_rows, prev = -1;
+            if (i < count) {
+                const uint64_t k = key[j];
+                if (kCountLo) atomicAdd(&lo_count[(uint32_t)k], 1u);
+                cur = (int64_t)(uint32_t)(k >> 32) - (int64_t)base;
+                if (cur < 0 || cur >= (int64_t)n_rows || (uint32_t)k >= lo_bound) {
+                    if (err) atomicExch(err, 2u);
+                    cur = (int64_t)n_rows;
+                }
             }
-        }
-        if (i > 0) {
-            prev = (int64_t)(uint32_t)(keys[i - 1] >> 32) - (int64_t)base;
-            if (prev < 0 || prev >= (int64_t)n_rows) prev = (int64_t)n_rows;
-        }
-        if (cur - prev > kGapShort) {
-            const uint32_t g = atomicAdd(n_gaps, 1u);
-            gaps[g] = RowGap{(uint32_t)(prev + 1), (uint32_t)cur, (uint32_t)i};
-        } else {
-            for (int64_t x = prev + 1; x <= cur; ++x) start[x] = (uint32_t)i;
+            if (i > 0) {
+                prev = (int64_t)(uint32_t)(key_prev[j] >> 32) - (int64_t)base;
+                if (prev < 0 || prev >= (int64_t)n_rows) prev = (int64_t)n_rows;
+            }
+            if (cur - prev > kGapShort) {
+                const uint32_t g = atomicAdd(n_gaps, 1u);
+                gaps[g] = RowGap{(uint32_t)(prev + 1), (uint32_t)cur, (uint32_t)i};
+            } else {
+                for (int64_t x = prev + 1; x <= cur; ++x) start[x] = (uint32_t)i;
+            }
         }
     }
 }
@@ -431,51 +449,43 @@ __global__ void __launch_bounds__(kThreads) row_gaps_kernel(const RowGap *__rest
     }
 }
 
+// lo_count[(uint32_t)keys[i]] += 1 for every key: the back-neighbour count of an edge list whose forward index exists
+constexpr int kEdgeLoads = 4;   // keys per thread in flight in the passes over the whole edge list
+__global__ void __launch_bounds__(kThreads) count_lo_kernel(const uint64_t *__restrict__ keys, uint64_t count, uint32_t *__restrict__ lo_count) {
+    const uint64_t stride = (uint64_t)gridDim.x * blockDim.x;
+    for (uint64_t i0 = (uint64_t)blockIdx.x * blockDim.x + threadIdx.x; i0 < count; i0 += stride * kEdgeLoads) {
+        uint64_t key[kEdgeLoads];
+#pragma unroll
+        for (int j = 0; j < kEdgeLoads; ++j) key[j] = i0 + j * stride < count ? keys[i0 + j * stride] : 0;
+#pragma unroll
+        for (int j = 0; j < kEdgeLoads; ++j)
+            if (i0 + j * stride < count) atomicAdd(&lo_count[(uint32_t)key[j]], 1u);
+    }
+}
+
+// deg[v] = forward neighbours (a run of the edge list) + back neighbours (counted)
 struct DegreeIn {
     const uint32_t *fwd_start;
-    const uint32_t *back_start;
+    const uint32_t *back_cnt;
     __device__ uint64_t operator()(uint64_t v) const {
-        return (uint64_t)(fwd_start[v + 1] - fwd_start[v]) + (uint64_t)(back_start[v + 1] - back_start[v]);
+        return (uint64_t)(fwd_start[v + 1] - fwd_start[v]) + (uint64_t)back_cnt[v];
     }
 };
+// row_ptr[v] (row_ptr[n] too, from the last vertex), deg[v], and the max degree: one atomic per warp that raises it
 struct DegreeOut {
     uint64_t *row_ptr;
     int32_t *deg;
+    int32_t *max_deg;
+    uint64_t n;
     __device__ void operator()(uint64_t v, uint64_t prefix, uint64_t d) const {
         row_ptr[v] = prefix;
         deg[v] = (int32_t)d;
+        if (v + 1 == n) row_ptr[n] = prefix + d;
+        const uint32_t active = __activemask();
+        const int32_t m = __reduce_max_sync(active, (int32_t)d);
+        if (lane_id() == (uint32_t)__ffs(active) - 1u && m > *(volatile int32_t *)max_deg) atomicMax(max_deg, m);
     }
 };
-
-// max of an int32 array: warp shuffle -> one atomic per warp
-__global__ void __launch_bounds__(kThreads) reduce_max_i32_kernel(const int32_t *__restrict__ x, uint64_t n,
-                                                                  int32_t *__restrict__ out) {
-    int32_t m = INT32_MIN;
-    for (uint64_t i = (uint64_t)blockIdx.x * blockDim.x + threadIdx.x; i < n; i += (uint64_t)gridDim.x * blockDim.x)
-        m = max(m, x[i]);
-    m = warp_reduce_max(m);
-    if (lane_id() == 0 && m != INT32_MIN) atomicMax(out, m);
-}
-
-// Row v = [back neighbours (< v, ascending) | forward neighbours (> v, ascending)].
-__global__ void __launch_bounds__(kThreads) fill_col_kernel(const uint64_t *__restrict__ edges,
-                                                            const uint64_t *__restrict__ swapped, uint64_t n_edges,
-                                                            const uint64_t *__restrict__ row_ptr,
-                                                            const uint32_t *__restrict__ fwd_start,
-                                                            const uint32_t *__restrict__ back_start,
-                                                            uint32_t *__restrict__ col) {
-    for (uint64_t i = (uint64_t)blockIdx.x * blockDim.x + threadIdx.x; i < n_edges; i += (uint64_t)gridDim.x * blockDim.x) {
-        uint64_t e = edges[i];
-        uint32_t u = (uint32_t)(e >> 32);
-        uint64_t nback = back_start[u + 1] - back_start[u];
-        col[row_ptr[u] + nback + (i - fwd_start[u])] = (uint32_t)e;
-        uint64_t s = swapped[i];
-        uint32_t v = (uint32_t)(s >> 32);
-        col[row_ptr[v] + (i - back_start[v])] = (uint32_t)s;
-    }
-}
-
-__global__ void set_u64_kernel(uint64_t *p, uint64_t v) { *p = v; }
 
 // keys sorted by high word: idx[j] = first position whose high word is >= bounds[j]
 __global__ void lower_bounds_kernel(const uint64_t *__restrict__ keys, uint64_t count, const uint32_t *__restrict__ bounds,
@@ -858,15 +868,20 @@ int pairs_to_edges(kombgpu_ctx *ctx, const uint32_t *u, const uint32_t *v, uint6
 }
 
 int row_starts(kombgpu_ctx *ctx, const uint64_t *keys, uint64_t count, uint32_t base, uint32_t n_rows, uint32_t lo_bound, uint32_t *start,
-               uint32_t *err_dev) {
+               uint32_t *err_dev, uint32_t *lo_count) {
     // a gap longer than kGapShort rows is recorded: at most n_rows / kGapShort + 1 of them
     DevBuf<RowGap> gaps;
     DevBuf<uint32_t> n_gaps(ctx, 1);
     KG_ALLOC(ctx, gaps, (size_t)n_rows / (size_t)kGapShort + 2);
     if (!n_gaps) return ctx_fail(ctx, KOMBGPU_ENOMEM, "workspace");
     KG_CUDA(ctx, cudaMemsetAsync(n_gaps.p, 0, sizeof(uint32_t), ctx->stream));
-    KG_LAUNCH(ctx, row_bounds_kernel, min(grid_for(count + 1, kThreads), 148u * 16u), kThreads, 0, keys, count, base, n_rows, lo_bound, start,
-              gaps.p, n_gaps.p, err_dev);
+    const uint32_t grid = min(grid_for(count + 1, kThreads), 148u * 16u);
+    if (lo_count)
+        KG_LAUNCH(ctx, row_bounds_kernel<true>, grid, kThreads, 0, keys, count, base, n_rows, lo_bound, start, gaps.p, n_gaps.p, err_dev,
+                  lo_count);
+    else
+        KG_LAUNCH(ctx, row_bounds_kernel<false>, grid, kThreads, 0, keys, count, base, n_rows, lo_bound, start, gaps.p, n_gaps.p, err_dev,
+                  nullptr);
     KG_LAUNCH(ctx, row_gaps_kernel, 148u * 4u, kThreads, 0, gaps.p, n_gaps.p, start);
     return KOMBGPU_OK;
 }
@@ -879,20 +894,29 @@ int forward_index(kombgpu_ctx *ctx, const uint64_t *edges, uint64_t E, uint32_t 
     return KOMBGPU_OK;
 }
 
-// unique simple edges (sorted, u < v) -> CSR of the symmetric graph
+// unique simple edges (sorted, u < v) -> CSR of the symmetric graph.  Row v = [back neighbours (< v, ascending) |
+// forward neighbours (> v, ascending)].  The forward halves are the edge list's own runs; the back halves come from a
+// stable sort of the edge list on v, whose last pass writes col directly: with back_cnt[v] the number of edges (., v)
+// and row_ptr the scan of deg = fwd + back, row_ptr[v] - (back entries before row v) = fwd_start[v], so the entry at
+// position j of the v-sorted order goes to col[fwd_start[v] + j].
 int csr_from_edges(kombgpu_ctx *ctx, DevBuf<uint64_t> &edges, uint64_t E, uint32_t n, kombgpu_graph *g) {
     g->n = n;
     g->n_edges = E;
     g->st.n_edges = E;
     g->st.n_vertices = n;
-    DevBuf<uint64_t> sw_a, sw_b;
-    uint64_t *swapped = nullptr;
-    KG_TRY(swapped_sorted(ctx, edges.p, E, n, sw_a, sw_b, &swapped));
-    DevBuf<uint32_t> back_start;
-    KG_ALLOC(ctx, back_start, (size_t)n + 1);
-    if (!g->fwd_start) KG_TRY(forward_index(ctx, edges.p, E, n, &g->fwd_start));   // kept: the CSR form of the edge list
+    // one read of the edge list: back_cnt, and the forward index when no earlier stage built it
+    DevBuf<uint32_t> back_cnt;
+    KG_ALLOC(ctx, back_cnt, n);
+    KG_CUDA(ctx, cudaMemsetAsync(back_cnt.p, 0, (size_t)n * sizeof(uint32_t), ctx->stream));
+    if (!g->fwd_start) {   // kept: the CSR form of the edge list
+        DevBuf<uint32_t> fwd_start;
+        KG_ALLOC(ctx, fwd_start, (size_t)n + 1);
+        KG_TRY(row_starts(ctx, edges.p, E, 0u, n, 0xffffffffu, fwd_start.p, nullptr, back_cnt.p));
+        g->fwd_start = fwd_start.take();
+    } else if (E) {
+        KG_LAUNCH(ctx, count_lo_kernel, min(grid_for(E, kThreads), 148u * 16u), kThreads, 0, edges.p, E, back_cnt.p);
+    }
     const uint32_t *fwd_start_p = g->fwd_start;
-    KG_TRY(row_starts(ctx, swapped, E, 0u, n, 0xffffffffu, back_start.p, nullptr));
 
     DevBuf<uint64_t> row_ptr;
     DevBuf<int32_t> deg, max_deg(ctx, 1);
@@ -902,13 +926,27 @@ int csr_from_edges(kombgpu_ctx *ctx, DevBuf<uint64_t> &edges, uint64_t E, uint32
     KG_ALLOC(ctx, col, 2 * E);
     if (!max_deg) return ctx_fail(ctx, KOMBGPU_ENOMEM, "workspace");
     KG_CUDA(ctx, cudaMemsetAsync(max_deg.p, 0, sizeof(int32_t), ctx->stream));
-    KG_TRY((device_scan<uint64_t>(ctx, n, DegreeIn{fwd_start_p, back_start.p}, DegreeOut{row_ptr.p, deg.p},
+    if (n == 0) KG_CUDA(ctx, cudaMemsetAsync(row_ptr.p, 0, sizeof(uint64_t), ctx->stream));
+    KG_TRY((device_scan<uint64_t>(ctx, n, DegreeIn{fwd_start_p, back_cnt.p}, DegreeOut{row_ptr.p, deg.p, max_deg.p, n},
                                   (uint64_t *)nullptr)));
-    if (n) KG_LAUNCH(ctx, reduce_max_i32_kernel, min(grid_for(n, kThreads), 148u * 8u), kThreads, 0, deg.p, (uint64_t)n, max_deg.p);
-    KG_LAUNCH(ctx, set_u64_kernel, 1, 1, 0, row_ptr.p + n, 2 * E);
-    if (E)
-        KG_LAUNCH(ctx, fill_col_kernel, min(grid_for(E, kThreads), 148u * 16u), kThreads, 0, edges.p, swapped, E, row_ptr.p,
-                  fwd_start_p, back_start.p, col.p);
+    // the v-sort reads the edge list in place, writing the forward halves as it goes (pass 1), takes its digit counts from
+    // back_cnt, and its last pass writes the back halves (b is scratch from 2 passes on, a from 3)
+    {
+        RadixPass passes[8];
+        const int np = plan_radix_passes(0, bits_for(n > 0 ? n - 1 : 0), 0, 0, passes);
+        DevBuf<uint64_t> a, b;
+        if (E >= 2 && np >= 2) KG_ALLOC(ctx, b, E);
+        if (E >= 2 && np >= 3) KG_ALLOC(ctx, a, E);
+        SortOptions opt;
+        opt.first = edges.p;
+        opt.counts = back_cnt.p;
+        opt.n_counts = n;
+        opt.col_base = fwd_start_p;
+        opt.col = col.p;
+        opt.fwd_row_ptr = row_ptr.p;
+        uint64_t *unused = nullptr;
+        KG_TRY(radix_sort_u64(ctx, a.p, b.p, E, passes, np, &unused, &opt));
+    }
     KG_TRY(read_back(ctx, max_deg.p, &g->st.max_degree, 1));
     g->edges = edges.take();
     g->row_ptr = row_ptr.take();

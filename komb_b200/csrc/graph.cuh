@@ -104,9 +104,9 @@ int unique_edges(kombgpu_ctx *ctx, const uint64_t *keys, uint64_t count, DevBuf<
                  DevBuf<uint32_t> *mult);
 // keys sorted by high word in [base, base + n_rows): start[x] = first index whose high word is >= base + x, x in [0, n_rows];
 // long runs of empty rows are filled by whole CTAs.  *err_dev (optional) is set to 2 when a key is out of range or its
-// low word is >= lo_bound.
+// low word is >= lo_bound.  lo_count (optional, zeroed by the caller, valid keys only): lo_count[low word] += 1 per key.
 int row_starts(kombgpu_ctx *ctx, const uint64_t *keys, uint64_t count, uint32_t base, uint32_t n_rows, uint32_t lo_bound, uint32_t *start,
-               uint32_t *err_dev);
+               uint32_t *err_dev, uint32_t *lo_count = nullptr);
 // fwd_start[x] = first edge whose source is >= x, x in [0, n]  (the edge list is sorted by source)
 int forward_index(kombgpu_ctx *ctx, const uint64_t *edges, uint64_t n_edges, uint32_t n, uint32_t **fwd_start_out);
 int swapped_sorted(kombgpu_ctx *ctx, const uint64_t *edges, uint64_t n_edges, uint32_t n_vertices, DevBuf<uint64_t> &a,

@@ -21,10 +21,29 @@ struct RadixPass {
 // fewest passes of at most 8 bits (equal widths), least significant first.
 int plan_radix_passes(int lo0, int hi0, int lo1, int hi1, RadixPass *out /* >= 8 entries */);
 
+// What a sort may take besides its keys, all optional.
+struct SortOptions {
+    // Pass 1 reads the keys here and leaves them unchanged; `a` is then only scratch (needed from 3 passes on, or
+    // from 2 without `col`).
+    const uint64_t *first = nullptr;
+    // counts[x], x < n_counts: the number of keys whose low word is x, when every pass's digit lies in the low word.
+    // The digit histograms come from these instead of from a read of the keys.
+    const uint32_t *counts = nullptr;
+    uint32_t n_counts = 0;
+    // The last pass writes no keys: the key (hi << 32 | lo) at sorted position pos stores hi at col[col_base[lo] + pos]
+    // (the back half of every CSR row, keys sorted on lo).  With fewer than 2 keys or no passes they go there unsorted.
+    const uint32_t *col_base = nullptr;
+    uint32_t *col = nullptr;
+    // With col: pass 1 (or, without passes, the unsorted store) also writes the forward half of every row as it reads
+    // the keys, which are then the u-sorted edge list with col_base its row starts: key i = (u << 32 | v) stores v at
+    // col[i + fwd_row_ptr[u + 1] - col_base[u + 1]].
+    const uint64_t *fwd_row_ptr = nullptr;
+};
+
 // Stable LSD radix sort.  `a` holds the keys, `b` is scratch of the same size;
-// returns in *sorted whichever of the two holds the result.
+// returns in *sorted whichever of the two holds the result (nullptr when opt->col takes it).
 int radix_sort_u64(kombgpu_ctx *ctx, uint64_t *a, uint64_t *b, uint64_t n, const RadixPass *passes,
-                   int n_passes, uint64_t **sorted);
+                   int n_passes, uint64_t **sorted, const SortOptions *opt = nullptr);
 
 #ifdef __CUDACC__
 

@@ -1,5 +1,5 @@
-// sort.cu — stable LSD radix sort of 64-bit keys (unitig pairs, swapped edges, CORE-A rank keys, and hits
-// when they do not arrive in read order).  Integer, HBM-bound.
+// sort.cu — stable LSD radix sort of 64-bit keys (unitig pairs, edges by their second endpoint, CORE-A rank keys, and
+// hits when they do not arrive in read order).  Integer, HBM-bound.
 //
 // Single-read passes (radix_sweep_kernel, "onesweep"): one kernel histograms every pass's digit up front, then each
 // pass reads the keys once and writes them once; tiles learn their global offsets by a decoupled look-back over
@@ -9,6 +9,8 @@
 // ballot-per-digit-bit ranking (profiles/r1/r1o_sweep_*).  MATCH.ANY ranks a key in one instruction but runs on the ADU
 // pipe and made every mix of the two slower (round 1).  Measurements of the passes and of the tile geometries that lost
 // to the one below are in DESIGN.md §4 "Sort".
+#include <type_traits>
+
 #include "kombgpu_debug.h"
 #include "primitives.cuh"
 
@@ -134,12 +136,40 @@ struct SweepSmem {
     uint32_t tile;
 };
 
+// Where a pass puts key k at its sorted position pos: every pass but a sink's last one writes the key array `out`.
+struct StoreKeys {
+    __device__ __forceinline__ void operator()(uint64_t *__restrict__ out, uint64_t pos, uint64_t k) const { out[pos] = k; }
+};
+// The CSR's back half (SortOptions::col): the v-sorted edge (u << 32 | v) at position pos is u, at col[col_base[v] + pos]
+struct StoreCol {
+    const uint32_t *col_base;
+    uint32_t *col;
+    __device__ __forceinline__ void operator()(uint64_t *, uint64_t pos, uint64_t k) const {
+        col[(uint64_t)col_base[(uint32_t)k] + pos] = (uint32_t)(k >> 32);
+    }
+};
+
+// What the first pass may do with each key it reads, besides sorting it (SortOptions::fwd_row_ptr)
+struct NoVisit {};
+// The CSR's forward half: edge i = (u << 32 | v) of the u-sorted list is v, at col[i + row_ptr[u + 1] - col_base[u + 1]]
+struct VisitFwdCol {
+    const uint64_t *row_ptr;
+    const uint32_t *col_base;
+    uint32_t *col;
+    __device__ __forceinline__ void operator()(uint64_t i, uint64_t k) const {
+        const uint32_t u1 = (uint32_t)(k >> 32) + 1u;
+        col[i + row_ptr[u1] - col_base[u1]] = (uint32_t)k;
+    }
+};
+
 // W: status word (StatusWord).  kBits: digit width known at compile time (8), or 0 = read it from `mask`.
-template <typename W, int kBits>
+// Store: where the sorted keys go (StoreKeys, or StoreCol in the last pass of a CSR sort).  Visit: called on every key
+// as it is read (NoVisit, or VisitFwdCol in the first pass of a CSR sort).
+template <typename W, int kBits, typename Store, typename Visit>
 __global__ void __launch_bounds__(kSweepThreads, kSweepMinBlocks) radix_sweep_kernel(const uint64_t *__restrict__ in, uint64_t *__restrict__ out,
                                                                     uint64_t n, DigitSpec dg,
                                                                     const uint32_t *__restrict__ digit_base,  // exclusive global histogram of this pass
-                                                                    W *status, uint32_t *tile_counter) {
+                                                                    W *status, uint32_t *tile_counter, Store store, Visit visit) {
     using SW = StatusWord<W>;
     constexpr int kWarps = kSweepThreads / 32;
     extern __shared__ __align__(16) unsigned char s_raw[];
@@ -217,6 +247,13 @@ __global__ void __launch_bounds__(kSweepThreads, kSweepMinBlocks) radix_sweep_ke
             s.keys[s.digit_local[d] + s.warp_cnt[warp][d] + rank[j]] = key[j];
         }
     }
+    if constexpr (!std::is_same_v<Visit, NoVisit>) {   // after the ranking, whose registers are free again
+#pragma unroll
+        for (int j = 0; j < kSweepItems; ++j) {
+            const uint32_t e = warp_base + j * 32 + lane;
+            if (e < tile_count) visit(tile_base + e, key[j]);
+        }
+    }
     for (uint32_t d = threadIdx.x; d <= mask; d += kSweepThreads) {
         uint32_t excl = 0;
         if (tile > 0) {
@@ -242,16 +279,72 @@ __global__ void __launch_bounds__(kSweepThreads, kSweepMinBlocks) radix_sweep_ke
     for (uint32_t i = threadIdx.x; i < tile_count; i += kSweepThreads) {
         const uint64_t k = s.keys[i];
         const uint32_t d = dg(k);
-        out[(uint64_t)(s.digit_global[d] + i)] = k;
+        store(out, (uint64_t)(s.digit_global[d] + i), k);
     }
 }
 
-template <typename W>
+template <typename W, typename Store = StoreKeys, typename Visit = NoVisit>
 int sweep_pass(kombgpu_ctx *ctx, const uint64_t *src, uint64_t *dst, uint64_t n, const RadixPass &pass, const DigitSpec &dg,
-               const uint32_t *digit_base, W *status, uint32_t *tile_counter) {
-    auto *kernel = pass.bits + pass.bits2 == 8 ? radix_sweep_kernel<W, 8> : radix_sweep_kernel<W, 0>;
+               const uint32_t *digit_base, W *status, uint32_t *tile_counter, Store store = Store{}, Visit visit = Visit{}) {
+    auto *kernel = pass.bits + pass.bits2 == 8 ? radix_sweep_kernel<W, 8, Store, Visit> : radix_sweep_kernel<W, 0, Store, Visit>;
     KG_LAUNCH(ctx, kernel, ceil_div_u64(n, kSweepTile), kSweepThreads, sizeof(SweepSmem), src, dst, n, dg, digit_base, status,
-              tile_counter);
+              tile_counter, store, visit);
+    return KOMBGPU_OK;
+}
+
+// one pass: the key array or the CSR sink, with or without the first pass's visit
+template <typename W>
+int sweep_pass_opt(kombgpu_ctx *ctx, const uint64_t *src, uint64_t *dst, uint64_t n, const RadixPass &pass, const DigitSpec &dg,
+                   const uint32_t *digit_base, W *status, uint32_t *tile_counter, bool to_col, bool visit, const SortOptions &o) {
+    const StoreCol sc{o.col_base, o.col};
+    const VisitFwdCol vf{o.fwd_row_ptr, o.col_base, o.col};
+    if (to_col && visit) return sweep_pass(ctx, src, nullptr, n, pass, dg, digit_base, status, tile_counter, sc, vf);
+    if (to_col) return sweep_pass(ctx, src, nullptr, n, pass, dg, digit_base, status, tile_counter, sc);
+    if (visit) return sweep_pass(ctx, src, dst, n, pass, dg, digit_base, status, tile_counter, StoreKeys{}, vf);
+    return sweep_pass(ctx, src, dst, n, pass, dg, digit_base, status, tile_counter);
+}
+
+// hist[p * 256 + d] += counts[x] for every x < m whose pass-p digit is d: the histograms of keys whose digits all lie in
+// their low word, from the number of keys per low word (neighbouring x share their high digits: one atomic per warp)
+__global__ void __launch_bounds__(kRsThreads) radix_count_hist_kernel(const uint32_t *__restrict__ counts, uint32_t m, PassList pl,
+                                                                      uint32_t *__restrict__ hist) {
+    __shared__ uint32_t s_hist[kMaxPasses * kRadix];
+    for (int i = threadIdx.x; i < pl.n * kRadix; i += kRsThreads) s_hist[i] = 0;
+    __syncthreads();
+    const uint32_t lane = lane_id();
+    for (uint64_t base = (uint64_t)blockIdx.x * kRsThreads; base < m; base += (uint64_t)gridDim.x * kRsThreads) {
+        const uint64_t x = base + threadIdx.x;
+        const uint32_t c = x < m ? counts[x] : 0u;
+        for (int p = 0; p < pl.n; ++p) {
+            const uint32_t d = pl.dg[p](x);
+            const uint32_t d0 = __shfl_sync(kFullMask, d, 0);
+            if (__all_sync(kFullMask, d == d0)) {
+                const uint32_t sum = warp_reduce_add(c);
+                if (lane == 0 && sum) atomicAdd(&s_hist[p * kRadix + d0], sum);
+            } else if (c) {
+                atomicAdd(&s_hist[p * kRadix + d], c);
+            }
+        }
+    }
+    __syncthreads();
+    for (int i = threadIdx.x; i < pl.n * kRadix; i += kRsThreads)
+        if (s_hist[i]) atomicAdd(&hist[i], s_hist[i]);
+}
+
+// a sort without passes (fewer than 2 keys, or no digit bits): the keys are visited and go through the sink in their order
+__global__ void store_unsorted_kernel(const uint64_t *__restrict__ keys, uint64_t n, StoreCol store, VisitFwdCol visit, bool do_visit) {
+    for (uint64_t i = (uint64_t)blockIdx.x * blockDim.x + threadIdx.x; i < n; i += (uint64_t)gridDim.x * blockDim.x) {
+        if (do_visit) visit(i, keys[i]);
+        store(nullptr, i, keys[i]);
+    }
+}
+
+template <typename Store, typename Visit>
+int set_sweep_attrs(kombgpu_ctx *ctx) {
+    KG_CUDA(ctx, cudaFuncSetAttribute(radix_sweep_kernel<uint32_t, 8, Store, Visit>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)sizeof(SweepSmem)));
+    KG_CUDA(ctx, cudaFuncSetAttribute(radix_sweep_kernel<uint32_t, 0, Store, Visit>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)sizeof(SweepSmem)));
+    KG_CUDA(ctx, cudaFuncSetAttribute(radix_sweep_kernel<uint64_t, 8, Store, Visit>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)sizeof(SweepSmem)));
+    KG_CUDA(ctx, cudaFuncSetAttribute(radix_sweep_kernel<uint64_t, 0, Store, Visit>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)sizeof(SweepSmem)));
     return KOMBGPU_OK;
 }
 
@@ -276,16 +369,27 @@ int plan_radix_passes(int lo0, int hi0, int lo1, int hi1, RadixPass *out) {
 }
 
 int radix_sort_u64(kombgpu_ctx *ctx, uint64_t *a, uint64_t *b, uint64_t n, const RadixPass *passes, int n_passes,
-                   uint64_t **sorted) {
-    *sorted = a;
-    if (n < 2 || n_passes == 0) return KOMBGPU_OK;
+                   uint64_t **sorted, const SortOptions *opt) {
+    static const SortOptions kNone{};
+    if (!opt) opt = &kNone;
+    const bool to_col = opt->col != nullptr;
+    const uint64_t *first = opt->first ? opt->first : a;
+    *sorted = to_col ? nullptr : a;
+    if (n < 2 || n_passes == 0) {
+        if (to_col && n)
+            KG_LAUNCH(ctx, store_unsorted_kernel, min(ceil_div_u64(n, 256), 148u * 16u), 256, 0, first, n, StoreCol{opt->col_base, opt->col},
+                      VisitFwdCol{opt->fwd_row_ptr, opt->col_base, opt->col}, opt->fwd_row_ptr != nullptr);
+        else if (opt->first && n)
+            KG_CUDA(ctx, cudaMemcpyAsync(a, first, n * sizeof(uint64_t), cudaMemcpyDeviceToDevice, ctx->stream));
+        return KOMBGPU_OK;
+    }
     if (n >= (1ull << 32)) return ctx_fail(ctx, KOMBGPU_EINVAL, "radix_sort_u64: %llu keys exceed the 2^32 per-array limit", (unsigned long long)n);
     if (n_passes > kMaxPasses) return ctx_fail(ctx, KOMBGPU_EINVAL, "radix_sort_u64: %d passes exceed %d", n_passes, kMaxPasses);
     if (!ctx->sort_attr_set) {   // function attributes are per device: once per context, not per process
-        KG_CUDA(ctx, cudaFuncSetAttribute(radix_sweep_kernel<uint32_t, 8>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)sizeof(SweepSmem)));
-        KG_CUDA(ctx, cudaFuncSetAttribute(radix_sweep_kernel<uint32_t, 0>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)sizeof(SweepSmem)));
-        KG_CUDA(ctx, cudaFuncSetAttribute(radix_sweep_kernel<uint64_t, 8>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)sizeof(SweepSmem)));
-        KG_CUDA(ctx, cudaFuncSetAttribute(radix_sweep_kernel<uint64_t, 0>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)sizeof(SweepSmem)));
+        KG_TRY((set_sweep_attrs<StoreKeys, NoVisit>(ctx)));
+        KG_TRY((set_sweep_attrs<StoreCol, NoVisit>(ctx)));
+        KG_TRY((set_sweep_attrs<StoreKeys, VisitFwdCol>(ctx)));
+        KG_TRY((set_sweep_attrs<StoreCol, VisitFwdCol>(ctx)));
         ctx->sort_attr_set = true;
     }
     // Workspace, in 32-bit words: [n_passes x 256 digit histograms | kMaxPasses tile counters | status words].  Below 2^30
@@ -302,23 +406,32 @@ int radix_sort_u64(kombgpu_ctx *ctx, uint64_t *a, uint64_t *b, uint64_t n, const
     PassList pl{};
     pl.n = n_passes;
     for (int p = 0; p < n_passes; ++p) pl.dg[p] = DigitSpec::of(passes[p]);
-    uint64_t *src = a, *dst = b;
-    const uint32_t hist_grid = min(ceil_div_u64(n, kRsTile), (uint32_t)ctx->sm_count * 4u);
-    KG_LAUNCH(ctx, radix_global_hist_kernel, hist_grid, kRsThreads, 0, src, n, pl, ws.p);
+    if (opt->counts) {
+        const uint32_t m = opt->n_counts;
+        if (m) KG_LAUNCH(ctx, radix_count_hist_kernel, min(ceil_div_u64(m, kRsThreads), (uint32_t)ctx->sm_count * 4u), kRsThreads, 0,
+                         opt->counts, m, pl, ws.p);
+    } else {
+        const uint32_t hist_grid = min(ceil_div_u64(n, kRsTile), (uint32_t)ctx->sm_count * 4u);
+        KG_LAUNCH(ctx, radix_global_hist_kernel, hist_grid, kRsThreads, 0, first, n, pl, ws.p);
+    }
     KG_LAUNCH(ctx, radix_hist_scan_kernel, n_passes, kRadix, 0, ws.p);
+    // ping-pong: pass 0 reads `first` (a, or the caller's const keys) and writes b; later passes alternate b and a
+    const uint64_t *src = first;
+    uint64_t *dst = b;
     for (int p = 0; p < n_passes; ++p) {
         const uint32_t *digit_base = ws.p + (size_t)p * kRadix;
         uint32_t *counter = ws.p + (size_t)n_passes * kRadix + p;
-        if (wide) {
-            uint64_t *status = reinterpret_cast<uint64_t *>(ws.p + head);
-            if (p > 0) KG_CUDA(ctx, cudaMemsetAsync(status, 0, region * sizeof(uint64_t), ctx->stream));
-            KG_TRY(sweep_pass(ctx, src, dst, n, passes[p], pl.dg[p], digit_base, status, counter));
-        } else {
-            KG_TRY(sweep_pass(ctx, src, dst, n, passes[p], pl.dg[p], digit_base, ws.p + head + (size_t)p * region, counter));
-        }
-        uint64_t *t = src; src = dst; dst = t;
+        uint64_t *status64 = reinterpret_cast<uint64_t *>(ws.p + head);
+        uint32_t *status32 = ws.p + head + (size_t)p * region;
+        if (wide && p > 0) KG_CUDA(ctx, cudaMemsetAsync(status64, 0, region * sizeof(uint64_t), ctx->stream));
+        const bool last_to_col = to_col && p == n_passes - 1, visit = p == 0 && opt->fwd_row_ptr;
+        if (wide) KG_TRY(sweep_pass_opt(ctx, src, dst, n, passes[p], pl.dg[p], digit_base, status64, counter, last_to_col, visit, *opt));
+        else KG_TRY(sweep_pass_opt(ctx, src, dst, n, passes[p], pl.dg[p], digit_base, status32, counter, last_to_col, visit, *opt));
+        if (last_to_col) break;
+        *sorted = dst;
+        src = dst;
+        dst = dst == b ? a : b;
     }
-    *sorted = src;
     return KOMBGPU_OK;
 }
 
